@@ -15,9 +15,16 @@ Workloads (config.workload):
   igrf            BASELINE configs[1]: 10^8 random LEO points through K1 (evals/s).
 The default line also carries `sweep`, `tvlqr16k` and `igrf12` blocks (one timed pass each) unless --no-extras.
 
-  python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--workload ...] [--trials T]
+  python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--workload ...] [--trials T] [--dump-outputs DIR]
 For N > 1 launch under torchrun (one rank per GPU).  Rank 0 prints ONE JSON line.
 --impl reference: the reference algorithm on the host cores (the C++ oracle; Julia is not in the image), rank 0 only.
+--dump-outputs DIR: after the timed steps, rank 0 writes what the last timed step returned as DIR/<name>.npy (float64), so
+  that two builds can be compared output by output on identical seeded inputs.  row.npy holds the row of the full output
+  each dumped row comes from; outputs over 64 MB in all are a fixed seeded sample of rows.
+    mc_fixed_orbit, mc_sweep  one file per outcome-record field (status ... flops) of the gathered outcomes, and
+                              stats.npy (the reduced statistics vector, fields in parallel.STAT_FIELDS order)
+    tvlqr16k                  n_sim.npy, slew_time.npy per slew
+    igrf                      B_north.npy, B_east.npy, B_down.npy (nT) per point of rank 0
 """
 import argparse
 import json
@@ -32,6 +39,7 @@ import numpy as np
 
 ROOT = os.path.dirname(os.path.abspath(__file__))
 sys.path.insert(0, ROOT)
+sys.dont_write_bytecode = True      # the benchmark writes nothing into the tree it runs from (it may be read-only)
 
 GM = 3.986004418E14 * (1 / 1000) ** 3
 J_1U = np.diag([0.00125] * 3)
@@ -66,6 +74,24 @@ try:
 except Exception:
     pass
 STATUS = ["converged", "max_outer", "cost_blowup", "reg_max", "nan", "no_cutoff"]
+DUMP_BYTES = 60 << 20                # --dump-outputs: array data of all files; with the .npy headers < 64 MB
+
+
+def dump_rows(n, row_bytes, budget=DUMP_BYTES):
+    """Rows of an n-row output that --dump-outputs writes: all of them, or a fixed seeded sample within `budget` bytes."""
+    cap = budget // row_bytes
+    if n <= cap:
+        return np.arange(n)
+    return np.sort(np.random.default_rng(SEED).choice(n, size=cap, replace=False, shuffle=False))
+
+
+def write_dump(directory, arrays):
+    """directory/<name>.npy in float64 for every array."""
+    arrays = {k: np.asarray(v, dtype=np.float64) for k, v in arrays.items()}
+    assert sum(v.nbytes for v in arrays.values()) <= DUMP_BYTES
+    os.makedirs(directory, exist_ok=True)
+    for k, v in arrays.items():
+        np.save(os.path.join(directory, k + ".npy"), v)
 
 
 # --------------------------------------------------------------------------- synthetic ensembles
@@ -259,7 +285,10 @@ def main():
     ap.add_argument("--points", type=int, default=100_000_000, help="igrf workload: points per GPU")
     ap.add_argument("--no-cpu-baseline", action="store_true")
     ap.add_argument("--no-extras", action="store_true", help="default line without the sweep / tvlqr16k / igrf12 blocks")
+    ap.add_argument("--dump-outputs", metavar="DIR", help="write the outputs of the last timed step as DIR/<name>.npy (see the module docstring)")
     a = ap.parse_args()
+    if a.steps < 1:
+        ap.error("--steps must be at least 1")
     rank = int(os.environ.get("RANK", "0"))
     local_rank = int(os.environ.get("LOCAL_RANK", "0"))
     world = int(os.environ.get("WORLD_SIZE", "1"))
@@ -329,7 +358,7 @@ def main():
     hbm_src = "MEASURED_PEAKS.json" if "hbm_gbs" in peaks else "fallback (B200_PROFILING.md)"
 
     # ---- K1 throughput (BASELINE's second metric): device-resident inputs after their own warm-up, and host-buffer e2e
-    def igrf_block(n, reps, with_e2e=True):
+    def igrf_block(n, reps, with_e2e=True, dump=None):
         g = torch.Generator(device=dev).manual_seed(SEED + rank)
         u = torch.rand(3, n, generator=g, device=dev, dtype=torch.float64)
         lat = torch.asin(2 * u[0] - 1)
@@ -342,6 +371,11 @@ def main():
             eng.igrf12_batch(2019.0, r, lat, lon, out=o)
             if i >= 3:
                 ms.append(eng.last_kernel_ms())
+        if dump and rank == 0:
+            eng.synchronize()
+            rows = dump_rows(n, 4 * 8)
+            sel = torch.from_numpy(rows).to(dev)
+            write_dump(dump, dict(row=rows, **{k: b[sel].cpu().numpy() for k, b in zip(("B_north", "B_east", "B_down"), o)}))
         kms = max_over_ranks(float(np.mean(ms)))
         blk = {"evals_per_s": world * n / (kms * 1e-3), "points_per_gpu": n, "ms": kms,
                "roofline": {"bound": "fp64", "achieved": FL_IGRF * n / (kms * 1e-3) / 1e12, "peak": peak_fp64, "unit": "TFLOP/s",
@@ -372,7 +406,7 @@ def main():
         clk = ClockSampler(local_rank)
         clk.start()
         l0 = eng.launch_count()
-        blk = igrf_block(n, max(1, a.steps))
+        blk = igrf_block(n, a.steps, dump=a.dump_outputs)
         launches = eng.launch_count() - l0
         clocks = clk.stop()
         line = {"metric": metric, "value": blk["evals_per_s"], "unit": unit, "n_gpus": world, "steps": a.steps, "warmup": 3,
@@ -393,7 +427,7 @@ def main():
         return 0
 
     # ---- Monte-Carlo workloads ------------------------------------------------------------------------------------
-    def mc_pass(workload, n, steps, warmup, keep=False):
+    def mc_pass(workload, n, steps, warmup, keep=False, dump=None):
         """`warmup` untimed + `steps` timed passes of ts_monte_carlo_run over this rank's shard; returns a result dict."""
         tr = make_trials(workload, n, rank)
         cfg = mc_config(host, tr, n)
@@ -435,6 +469,10 @@ def main():
         wall = max_over_ranks(time.perf_counter() - t0)
         launches = eng.launch_count() - l0
         out, st, allout, vec = last
+        if dump and rank == 0:
+            fields = host.OUTCOME_DTYPE.names
+            rows = dump_rows(len(allout), 8 * (1 + len(fields)), DUMP_BYTES - vec.nbytes)
+            write_dump(dump, dict(row=rows, stats=vec, **{f: allout[f][rows] for f in fields}))
         dev_s = max_over_ranks(float(np.mean(acc["dev_ms"])) * 1e-3)      # device time of the kernels (CUDA events), max over ranks
         solve_s = float(np.mean(acc["solve"])) * 1e-3
         act = allout["status"] != 5
@@ -468,7 +506,7 @@ def main():
         res["d2h"] = int(n * 64 + 8 * len(fo))
         return res
 
-    def tvlqr_block(n_tv, reps):
+    def tvlqr_block(n_tv, reps, dump=None):
         """K4 alone on the first n_tv optimised slews of the run whose trajectories are resident (keep_trajectories)."""
         tj = eng.mc_trajectories(last_sweep["n"], want=("X", "U", "B_eci"))
         ko, ro = tj["knot_offs"], tj["row_offs"]
@@ -497,6 +535,9 @@ def main():
             if i >= 1:
                 walls.append(time.perf_counter() - t0)
                 kms.append(eng.last_kernel_ms())
+        if dump and rank == 0:
+            rows = dump_rows(n_ok, 3 * 8)
+            write_dump(dump, dict(row=rows, n_sim=r[4][rows], slew_time=r[5][rows]))
         k_s = max_over_ranks(float(np.mean(kms)) * 1e-3)
         w_s = max_over_ranks(float(np.mean(walls)))
         knots = float(np.sum(N_i - 1))
@@ -517,12 +558,12 @@ def main():
         n_sw = 2 * (a.trials or 2048)
         sw = mc_pass("mc_sweep", n_sw, 1, 0, keep=True)
         last_sweep.update(n=n_sw, out=sw["out"], tr=sw["tr"])
-        blk = tvlqr_block(a.trials or 2048, max(1, a.steps))
+        blk = tvlqr_block(a.trials or 2048, a.steps, dump=a.dump_outputs)
         clocks = clk.stop()
         line = {"metric": metric, "value": blk["slews_per_s"], "unit": unit, "n_gpus": world, "steps": a.steps, "warmup": 1,
                 "ms_per_step": blk["ms"], "higher_is_better": True, "scaling": "weak", "vs_baseline": None, "dtype": "f64", "data": "synthetic",
                 "config": {"workload": blk["workload"], "trials_per_gpu": blk["slews_per_gpu"]}, "roofline": blk["roofline"], "e2e": blk["e2e"],
-                "gpu_launches": max(1, a.steps), "clocks": clocks}
+                "gpu_launches": a.steps, "clocks": clocks}
         if rank == 0:
             print(json.dumps(line))
         if world > 1:
@@ -530,7 +571,7 @@ def main():
         return 0
 
     n = a.trials or (4096 if a.workload == "mc_fixed_orbit" else 8192)
-    main_r = mc_pass(a.workload, n, a.steps, a.warmup)
+    main_r = mc_pass(a.workload, n, a.steps, a.warmup, dump=a.dump_outputs)
     clocks = clk.stop()
     line = {"metric": metric, "value": main_r["value"], "unit": unit, "n_gpus": world, "steps": a.steps, "warmup": a.warmup,
             "ms_per_step": main_r["wall_step_s"] * 1e3, "higher_is_better": True, "scaling": "weak", "vs_baseline": None, "dtype": "f64",
