@@ -37,6 +37,7 @@ extern "C" {
 #define TS_ERR_ARG (-2)       /* bad argument (null pointer, negative size, ...) */
 #define TS_ERR_DATE (-3)      /* igrf12: date outside [1900, 2025]        (igrf.jl:80-81) */
 #define TS_ERR_DOMAIN (-4)    /* igrf12: |lat| > pi/2 or |lon| > pi at >=1 point (igrf.jl:84-88);
+                                 field map: a non-finite index at >=1 point;
                                  the offending outputs are NaN, the rest are valid */
 #define TS_ERR_NOMEM (-5)
 
@@ -315,6 +316,18 @@ int ts_mc_fetch_trajectories(ts_ctx* ctx, double* X, double* U, double* X_sim, d
  * Returns TS_ERR_DATE for dates outside [1900, 2025] (igrf.jl:343-345).                                              */
 int ts_igrf12syn_batch(ts_ctx* ctx, int isv, double date, int itype, int64_t n, const double* alt_km, const double* colat_deg,
                        const double* elong_deg, double* x, double* y, double* z, double* f, int pointers_are_device);
+
+/* ---- K8: cubic B-spline interpolant of the igrf_data field map -------------------------------- *
+ * extrapolate(interpolate(A, BSpline(Cubic(Reflect(OnCell())))), Periodic()) [src/magnetic_toolbox.jl:124-125] of an
+ * n0 x n1 x 3 map A (e.g. the lat/long map of igrf_data, :108-121), under rules FM1..FM4 of DESIGN.md section 4 (K8).
+ * 2 <= n0, n1 <= 2^20.  ts_field_map_prefilter (FM1): grid (n0 x n1 x 3) -> coefs ((n0+2) x (n1+2) x 3), each component
+ * on its own.  ts_field_map_eval_batch (FM2, FM3): x0, x1 (n each, 1-based fractional indices along axis 0 / 1, any real
+ * value: both axes wrap with period n0 / n1) -> out (n x 3: all three components; FM4, the integer component index with
+ * period 3, is the caller's choice of column).  A non-finite index gives a NaN row and TS_ERR_DOMAIN; the other rows
+ * are valid.                                                                                                         */
+int ts_field_map_prefilter(ts_ctx* ctx, int64_t n0, int64_t n1, const double* grid, double* coefs, int pointers_are_device);
+int ts_field_map_eval_batch(ts_ctx* ctx, int64_t n0, int64_t n1, const double* coefs, int64_t n, const double* x0,
+                            const double* x1, double* out, int pointers_are_device);
 
 /* ---- several GPUs of one node behind one handle ---------------------------------------------- *
  * ts_create_multi owns one ts_ctx per device, one host thread per device while a call runs, and (for n_devices > 1)

@@ -149,6 +149,42 @@ function igrf_data(altitude, year::Int64)
     end
     MagFieldMap(mag_field)
 end
+# igrf_interpolant(altitude, year): the cubic B-spline of that map   reference src/magnetic_toolbox.jl:124-125
+# extrapolate(interpolate(A, BSpline(Cubic(Reflect(OnCell())))), Periodic()) under rules FM1..FM4 (DESIGN.md section 4,
+# K8): real i, j (periodic), integer c (period 3).  coefs is the 3 x (n1+2) x (n0+2) Julia array whose memory is the
+# row-major (n0+2) x (n1+2) x 3 coefficient array of ts_field_map_prefilter.  Each call copies it to the GPU, so
+# evaluate many points per field_map_eval call.
+struct MagFieldInterpolant
+    coefs::Array{Float64,3}
+    n0::Int64
+    n1::Int64
+    e::Engine
+end
+function field_map_prefilter(grid::Array{Float64,3}; e::Engine = engine())
+    n0, n1, _ = size(grid)
+    g = permutedims(grid, (3, 2, 1))            # n0 x n1 x 3 (Julia) -> row-major n0 x n1 x 3 (C)
+    C = Array{Float64}(undef, 3, n1 + 2, n0 + 2)
+    rc = ccall((:ts_field_map_prefilter, LIB), Cint, (Ptr{Cvoid}, Int64, Int64, Ptr{Float64}, Ptr{Float64}, Cint),
+               e.h, n0, n1, g, C, 0)
+    check(e, rc)
+    MagFieldInterpolant(C, n0, n1, e)
+end
+# the spline at the 1-based indices (i[p], j[p]) -> 3 x n (north, east, down)
+function field_map_eval(m::MagFieldInterpolant, i::Vector{Float64}, j::Vector{Float64})
+    n = length(i)
+    length(j) == n || error("field_map_eval: i and j must have the same length")
+    out = Matrix{Float64}(undef, 3, n)
+    rc = ccall((:ts_field_map_eval_batch, LIB), Cint,
+               (Ptr{Cvoid}, Int64, Int64, Ptr{Float64}, Int64, Ptr{Float64}, Ptr{Float64}, Ptr{Float64}, Cint),
+               m.e.h, m.n0, m.n1, m.coefs, n, i, j, out, 0)
+    check(m.e, rc)
+    out
+end
+function (m::MagFieldInterpolant)(i, j, c)
+    isinteger(c) || error("mag_field(i,j,c): the component index c must be an integer")
+    field_map_eval(m, [Float64(i)], [Float64(j)])[mod(Int(c) - 1, 3) + 1, 1]
+end
+igrf_interpolant(altitude, year::Int64; e::Engine = engine()) = field_map_prefilter(igrf_data(altitude, year).grid; e = e)
 
 # ----------------------------------------------------------------------------- K2: orbit + field table
 # magnetic_simulation(p,t0,tf,N,mag_field)                  reference src/magnetic_toolbox.jl:33-106
@@ -401,6 +437,6 @@ hat(x) = [0 -x[3] x[2]; x[3] 0 -x[1]; -x[2] x[1] 0]                             
 export Engine, params, input_parameters, igrf12, igrf12_batch, igrf_data, magnetic_simulation, magnetic_gramian, kep_ECI, OrbitPlotter,
        legendre, dlegendre, DerivFunction, gain_simulator, attitude_dynamics,
        condition_based_time, eigen_axis_slew, bryson_weights, solve_slew, attitude_simulation, monte_carlo, qmult, qrot, q_inv, hat,
-       igrf12syn, attitude_dynamics_linear, psiaki_pd_simulation
+       igrf12syn, attitude_dynamics_linear, psiaki_pd_simulation, igrf_interpolant, field_map_prefilter, field_map_eval
 
 end # module

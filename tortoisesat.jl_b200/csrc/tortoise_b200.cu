@@ -10,6 +10,7 @@
 #include "k5_unitops.cuh"
 #include "k6_igrf12syn.cuh"
 #include "k7_comparison.cuh"
+#include "k8_field_map.cuh"
 
 #include <algorithm>
 #include <numeric>
@@ -58,7 +59,7 @@ struct HostIO {
 
 extern "C" {
 
-int ts_version(void) { return 100; }
+int ts_version(void) { return 101; }
 
 int ts_create(ts_ctx** out, int device_id) {
   if (!out) return TS_ERR_ARG;
@@ -355,6 +356,88 @@ int ts_igrf12syn_batch(ts_ctx* c, int isv, double date, int itype, int64_t n, co
   if ((rc = dev_back(c, ox, x, b)) || (rc = dev_back(c, oy, y, b)) || (rc = dev_back(c, oz, z, b)) || (rc = dev_back(c, of, f, b))) return rc;
   TS_CUDA(c, cudaStreamSynchronize(c->stream));
   tm.read();
+  return TS_OK;
+}
+
+// ---------------------------------------------------------------------------- K8
+static int field_map_dims(ts_ctx* c, const char* fn, int64_t n0, int64_t n1) {
+  if (n0 < 2 || n1 < 2 || n0 > K8_MAX_AXIS || n1 > K8_MAX_AXIS)
+    return fail(c, TS_ERR_ARG, "%s: n0 = %lld and n1 = %lld must lie in [2, %lld]", fn, (long long)n0, (long long)n1,
+                (long long)K8_MAX_AXIS);
+  return TS_OK;
+}
+
+// FM1: Thomas solves along axis 1 (j) for every data row, then along axis 0 (i) for every padded column.  The j-lines
+// are made columns by a tiled transpose into a (n1+2) x n0 x 3 buffer, solved in place, and transposed into rows
+// 1..n0 of C, where the i-pass solves in place.
+int ts_field_map_prefilter(ts_ctx* c, int64_t n0, int64_t n1, const double* grid, double* coefs, int pad) {
+  if (!c) return TS_ERR_ARG;
+  if (!grid || !coefs) return fail(c, TS_ERR_ARG, "ts_field_map_prefilter: null array");
+  int rc;
+  if ((rc = field_map_dims(c, "ts_field_map_prefilter", n0, n1))) return rc;
+  TS_CUDA(c, cudaSetDevice(c->device));
+  const size_t b_in = (size_t)n0 * n1 * 3 * sizeof(double), b_out = (size_t)(n0 + 2) * (n1 + 2) * 3 * sizeof(double);
+  std::vector<double> inv((size_t)(n0 + n1));
+  k8_thomas_factors(n0, inv.data());
+  k8_thomas_factors(n1, inv.data() + n0);
+  DevBuf dg, dc, dt, df;
+  if ((rc = dev_in(c, dg, grid, b_in, pad)) || (rc = dev_out(c, dc, coefs, b_out, pad)) ||
+      (rc = dev_in(c, df, inv.data(), inv.size() * sizeof(double), 0)))
+    return rc;
+  const size_t b_t = (size_t)(n1 + 2) * n0 * 3 * sizeof(double);
+  cudaError_t e = cudaMalloc(&dt.d, b_t);
+  if (e != cudaSuccess) return fail(c, TS_ERR_NOMEM, "cudaMalloc(%zu) failed: %s", b_t, cudaGetErrorString(e));
+  dt.owned = true;
+  double *G = (double*)dg.d, *Cf = (double*)dc.d, *T = (double*)dt.d;
+  const double *inv0 = (const double*)df.d, *inv1 = inv0 + n0;
+  const dim3 tb(K8_TILE, 8);
+  KernelTimer tm(c);
+  k8_transpose3<<<dim3((unsigned)((n1 + K8_TILE - 1) / K8_TILE), (unsigned)((n0 + K8_TILE - 1) / K8_TILE)), tb, 0, c->stream>>>(
+      G, n0, n1, T + n0 * 3, n0 * 3);
+  k8_prefilter_cols<<<(unsigned)((n0 * 3 + 127) / 128), 128, 0, c->stream>>>(T, n1, n0 * 3, inv1);
+  k8_transpose3<<<dim3((unsigned)((n0 + K8_TILE - 1) / K8_TILE), (unsigned)((n1 + 2 + K8_TILE - 1) / K8_TILE)), tb, 0, c->stream>>>(
+      T, n1 + 2, n0, Cf + (n1 + 2) * 3, (n1 + 2) * 3);
+  k8_prefilter_cols<<<(unsigned)(((n1 + 2) * 3 + 127) / 128), 128, 0, c->stream>>>(Cf, n0, (n1 + 2) * 3, inv0);
+  tm.stop();
+  c->launches += 4;
+  TS_CUDA(c, cudaGetLastError());
+  if ((rc = dev_back(c, dc, coefs, b_out))) return rc;
+  TS_CUDA(c, cudaStreamSynchronize(c->stream));
+  tm.read();
+  return TS_OK;
+}
+
+// FM2 + FM3 at n points; FM4 (the component index) is left to the caller: every row holds all three components.
+int ts_field_map_eval_batch(ts_ctx* c, int64_t n0, int64_t n1, const double* coefs, int64_t n, const double* x0,
+                            const double* x1, double* out, int pad) {
+  if (!c) return TS_ERR_ARG;
+  if (n < 0 || !coefs || (n > 0 && (!x0 || !x1 || !out))) return fail(c, TS_ERR_ARG, "ts_field_map_eval_batch: null array or n<0");
+  int rc;
+  if ((rc = field_map_dims(c, "ts_field_map_eval_batch", n0, n1))) return rc;
+  if (n == 0) return TS_OK;
+  TS_CUDA(c, cudaSetDevice(c->device));
+  const size_t b_c = (size_t)(n0 + 2) * (n1 + 2) * 3 * sizeof(double), b = (size_t)n * sizeof(double);
+  DevBuf dc, da, db, dout;
+  if ((rc = dev_in(c, dc, coefs, b_c, pad)) || (rc = dev_in(c, da, x0, b, pad)) || (rc = dev_in(c, db, x1, b, pad)) ||
+      (rc = dev_out(c, dout, out, 3 * b, pad)))
+    return rc;
+  const int64_t nodes = (n0 + 2) * (n1 + 2);
+  void* c4;
+  if ((rc = scratch_reserve(c, 27, (size_t)nodes * 4 * sizeof(double), &c4))) return rc;   // slot 27: K8 only
+  TS_CUDA(c, cudaMemsetAsync(c->d_flag, 0, sizeof(int), c->stream));
+  KernelTimer tm(c);
+  k8_pad4<<<(unsigned)((nodes + 255) / 256), 256, 0, c->stream>>>((const double*)dc.d, nodes, (double*)c4);
+  k8_field_map_eval<<<(unsigned)((n + K8_THREADS - 1) / K8_THREADS), K8_THREADS, 0, c->stream>>>(
+      (const double*)c4, n0, n1, n, (const double*)da.d, (const double*)db.d, (double*)dout.d, c->d_flag);
+  tm.stop();
+  c->launches += 2;
+  TS_CUDA(c, cudaGetLastError());
+  if ((rc = dev_back(c, dout, out, 3 * b))) return rc;
+  int bad = 0;
+  TS_CUDA(c, cudaMemcpyAsync(&bad, c->d_flag, sizeof(int), cudaMemcpyDeviceToHost, c->stream));
+  TS_CUDA(c, cudaStreamSynchronize(c->stream));
+  tm.read();
+  if (bad) return fail(c, TS_ERR_DOMAIN, "ts_field_map_eval_batch: non-finite index (the rows of those points are NaN)");
   return TS_OK;
 }
 

@@ -3,6 +3,7 @@
 Reference interface mirrored here (file:line in /root/reference/src):
   igrf12(date, r, lat, lon)                       igrf.jl:67-274
   igrf_data(altitude, year)                       magnetic_toolbox.jl:108-127
+  its cubic B-spline interpolant                  magnetic_toolbox.jl:124-125   (MagFieldMap.interpolant)
 (more entry points are added with each kernel)
 """
 import ctypes as C
@@ -157,6 +158,8 @@ def load_library():
     L.ts_multi_ctx.restype = C.c_void_p
     L.ts_multi_monte_carlo_run.argtypes = [C.c_void_p, C.POINTER(McConfig)] + [C.c_void_p] * 8 + [C.POINTER(McStats)]
     L.ts_igrf12_batch.argtypes = [C.c_void_p, C.c_double, C.c_int64] + [C.c_void_p] * 6 + [C.c_int]
+    L.ts_field_map_prefilter.argtypes = [C.c_void_p, C.c_int64, C.c_int64, C.c_void_p, C.c_void_p, C.c_int]
+    L.ts_field_map_eval_batch.argtypes = [C.c_void_p, C.c_int64, C.c_int64, C.c_void_p, C.c_int64] + [C.c_void_p] * 3 + [C.c_int]
     L.ts_magnetic_simulation_batch.argtypes = [C.c_void_p, C.c_int64] + [C.c_void_p] * 7 + [C.c_int]
     L.ts_magnetic_gramian_batch.argtypes = [C.c_void_p, C.c_int64] + [C.c_void_p] * 5 + [C.c_int]
     L.ts_condition_based_time_batch.argtypes = [C.c_void_p, C.c_int64] + [C.c_void_p] * 5 + [C.c_int]
@@ -190,6 +193,46 @@ def _ptr(a):
     if isinstance(a, np.ndarray):
         return a.ctypes.data
     return a.data_ptr()  # torch tensor
+
+
+def _is_tensor(a):
+    return not isinstance(a, np.ndarray) and hasattr(a, "data_ptr")
+
+
+def _cuda_f64(t):
+    """a torch CUDA float64 tensor, contiguous (device-pointer path)"""
+    if not _is_tensor(t) or not t.is_cuda or str(t.dtype) != "torch.float64":
+        raise ValueError("the device path takes torch CUDA float64 tensors")
+    return t.contiguous()
+
+
+def _wait_for_torch(t):
+    """The library runs on its own non-blocking stream: work torch has queued on the tensors (a copy, a random fill)
+    must be finished before the library reads them."""
+    import torch
+    torch.cuda.current_stream(t.device).synchronize()
+
+
+def _check_out(out, count):
+    """a caller-provided output must be contiguous float64 storage of `count` values"""
+    if _is_tensor(out):
+        ok = out.is_cuda and str(out.dtype) == "torch.float64" and out.is_contiguous() and out.numel() == count
+    else:
+        ok = isinstance(out, np.ndarray) and out.dtype == np.float64 and out.flags.c_contiguous and out.size == count
+    if not ok:
+        raise ValueError("out must be contiguous float64 storage of %d values on the input's side" % count)
+
+
+def _field_map_grid_dims(shape):
+    if len(shape) != 3 or shape[2] != 3 or shape[0] < 2 or shape[1] < 2:
+        raise ValueError("the field map grid must be n0 x n1 x 3 with n0, n1 >= 2, got %s" % (tuple(shape),))
+    return int(shape[0]), int(shape[1])
+
+
+def _field_map_coef_dims(shape):
+    if len(shape) != 3 or shape[2] != 3 or shape[0] < 4 or shape[1] < 4:
+        raise ValueError("field map coefficients must be (n0+2) x (n1+2) x 3 with n0, n1 >= 2, got %s" % (tuple(shape),))
+    return int(shape[0]) - 2, int(shape[1]) - 2
 
 
 class Engine:
@@ -271,6 +314,55 @@ class Engine:
                                              _ptr(Bd), 1))
         return Bn, Be, Bd
 
+    # -- K8 ---------------------------------------------------------------
+    def field_map_prefilter(self, grid, out=None):
+        """FM1 (DESIGN section 4, K8) of the cubic B-spline of magnetic_toolbox.jl:124-125: n0 x n1 x 3 grid ->
+        (n0+2) x (n1+2) x 3 coefficients.  numpy in -> numpy out (host path), or a torch CUDA float64 tensor in ->
+        a tensor out (device path; `out` is allocated when not given)."""
+        if _is_tensor(grid):
+            n0, n1 = _field_map_grid_dims(grid.shape)
+            grid = _cuda_f64(grid)
+            if out is None:
+                import torch
+                out = torch.empty((n0 + 2, n1 + 2, 3), dtype=torch.float64, device=grid.device)
+            _check_out(out, (n0 + 2) * (n1 + 2) * 3)
+            _wait_for_torch(grid)
+            self._check(self.lib.ts_field_map_prefilter(self.h, n0, n1, _ptr(grid), _ptr(out), 1))
+            return out
+        grid = _f64(grid)
+        n0, n1 = _field_map_grid_dims(grid.shape)
+        out = np.empty((n0 + 2, n1 + 2, 3)) if out is None else out
+        _check_out(out, (n0 + 2) * (n1 + 2) * 3)
+        self._check(self.lib.ts_field_map_prefilter(self.h, n0, n1, _ptr(grid), _ptr(out), 0))
+        return out
+
+    def field_map_eval_batch(self, coefs, x0, x1, out=None):
+        """FM2 + FM3: the spline with coefficients `coefs` ((n0+2) x (n1+2) x 3) at the 1-based fractional indices
+        (x0[p], x1[p]) -> n x 3 (all three components).  Host arrays -> numpy out; torch CUDA float64 tensors (coefs,
+        x0, x1) -> a tensor out.  A non-finite index raises TortoiseError (code TS_ERR_DOMAIN) after the other rows of
+        `out` (if given) have been written; the offending rows are NaN."""
+        if _is_tensor(coefs):
+            n0, n1 = _field_map_coef_dims(coefs.shape)
+            coefs, x0, x1 = _cuda_f64(coefs), _cuda_f64(x0).reshape(-1), _cuda_f64(x1).reshape(-1)
+            n = x0.numel()
+            if x1.numel() != n:
+                raise ValueError("x0 and x1 must have the same length")
+            if out is None:
+                import torch
+                out = torch.empty((n, 3), dtype=torch.float64, device=coefs.device)
+            _check_out(out, n * 3)
+            _wait_for_torch(coefs)
+            self._check(self.lib.ts_field_map_eval_batch(self.h, n0, n1, _ptr(coefs), n, _ptr(x0), _ptr(x1), _ptr(out), 1))
+            return out
+        coefs = _f64(coefs)
+        n0, n1 = _field_map_coef_dims(coefs.shape)
+        x0, x1 = _f64(np.atleast_1d(x0)).reshape(-1), _f64(np.atleast_1d(x1)).reshape(-1)
+        if x0.shape != x1.shape:
+            raise ValueError("x0 and x1 must have the same length")
+        out = np.empty((x0.shape[0], 3)) if out is None else out
+        _check_out(out, x0.shape[0] * 3)
+        self._check(self.lib.ts_field_map_eval_batch(self.h, n0, n1, _ptr(coefs), x0.shape[0], _ptr(x0), _ptr(x1), _ptr(out), 0))
+        return out
 
     # -- K2 ---------------------------------------------------------------
     def magnetic_simulation_batch(self, kep6, opts, rows_limit=None, want_pos=False):
@@ -603,11 +695,16 @@ class MagFieldMap:
     array in a cubic B-spline interpolant with periodic extrapolation (magnetic_toolbox.jl:124-125)
     but only ever evaluates it at integer grid nodes, where an interpolating spline returns the
     data itself: this object returns the node values and wraps indices periodically (period n per
-    axis, 3 for the component axis).  Non-integer arguments are rejected -- the reference has no
-    caller for them and its boundary condition (Cubic(Reflect(OnCell()))) is not pinned by any test."""
+    axis, 3 for the component axis).  Non-integer arguments are rejected here; ``interpolant()``
+    gives the spline itself, which takes fractional spatial indices."""
 
     def __init__(self, grid):
         self.grid = np.ascontiguousarray(grid, dtype=np.float64)
+
+    def interpolant(self, engine=None):
+        """The cubic B-spline of magnetic_toolbox.jl:124-125 over this map (FM1..FM4, DESIGN section 4, K8), prefiltered
+        on the GPU and kept there."""
+        return MagFieldInterpolant(self.grid, engine or default_engine())
 
     def __call__(self, i, j, c):
         for v in (i, j, c):
@@ -625,6 +722,37 @@ class MagFieldMap:
 
     def __getitem__(self, idx):
         return self.grid[idx]
+
+
+class MagFieldInterpolant:
+    """extrapolate(interpolate(A, BSpline(Cubic(Reflect(OnCell())))), Periodic()) of an n0 x n1 x 3 map
+    (magnetic_toolbox.jl:124-125), rules FM1..FM4 of DESIGN section 4 (K8).  The coefficients stay on the GPU as a torch
+    CUDA tensor (``coefs``, (n0+2) x (n1+2) x 3) and every evaluation runs through the device-pointer path.
+
+    ``mag(i, j, c)``: real 1-based i, j (periodic, period n0 / n1), integer c (period 3; a fractional c is rejected,
+    it would blend north, east and down) -> float.  ``mag.eval(i, j)``: arrays -> n x 3 (numpy for host inputs, a
+    tensor for torch CUDA inputs).  A non-finite index raises TortoiseError."""
+
+    def __init__(self, grid, engine):
+        import torch
+        self.engine = engine
+        self.device = torch.device("cuda", engine.device)
+        g = torch.as_tensor(np.ascontiguousarray(grid, dtype=np.float64)).to(self.device)
+        self.coefs = engine.field_map_prefilter(g)
+        self.shape = tuple(g.shape)
+
+    def eval(self, i, j):
+        import torch
+        if _is_tensor(i):
+            return self.engine.field_map_eval_batch(self.coefs, i, j)
+        x0 = torch.as_tensor(_f64(np.atleast_1d(i)).reshape(-1)).to(self.device)
+        x1 = torch.as_tensor(_f64(np.atleast_1d(j)).reshape(-1)).to(self.device)
+        return self.engine.field_map_eval_batch(self.coefs, x0, x1).cpu().numpy()
+
+    def __call__(self, i, j, c):
+        if int(c) != c:
+            raise ValueError("mag_field(i,j,c): the component index c must be an integer")
+        return float(self.eval(float(i), float(j))[0, (int(c) - 1) % 3])
 
 
 def igrf_data(altitude, year, n=1000):
