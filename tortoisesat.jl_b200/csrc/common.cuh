@@ -11,6 +11,32 @@
 
 #include "../../include/tortoise_b200.h"
 
+namespace ts {
+// Grow-only device scratch slots of a context.  Most slots hold one call's working storage and are shared between
+// entries: whatever a call leaves in them is dead once it returns.  Storage that a later call reads (the readers are
+// ts_k3_last_* and ts_mc_fetch_trajectories) lives in a slot that no other entry writes.
+enum Slot : int {
+  SLOT_POSITIONS,                          // K2 orbit positions (ts_magnetic_simulation_batch without `pos`, Monte-Carlo)
+  SLOT_ARGS_A, SLOT_ARGS_B, SLOT_ARGS_C,   // a call's small per-trial inputs; C also K3 outcomes and slew-prep outputs
+  SLOT_CUTOFF,                             // gramian / condition-time cutoffs
+  SLOT_PER_TRIAL,                          // tf_index, the K3 queue order, K4 N_sim + slew_time
+  SLOT_K3_ARENA, SLOT_ROWS_A, SLOT_ROWS_B, // K3 trajectory arena; per-row outputs (slew-prep guesses, Monte-Carlo scoping field)
+  SLOT_K4_GAINS,                           // K4 gains when the caller passes none
+  SLOT_ORBIT_BLOCK, SLOT_ROW_LIMITS,       // Monte-Carlo per-orbit block and table row limits
+  SLOT_PACKED_I64, SLOT_PACKED_F64,        // Monte-Carlo packed per-trial arrays
+  SLOT_STREAM_IDS,                         // Monte-Carlo Philox stream ids
+  SLOT_PARK_STATE, SLOT_PARK_DATA,         // K3 parking places (read by ts_k3_last_parked) and parked trajectories
+  SLOT_PIPE_A, SLOT_PIPE_B,                // K1 host-pointer pipeline stages
+  SLOT_K3_CYCLES,                          // K3 cycle counters (read by ts_k3_last_cycles)
+  SLOT_KEPT_XSIM, SLOT_KEPT_USIM, SLOT_KEPT_BLOCK,   // Monte-Carlo kept trajectories (read by ts_mc_fetch_trajectories)
+  SLOT_K3_WARP_OFFS, SLOT_K3_WARP_CAPS, SLOT_K3_POOL, // K3 per-warp arena offsets and capacities, straggler pool
+  SLOT_LIN_RECORDS,                        // K4 linearisation records
+  SLOT_TABLE,                              // a call's lookup table: K4 linearisation offsets, K8 padded coefficients
+  SLOT_K3_COUNTERS,                        // K3 queue and park counters (read by ts_k3_last_split / ts_k3_last_parked)
+  SLOT_COUNT
+};
+}  // namespace ts
+
 struct ts_ctx {
   int device = 0;
   int sm_count = 0;
@@ -20,7 +46,7 @@ struct ts_ctx {
   unsigned* d_k3_parked = nullptr;                     // device word holding the number of parked trials of the last K3 run
   bool k3_timed = false;
   int k3_park_cap = 0;                                 // parking places of the last K3 run
-  int64_t k3_diag_n = 0;                               // trials covered by the K3 cycle diagnostics (scratch slot 19)
+  int64_t k3_diag_n = 0;                               // trials covered by the K3 cycle diagnostics (SLOT_K3_CYCLES)
   cudaStream_t pipe[2] = {nullptr, nullptr};           // K1 host-pointer path: double-buffered copy/compute pipeline
   cudaEvent_t pipe_ev = nullptr;
   char err[512] = {0};
@@ -40,8 +66,8 @@ struct ts_ctx {
     double *d_X = nullptr, *d_U = nullptr, *d_Xs = nullptr, *d_Us = nullptr, *d_B = nullptr;
   } mc_last;
   // grow-only scratch arenas
-  void* scratch[32] = {};
-  size_t scratch_bytes[32] = {};
+  void* scratch[ts::SLOT_COUNT] = {};
+  size_t scratch_bytes[ts::SLOT_COUNT] = {};
 };
 
 namespace ts {
@@ -64,7 +90,7 @@ inline int fail(ts_ctx* ctx, int code, const char* fmt, ...) {
   } while (0)
 
 // grow-only device scratch slot
-inline int scratch_reserve(ts_ctx* ctx, int slot, size_t bytes, void** out) {
+inline int scratch_reserve(ts_ctx* ctx, Slot slot, size_t bytes, void** out) {
   if (ctx->scratch_bytes[slot] < bytes) {
     if (ctx->scratch[slot]) cudaFree(ctx->scratch[slot]);
     ctx->scratch[slot] = nullptr;
@@ -77,47 +103,76 @@ inline int scratch_reserve(ts_ctx* ctx, int slot, size_t bytes, void** out) {
   return TS_OK;
 }
 
-// RAII-less helper for "host or device pointer" arguments: stages host arrays
-// into device memory owned by the call and copies results back.
-struct DevBuf {
-  void* d = nullptr;
-  bool owned = false;
-  ~DevBuf() {
-    if (owned && d) cudaFree(d);
+// A call's arrays.  in / out pass device pointers through (pointers_are_device) or stage host arrays into device
+// memory the call owns; out and back queue the copies of results into host arrays.  start() opens the timed window of
+// ts_last_kernel_ms.  finish() ends the call: it closes that window, checks the launches, runs the queued copies,
+// synchronises the stream once and reads the time.  The first failure sticks in rc and makes the rest no-ops.
+struct Staging {
+  struct Back {
+    void* host;
+    const void* dev;
+    size_t bytes;
+  };
+  ts_ctx* c;
+  const int pointers_are_device;
+  int rc = TS_OK;
+  bool timed = false;
+  std::vector<void*> owned;
+  std::vector<Back> backs;
+  Staging(ts_ctx* ctx, int pointers_are_device) : c(ctx), pointers_are_device(pointers_are_device) {}
+  ~Staging() {
+    for (void* p : owned) cudaFree(p);
+  }
+  void* alloc(size_t bytes) {
+    void* d = nullptr;
+    if (rc) return nullptr;
+    cudaError_t e = cudaMalloc(&d, bytes);
+    if (e != cudaSuccess) {
+      rc = fail(c, TS_ERR_NOMEM, "cudaMalloc(%zu) failed: %s", bytes, cudaGetErrorString(e));
+      return nullptr;
+    }
+    owned.push_back(d);
+    return d;
+  }
+  template <class T> const T* in(const T* p, size_t count) {
+    if (!p || pointers_are_device || count == 0) return p;
+    T* d = (T*)alloc(count * sizeof(T));
+    if (!d) return nullptr;
+    cudaError_t e = cudaMemcpyAsync(d, p, count * sizeof(T), cudaMemcpyHostToDevice, c->stream);
+    if (e != cudaSuccess) rc = fail(c, TS_ERR_CUDA, "H2D copy failed: %s", cudaGetErrorString(e));
+    return d;
+  }
+  template <class T> T* out(T* p, size_t count) {
+    if (!p || pointers_are_device || count == 0) return p;
+    T* d = (T*)alloc(count * sizeof(T));
+    back(p, d, count);
+    return d;
+  }
+  template <class T> void back(T* host, const T* dev, size_t count) {
+    if (!rc && count) backs.push_back({host, dev, count * sizeof(T)});
+  }
+  void start() {
+    timed = true;
+    cudaEventRecord(c->ev0, c->stream);
+  }
+  int finish() {
+    if (rc) return rc;
+    if (timed) cudaEventRecord(c->ev1, c->stream);
+    TS_CUDA(c, cudaGetLastError());
+    for (const Back& b : backs) {
+      cudaError_t e = cudaMemcpyAsync(b.host, b.dev, b.bytes, cudaMemcpyDeviceToHost, c->stream);
+      if (e != cudaSuccess) return fail(c, TS_ERR_CUDA, "D2H copy failed: %s", cudaGetErrorString(e));
+    }
+    TS_CUDA(c, cudaStreamSynchronize(c->stream));
+    float ms = 0.f;
+    if (timed && cudaEventElapsedTime(&ms, c->ev0, c->ev1) == cudaSuccess) c->last_kernel_ms = ms;
+    return TS_OK;
   }
 };
-inline int dev_in(ts_ctx* ctx, DevBuf& b, const void* p, size_t bytes, int is_device) {
-  if (is_device || bytes == 0) {
-    b.d = const_cast<void*>(p);
-    return TS_OK;
-  }
-  cudaError_t e = cudaMalloc(&b.d, bytes);
-  if (e != cudaSuccess) return fail(ctx, TS_ERR_NOMEM, "cudaMalloc(%zu) failed: %s", bytes, cudaGetErrorString(e));
-  b.owned = true;
-  e = cudaMemcpyAsync(b.d, p, bytes, cudaMemcpyHostToDevice, ctx->stream);
-  if (e != cudaSuccess) return fail(ctx, TS_ERR_CUDA, "H2D copy failed: %s", cudaGetErrorString(e));
-  return TS_OK;
-}
-inline int dev_out(ts_ctx* ctx, DevBuf& b, void* p, size_t bytes, int is_device) {
-  if (is_device || bytes == 0 || p == nullptr) {
-    b.d = p;
-    return TS_OK;
-  }
-  cudaError_t e = cudaMalloc(&b.d, bytes);
-  if (e != cudaSuccess) return fail(ctx, TS_ERR_NOMEM, "cudaMalloc(%zu) failed: %s", bytes, cudaGetErrorString(e));
-  b.owned = true;
-  return TS_OK;
-}
-inline int dev_back(ts_ctx* ctx, DevBuf& b, void* p, size_t bytes) {
-  if (!b.owned || bytes == 0) return TS_OK;
-  cudaError_t e = cudaMemcpyAsync(p, b.d, bytes, cudaMemcpyDeviceToHost, ctx->stream);
-  if (e != cudaSuccess) return fail(ctx, TS_ERR_CUDA, "D2H copy failed: %s", cudaGetErrorString(e));
-  return TS_OK;
-}
 
 // small host array -> device scratch slot
 template <class T>
-inline int upload(ts_ctx* c, int slot, const T* host, size_t count, T** dev) {
+inline int upload(ts_ctx* c, Slot slot, const T* host, size_t count, T** dev) {
   void* d = nullptr;
   int rc = scratch_reserve(c, slot, count * sizeof(T) + 16, &d);
   if (rc) return rc;
@@ -125,16 +180,5 @@ inline int upload(ts_ctx* c, int slot, const T* host, size_t count, T** dev) {
   *dev = (T*)d;
   return TS_OK;
 }
-
-struct KernelTimer {
-  ts_ctx* c;
-  explicit KernelTimer(ts_ctx* ctx) : c(ctx) { cudaEventRecord(c->ev0, c->stream); }
-  void stop() { cudaEventRecord(c->ev1, c->stream); }
-  // call after the stream has been synchronised
-  void read() {
-    float ms = 0.f;
-    if (cudaEventElapsedTime(&ms, c->ev0, c->ev1) == cudaSuccess) c->last_kernel_ms = ms;
-  }
-};
 
 }  // namespace ts

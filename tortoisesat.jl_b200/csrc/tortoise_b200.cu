@@ -22,41 +22,6 @@ namespace ts {
 
 using namespace ts;
 
-// generic helper: host inputs -> device scratch, one kernel, outputs back
-struct HostIO {
-  ts_ctx* c;
-  std::vector<std::pair<void*, std::pair<void*, size_t>>> outs;
-  std::vector<void*> bufs;
-  int rc = TS_OK;
-  explicit HostIO(ts_ctx* ctx) : c(ctx) {}
-  ~HostIO() { for (void* p : bufs) cudaFree(p); }
-  template <class T> T* in(const T* h, size_t count) {
-    if (rc || !h || count == 0) return nullptr;
-    void* d = nullptr;
-    if (cudaMalloc(&d, count * sizeof(T)) != cudaSuccess) { rc = fail(c, TS_ERR_NOMEM, "cudaMalloc failed"); return nullptr; }
-    bufs.push_back(d);
-    cudaMemcpyAsync(d, h, count * sizeof(T), cudaMemcpyHostToDevice, c->stream);
-    return (T*)d;
-  }
-  template <class T> T* out(T* h, size_t count) {
-    if (rc || !h || count == 0) return nullptr;
-    void* d = nullptr;
-    if (cudaMalloc(&d, count * sizeof(T)) != cudaSuccess) { rc = fail(c, TS_ERR_NOMEM, "cudaMalloc failed"); return nullptr; }
-    bufs.push_back(d);
-    outs.push_back({d, {h, count * sizeof(T)}});
-    return (T*)d;
-  }
-  int finish() {
-    if (rc) return rc;
-    c->launches++;
-    TS_CUDA(c, cudaGetLastError());
-    for (auto& o : outs) TS_CUDA(c, cudaMemcpyAsync(o.second.first, o.first, o.second.second, cudaMemcpyDeviceToHost, c->stream));
-    TS_CUDA(c, cudaStreamSynchronize(c->stream));
-    return TS_OK;
-  }
-};
-
-
 extern "C" {
 
 int ts_version(void) { return 101; }
@@ -105,7 +70,7 @@ int ts_create(ts_ctx** out, int device_id) {
 void ts_destroy(ts_ctx* c) {
   if (!c) return;
   cudaSetDevice(c->device);
-  for (int i = 0; i < 32; ++i)
+  for (int i = 0; i < SLOT_COUNT; ++i)
     if (c->scratch[i]) cudaFree(c->scratch[i]);
   if (c->d_tabG) cudaFree(c->d_tabG);
   if (c->d_tabH) cudaFree(c->d_tabH);
@@ -149,7 +114,7 @@ int ts_k3_last_split(ts_ctx* c, double* persistent_ms, double* straggler_ms, int
 int ts_k3_last_parked(ts_ctx* c, int64_t cap, int64_t* trial, int32_t* outer_at_park, int32_t* inner_at_park, int64_t* n_out) {
   if (!c || !n_out || cap < 0 || (cap > 0 && (!trial || !outer_at_park || !inner_at_park))) return TS_ERR_ARG;
   *n_out = 0;
-  if (!c->k3_timed || !c->d_k3_parked || c->k3_park_cap <= 0 || !c->scratch[15]) return TS_OK;
+  if (!c->k3_timed || !c->d_k3_parked || c->k3_park_cap <= 0 || !c->scratch[SLOT_PARK_STATE]) return TS_OK;
   TS_CUDA(c, cudaSetDevice(c->device));
   TS_CUDA(c, cudaStreamSynchronize(c->stream));
   unsigned np = 0;
@@ -159,8 +124,8 @@ int ts_k3_last_parked(ts_ctx* c, int64_t cap, int64_t* trial, int32_t* outer_at_
   std::vector<TrialState> st(n);
   std::vector<int64_t> tr(n);
   if (n) {
-    TS_CUDA(c, cudaMemcpy(st.data(), c->scratch[15], n * sizeof(TrialState), cudaMemcpyDeviceToHost));
-    TS_CUDA(c, cudaMemcpy(tr.data(), (const char*)c->scratch[15] + pc * sizeof(TrialState), n * 8, cudaMemcpyDeviceToHost));
+    TS_CUDA(c, cudaMemcpy(st.data(), c->scratch[SLOT_PARK_STATE], n * sizeof(TrialState), cudaMemcpyDeviceToHost));
+    TS_CUDA(c, cudaMemcpy(tr.data(), (const char*)c->scratch[SLOT_PARK_STATE] + pc * sizeof(TrialState), n * 8, cudaMemcpyDeviceToHost));
   }
   for (size_t i = 0; i < n; ++i) {
     trial[i] = tr[i];
@@ -173,10 +138,10 @@ int ts_k3_last_parked(ts_ctx* c, int64_t cap, int64_t* trial, int32_t* outer_at_
 
 int ts_k3_last_cycles(ts_ctx* c, int64_t n_trials, double* cycles3) {
   if (!c || !cycles3 || n_trials < 0) return TS_ERR_ARG;
-  if (n_trials > c->k3_diag_n || !c->scratch[19]) return fail(c, TS_ERR_ARG, "ts_k3_last_cycles: the last solve covered %lld trials", (long long)c->k3_diag_n);
+  if (n_trials > c->k3_diag_n || !c->scratch[SLOT_K3_CYCLES]) return fail(c, TS_ERR_ARG, "ts_k3_last_cycles: the last solve covered %lld trials", (long long)c->k3_diag_n);
   TS_CUDA(c, cudaSetDevice(c->device));
   TS_CUDA(c, cudaStreamSynchronize(c->stream));
-  TS_CUDA(c, cudaMemcpy(cycles3, c->scratch[19], (size_t)n_trials * 3 * sizeof(double), cudaMemcpyDeviceToHost));
+  TS_CUDA(c, cudaMemcpy(cycles3, c->scratch[SLOT_K3_CYCLES], (size_t)n_trials * 3 * sizeof(double), cudaMemcpyDeviceToHost));
   return TS_OK;
 }
 
@@ -200,13 +165,11 @@ int ts_fp64_peak_probe(ts_ctx* c, double* tflops_out) {
   const int iters = 4096, blocks = c->sm_count * 8, threads = 256;
   double best = 0.0;
   for (int rep = 0; rep < 4; ++rep) {
-    KernelTimer t(c);
+    Staging io(c, 0);
+    io.start();
     fp64_peak_kernel<<<blocks, threads, 0, c->stream>>>((double*)c->d_flag + 1, iters, 1.0000001, 1e-9);
-    t.stop();
     c->launches++;
-    TS_CUDA(c, cudaGetLastError());
-    TS_CUDA(c, cudaStreamSynchronize(c->stream));
-    t.read();
+    if (int rc = io.finish()) return rc;
     const double flops = 2.0 * 8 * 16 * (double)iters * (double)blocks * threads;
     const double tf = flops / (c->last_kernel_ms * 1e-3) / 1e12;
     if (rep > 0 && tf > best) best = tf;
@@ -228,6 +191,20 @@ int ts_fp64_latency_probe(ts_ctx* c, double* cycles4) {
   TS_CUDA(c, cudaMemcpy(cycles4, d + 1, 4 * sizeof(double), cudaMemcpyDeviceToHost));
   return TS_OK;
 }
+
+// the dates igrf12 / igrf12syn accept
+static bool igrf_date_ok(double date) { return date >= 1900.0 && date <= 2025.0; }
+
+// Reads back c->d_flag after the call's other results and turns a set flag into TS_ERR_DOMAIN (K1, K8).
+static int finish_domain_checked(ts_ctx* c, Staging& io, const char* msg) {
+  int bad = 0;
+  io.back(&bad, (const int*)c->d_flag, 1);
+  if (int rc = io.finish()) return rc;
+  return bad ? fail(c, TS_ERR_DOMAIN, "%s", msg) : TS_OK;
+}
+
+static const char* const K1_DOMAIN_MSG =
+    "The latitude must be between -pi/2 and +pi/2 rad and the longitude between -pi and +pi rad.";
 
 // the call's coefficient table (c->d_gh_stage), queued on the context's stream ahead of the K1 launches that read it
 static void k1_stage(ts_ctx* c, double date) {
@@ -260,7 +237,7 @@ static int igrf12_host_pipeline(ts_ctx* c, double date, int64_t n, const double*
   int rc;
   for (int i = 0; i < 2; ++i) {
     void* p;
-    if ((rc = scratch_reserve(c, 17 + i, (size_t)chunk * 6 * sizeof(double), &p))) return rc;
+    if ((rc = scratch_reserve(c, i ? SLOT_PIPE_B : SLOT_PIPE_A, (size_t)chunk * 6 * sizeof(double), &p))) return rc;
     stage[i] = (double*)p;
   }
   TS_CUDA(c, cudaMemsetAsync(c->d_flag, 0, sizeof(int), c->stream));
@@ -300,63 +277,48 @@ static int igrf12_host_pipeline(ts_ctx* c, double date, int64_t n, const double*
     if (e) cudaEventDestroy(e);
   if (err != cudaSuccess) return fail(c, TS_ERR_CUDA, "ts_igrf12_batch (host pipeline): %s", cudaGetErrorString(err));
   c->last_kernel_ms = ms_sum;
-  int bad = 0;
-  TS_CUDA(c, cudaMemcpyAsync(&bad, c->d_flag, sizeof(int), cudaMemcpyDeviceToHost, c->stream));
-  TS_CUDA(c, cudaStreamSynchronize(c->stream));
-  if (bad) return fail(c, TS_ERR_DOMAIN, "The latitude must be between -pi/2 and +pi/2 rad and the longitude between -pi and +pi rad.");
-  return TS_OK;
+  Staging io(c, 0);
+  return finish_domain_checked(c, io, K1_DOMAIN_MSG);
 }
 
 int ts_igrf12_batch(ts_ctx* c, double date, int64_t n, const double* r_m, const double* lat, const double* lon, double* Bn,
                     double* Be, double* Bd, int pointers_are_device) {
   if (!c) return TS_ERR_ARG;
   if (n < 0 || (n > 0 && (!r_m || !lat || !lon || !Bn || !Be || !Bd))) return fail(c, TS_ERR_ARG, "ts_igrf12_batch: null array or n<0");
-  if (!(date >= 1900.0 && date <= 2025.0))
+  if (!igrf_date_ok(date))
     return fail(c, TS_ERR_DATE, "This IGRF version will not work for years outside the interval [1900, 2025).");
   if (n == 0) return TS_OK;
   TS_CUDA(c, cudaSetDevice(c->device));
   if (!pointers_are_device) return igrf12_host_pipeline(c, date, n, r_m, lat, lon, Bn, Be, Bd);
   TS_CUDA(c, cudaMemsetAsync(c->d_flag, 0, sizeof(int), c->stream));
-  KernelTimer t(c);
+  Staging io(c, pointers_are_device);
+  io.start();
   k1_stage(c, date);
   k1_launch(c, c->stream, date, n, r_m, lat, lon, Bn, Be, Bd);
-  t.stop();
-  TS_CUDA(c, cudaGetLastError());
-  int bad = 0;
-  TS_CUDA(c, cudaMemcpyAsync(&bad, c->d_flag, sizeof(int), cudaMemcpyDeviceToHost, c->stream));
-  TS_CUDA(c, cudaStreamSynchronize(c->stream));
-  t.read();
-  if (bad) return fail(c, TS_ERR_DOMAIN, "The latitude must be between -pi/2 and +pi/2 rad and the longitude between -pi and +pi rad.");
-  return TS_OK;
+  return finish_domain_checked(c, io, K1_DOMAIN_MSG);
 }
 
 // igrf12syn(isv,date,itype,alt,colat,elong) [src/igrf.jl:335-534] at n points
 int ts_igrf12syn_batch(ts_ctx* c, int isv, double date, int itype, int64_t n, const double* alt_km, const double* colat_deg,
-                       const double* elong_deg, double* x, double* y, double* z, double* f, int pad) {
+                       const double* elong_deg, double* x, double* y, double* z, double* f, int pointers_are_device) {
   if (!c) return TS_ERR_ARG;
   if (n < 0 || (n > 0 && (!alt_km || !colat_deg || !elong_deg || !x || !y || !z || !f))) return fail(c, TS_ERR_ARG, "ts_igrf12syn_batch: null array or n<0");
   if (isv != 0 && isv != 1) return fail(c, TS_ERR_ARG, "ts_igrf12syn_batch: isv must be 0 or 1");
   if (itype != 1 && itype != 2) return fail(c, TS_ERR_ARG, "ts_igrf12syn_batch: itype must be 1 (geodetic) or 2 (geocentric)");
-  if (!(date >= 1900.0 && date <= 2025.0))
+  if (!igrf_date_ok(date))
     return fail(c, TS_ERR_DATE, "This IGRF version will not work for years outside the interval [1900, 2025).");
   if (n == 0) return TS_OK;
   TS_CUDA(c, cudaSetDevice(c->device));
-  int rc;
-  DevBuf da, dc, de, ox, oy, oz, of;
-  const size_t b = (size_t)n * sizeof(double);
-  if ((rc = dev_in(c, da, alt_km, b, pad)) || (rc = dev_in(c, dc, colat_deg, b, pad)) || (rc = dev_in(c, de, elong_deg, b, pad))) return rc;
-  if ((rc = dev_out(c, ox, x, b, pad)) || (rc = dev_out(c, oy, y, b, pad)) || (rc = dev_out(c, oz, z, b, pad)) || (rc = dev_out(c, of, f, b, pad))) return rc;
+  Staging io(c, pointers_are_device);
+  const size_t m = (size_t)n;
+  const double *da = io.in(alt_km, m), *dc = io.in(colat_deg, m), *de = io.in(elong_deg, m);
+  double *ox = io.out(x, m), *oy = io.out(y, m), *oz = io.out(z, m), *of = io.out(f, m);
+  if (io.rc) return io.rc;
   const SynEpoch ep = igrf12syn_epoch(isv, date);
-  KernelTimer tm(c);
-  k6_igrf12syn<<<(unsigned)((n + 127) / 128), 128, 0, c->stream>>>(c->d_tabGH, ep, itype, n, (const double*)da.d, (const double*)dc.d,
-                                                                   (const double*)de.d, (double*)ox.d, (double*)oy.d, (double*)oz.d, (double*)of.d);
-  tm.stop();
+  io.start();
+  k6_igrf12syn<<<(unsigned)((n + 127) / 128), 128, 0, c->stream>>>(c->d_tabGH, ep, itype, n, da, dc, de, ox, oy, oz, of);
   c->launches++;
-  TS_CUDA(c, cudaGetLastError());
-  if ((rc = dev_back(c, ox, x, b)) || (rc = dev_back(c, oy, y, b)) || (rc = dev_back(c, oz, z, b)) || (rc = dev_back(c, of, f, b))) return rc;
-  TS_CUDA(c, cudaStreamSynchronize(c->stream));
-  tm.read();
-  return TS_OK;
+  return io.finish();
 }
 
 // ---------------------------------------------------------------------------- K8
@@ -370,80 +332,76 @@ static int field_map_dims(ts_ctx* c, const char* fn, int64_t n0, int64_t n1) {
 // FM1: Thomas solves along axis 1 (j) for every data row, then along axis 0 (i) for every padded column.  The j-lines
 // are made columns by a tiled transpose into a (n1+2) x n0 x 3 buffer, solved in place, and transposed into rows
 // 1..n0 of C, where the i-pass solves in place.
-int ts_field_map_prefilter(ts_ctx* c, int64_t n0, int64_t n1, const double* grid, double* coefs, int pad) {
+int ts_field_map_prefilter(ts_ctx* c, int64_t n0, int64_t n1, const double* grid, double* coefs, int pointers_are_device) {
   if (!c) return TS_ERR_ARG;
   if (!grid || !coefs) return fail(c, TS_ERR_ARG, "ts_field_map_prefilter: null array");
   int rc;
   if ((rc = field_map_dims(c, "ts_field_map_prefilter", n0, n1))) return rc;
   TS_CUDA(c, cudaSetDevice(c->device));
-  const size_t b_in = (size_t)n0 * n1 * 3 * sizeof(double), b_out = (size_t)(n0 + 2) * (n1 + 2) * 3 * sizeof(double);
   std::vector<double> inv((size_t)(n0 + n1));
   k8_thomas_factors(n0, inv.data());
   k8_thomas_factors(n1, inv.data() + n0);
-  DevBuf dg, dc, dt, df;
-  if ((rc = dev_in(c, dg, grid, b_in, pad)) || (rc = dev_out(c, dc, coefs, b_out, pad)) ||
-      (rc = dev_in(c, df, inv.data(), inv.size() * sizeof(double), 0)))
-    return rc;
-  const size_t b_t = (size_t)(n1 + 2) * n0 * 3 * sizeof(double);
-  cudaError_t e = cudaMalloc(&dt.d, b_t);
-  if (e != cudaSuccess) return fail(c, TS_ERR_NOMEM, "cudaMalloc(%zu) failed: %s", b_t, cudaGetErrorString(e));
-  dt.owned = true;
-  double *G = (double*)dg.d, *Cf = (double*)dc.d, *T = (double*)dt.d;
-  const double *inv0 = (const double*)df.d, *inv1 = inv0 + n0;
+  Staging io(c, pointers_are_device), host(c, 0);   // the factors are always a host array
+  const double* G = io.in(grid, (size_t)n0 * n1 * 3);
+  double* Cf = io.out(coefs, (size_t)(n0 + 2) * (n1 + 2) * 3);
+  const double* inv0 = host.in(inv.data(), inv.size());
+  double* T = (double*)io.alloc((size_t)(n1 + 2) * n0 * 3 * sizeof(double));
+  if (io.rc || host.rc) return io.rc ? io.rc : host.rc;
+  const double* inv1 = inv0 + n0;
   const dim3 tb(K8_TILE, 8);
-  KernelTimer tm(c);
+  io.start();
   k8_transpose3<<<dim3((unsigned)((n1 + K8_TILE - 1) / K8_TILE), (unsigned)((n0 + K8_TILE - 1) / K8_TILE)), tb, 0, c->stream>>>(
       G, n0, n1, T + n0 * 3, n0 * 3);
   k8_prefilter_cols<<<(unsigned)((n0 * 3 + 127) / 128), 128, 0, c->stream>>>(T, n1, n0 * 3, inv1);
   k8_transpose3<<<dim3((unsigned)((n0 + K8_TILE - 1) / K8_TILE), (unsigned)((n1 + 2 + K8_TILE - 1) / K8_TILE)), tb, 0, c->stream>>>(
       T, n1 + 2, n0, Cf + (n1 + 2) * 3, (n1 + 2) * 3);
   k8_prefilter_cols<<<(unsigned)(((n1 + 2) * 3 + 127) / 128), 128, 0, c->stream>>>(Cf, n0, (n1 + 2) * 3, inv0);
-  tm.stop();
   c->launches += 4;
-  TS_CUDA(c, cudaGetLastError());
-  if ((rc = dev_back(c, dc, coefs, b_out))) return rc;
-  TS_CUDA(c, cudaStreamSynchronize(c->stream));
-  tm.read();
-  return TS_OK;
+  return io.finish();
 }
 
 // FM2 + FM3 at n points; FM4 (the component index) is left to the caller: every row holds all three components.
 int ts_field_map_eval_batch(ts_ctx* c, int64_t n0, int64_t n1, const double* coefs, int64_t n, const double* x0,
-                            const double* x1, double* out, int pad) {
+                            const double* x1, double* out, int pointers_are_device) {
   if (!c) return TS_ERR_ARG;
   if (n < 0 || !coefs || (n > 0 && (!x0 || !x1 || !out))) return fail(c, TS_ERR_ARG, "ts_field_map_eval_batch: null array or n<0");
   int rc;
   if ((rc = field_map_dims(c, "ts_field_map_eval_batch", n0, n1))) return rc;
   if (n == 0) return TS_OK;
   TS_CUDA(c, cudaSetDevice(c->device));
-  const size_t b_c = (size_t)(n0 + 2) * (n1 + 2) * 3 * sizeof(double), b = (size_t)n * sizeof(double);
-  DevBuf dc, da, db, dout;
-  if ((rc = dev_in(c, dc, coefs, b_c, pad)) || (rc = dev_in(c, da, x0, b, pad)) || (rc = dev_in(c, db, x1, b, pad)) ||
-      (rc = dev_out(c, dout, out, 3 * b, pad)))
-    return rc;
   const int64_t nodes = (n0 + 2) * (n1 + 2);
+  Staging io(c, pointers_are_device);
+  const double *dc = io.in(coefs, (size_t)nodes * 3), *da = io.in(x0, (size_t)n), *db = io.in(x1, (size_t)n);
+  double* dout = io.out(out, (size_t)n * 3);
+  if (io.rc) return io.rc;
   void* c4;
-  if ((rc = scratch_reserve(c, 27, (size_t)nodes * 4 * sizeof(double), &c4))) return rc;   // slot 27: K8 only
+  if ((rc = scratch_reserve(c, SLOT_TABLE, (size_t)nodes * 4 * sizeof(double), &c4))) return rc;
   TS_CUDA(c, cudaMemsetAsync(c->d_flag, 0, sizeof(int), c->stream));
-  KernelTimer tm(c);
-  k8_pad4<<<(unsigned)((nodes + 255) / 256), 256, 0, c->stream>>>((const double*)dc.d, nodes, (double*)c4);
+  io.start();
+  k8_pad4<<<(unsigned)((nodes + 255) / 256), 256, 0, c->stream>>>(dc, nodes, (double*)c4);
   k8_field_map_eval<<<(unsigned)((n + K8_THREADS - 1) / K8_THREADS), K8_THREADS, 0, c->stream>>>(
-      (const double*)c4, n0, n1, n, (const double*)da.d, (const double*)db.d, (double*)dout.d, c->d_flag);
-  tm.stop();
+      (const double*)c4, n0, n1, n, da, db, dout, c->d_flag);
   c->launches += 2;
-  TS_CUDA(c, cudaGetLastError());
-  if ((rc = dev_back(c, dout, out, 3 * b))) return rc;
-  int bad = 0;
-  TS_CUDA(c, cudaMemcpyAsync(&bad, c->d_flag, sizeof(int), cudaMemcpyDeviceToHost, c->stream));
-  TS_CUDA(c, cudaStreamSynchronize(c->stream));
-  tm.read();
-  if (bad) return fail(c, TS_ERR_DOMAIN, "ts_field_map_eval_batch: non-finite index (the rows of those points are NaN)");
-  return TS_OK;
+  return finish_domain_checked(c, io, "ts_field_map_eval_batch: non-finite index (the rows of those points are NaN)");
 }
 
 // ---------------------------------------------------------------------------- K2
 static_assert(sizeof(ts_field_opts) == sizeof(ts_field_opts_dev), "field opts layout");
 
+// K2b over `rows` table rows from row `lo` of n orbits: one launch per IGRF degree present (any13 / any10); `skip`
+// (nullable) leaves out the orbits whose cutoff index is already set
+static void k2b_launch(ts_ctx* c, bool any13, bool any10, int64_t n, int64_t rows, const ts_field_opts_dev* fo, const int64_t* offs,
+                       const int64_t* lim, const double* pos, double* B, int64_t lo = 0, const int64_t* skip = nullptr) {
+  const dim3 grid((unsigned)n, (unsigned)((rows + K2B_THREADS - 1) / K2B_THREADS));
+  if (any13) {
+    k2b_field_rows<13><<<grid, K2B_THREADS, 0, c->stream>>>(c->d_tabG, c->d_tabH, fo, offs, lim, pos, B, 13, lo, skip);
+    c->launches++;
+  }
+  if (any10) {
+    k2b_field_rows<10><<<grid, K2B_THREADS, 0, c->stream>>>(c->d_tabG, c->d_tabH, fo, offs, lim, pos, B, 10, lo, skip);
+    c->launches++;
+  }
+}
 
 int ts_magnetic_simulation_batch(ts_ctx* c, int64_t n_trials, const double* kep6, const ts_field_opts* opts,
                                  const int64_t* B_offs, const int64_t* rows_limit, double* B_eci, double* pos, double* vel,
@@ -455,7 +413,7 @@ int ts_magnetic_simulation_batch(ts_ctx* c, int64_t n_trials, const double* kep6
   bool any13 = false, any10 = false;
   int64_t maxN = 0;
   for (int64_t t = 0; t < n_trials; ++t) {
-    if (!(opts[t].igrf_date >= 1900.0 && opts[t].igrf_date <= 2025.0))
+    if (!igrf_date_ok(opts[t].igrf_date))
       return fail(c, TS_ERR_DATE, "trial %lld: IGRF date outside [1900, 2025]", (long long)t);
     if (opts[t].N < 1 || B_offs[t + 1] - B_offs[t] < 2 * opts[t].N)
       return fail(c, TS_ERR_ARG, "trial %lld: N < 1 or B_offs does not leave 2N rows", (long long)t);
@@ -465,50 +423,33 @@ int ts_magnetic_simulation_batch(ts_ctx* c, int64_t n_trials, const double* kep6
   TS_CUDA(c, cudaSetDevice(c->device));
   const int64_t total_rows = B_offs[n_trials];
   int rc;
-  DevBuf dkep, dB, dpos, dvel;
-  if ((rc = dev_in(c, dkep, kep6, (size_t)n_trials * 6 * sizeof(double), pointers_are_device))) return rc;
-  if ((rc = dev_out(c, dB, B_eci, (size_t)total_rows * 3 * sizeof(double), pointers_are_device))) return rc;
-  const size_t pos_bytes = (size_t)(total_rows + n_trials) * 3 * sizeof(double);
-  double* d_pos = nullptr;
-  if (pos) {
-    if ((rc = dev_out(c, dpos, pos, pos_bytes, pointers_are_device))) return rc;
-    d_pos = (double*)dpos.d;
-  } else {
+  Staging io(c, pointers_are_device);
+  const double* d_kep = io.in(kep6, (size_t)n_trials * 6);
+  double* d_B = io.out(B_eci, (size_t)total_rows * 3);
+  const size_t pos_count = (size_t)(total_rows + n_trials) * 3;
+  double* d_pos = io.out(pos, pos_count);
+  if (io.rc) return io.rc;
+  if (!pos) {
     void* p = nullptr;
-    if ((rc = scratch_reserve(c, 0, pos_bytes, &p))) return rc;
+    if ((rc = scratch_reserve(c, SLOT_POSITIONS, pos_count * sizeof(double), &p))) return rc;
     d_pos = (double*)p;
   }
-  if (vel && (rc = dev_out(c, dvel, vel, pos_bytes, pointers_are_device))) return rc;
+  double* d_vel = io.out(vel, pos_count);
+  if (io.rc) return io.rc;
   ts_field_opts_dev* d_opts = nullptr;
   int64_t *d_offs = nullptr, *d_lim = nullptr;
-  if ((rc = upload(c, 1, (const ts_field_opts_dev*)opts, (size_t)n_trials, &d_opts))) return rc;
-  if ((rc = upload(c, 2, B_offs, (size_t)n_trials + 1, &d_offs))) return rc;
-  if (rows_limit && (rc = upload(c, 3, rows_limit, (size_t)n_trials, &d_lim))) return rc;
-  KernelTimer tm(c);
-  k2a_orbit_euler<<<(unsigned)((n_trials + 127) / 128), 128, 0, c->stream>>>(n_trials, (const double*)dkep.d, d_opts, d_offs, d_lim,
-                                                                             d_pos, vel ? (double*)dvel.d : nullptr);
+  if ((rc = upload(c, SLOT_ARGS_A, (const ts_field_opts_dev*)opts, (size_t)n_trials, &d_opts))) return rc;
+  if ((rc = upload(c, SLOT_ARGS_B, B_offs, (size_t)n_trials + 1, &d_offs))) return rc;
+  if (rows_limit && (rc = upload(c, SLOT_ARGS_C, rows_limit, (size_t)n_trials, &d_lim))) return rc;
+  io.start();
+  k2a_orbit_euler<<<(unsigned)((n_trials + 127) / 128), 128, 0, c->stream>>>(n_trials, d_kep, d_opts, d_offs, d_lim, d_pos, d_vel);
   c->launches++;
-  dim3 grid((unsigned)n_trials, (unsigned)((2 * maxN + K2B_THREADS - 1) / K2B_THREADS));
-  if (any13) {
-    k2b_field_rows<13><<<grid, K2B_THREADS, 0, c->stream>>>(c->d_tabG, c->d_tabH, d_opts, d_offs, d_lim, d_pos, (double*)dB.d, 13);
-    c->launches++;
-  }
-  if (any10) {
-    k2b_field_rows<10><<<grid, K2B_THREADS, 0, c->stream>>>(c->d_tabG, c->d_tabH, d_opts, d_offs, d_lim, d_pos, (double*)dB.d, 10);
-    c->launches++;
-  }
-  tm.stop();
-  TS_CUDA(c, cudaGetLastError());
-  if ((rc = dev_back(c, dB, B_eci, (size_t)total_rows * 3 * sizeof(double)))) return rc;
-  if (pos && (rc = dev_back(c, dpos, pos, pos_bytes))) return rc;
-  if (vel && (rc = dev_back(c, dvel, vel, pos_bytes))) return rc;
-  TS_CUDA(c, cudaStreamSynchronize(c->stream));
-  tm.read();
-  return TS_OK;
+  k2b_launch(c, any13, any10, n_trials, 2 * maxN, d_opts, d_offs, d_lim, d_pos, d_B);
+  return io.finish();
 }
 
 static int gramian_common(ts_ctx* c, int64_t n_trials, const double* B_eci, const int64_t* B_offs, const int64_t* rows,
-                          const double* dt, const double* cutoff, double* G, int64_t* tf_index, int pad) {
+                          const double* dt, const double* cutoff, double* G, int64_t* tf_index, int pointers_are_device) {
   if (!c) return TS_ERR_ARG;
   if (n_trials < 0 || (n_trials > 0 && (!B_eci || !B_offs || !rows || !dt))) return fail(c, TS_ERR_ARG, "gramian: null argument");
   if (n_trials == 0) return TS_OK;
@@ -516,47 +457,42 @@ static int gramian_common(ts_ctx* c, int64_t n_trials, const double* B_eci, cons
   int64_t total = 0;
   for (int64_t t = 0; t < n_trials; ++t) total = (B_offs[t] + rows[t] > total) ? B_offs[t] + rows[t] : total;
   int rc;
-  DevBuf dB, dG;
-  if ((rc = dev_in(c, dB, B_eci, (size_t)total * 3 * sizeof(double), pad))) return rc;
-  if (G && (rc = dev_out(c, dG, G, (size_t)total * 9 * sizeof(double), pad))) return rc;
+  Staging io(c, pointers_are_device);
+  const double* d_B = io.in(B_eci, (size_t)total * 3);
+  double* d_G = io.out(G, (size_t)total * 9);
+  if (io.rc) return io.rc;
   int64_t *d_offs, *d_rows, *d_idx = nullptr;
   double *d_dt, *d_cut = nullptr;
-  if ((rc = upload(c, 1, B_offs, (size_t)n_trials, &d_offs))) return rc;
-  if ((rc = upload(c, 2, rows, (size_t)n_trials, &d_rows))) return rc;
-  if ((rc = upload(c, 3, dt, (size_t)n_trials, &d_dt))) return rc;
-  if (cutoff && (rc = upload(c, 4, cutoff, (size_t)n_trials, &d_cut))) return rc;
+  if ((rc = upload(c, SLOT_ARGS_A, B_offs, (size_t)n_trials, &d_offs))) return rc;
+  if ((rc = upload(c, SLOT_ARGS_B, rows, (size_t)n_trials, &d_rows))) return rc;
+  if ((rc = upload(c, SLOT_ARGS_C, dt, (size_t)n_trials, &d_dt))) return rc;
+  if (cutoff && (rc = upload(c, SLOT_CUTOFF, cutoff, (size_t)n_trials, &d_cut))) return rc;
   if (tf_index) {
     void* p;
-    if ((rc = scratch_reserve(c, 5, (size_t)n_trials * sizeof(int64_t), &p))) return rc;
+    if ((rc = scratch_reserve(c, SLOT_PER_TRIAL, (size_t)n_trials * sizeof(int64_t), &p))) return rc;
     d_idx = (int64_t*)p;
+    io.back(tf_index, d_idx, (size_t)n_trials);
   }
-  KernelTimer tm(c);
-  k2c_gramian_cutoff<<<(unsigned)((n_trials + 127) / 128), 128, 0, c->stream>>>(n_trials, (const double*)dB.d, d_offs, d_rows, d_dt,
-                                                                                d_cut, G ? (double*)dG.d : nullptr, d_idx);
-  tm.stop();
+  io.start();
+  k2c_gramian_cutoff<<<(unsigned)((n_trials + 127) / 128), 128, 0, c->stream>>>(n_trials, d_B, d_offs, d_rows, d_dt, d_cut, d_G, d_idx);
   c->launches++;
-  TS_CUDA(c, cudaGetLastError());
-  if (G && (rc = dev_back(c, dG, G, (size_t)total * 9 * sizeof(double)))) return rc;
-  if (tf_index) TS_CUDA(c, cudaMemcpyAsync(tf_index, d_idx, (size_t)n_trials * sizeof(int64_t), cudaMemcpyDeviceToHost, c->stream));
-  TS_CUDA(c, cudaStreamSynchronize(c->stream));
-  tm.read();
-  return TS_OK;
+  return io.finish();
 }
 
 int ts_magnetic_gramian_batch(ts_ctx* c, int64_t n_trials, const double* B_eci, const int64_t* B_offs, const int64_t* rows,
-                              const double* dt, double* G, int pad) {
+                              const double* dt, double* G, int pointers_are_device) {
   if (c && !G) return fail(c, TS_ERR_ARG, "ts_magnetic_gramian_batch: G is null");
-  return gramian_common(c, n_trials, B_eci, B_offs, rows, dt, nullptr, G, nullptr, pad);
+  return gramian_common(c, n_trials, B_eci, B_offs, rows, dt, nullptr, G, nullptr, pointers_are_device);
 }
 
 int ts_condition_cutoff_batch(ts_ctx* c, int64_t n_trials, const double* B_eci, const int64_t* B_offs, const int64_t* rows,
-                              const double* dt, const double* cutoff, int64_t* tf_index, int pad) {
+                              const double* dt, const double* cutoff, int64_t* tf_index, int pointers_are_device) {
   if (c && (!cutoff || !tf_index)) return fail(c, TS_ERR_ARG, "ts_condition_cutoff_batch: null argument");
-  return gramian_common(c, n_trials, B_eci, B_offs, rows, dt, cutoff, nullptr, tf_index, pad);
+  return gramian_common(c, n_trials, B_eci, B_offs, rows, dt, cutoff, nullptr, tf_index, pointers_are_device);
 }
 
 int ts_condition_based_time_batch(ts_ctx* c, int64_t n_trials, const double* G, const int64_t* offs, const int64_t* rows,
-                                  const double* cutoff, int64_t* tf_index, int pad) {
+                                  const double* cutoff, int64_t* tf_index, int pointers_are_device) {
   if (!c) return TS_ERR_ARG;
   if (n_trials < 0 || (n_trials > 0 && (!G || !offs || !rows || !cutoff || !tf_index)))
     return fail(c, TS_ERR_ARG, "ts_condition_based_time_batch: null argument");
@@ -565,25 +501,22 @@ int ts_condition_based_time_batch(ts_ctx* c, int64_t n_trials, const double* G, 
   int64_t total = 0;
   for (int64_t t = 0; t < n_trials; ++t) total = (offs[t] + rows[t] > total) ? offs[t] + rows[t] : total;
   int rc;
-  DevBuf dG;
-  if ((rc = dev_in(c, dG, G, (size_t)total * 9 * sizeof(double), pad))) return rc;
+  Staging io(c, pointers_are_device);
+  const double* d_G = io.in(G, (size_t)total * 9);
+  if (io.rc) return io.rc;
   int64_t *d_offs, *d_rows, *d_idx;
   double* d_cut;
-  if ((rc = upload(c, 1, offs, (size_t)n_trials, &d_offs))) return rc;
-  if ((rc = upload(c, 2, rows, (size_t)n_trials, &d_rows))) return rc;
-  if ((rc = upload(c, 4, cutoff, (size_t)n_trials, &d_cut))) return rc;
+  if ((rc = upload(c, SLOT_ARGS_A, offs, (size_t)n_trials, &d_offs))) return rc;
+  if ((rc = upload(c, SLOT_ARGS_B, rows, (size_t)n_trials, &d_rows))) return rc;
+  if ((rc = upload(c, SLOT_CUTOFF, cutoff, (size_t)n_trials, &d_cut))) return rc;
   void* p;
-  if ((rc = scratch_reserve(c, 5, (size_t)n_trials * sizeof(int64_t), &p))) return rc;
+  if ((rc = scratch_reserve(c, SLOT_PER_TRIAL, (size_t)n_trials * sizeof(int64_t), &p))) return rc;
   d_idx = (int64_t*)p;
-  KernelTimer tm(c);
-  k2d_condition_time<<<(unsigned)((n_trials + 127) / 128), 128, 0, c->stream>>>(n_trials, (const double*)dG.d, d_offs, d_rows, d_cut, d_idx);
-  tm.stop();
+  io.back(tf_index, d_idx, (size_t)n_trials);
+  io.start();
+  k2d_condition_time<<<(unsigned)((n_trials + 127) / 128), 128, 0, c->stream>>>(n_trials, d_G, d_offs, d_rows, d_cut, d_idx);
   c->launches++;
-  TS_CUDA(c, cudaGetLastError());
-  TS_CUDA(c, cudaMemcpyAsync(tf_index, d_idx, (size_t)n_trials * sizeof(int64_t), cudaMemcpyDeviceToHost, c->stream));
-  TS_CUDA(c, cudaStreamSynchronize(c->stream));
-  tm.read();
-  return TS_OK;
+  return io.finish();
 }
 
 // ---------------------------------------------------------------------------- K3
@@ -709,7 +642,7 @@ static int k3_launch(ts_ctx* c, K3Args& a, const int64_t* N_i_host, const double
   }
   int rc;
   int64_t* d_order = nullptr;
-  if ((rc = upload(c, 5, order.data(), (size_t)n_trials, &d_order))) return rc;
+  if ((rc = upload(c, SLOT_PER_TRIAL, order.data(), (size_t)n_trials, &d_order))) return rc;
   void *p_work, *p_q, *p_diag;
   Nmax += (Nmax & 1);  // even: keeps every per-knot record 16-byte aligned for the asynchronous copies
   // ragged arena: warp w's four slots are sized for its static first group (the w-th of the horizon-sorted queue; the
@@ -731,13 +664,13 @@ static int k3_launch(ts_ctx* c, K3Args& a, const int64_t* N_i_host, const double
       arena += 4 * cap * K3_SLOT_DOUBLES_PER_KNOT;
     }
   }
-  if ((rc = scratch_reserve(c, 6, (size_t)(arena + 2) * sizeof(double) + 256, &p_work))) return rc;
+  if ((rc = scratch_reserve(c, SLOT_K3_ARENA, (size_t)(arena + 2) * sizeof(double) + 256, &p_work))) return rc;
   long long* d_woff = nullptr;
   int* d_wcap = nullptr;
-  if ((rc = upload(c, 23, warp_off.data(), (size_t)n_warps, &d_woff))) return rc;
-  if ((rc = upload(c, 24, warp_cap.data(), (size_t)n_warps, &d_wcap))) return rc;
-  if ((rc = scratch_reserve(c, 4, 128, &p_q))) return rc;
-  if ((rc = scratch_reserve(c, 19, (size_t)n_trials * 3 * sizeof(double) + 64, &p_diag))) return rc;
+  if ((rc = upload(c, SLOT_K3_WARP_OFFS, warp_off.data(), (size_t)n_warps, &d_woff))) return rc;
+  if ((rc = upload(c, SLOT_K3_WARP_CAPS, warp_cap.data(), (size_t)n_warps, &d_wcap))) return rc;
+  if ((rc = scratch_reserve(c, SLOT_K3_COUNTERS, 128, &p_q))) return rc;
+  if ((rc = scratch_reserve(c, SLOT_K3_CYCLES, (size_t)n_trials * 3 * sizeof(double) + 64, &p_diag))) return rc;
   {
     unsigned long long h_q[16] = {0};
     h_q[0] = (unsigned long long)(4 * n_warps);   // the dynamic queue starts behind the static first groups
@@ -786,7 +719,7 @@ static int k3_launch(ts_ctx* c, K3Args& a, const int64_t* N_i_host, const double
     // (no region is ever re-used); the parking places are limited to what fits 60% of the free device memory
     size_t free_b = 0, total_b = 0;
     TS_CUDA(c, cudaMemGetInfo(&free_b, &total_b));
-    const double budget = 0.6 * (double)(free_b + c->scratch_bytes[16] + c->scratch_bytes[25]) / 8.0;
+    const double budget = 0.6 * (double)(free_b + c->scratch_bytes[SLOT_PARK_DATA] + c->scratch_bytes[SLOT_K3_POOL]) / 8.0;
     double need = 0.0, pool_need = 0.0;
     int64_t cap_fit = 0;
     for (int64_t i = 0; i < cap; ++i) {
@@ -799,11 +732,11 @@ static int k3_launch(ts_ctx* c, K3Args& a, const int64_t* N_i_host, const double
     }
     cap = cap_fit;
     void *p_ps, *p_pd, *p_pool;
-    if ((rc = scratch_reserve(c, 25, (size_t)pool_need * sizeof(double) + 256, &p_pool))) return rc;
+    if ((rc = scratch_reserve(c, SLOT_K3_POOL, (size_t)pool_need * sizeof(double) + 256, &p_pool))) return rc;
     a.pool = (double*)p_pool;
     a.pool_cap = (long long)pool_need;
-    if ((rc = scratch_reserve(c, 15, (size_t)cap * (sizeof(TrialState) + 8 + 8 + 4) + 64, &p_ps))) return rc;
-    if ((rc = scratch_reserve(c, 16, (size_t)need * sizeof(double) + 64, &p_pd))) return rc;
+    if ((rc = scratch_reserve(c, SLOT_PARK_STATE, (size_t)cap * (sizeof(TrialState) + 8 + 8 + 4) + 64, &p_ps))) return rc;
+    if ((rc = scratch_reserve(c, SLOT_PARK_DATA, (size_t)need * sizeof(double) + 64, &p_pd))) return rc;
     a.park_cap = (int)cap;
     a.park_state = (TrialState*)p_ps;
     a.park_trial = (int64_t*)((char*)p_ps + (size_t)cap * sizeof(TrialState));
@@ -840,7 +773,7 @@ int ts_alilqr_solve_batch(ts_ctx* c, int64_t n_trials, const int64_t* N_i, const
                           const double* xf, const double* Jmat, const double* Qd, const double* Qfd, const double* Rd,
                           const double* B_eci, const int64_t* B_offs, const int64_t* B_rows, const double* index_scale,
                           const double* clock_rate, double dt, const double* U0, const ts_ilqr_opts* opts, double* X,
-                          double* U, double* K, ts_trial_outcome* out, int pad) {
+                          double* U, double* K, ts_trial_outcome* out, int pointers_are_device) {
   if (!c) return TS_ERR_ARG;
   if (n_trials < 0 || (n_trials > 0 && (!N_i || !offs || !x0 || !xf || !Jmat || !Qd || !Qfd || !Rd || !B_eci || !B_offs || !B_rows ||
                                         !index_scale || !clock_rate || !X || !U || !out)))
@@ -864,12 +797,14 @@ int ts_alilqr_solve_batch(ts_ctx* c, int64_t n_trials, const int64_t* N_i, const
   }
   TS_CUDA(c, cudaSetDevice(c->device));
   int rc;
-  DevBuf dB, dU0, dX, dU, dK;
-  if ((rc = dev_in(c, dB, B_eci, (size_t)total_rows * 3 * sizeof(double), pad))) return rc;
-  if (U0 && (rc = dev_in(c, dU0, U0, (size_t)total_knots * 3 * sizeof(double), pad))) return rc;
-  if ((rc = dev_out(c, dX, X, (size_t)total_knots * 8 * sizeof(double), pad))) return rc;
-  if ((rc = dev_out(c, dU, U, (size_t)total_knots * 3 * sizeof(double), pad))) return rc;
-  if (K && (rc = dev_out(c, dK, K, (size_t)total_knots * 24 * sizeof(double), pad))) return rc;
+  Staging io(c, pointers_are_device);
+  K3Args a;
+  a.B_eci = io.in(B_eci, (size_t)total_rows * 3);
+  a.U0 = io.in(U0, (size_t)total_knots * 3);
+  a.X = io.out(X, (size_t)total_knots * 8);
+  a.U = io.out(U, (size_t)total_knots * 3);
+  a.K = io.out(K, (size_t)total_knots * 24);
+  if (io.rc) return io.rc;
   // per-trial small arrays -> one packed upload
   const size_t T = (size_t)n_trials;
   const size_t n_i64 = 4 * T, n_f64 = (8 + 8 + 9 + 8 + 8 + 3 + 1 + 1) * T;
@@ -885,37 +820,41 @@ int ts_alilqr_solve_batch(ts_ctx* c, int64_t n_trials, const int64_t* N_i, const
                o_is = put(index_scale, 1), o_cr = put(clock_rate, 1);
   int64_t* d_i = nullptr;
   double* d_f = nullptr;
-  if ((rc = upload(c, 1, hi.data(), n_i64, &d_i))) return rc;
-  if ((rc = upload(c, 2, hf.data(), n_f64, &d_f))) return rc;
+  if ((rc = upload(c, SLOT_ARGS_A, hi.data(), n_i64, &d_i))) return rc;
+  if ((rc = upload(c, SLOT_ARGS_B, hf.data(), n_f64, &d_f))) return rc;
   void* p_out;
-  if ((rc = scratch_reserve(c, 3, T * sizeof(ts_trial_outcome), &p_out))) return rc;
-  K3Args a;
+  if ((rc = scratch_reserve(c, SLOT_ARGS_C, T * sizeof(ts_trial_outcome), &p_out))) return rc;
   a.n_trials = n_trials;
   a.N_i = d_i + 0 * T; a.offs = d_i + 1 * T; a.B_offs = d_i + 2 * T; a.B_rows = d_i + 3 * T;
   a.x0 = d_f + o_x0; a.xf = d_f + o_xf; a.Jmat = d_f + o_J; a.Qd = d_f + o_Qd; a.Qfd = d_f + o_Qfd; a.Rd = d_f + o_Rd;
   a.index_scale = d_f + o_is; a.clock_rate = d_f + o_cr;
-  a.B_eci = (const double*)dB.d;
   a.dt = dt;
-  a.U0 = U0 ? (const double*)dU0.d : nullptr;
   memcpy(&a.opts, &o, sizeof(o));
-  a.X = (double*)dX.d; a.U = (double*)dU.d; a.K = K ? (double*)dK.d : nullptr;
   a.out = (ts_trial_outcome_dev*)p_out;
+  io.back(out, (const ts_trial_outcome*)p_out, T);
   std::vector<double> diff(T);
   for (size_t t = 0; t < T; ++t) diff[t] = slew_angle(x0 + 8 * t, xf + 8 * t);
-  KernelTimer tm(c);
+  io.start();
   if ((rc = k3_launch(c, a, N_i, diff.data(), all_inertia_diagonal(Jmat, n_trials)))) return rc;
-  tm.stop();
-  if ((rc = dev_back(c, dX, X, (size_t)total_knots * 8 * sizeof(double)))) return rc;
-  if ((rc = dev_back(c, dU, U, (size_t)total_knots * 3 * sizeof(double)))) return rc;
-  if (K && (rc = dev_back(c, dK, K, (size_t)total_knots * 24 * sizeof(double)))) return rc;
-  TS_CUDA(c, cudaMemcpyAsync(out, p_out, T * sizeof(ts_trial_outcome), cudaMemcpyDeviceToHost, c->stream));
-  TS_CUDA(c, cudaStreamSynchronize(c->stream));
-  tm.read();
-  return TS_OK;
+  return io.finish();
 }
 
 // ---------------------------------------------------------------------------- prep + K4
 static_assert(sizeof(ts_tvlqr_opts) == sizeof(ts_tvlqr_opts_dev), "tvlqr opts layout");
+
+// K4's linearisation table: lin_offs (the prefix sum of the n trials' N_i - 1 steps, uploaded) and the records AB
+// (54 doubles per step) + clk (one per step)
+static int k4_lin_table(ts_ctx* c, const int64_t* N_i, size_t n, K4Args& a) {
+  std::vector<int64_t> lin(n + 1, 0);
+  for (size_t t = 0; t < n; ++t) lin[t + 1] = lin[t] + (N_i[t] - 1);
+  int64_t* d_lin;
+  void* p_ab;
+  int rc;
+  if ((rc = upload(c, SLOT_TABLE, lin.data(), n + 1, &d_lin))) return rc;
+  if ((rc = scratch_reserve(c, SLOT_LIN_RECORDS, (size_t)lin[n] * 55 * 8 + 64, &p_ab))) return rc;
+  a.AB = (double*)p_ab; a.clk = a.AB + (size_t)lin[n] * 54; a.lin_offs = d_lin; a.lin_total = lin[n];
+  return TS_OK;
+}
 
 void ts_tvlqr_default_opts(ts_tvlqr_opts* o) {
   if (!o) return;
@@ -947,37 +886,34 @@ int ts_slew_weights_batch(ts_ctx* c, int64_t n, const double* x0, const double* 
   double* d_f;
   int64_t* d_g = nullptr;
   int rc;
-  if ((rc = upload(c, 1, hf.data(), hf.size(), &d_f))) return rc;
-  if (goffs && (rc = upload(c, 2, goffs, T, &d_g))) return rc;
+  if ((rc = upload(c, SLOT_ARGS_A, hf.data(), hf.size(), &d_f))) return rc;
+  if (goffs && (rc = upload(c, SLOT_ARGS_B, goffs, T, &d_g))) return rc;
   void *p_o, *p_w = nullptr, *p_q = nullptr;
-  if ((rc = scratch_reserve(c, 3, 19 * T * 8, &p_o))) return rc;
-  if (w_guess && (rc = scratch_reserve(c, 7, (size_t)total * 3 * 8, &p_w))) return rc;
-  if (q_guess && (rc = scratch_reserve(c, 8, (size_t)total * 4 * 8, &p_q))) return rc;
+  if ((rc = scratch_reserve(c, SLOT_ARGS_C, 19 * T * 8, &p_o))) return rc;
+  if (w_guess && (rc = scratch_reserve(c, SLOT_ROWS_A, (size_t)total * 3 * 8, &p_w))) return rc;
+  if (q_guess && (rc = scratch_reserve(c, SLOT_ROWS_B, (size_t)total * 4 * 8, &p_q))) return rc;
   PrepArgs a;
   a.n_trials = n; a.x0 = d_f; a.xf = d_f + 8 * T; a.Jmat = d_f + 16 * T; a.t_final = d_f + 25 * T;
   a.t0 = t0; a.dt = dt; a.alpha = alpha; a.beta = beta; a.conj_fix = eigen_axis_fix ? 1 : 0;
   a.Qd = (double*)p_o; a.Qfd = a.Qd + 8 * T; a.Rd = a.Qd + 16 * T;
   a.goffs = d_g; a.w_guess = (double*)p_w; a.q_guess = (double*)p_q;
-  KernelTimer tm(c);
+  Staging io(c, 0);
+  io.back(Qd, a.Qd, 8 * T);
+  io.back(Qfd, a.Qfd, 8 * T);
+  io.back(Rd, a.Rd, 3 * T);
+  if (w_guess) io.back(w_guess, a.w_guess, (size_t)total * 3);
+  if (q_guess) io.back(q_guess, a.q_guess, (size_t)total * 4);
+  io.start();
   k_slew_prep<<<(unsigned)((n + 127) / 128), 128, 0, c->stream>>>(a);
-  tm.stop();
   c->launches++;
-  TS_CUDA(c, cudaGetLastError());
-  TS_CUDA(c, cudaMemcpyAsync(Qd, a.Qd, 8 * T * 8, cudaMemcpyDeviceToHost, c->stream));
-  TS_CUDA(c, cudaMemcpyAsync(Qfd, a.Qfd, 8 * T * 8, cudaMemcpyDeviceToHost, c->stream));
-  TS_CUDA(c, cudaMemcpyAsync(Rd, a.Rd, 3 * T * 8, cudaMemcpyDeviceToHost, c->stream));
-  if (w_guess) TS_CUDA(c, cudaMemcpyAsync(w_guess, p_w, (size_t)total * 3 * 8, cudaMemcpyDeviceToHost, c->stream));
-  if (q_guess) TS_CUDA(c, cudaMemcpyAsync(q_guess, p_q, (size_t)total * 4 * 8, cudaMemcpyDeviceToHost, c->stream));
-  TS_CUDA(c, cudaStreamSynchronize(c->stream));
-  tm.read();
-  return TS_OK;
+  return io.finish();
 }
 
 int ts_tvlqr_sim_batch(ts_ctx* c, int64_t n, const int64_t* N_i, const int64_t* offs, const double* X_lqr, const double* U_lqr,
                        const double* x0_lqr, const double* Jmat, const double* B_eci, const int64_t* B_offs, const int64_t* B_rows,
                        const double* index_scale, const double* clock_rate, const double* t_final, const double* q_final,
                        const uint32_t* stream_id, const ts_tvlqr_opts* opts, const double* noise, double* X_sim, double* U_sim,
-                       double* dX, double* K, int64_t* N_sim, double* slew_time, int pad) {
+                       double* dX, double* K, int64_t* N_sim, double* slew_time, int pointers_are_device) {
   if (!c) return TS_ERR_ARG;
   if (n < 0 || (n > 0 && (!N_i || !offs || !X_lqr || !U_lqr || !x0_lqr || !Jmat || !B_eci || !B_offs || !B_rows || !index_scale ||
                           !clock_rate || !t_final || !q_final)))
@@ -996,22 +932,21 @@ int ts_tvlqr_sim_batch(ts_ctx* c, int64_t n, const int64_t* N_i, const int64_t* 
     rows = std::max(rows, B_offs[t] + B_rows[t]);
   }
   int rc;
-  DevBuf dX_, dU_, dB, dNz, oX, oU, odX, oK;
-  if ((rc = dev_in(c, dX_, X_lqr, (size_t)knots * 8 * 8, pad))) return rc;
-  if ((rc = dev_in(c, dU_, U_lqr, (size_t)knots * 3 * 8, pad))) return rc;
-  if ((rc = dev_in(c, dB, B_eci, (size_t)rows * 3 * 8, pad))) return rc;
-  if (o.noise_mode == 1 && (rc = dev_in(c, dNz, noise, (size_t)knots * 36 * 8, pad))) return rc;
-  if (X_sim && (rc = dev_out(c, oX, X_sim, (size_t)knots * 8 * 8, pad))) return rc;
-  if (U_sim && (rc = dev_out(c, oU, U_sim, (size_t)knots * 3 * 8, pad))) return rc;
-  if (dX && (rc = dev_out(c, odX, dX, (size_t)knots * 6 * 8, pad))) return rc;
-  double* dK = nullptr;
-  if (K) {
-    if ((rc = dev_out(c, oK, K, (size_t)knots * 18 * 8, pad))) return rc;
-    dK = (double*)oK.d;
-  } else {
+  Staging io(c, pointers_are_device);
+  K4Args a;
+  a.X_lqr = io.in(X_lqr, (size_t)knots * 8);
+  a.U_lqr = io.in(U_lqr, (size_t)knots * 3);
+  a.B_eci = io.in(B_eci, (size_t)rows * 3);
+  a.noise = io.in(o.noise_mode == 1 ? noise : nullptr, (size_t)knots * 36);
+  a.X_sim = io.out(X_sim, (size_t)knots * 8);
+  a.U_sim = io.out(U_sim, (size_t)knots * 3);
+  a.dX = io.out(dX, (size_t)knots * 6);
+  a.K = io.out(K, (size_t)knots * 18);
+  if (io.rc) return io.rc;
+  if (!K) {
     void* p;
-    if ((rc = scratch_reserve(c, 9, (size_t)knots * 18 * 8, &p))) return rc;
-    dK = (double*)p;
+    if ((rc = scratch_reserve(c, SLOT_K4_GAINS, (size_t)knots * 18 * 8, &p))) return rc;
+    a.K = (double*)p;
   }
   std::vector<int64_t> hi(4 * T);
   memcpy(&hi[0], N_i, T * 8); memcpy(&hi[T], offs, T * 8); memcpy(&hi[2 * T], B_offs, T * 8); memcpy(&hi[3 * T], B_rows, T * 8);
@@ -1019,42 +954,23 @@ int ts_tvlqr_sim_batch(ts_ctx* c, int64_t n, const int64_t* N_i, const int64_t* 
   memcpy(&hf[0], x0_lqr, 8 * T * 8); memcpy(&hf[8 * T], Jmat, 9 * T * 8); memcpy(&hf[17 * T], index_scale, T * 8);
   memcpy(&hf[18 * T], clock_rate, T * 8); memcpy(&hf[19 * T], t_final, T * 8); memcpy(&hf[20 * T], q_final, 4 * T * 8);
   int64_t* d_i; double* d_f; uint32_t* d_s = nullptr;
-  if ((rc = upload(c, 1, hi.data(), hi.size(), &d_i))) return rc;
-  if ((rc = upload(c, 2, hf.data(), hf.size(), &d_f))) return rc;
-  if (stream_id && (rc = upload(c, 3, stream_id, T, &d_s))) return rc;
+  if ((rc = upload(c, SLOT_ARGS_A, hi.data(), hi.size(), &d_i))) return rc;
+  if ((rc = upload(c, SLOT_ARGS_B, hf.data(), hf.size(), &d_f))) return rc;
+  if (stream_id && (rc = upload(c, SLOT_ARGS_C, stream_id, T, &d_s))) return rc;
   void* p_o;
-  if ((rc = scratch_reserve(c, 5, T * 16, &p_o))) return rc;
-  K4Args a;
+  if ((rc = scratch_reserve(c, SLOT_PER_TRIAL, T * 16, &p_o))) return rc;
   a.n_trials = n; a.N_i = d_i; a.offs = d_i + T; a.B_offs = d_i + 2 * T; a.B_rows = d_i + 3 * T;
-  a.X_lqr = (const double*)dX_.d; a.U_lqr = (const double*)dU_.d; a.x0_lqr = d_f; a.Jmat = d_f + 8 * T;
-  a.B_eci = (const double*)dB.d; a.index_scale = d_f + 17 * T; a.clock_rate = d_f + 18 * T; a.t_final = d_f + 19 * T;
+  a.x0_lqr = d_f; a.Jmat = d_f + 8 * T;
+  a.index_scale = d_f + 17 * T; a.clock_rate = d_f + 18 * T; a.t_final = d_f + 19 * T;
   a.q_final = d_f + 20 * T; a.stream_id = d_s;
   memcpy(&a.opts, &o, sizeof(o));
-  a.noise = (o.noise_mode == 1) ? (const double*)dNz.d : nullptr;
-  a.X_sim = X_sim ? (double*)oX.d : nullptr; a.U_sim = U_sim ? (double*)oU.d : nullptr; a.dX = dX ? (double*)odX.d : nullptr;
-  a.K = dK; a.N_sim = (int64_t*)p_o; a.slew_time = (double*)((int64_t*)p_o + T);
-  {
-    std::vector<int64_t> lin((size_t)T + 1, 0);
-    for (size_t t = 0; t < T; ++t) lin[t + 1] = lin[t] + (N_i[t] - 1);
-    int64_t* d_lin;
-    void* p_ab;
-    if ((rc = upload(c, 27, lin.data(), T + 1, &d_lin))) return rc;
-    if ((rc = scratch_reserve(c, 26, (size_t)lin[T] * 55 * 8 + 64, &p_ab))) return rc;
-    a.AB = (double*)p_ab; a.clk = a.AB + (size_t)lin[T] * 54; a.lin_offs = d_lin; a.lin_total = lin[T];
-  }
-  KernelTimer tm(c);
+  a.N_sim = (int64_t*)p_o; a.slew_time = (double*)((int64_t*)p_o + T);
+  if (N_sim) io.back(N_sim, a.N_sim, T);
+  if (slew_time) io.back(slew_time, a.slew_time, T);
+  if ((rc = k4_lin_table(c, N_i, T, a))) return rc;
+  io.start();
   k4_launch(c, a);
-  tm.stop();
-  TS_CUDA(c, cudaGetLastError());
-  if (X_sim && (rc = dev_back(c, oX, X_sim, (size_t)knots * 8 * 8))) return rc;
-  if (U_sim && (rc = dev_back(c, oU, U_sim, (size_t)knots * 3 * 8))) return rc;
-  if (dX && (rc = dev_back(c, odX, dX, (size_t)knots * 6 * 8))) return rc;
-  if (K && (rc = dev_back(c, oK, K, (size_t)knots * 18 * 8))) return rc;
-  if (N_sim) TS_CUDA(c, cudaMemcpyAsync(N_sim, a.N_sim, T * 8, cudaMemcpyDeviceToHost, c->stream));
-  if (slew_time) TS_CUDA(c, cudaMemcpyAsync(slew_time, a.slew_time, T * 8, cudaMemcpyDeviceToHost, c->stream));
-  TS_CUDA(c, cudaStreamSynchronize(c->stream));
-  tm.read();
-  return TS_OK;
+  return io.finish();
 }
 
 // ---------------------------------------------------------------------------- fused Monte-Carlo
@@ -1091,19 +1007,19 @@ int ts_monte_carlo_run(ts_ctx* c, const ts_mc_config* cfg, const double* kep6, c
   for (int64_t f = 0; f < nf; ++f) {
     fo[f] = fopts[f];
     fo[f].t0 = cfg->t0; fo[f].tf = cfg->tf; fo[f].N = cfg->N_scope;
-    if (!(fo[f].igrf_date >= 1900.0 && fo[f].igrf_date <= 2025.0)) return fail(c, TS_ERR_DATE, "orbit %lld: IGRF date outside [1900, 2025]", (long long)f);
+    if (!igrf_date_ok(fo[f].igrf_date)) return fail(c, TS_ERR_DATE, "orbit %lld: IGRF date outside [1900, 2025]", (long long)f);
     (igrf_nmax_for_date(fo[f].igrf_date) == 13 ? any13 : any10) = true;
     offs_s[f] = 2 * cfg->N_scope * f;
   }
   offs_s[nf] = 2 * cfg->N_scope * nf;
   double* d_kep; ts_field_opts_dev* d_fo; int64_t* d_offs_s;
-  if ((rc = upload(c, 1, kep6, 6 * NF, &d_kep))) return rc;
-  if ((rc = upload(c, 2, (const ts_field_opts_dev*)fo.data(), NF, &d_fo))) return rc;
-  if ((rc = upload(c, 3, offs_s.data(), NF + 1, &d_offs_s))) return rc;
+  if ((rc = upload(c, SLOT_ARGS_A, kep6, 6 * NF, &d_kep))) return rc;
+  if ((rc = upload(c, SLOT_ARGS_B, (const ts_field_opts_dev*)fo.data(), NF, &d_fo))) return rc;
+  if ((rc = upload(c, SLOT_ARGS_C, offs_s.data(), NF + 1, &d_offs_s))) return rc;
   void *p_pos, *p_Bs, *p_sm;
-  if ((rc = scratch_reserve(c, 0, (size_t)(offs_s[nf] + nf) * 3 * 8, &p_pos))) return rc;
-  if ((rc = scratch_reserve(c, 7, (size_t)offs_s[nf] * 3 * 8, &p_Bs))) return rc;
-  if ((rc = scratch_reserve(c, 10, NF * 80, &p_sm))) return rc;
+  if ((rc = scratch_reserve(c, SLOT_POSITIONS, (size_t)(offs_s[nf] + nf) * 3 * 8, &p_pos))) return rc;
+  if ((rc = scratch_reserve(c, SLOT_ROWS_A, (size_t)offs_s[nf] * 3 * 8, &p_Bs))) return rc;
+  if ((rc = scratch_reserve(c, SLOT_ORBIT_BLOCK, NF * 80, &p_sm))) return rc;
   std::vector<int64_t> rows_s(NF, 2 * cfg->N_scope);
   std::vector<double> dts(NF, (cfg->tf - cfg->t0) / (double)cfg->N_scope), cuts(NF, cfg->cutoff);
   int64_t* d_rows_s = (int64_t*)p_sm;
@@ -1125,10 +1041,7 @@ int ts_monte_carlo_run(ts_ctx* c, const ts_mc_config* cfg, const double* kep6, c
     for (int pass = 0; pass < 2; ++pass) {
       const int64_t lo = pass ? SA : 0, hi = pass ? S2 : SA;
       if (hi <= lo) break;
-      const int64_t* skip = pass ? d_idx : nullptr;
-      dim3 grid((unsigned)nf, (unsigned)((hi - lo + K2B_THREADS - 1) / K2B_THREADS));
-      if (any13) { k2b_field_rows<13><<<grid, K2B_THREADS, 0, c->stream>>>(c->d_tabG, c->d_tabH, d_fo, d_offs_s, nullptr, (double*)p_pos, (double*)p_Bs, 13, lo, skip); c->launches++; }
-      if (any10) { k2b_field_rows<10><<<grid, K2B_THREADS, 0, c->stream>>>(c->d_tabG, c->d_tabH, d_fo, d_offs_s, nullptr, (double*)p_pos, (double*)p_Bs, 10, lo, skip); c->launches++; }
+      k2b_launch(c, any13, any10, nf, hi - lo, d_fo, d_offs_s, nullptr, (double*)p_pos, (double*)p_Bs, lo, pass ? d_idx : nullptr);
       k2c_cutoff_scan<<<(unsigned)nf, K2C_THREADS, 0, c->stream>>>((double*)p_Bs, d_offs_s, d_rows_s, d_dts, d_cuts, lo, hi, d_carry, d_idx);
       c->launches++;
     }
@@ -1184,11 +1097,11 @@ int ts_monte_carlo_run(ts_ctx* c, const ts_mc_config* cfg, const double* kep6, c
   if (na > 0) {
     // ---- stage 2: fine field tables
     ts_field_opts_dev* d_fo2; int64_t *d_offs_f, *d_lim;
-    if ((rc = upload(c, 2, (const ts_field_opts_dev*)fo2.data(), NF, &d_fo2))) return rc;
-    if ((rc = upload(c, 3, offs_f.data(), NF + 1, &d_offs_f))) return rc;
-    if ((rc = upload(c, 11, lim.data(), NF, &d_lim))) return rc;
+    if ((rc = upload(c, SLOT_ARGS_B, (const ts_field_opts_dev*)fo2.data(), NF, &d_fo2))) return rc;
+    if ((rc = upload(c, SLOT_ARGS_C, offs_f.data(), NF + 1, &d_offs_f))) return rc;
+    if ((rc = upload(c, SLOT_ROW_LIMITS, lim.data(), NF, &d_lim))) return rc;
     void* p_pos2;
-    if ((rc = scratch_reserve(c, 0, std::max((size_t)(offs_s[nf] + nf) * 3 * 8, (size_t)(offs_f[nf] + nf) * 3 * 8), &p_pos2))) return rc;
+    if ((rc = scratch_reserve(c, SLOT_POSITIONS, std::max((size_t)(offs_s[nf] + nf) * 3 * 8, (size_t)(offs_f[nf] + nf) * 3 * 8), &p_pos2))) return rc;
     // per-trial layout
     std::vector<int64_t> hi(4 * NA + 1);
     std::vector<double> hf((8 + 8 + 9 + 1 + 1 + 1 + 8 + 4) * NA);
@@ -1228,13 +1141,13 @@ int ts_monte_carlo_run(ts_ctx* c, const ts_mc_config* cfg, const double* kep6, c
     }
     hi[4 * NA] = knots;
     int64_t* d_i; double* d_f;
-    if ((rc = upload(c, 12, hi.data(), hi.size(), &d_i))) return rc;
-    if ((rc = upload(c, 13, hf.data(), hf.size(), &d_f))) return rc;
+    if ((rc = upload(c, SLOT_PACKED_I64, hi.data(), hi.size(), &d_i))) return rc;
+    if ((rc = upload(c, SLOT_PACKED_F64, hf.data(), hf.size(), &d_f))) return rc;
     // device block: fine field tables, weights, X, U, outcomes, slew times
     const size_t b_B = (size_t)offs_f[nf] * 3 * 8, b_w = 19 * NA * 8, b_X = (size_t)knots * 8 * 8, b_U = (size_t)knots * 3 * 8,
                  b_o = NA * sizeof(ts_trial_outcome), b_s = NA * 16;
     void* p_blk;
-    if ((rc = scratch_reserve(c, 22, b_B + b_w + b_X + b_U + b_o + b_s + 512, &p_blk))) return rc;   // slot 22: only this path uses it (kept trajectories)
+    if ((rc = scratch_reserve(c, SLOT_KEPT_BLOCK, b_B + b_w + b_X + b_U + b_o + b_s + 512, &p_blk))) return rc;
     char* w = (char*)p_blk;
     double* d_Bf = (double*)w; w += b_B;
     double* d_Qd = (double*)w; w += b_w;
@@ -1248,9 +1161,7 @@ int ts_monte_carlo_run(ts_ctx* c, const ts_mc_config* cfg, const double* kep6, c
     {
       int64_t maxlim = 1;
       for (int64_t f = 0; f < nf; ++f) maxlim = std::max(maxlim, 2 * std::max<int64_t>(Nf[f], 1));
-      dim3 grid((unsigned)nf, (unsigned)((maxlim + K2B_THREADS - 1) / K2B_THREADS));
-      if (any13) { k2b_field_rows<13><<<grid, K2B_THREADS, 0, c->stream>>>(c->d_tabG, c->d_tabH, d_fo2, d_offs_f, d_lim, (double*)p_pos2, d_Bf, 13); c->launches++; }
-      if (any10) { k2b_field_rows<10><<<grid, K2B_THREADS, 0, c->stream>>>(c->d_tabG, c->d_tabH, d_fo2, d_offs_f, d_lim, (double*)p_pos2, d_Bf, 10); c->launches++; }
+      k2b_launch(c, any13, any10, nf, maxlim, d_fo2, d_offs_f, d_lim, (double*)p_pos2, d_Bf);
     }
     cudaEventRecord(e[2], c->stream);
     // ---- stage 3: eigen-axis guess + Bryson weights
@@ -1275,21 +1186,18 @@ int ts_monte_carlo_run(ts_ctx* c, const ts_mc_config* cfg, const double* kep6, c
     for (int64_t aa = 0; aa < na; ++aa) diff[aa] = slew_angle(x0 + 8 * act[aa], xf + 8 * act[aa]);
     // everything stage 5 needs is reserved and uploaded BEFORE the solve is queued: a cudaMalloc between the two would
     // wait for the solve and put its host latency on the device timeline
-    void *p_K = nullptr, *p_ab = nullptr, *p_xs = nullptr, *p_us = nullptr;
+    void *p_K = nullptr, *p_xs = nullptr, *p_us = nullptr;
     uint32_t* d_sid = nullptr;
-    int64_t* d_lin = nullptr;
-    std::vector<int64_t> lin(NA + 1, 0);
+    K4Args k4;
     if (cfg->run_tvlqr) {
-      if ((rc = scratch_reserve(c, 9, (size_t)knots * 18 * 8, &p_K))) return rc;
+      if ((rc = scratch_reserve(c, SLOT_K4_GAINS, (size_t)knots * 18 * 8, &p_K))) return rc;
       std::vector<uint32_t> sid(NA);
       for (int64_t a = 0; a < na; ++a) sid[a] = stream_id ? stream_id[act[a]] : (uint32_t)act[a];
-      if ((rc = upload(c, 14, sid.data(), NA, &d_sid))) return rc;
-      for (size_t a2 = 0; a2 < NA; ++a2) lin[a2 + 1] = lin[a2] + (hi[a2] - 1);
-      if ((rc = upload(c, 27, lin.data(), NA + 1, &d_lin))) return rc;
-      if ((rc = scratch_reserve(c, 26, (size_t)lin[NA] * 55 * 8 + 64, &p_ab))) return rc;
+      if ((rc = upload(c, SLOT_STREAM_IDS, sid.data(), NA, &d_sid))) return rc;
+      if ((rc = k4_lin_table(c, hi.data(), NA, k4))) return rc;
       if (cfg->keep_trajectories) {
-        if ((rc = scratch_reserve(c, 20, (size_t)knots * 8 * 8 + 64, &p_xs))) return rc;
-        if ((rc = scratch_reserve(c, 21, (size_t)knots * 3 * 8 + 64, &p_us))) return rc;
+        if ((rc = scratch_reserve(c, SLOT_KEPT_XSIM, (size_t)knots * 8 * 8 + 64, &p_xs))) return rc;
+        if ((rc = scratch_reserve(c, SLOT_KEPT_USIM, (size_t)knots * 3 * 8 + 64, &p_us))) return rc;
       }
     }
     if ((rc = k3_launch(c, ka, hi.data(), diff.data(), all_inertia_diagonal(Jmat, n)))) return rc;
@@ -1297,7 +1205,6 @@ int ts_monte_carlo_run(ts_ctx* c, const ts_mc_config* cfg, const double* kep6, c
     // ---- stage 5: TVLQR replay + slew-time rule
     double *d_Xs_keep = nullptr, *d_Us_keep = nullptr;
     if (cfg->run_tvlqr) {
-      K4Args k4;
       k4.n_trials = na; k4.N_i = d_i; k4.offs = d_i + NA; k4.B_offs = d_i + 2 * NA; k4.B_rows = d_i + 3 * NA;
       k4.X_lqr = d_X; k4.U_lqr = d_U; k4.x0_lqr = d_f + 28 * NA; k4.Jmat = d_f + 16 * NA; k4.B_eci = d_Bf;
       k4.index_scale = d_f + 26 * NA; k4.clock_rate = d_f + 27 * NA; k4.t_final = d_f + 25 * NA; k4.q_final = d_f + 36 * NA;
@@ -1314,7 +1221,6 @@ int ts_monte_carlo_run(ts_ctx* c, const ts_mc_config* cfg, const double* kep6, c
         d_Xs_keep = k4.X_sim; d_Us_keep = k4.U_sim;
       }
       k4.N_sim = d_nsim; k4.slew_time = d_slew;
-      k4.AB = (double*)p_ab; k4.clk = k4.AB + (size_t)lin[NA] * 54; k4.lin_offs = d_lin; k4.lin_total = lin[NA];
       k4_launch(c, k4);
     }
     cudaEventRecord(e[5], c->stream);
@@ -1411,12 +1317,14 @@ int ts_kep_eci_batch(ts_ctx* c, int64_t n, const double* kep6, const double* t0,
   if (n < 0 || (n > 0 && (!kep6 || !rv6))) return fail(c, TS_ERR_ARG, "ts_kep_eci_batch: null argument");
   if (n == 0) return TS_OK;
   TS_CUDA(c, cudaSetDevice(c->device));
-  HostIO io(c);
+  Staging io(c, 0);
   const double* dk = io.in(kep6, (size_t)n * 6);
   const double* dt0 = io.in(t0, (size_t)n);
   double* dr = io.out(rv6, (size_t)n * 6);
   if (io.rc) return io.rc;
+  io.start();
   k5_kep_eci<<<(unsigned)((n + 127) / 128), 128, 0, c->stream>>>(n, dk, dt0, GM, dr);
+  c->launches++;
   return io.finish();
 }
 
@@ -1425,11 +1333,13 @@ int ts_orbit_rhs_batch(ts_ctx* c, int64_t n, const double* x6, double* dx6) {
   if (n < 0 || (n > 0 && (!x6 || !dx6))) return fail(c, TS_ERR_ARG, "ts_orbit_rhs_batch: null argument");
   if (n == 0) return TS_OK;
   TS_CUDA(c, cudaSetDevice(c->device));
-  HostIO io(c);
+  Staging io(c, 0);
   const double* dx = io.in(x6, (size_t)n * 6);
   double* dd = io.out(dx6, (size_t)n * 6);
   if (io.rc) return io.rc;
+  io.start();
   k5_orbit_rhs<<<(unsigned)((n + 127) / 128), 128, 0, c->stream>>>(n, dx, dd);
+  c->launches++;
   return io.finish();
 }
 
@@ -1439,13 +1349,15 @@ int ts_legendre_schmidt_batch(ts_ctx* c, int64_t n, const double* theta, int n_m
   if (n_max < 1 || n_max > 13) return fail(c, TS_ERR_ARG, "n_max must be in [1, 13]");
   if (n == 0) return TS_OK;
   TS_CUDA(c, cudaSetDevice(c->device));
-  HostIO io(c);
+  Staging io(c, 0);
   const size_t d2 = (size_t)(n_max + 1) * (n_max + 1);
   const double* dth = io.in(theta, (size_t)n);
   double* dPd = io.out(P, (size_t)n * d2);
   double* ddP = io.out(dP, (size_t)n * d2);
   if (io.rc) return io.rc;
+  io.start();
   k5_legendre<<<(unsigned)((n + 63) / 64), 64, 0, c->stream>>>(n, dth, n_max, dPd, ddP);
+  c->launches++;
   return io.finish();
 }
 
@@ -1456,7 +1368,7 @@ int ts_dynamics_batch(ts_ctx* c, int mode, int64_t n, const double* x, const dou
   if (mode != 2 && B_rows < 1) return fail(c, TS_ERR_ARG, "ts_dynamics_batch: empty field table");
   if (n == 0) return TS_OK;
   TS_CUDA(c, cudaSetDevice(c->device));
-  HostIO io(c);
+  Staging io(c, 0);
   const int nx = (mode == 2) ? 7 : 8;
   const double* dxs = io.in(x, (size_t)n * nx);
   const double* du = io.in(u, (size_t)n * 3);
@@ -1464,7 +1376,9 @@ int ts_dynamics_batch(ts_ctx* c, int mode, int64_t n, const double* x, const dou
   const double* dJ = io.in(Jmat, 9);
   double* dd = io.out(dx, (size_t)n * nx);
   if (io.rc) return io.rc;
+  io.start();
   k5_dynamics<<<(unsigned)((n + 127) / 128), 128, 0, c->stream>>>(mode, n, dxs, du, dB, B_rows, index_scale, clock_rate, dJ, dd);
+  c->launches++;
   return io.finish();
 }
 
@@ -1474,14 +1388,16 @@ int ts_rk3_step_batch(ts_ctx* c, int64_t n, const double* x, const double* u, co
   if (n < 0 || B_rows < 1 || (n > 0 && (!x || !u || !B || !Jmat || !xn))) return fail(c, TS_ERR_ARG, "ts_rk3_step_batch: bad argument");
   if (n == 0) return TS_OK;
   TS_CUDA(c, cudaSetDevice(c->device));
-  HostIO io(c);
+  Staging io(c, 0);
   const double* dxs = io.in(x, (size_t)n * 8);
   const double* du = io.in(u, (size_t)n * 3);
   const double* dB = io.in(B, (size_t)B_rows * 3);
   const double* dJ = io.in(Jmat, 9);
   double* dd = io.out(xn, (size_t)n * 8);
   if (io.rc) return io.rc;
+  io.start();
   k5_rk3_step<<<(unsigned)((n + 127) / 128), 128, 0, c->stream>>>(n, dxs, du, dB, B_rows, index_scale, clock_rate, dJ, dt, dd);
+  c->launches++;
   return io.finish();
 }
 
@@ -1500,7 +1416,7 @@ int ts_psiaki_pd_batch(ts_ctx* c, int64_t n_trials, const int64_t* N_i, const in
     knots = std::max(knots, offs[t] + N_i[t]);
   }
   TS_CUDA(c, cudaSetDevice(c->device));
-  HostIO io(c);
+  Staging io(c, 0);
   K7Args a;
   a.n_trials = n_trials;
   a.N_i = io.in(N_i, (size_t)n_trials);
@@ -1515,7 +1431,9 @@ int ts_psiaki_pd_batch(ts_ctx* c, int64_t n_trials, const int64_t* N_i, const in
   a.M = io.out(M, (size_t)knots * 3);
   a.Qe = io.out(q_err, (size_t)knots * 4);
   if (io.rc) return io.rc;
+  io.start();
   k7_psiaki_pd_kernel<<<(unsigned)((n_trials + 63) / 64), 64, 0, c->stream>>>(a);
+  c->launches++;
   return io.finish();
 }
 
@@ -1525,7 +1443,7 @@ int ts_attitude_dynamics_linear_batch(ts_ctx* c, int64_t n, const double* x, con
   if (n < 0 || (n > 0 && (!x || !u || !x_linear || !B_B || !Jmat || !dx))) return fail(c, TS_ERR_ARG, "ts_attitude_dynamics_linear_batch: null argument");
   if (n == 0) return TS_OK;
   TS_CUDA(c, cudaSetDevice(c->device));
-  HostIO io(c);
+  Staging io(c, 0);
   const double* dxs = io.in(x, (size_t)n * 7);
   const double* du = io.in(u, (size_t)n * 3);
   const double* dl = io.in(x_linear, (size_t)n * 7);
@@ -1533,7 +1451,9 @@ int ts_attitude_dynamics_linear_batch(ts_ctx* c, int64_t n, const double* x, con
   const double* dJ = io.in(Jmat, 9);
   double* dd = io.out(dx, (size_t)n * 7);
   if (io.rc) return io.rc;
+  io.start();
   k7_attitude_dynamics_linear<<<(unsigned)((n + 127) / 128), 128, 0, c->stream>>>(n, dxs, du, dl, dB, dJ, dd);
+  c->launches++;
   return io.finish();
 }
 
