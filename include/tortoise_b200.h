@@ -220,6 +220,49 @@ int ts_alilqr_solve_batch(ts_ctx* ctx, int64_t n_trials, const int64_t* N_i, con
                           const double* clock_rate, double dt, const double* U0, const ts_ilqr_opts* opts, double* X,
                           double* U, double* K, ts_trial_outcome* out, int pointers_are_device);
 
+/* ---- K3 continuation: export the solver state and continue max-outer trials from it ----------------------- *
+ * The state of one finished trial (104 bytes).  The per-knot bound multipliers go alongside it in a ragged `lam`
+ * array of (sum N) x 6 doubles at offs[t]*6 (the layout of U; the last row of each trial is unused and zero).  Rules
+ * (DESIGN.md section 4, K3):
+ *  CS1 export: the state is what the solver holds after its final outer update.  At a TS_ST_MAX_OUTER end the dual,
+ *      goal-multiplier and penalty updates have been applied, so mu, lam_goal and lam are the values the next outer
+ *      iteration would use.
+ *  CS2 a trial continues when status == TS_ST_MAX_OUTER and outer_iters < opts->max_outer of the continuing call.
+ *      Every other trial passes through: its X, U and K rows are not written, its outcome is rebuilt from the state
+ *      (N from N_i, the rest of the record zero), its state and lam rows are copied to the outputs.
+ *  CS3 a continuing trial resumes with the next outer iteration: outer_iters + 1, a fresh inner solve, J_prev = the
+ *      cost of (X, U) under the imported multipliers (A7: the carried J), previous c_max = c_max.  The trajectory is
+ *      imported from X (columns 0-6; the clock column is recomputed) and U, not rolled out again.  Counters and costs
+ *      accumulate: a continued outcome reports totals over both calls.
+ *  CS4 "solve to M1, then continue to M2" equals "solve to M2" exactly when cost_tol_intermediate == cost_tol and
+ *      grad_tol_intermediate == grad_tol, or a4_no_intermediate = 1.  Otherwise outer iteration M1 ran with the final
+ *      tolerances in the first call and would have run with the intermediate ones in a direct solve to M2: a slightly
+ *      different, documented schedule (the defaults differ in cost_tol).
+ * The continuing call's opts apply to the continuation (raise max_outer, change penalty_max, ...).  The call does not
+ * check that X, U and lam come from the same solve as the state: that is the caller's contract.               */
+typedef struct ts_al_state {
+  double mu;           /* penalty after the last outer (dual + penalty) update                     */
+  double lam_goal[8];  /* goal-constraint multipliers after that update                            */
+  double J;            /* = ts_trial_outcome.J: cost at the last inner iteration (the A7 carry)    */
+  double c_max;        /* = ts_trial_outcome.c_max: violation at the last outer update              */
+  int32_t status, outer_iters, inner_iters, ls_rollouts;   /* as in ts_trial_outcome               */
+} ts_al_state;
+
+/* ts_alilqr_solve_batch with the state in and out.  state_in == NULL: a fresh solve, bit-identical to
+ * ts_alilqr_solve_batch (which is this call with four NULLs).  state_in set: X and U are inputs for the continuing
+ * trials (CS2) and outputs for all trials, and lam_in (required) holds the bound multipliers.  state_out (nullable)
+ * receives every trial's state and lam_out (nullable) its multipliers.  lam_in, lam_out, X, U and K follow
+ * pointers_are_device; state_in and state_out are HOST arrays of n_trials, like out.  A status outside 0-5 or
+ * outer_iters < 1 in state_in, or state_in without lam_in, is TS_ERR_ARG and nothing is written.  The continuing
+ * trials run on the one-warp-per-trial straggler kernels; TS_ERR_NOMEM (nothing written) if their parked records do not
+ * fit in device memory.  ts_k3_last_split reports 0 ms for the persistent kernel and every continuing trial as handed over.   */
+int ts_alilqr_solve_state_batch(ts_ctx* ctx, int64_t n_trials, const int64_t* N_i, const int64_t* offs, const double* x0,
+                                const double* xf, const double* Jmat, const double* Qd, const double* Qfd, const double* Rd,
+                                const double* B_eci, const int64_t* B_offs, const int64_t* B_rows, const double* index_scale,
+                                const double* clock_rate, double dt, const double* U0, const ts_ilqr_opts* opts, double* X,
+                                double* U, double* K, ts_trial_outcome* out, int pointers_are_device,
+                                const ts_al_state* state_in, const double* lam_in, ts_al_state* state_out, double* lam_out);
+
 /* ---- slew preparation: eigen-axis guess + Bryson weights ---------------------- *
  * eigen_axis_slew(x0,xf,t) [src/eigen_axis_slew.jl:1-38] over t = t0:dt:t_final[t], followed by
  * Bryson's rule [src/TortoiseSat.jl:157-168; alpha = 10 there, 0.1 in src/monte_carlo.jl:169;

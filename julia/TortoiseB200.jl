@@ -53,6 +53,10 @@ struct TrialOutcome         # ts_trial_outcome (64 bytes)
     status::Int32; outer_iters::Int32; inner_iters::Int32; ls_rollouts::Int32; N::Int64
     J::Float64; c_max::Float64; t_final::Float64; slew_time::Float64; flops::Float64
 end
+struct AlState              # ts_al_state (104 bytes): exported AL-iLQR solver state of one trial (CS1-CS4, DESIGN.md section 4)
+    mu::Float64; lam_goal::NTuple{8,Float64}; J::Float64; c_max::Float64
+    status::Int32; outer_iters::Int32; inner_iters::Int32; ls_rollouts::Int32
+end
 struct TvlqrOpts            # ts_tvlqr_opts
     dt::Float64; t0::Float64; tf::Float64
     Qd::NTuple{6,Float64}; Qfd::NTuple{6,Float64}; Rd::NTuple{3,Float64}
@@ -268,6 +272,29 @@ function solve_slew(x0, xf, J, Q, R, Qf, B_ECI, N::Integer, dt; N_field = N, tf_
     check(e, rc)
     X, U[:, 1:N-1], permutedims(K, (2, 1, 3))[:, :, 1:N-1], out[1]
 end
+# solve_slew that also returns the solver state and the bound multipliers (6 x N, last column zero), and continues from
+# them: pass `state`, `lam` and the X, U of an earlier call to run a slew that ended at max_outer on to opts.max_outer
+# (CS2, CS3).  A slew that does not continue passes through unchanged (its K is then zero).
+function solve_slew(x0, xf, J, Q, R, Qf, B_ECI, N::Integer, dt, state::Union{Nothing,AlState}; N_field = N, tf_scope = 5400.0,
+                    t0 = 0.0, U0 = nothing, opts::IlqrOpts = default_ilqr_opts(), lam = nothing, X_in = nothing, U_in = nothing,
+                    e::Engine = engine())
+    Bt = Matrix{Float64}(B_ECI'); X = zeros(8, N); U = zeros(3, N); K = zeros(8, 3, N)
+    if state !== nothing
+        X .= X_in; U[:, 1:N-1] .= U_in
+    end
+    out = Vector{TrialOutcome}(undef, 1); st_out = Vector{AlState}(undef, 1); lam_out = zeros(6, N)
+    rc = ccall((:ts_alilqr_solve_state_batch, LIB), Cint,
+               (Ptr{Cvoid}, Int64, Ptr{Int64}, Ptr{Int64}, Ptr{Float64}, Ptr{Float64}, Ptr{Float64}, Ptr{Float64}, Ptr{Float64},
+                Ptr{Float64}, Ptr{Float64}, Ptr{Int64}, Ptr{Int64}, Ptr{Float64}, Ptr{Float64}, Cdouble, Ptr{Float64},
+                Ref{IlqrOpts}, Ptr{Float64}, Ptr{Float64}, Ptr{Float64}, Ptr{TrialOutcome}, Cint,
+                Ptr{AlState}, Ptr{Float64}, Ptr{AlState}, Ptr{Float64}),
+               e.h, 1, Int64[N], Int64[0], collect(Float64, x0), collect(Float64, xf), vec(Matrix{Float64}(J')), diag(Q), diag(Qf),
+               diag(R), Bt, Int64[0], Int64[size(Bt, 2)], Float64[N_field], Float64[1 / (tf_scope - t0)], dt,
+               U0 === nothing ? C_NULL : U0, Ref(opts), X, U, K, out, 0,
+               state === nothing ? C_NULL : AlState[state], state === nothing ? C_NULL : Matrix{Float64}(lam), st_out, lam_out)
+    check(e, rc)
+    X, U[:, 1:N-1], permutedims(K, (2, 1, 3))[:, :, 1:N-1], out[1], st_out[1], lam_out
+end
 
 # ----------------------------------------------------------------------------- K4: TVLQR replay
 # attitude_simulation(f!,f_gains!,integration,X_lqr,U_lqr,dt_lqr,x0_lqr,t0,tf,Q_lqr,R_lqr,Qf_lqr) -> (X_sim,U_sim,dX,K)
@@ -437,6 +464,6 @@ hat(x) = [0 -x[3] x[2]; x[3] 0 -x[1]; -x[2] x[1] 0]                             
 export Engine, params, input_parameters, igrf12, igrf12_batch, igrf_data, magnetic_simulation, magnetic_gramian, kep_ECI, OrbitPlotter,
        legendre, dlegendre, DerivFunction, gain_simulator, attitude_dynamics,
        condition_based_time, eigen_axis_slew, bryson_weights, solve_slew, attitude_simulation, monte_carlo, qmult, qrot, q_inv, hat,
-       igrf12syn, attitude_dynamics_linear, psiaki_pd_simulation, igrf_interpolant, field_map_prefilter, field_map_eval
+       igrf12syn, attitude_dynamics_linear, psiaki_pd_simulation, igrf_interpolant, field_map_prefilter, field_map_eval, AlState
 
 end # module

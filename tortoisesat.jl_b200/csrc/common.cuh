@@ -33,6 +33,7 @@ enum Slot : int {
   SLOT_LIN_RECORDS,                        // K4 linearisation records
   SLOT_TABLE,                              // a call's lookup table: K4 linearisation offsets, K8 padded coefficients
   SLOT_K3_COUNTERS,                        // K3 queue and park counters (read by ts_k3_last_split / ts_k3_last_parked)
+  SLOT_AL_STATES,                          // K3 continuation: a call's imported and exported solver states
   SLOT_COUNT
 };
 }  // namespace ts
@@ -145,6 +146,13 @@ struct Staging {
   template <class T> T* out(T* p, size_t count) {
     if (!p || pointers_are_device || count == 0) return p;
     T* d = (T*)alloc(count * sizeof(T));
+    back(p, d, count);
+    return d;
+  }
+  // an array the call reads and writes in place: staged in, and copied back at finish()
+  template <class T> T* inout(T* p, size_t count) {
+    if (!p || pointers_are_device || count == 0) return p;
+    T* d = const_cast<T*>(in((const T*)p, count));
     back(p, d, count);
     return d;
   }

@@ -55,6 +55,11 @@ struct ts_trial_outcome_dev {
   int64_t N;
   double J, c_max, t_final, slew_time, flops;
 };
+// 104-byte solver state of a finished trial (C ABI: ts_al_state; rules CS1-CS4 in DESIGN.md section 4, K3)
+struct ts_al_state_dev {
+  double mu, lam_goal[8], J, c_max;
+  int32_t status, outer_iters, inner_iters, ls_rollouts;
+};
 
 namespace ts {
 
@@ -899,14 +904,13 @@ struct TrialState {
   int it, outer, dJ_zero, inner_total, ls_total, status, cur, phase, b0, pad_;
 };
 
-// setup: clock trajectory + stage field vectors (sequential, exact replica), multipliers, initial rollout, J_prev
+// the trial's tables: clock trajectory + stage field vectors of every knot (sequential, exact replica); returns max |clock|
+// in every lane.  Shared by a fresh start (solve_init) and a continuation (park_import_kernel, CS3).
 template <class Team>
-TS_FN void solve_init(Team& tm, const TrialIn& in, const ts_ilqr_opts_dev& o, const TrialWork& w, TrialState& st) {
-  const int lane = tm.lane();
+TS_FN double solve_tables(Team& tm, const TrialIn& in, const TrialWork& w) {
   const int N = in.N;
-  const double sc = o.stage_cost_dt ? in.dt : 1.0;
   double clk_absmax = 0.0;
-  if (lane == 0) {
+  if (tm.lane() == 0) {
     double x8 = in.clk0;
     for (int k = 0; k < N - 1; ++k) {
       const ClockStep cs = clock_rk3(x8, in.clock_rate, in.dt);
@@ -923,7 +927,16 @@ TS_FN void solve_init(Team& tm, const TrialIn& in, const ts_ilqr_opts_dev& o, co
     gptr(w.clk)[N - 1] = x8;
     clk_absmax = fmax(clk_absmax, fabs(x8));
   }
-  clk_absmax = tm.bcast(clk_absmax, 0);
+  return tm.bcast(clk_absmax, 0);
+}
+
+// setup: tables, multipliers, initial rollout, J_prev
+template <class Team>
+TS_FN void solve_init(Team& tm, const TrialIn& in, const ts_ilqr_opts_dev& o, const TrialWork& w, TrialState& st) {
+  const int lane = tm.lane();
+  const int N = in.N;
+  const double sc = o.stage_cost_dt ? in.dt : 1.0;
+  const double clk_absmax = solve_tables(tm, in, w);
   for (int i = lane; i < (N - 1) * 6; i += Team::W) gptr(w.lam)[i] = 0.0;
   tm.sync();
   if (lane == 0) {
@@ -968,6 +981,23 @@ TS_FN void solve_init(Team& tm, const TrialIn& in, const ts_ilqr_opts_dev& o, co
   st.J = st.J_prev;
   st.J_true = st.J_prev;
   st.phase = (o.max_outer < 1) ? PH_DONE : PH_BACKWARD;
+}
+
+// start of the next outer iteration on the trajectory xu_c, after an outer update (mu, lam_g and the bound multipliers
+// already updated).  Also the resume step of a continued solve (CS3, park_import_kernel).
+template <class Team>
+TS_FN void solve_next_outer(Team& tm, const TrialIn& in, const ts_ilqr_opts_dev& o, const TrialWork& w, TrialState& st,
+                            const double* xu_c, double sc) {
+  ++st.outer;
+  st.it = 0;
+  st.dJ_zero = 0;
+  st.rho = 0.0;
+  st.drho = 0.0;
+  double cm;
+  // J_true: the current trajectory's cost under the NEW multipliers; J_prev: the line-search reference of the next
+  // iteration -- the same number in the default reading, the carried-over cost under A7
+  st.J_true = trajectory_cost(tm, in, o, w, xu_c, sc, st.mu, st.lam_g, cm);
+  st.J_prev = o.a7_carry_cost ? st.J : st.J_true;
 }
 
 // inner-iteration bookkeeping once a forward pass has produced (Jn, grad): convergence tests, outer AL update
@@ -1031,16 +1061,7 @@ TS_FN void solve_after_forward(Team& tm, const TrialIn& in, const ts_ilqr_opts_d
   } else if (st.outer >= o.max_outer) {
     st.phase = PH_DONE;
   } else {
-    ++st.outer;
-    st.it = 0;
-    st.dJ_zero = 0;
-    st.rho = 0.0;
-    st.drho = 0.0;
-    double cm;
-    // J_true: the current trajectory's cost under the NEW multipliers; J_prev: the line-search reference of the next
-    // iteration -- the same number in the default reading, the carried-over cost under A7
-    st.J_true = trajectory_cost(tm, in, o, w, xu_c, sc, st.mu, st.lam_g, cm);
-    st.J_prev = o.a7_carry_cost ? st.J : st.J_true;
+    solve_next_outer(tm, in, o, w, st, xu_c, sc);
   }
 }
 
@@ -1136,6 +1157,43 @@ TS_HD void solve_finish(const TrialIn& in, const TrialState& st, ts_trial_outcom
   out.t_final = 0.0;    // filled by the fused Monte-Carlo path; the low-level solve has no field pass / replay
   out.slew_time = 0.0;
   out.flops = 0.0;
+}
+// CS1: the exported state of a finished trial is what the solver holds after its final outer update (at a MAX_OUTER end
+// solve_after_forward has applied the dual, goal-multiplier and penalty updates before it stops)
+TS_HD void solve_export(const TrialState& st, ts_al_state_dev& s) {
+  s.mu = st.mu;
+  for (int i = 0; i < 8; ++i) s.lam_goal[i] = st.lam_g[i];
+  s.J = st.J;
+  s.c_max = st.c_max;
+  s.status = st.status;
+  s.outer_iters = st.outer;
+  s.inner_iters = st.inner_total;
+  s.ls_rollouts = st.ls_total;
+}
+// CS3: resume a trial exported at a MAX_OUTER end.  Expects the trajectory in buffer 0 of w and the bound multipliers in
+// w.lam; rebuilds the tables as solve_init does and then runs the start of the next outer iteration exactly as
+// solve_after_forward does.  Counters and costs carry on from the exported values.
+template <class Team>
+TS_FN void solve_import(Team& tm, const TrialIn& in, const ts_ilqr_opts_dev& o, const TrialWork& w, const ts_al_state_dev& s,
+                        TrialState& st) {
+  st.clk_absmax = solve_tables(tm, in, w);
+  tm.sync();
+  st.mu = s.mu;
+  for (int i = 0; i < 8; ++i) st.lam_g[i] = s.lam_goal[i];
+  st.J = s.J;
+  st.c_max = s.c_max;
+  st.c_max_prev = s.c_max;
+  st.status = ST_MAX_OUTER;
+  st.outer = s.outer_iters;
+  st.inner_total = s.inner_iters;
+  st.ls_total = s.ls_rollouts;
+  st.cur = 0;
+  st.b0 = 0;
+  st.pad_ = 0;
+  st.dV1 = st.dV2 = 0.0;
+  st.cyc_bwd = st.cyc_fwd = st.cyc_lin = 0;
+  st.phase = PH_BACKWARD;
+  solve_next_outer(tm, in, o, w, st, xu_buf<Team::W>(w, 0), o.stage_cost_dt ? in.dt : 1.0);
 }
 // per-trial SM-cycle diagnostics (ts_k3_last_cycles): backward pass, forward pass, linearisation share of the backward pass
 TS_HD void solve_diag(const TrialState& st, double* diag3) {

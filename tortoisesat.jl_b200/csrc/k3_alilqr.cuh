@@ -111,6 +111,16 @@ struct GpuWideTeam {
   }
 };
 
+// Solver state in and out (ts_alilqr_solve_state_batch; CS1-CS3 in DESIGN.md section 4, K3).  Kept behind one pointer
+// of K3Args: the four-per-warp kernel sits at the register limit, and its allocation is sensitive to the parameter block.
+struct K3StateIO {
+  ts_al_state_dev* state_out;       // nullable; n_trials records
+  double* lam_out;                  // with state_out; ragged N x 6 at offs*6 (last row of a trial zero)
+  const ts_al_state_dev* state_in;  // continuation: n_trials records
+  const double* lam_in;             // continuation: ragged like lam_out
+  int64_t n_import;                 // continuation: trials park_import_kernel parks (places 0..n_import-1)
+  int64_t lam_doubles;              // continuation: length of lam_in / lam_out (host side only)
+};
 struct K3Args {
   int64_t n_trials;
   const int64_t* order;  // trial permutation (sorted by horizon), n_trials entries
@@ -168,6 +178,7 @@ struct K3Args {
   unsigned long long* park_used;  // doubles handed out
   unsigned long long* queue2; // work queue of the second launch
   int* park_order;            // [park_cap] parking places, longest remaining work first
+  const struct K3StateIO* sio;   // nullable: solver state in and out (ts_alilqr_solve_state_batch), in device memory
 };
 
 
@@ -205,11 +216,39 @@ __device__ __forceinline__ const TrialIn& k3_load_trial(const Team& tm, const K3
   return *inp;
 }
 
+// The four-per-warp kernels that export the solver state are instantiations of their own (Team::EXPORT): that kernel sits
+// at the register limit, and the export code changes its allocation in the per-knot loops, so the solves that export
+// nothing run kernels without it.  The general-inertia exporting instantiation also declares NO_LEND: without tail
+// sharing (which does not change results, tests/test_gpu_ilqr.py) its per-knot loops stay free of local memory; with it,
+// one reload landed in the rollout loop.
+template <class Team, class = void>
+struct team_export {
+  static constexpr bool value = false;
+};
+template <class Team>
+struct team_export<Team, decltype((void)Team::EXPORT)> {
+  static constexpr bool value = Team::EXPORT;
+};
+template <class Team, class = void>
+struct team_no_lend {
+  static constexpr bool value = false;
+};
+template <class Team>
+struct team_no_lend<Team, decltype((void)Team::NO_LEND)> {
+  static constexpr bool value = Team::NO_LEND;
+};
+
 // Writes a finished trial's results in the reference's shapes: X (N x 8 incl. clock), U, K (3 x 8 per knot).
 template <class Team>
 __device__ __forceinline__ void k3_store_results(const Team& tm, const K3Args& a, int64_t t, const TrialWork& w, int N, int cur,
                                                  const ts_trial_outcome_dev& oc, const TrialState& st) {
   if (tm.ln == 0 && a.diag) solve_diag(st, a.diag + t * 3);
+  if ((Team::W == 32 || team_export<Team>::value) && a.sio) {   // CS1 export
+    if (tm.ln == 0) solve_export(st, a.sio->state_out[t]);
+    double* Lo = a.sio->lam_out + a.offs[t] * 6;
+    for (int k = tm.ln; k < N; k += Team::W)
+      for (int i = 0; i < 6; ++i) Lo[(int64_t)k * 6 + i] = (k < N - 1) ? w.lam[(int64_t)k * 6 + i] : 0.0;
+  }
   const double* xu = xu_buf<Team::W>(w, cur);
   double* Xo = a.X + a.offs[t] * 8;
   double* Uo = a.U + a.offs[t] * 3;
@@ -288,6 +327,40 @@ __global__ void __launch_bounds__(K3_WARPS_PER_BLOCK * 32, 1) k3_alilqr_quat_dia
 #include "k3_alilqr_body.inc"
 }
 #undef K3_BODY_TEAM
+// the instantiations that export the solver state (K3StateIO)
+struct GpuTeamX : GpuTeam {
+  static constexpr bool EXPORT = true;
+  static constexpr bool NO_LEND = true;
+};
+#define K3_BODY_TEAM GpuTeamX
+__global__ void __launch_bounds__(K3_WARPS_PER_BLOCK * 32, 1) k3_alilqr_export_kernel(const K3Args a) {
+#include "k3_alilqr_body.inc"
+}
+#undef K3_BODY_TEAM
+struct GpuTeamDiagX : GpuTeamDiag {
+  static constexpr bool EXPORT = true;
+};
+struct GpuTeamQuatX : GpuTeamQuat {
+  static constexpr bool EXPORT = true;
+};
+struct GpuTeamQuatDiagX : GpuTeamQuatDiag {
+  static constexpr bool EXPORT = true;
+};
+#define K3_BODY_TEAM GpuTeamDiagX
+__global__ void __launch_bounds__(K3_WARPS_PER_BLOCK * 32, 1) k3_alilqr_diag_export_kernel(const K3Args a) {
+#include "k3_alilqr_body.inc"
+}
+#undef K3_BODY_TEAM
+#define K3_BODY_TEAM GpuTeamQuatX
+__global__ void __launch_bounds__(K3_WARPS_PER_BLOCK * 32, 1) k3_alilqr_quat_export_kernel(const K3Args a) {
+#include "k3_alilqr_body.inc"
+}
+#undef K3_BODY_TEAM
+#define K3_BODY_TEAM GpuTeamQuatDiagX
+__global__ void __launch_bounds__(K3_WARPS_PER_BLOCK * 32, 1) k3_alilqr_quat_diag_export_kernel(const K3Args a) {
+#include "k3_alilqr_body.inc"
+}
+#undef K3_BODY_TEAM
 // ---------------------------------------------------------------------------------------------
 // Second launch: every parked straggler is finished by ONE WHOLE WARP (32-lane team): 32 knots linearised per
 // chunk, all 21 line-search candidates in one batch, one warp per SM sub-partition when few trials are left.
@@ -327,6 +400,50 @@ __global__ void __launch_bounds__(1024, 1) k3_park_order_kernel(const K3Args a) 
   }
   __syncthreads();
   for (unsigned i = tid; i < n; i += 1024) a.park_order[atomicAdd(&start[bin_of(i)], 1)] = (int)i;
+}
+
+// ---------------------------------------------------------------------------------------------
+// Continuation (ts_alilqr_solve_state_batch with a state): one 8-lane team per continuing trial builds that trial's
+// parked form -- TrialState + the 27 N-double record k3_wide_kernel / k3_pair_kernel resume from -- in the park
+// buffers: the trial's tables (as solve_init builds them), the imported trajectory and multipliers, and the start of
+// its next outer iteration (CS3, solve_import).  Place i holds trial park_trial[i] at park_off[i] (set by the host).
+// Continuing trials are stragglers by construction: they go straight to the one-warp-per-trial launch.
+__global__ void __launch_bounds__(32, 1) park_import_kernel(const K3Args a) {
+  extern __shared__ __align__(16) double k3_smem[];
+  const int lane32 = threadIdx.x & 31;
+  const int team = lane32 >> 3;
+  const int64_t i = (int64_t)blockIdx.x * 4 + team;
+  if (i >= a.sio->n_import) return;   // team-uniform: the teams of a warp never synchronise with each other here
+  GpuTeam tm;
+  tm.ln = lane32 & 7;
+  tm.shift = team * 8;
+  tm.mask = 0xffu << tm.shift;
+  tm.sm = k3_smem + team * TEAM_SMEM_DOUBLES;
+  const int64_t t = a.park_trial[i];
+  const TrialIn& in = k3_load_trial(tm, a, t);
+  const int N = in.N;
+  const long long Ne = N + (N & 1);
+  double* pd = a.park_data + a.park_off[i];
+  TrialWork w;
+  w.Nmax = Ne;
+  w.xu = w.xu_warp = pd;
+  w.slot_stride = 0;
+  w.kd = nullptr;
+  w.lam = pd + 10 * Ne;
+  w.bk = pd + 16 * Ne;
+  w.clk = pd + 26 * Ne;
+  const double* X = a.X + a.offs[t] * 8;
+  const double* U = a.U + a.offs[t] * 3;
+  const double* L = a.sio->lam_in + a.offs[t] * 6;
+  for (int k = tm.ln; k < N; k += TEAM) {
+    const bool stage = k < N - 1;
+    for (int j = 0; j < 7; ++j) pd[(long long)k * 10 + j] = X[(long long)k * 8 + j];
+    for (int j = 0; j < 3; ++j) pd[(long long)k * 10 + 7 + j] = stage ? U[(long long)k * 3 + j] : 0.0;
+    for (int j = 0; j < 6; ++j) w.lam[(long long)k * 6 + j] = stage ? L[(long long)k * 6 + j] : 0.0;
+  }
+  TrialState st;
+  solve_import(tm, in, a.opts, w, a.sio->state_in[t], st);
+  if (tm.ln == 0) a.park_state[i] = st;
 }
 
 struct GpuWideQuatTeam : GpuWideTeam {

@@ -24,7 +24,7 @@ using namespace ts;
 
 extern "C" {
 
-int ts_version(void) { return 101; }
+int ts_version(void) { return 102; }
 
 int ts_create(ts_ctx** out, int device_id) {
   if (!out) return TS_ERR_ARG;
@@ -557,7 +557,10 @@ static bool all_inertia_diagonal(const double* Jmat, int64_t n) {
   return true;
 }
 
-static int k3_launch(ts_ctx* c, K3Args& a, const int64_t* N_i_host, const double* difficulty_host = nullptr, bool diag_inertia = false) {
+// cont (continuation, ts_alilqr_solve_state_batch with a state): the trials to continue.  They skip the first launch:
+// park_import_kernel parks them, and the one-warp-per-trial launch finishes them.
+static int k3_launch(ts_ctx* c, K3Args& a, const int64_t* N_i_host, const double* difficulty_host = nullptr, bool diag_inertia = false,
+                     const std::vector<int64_t>* cont = nullptr, K3StateIO* sio = nullptr) {
   const int64_t n_trials = a.n_trials;
   // the quaternion-aware variant (opts.quat_error) runs the same two-launch scheme on the QUAT instantiations
   const bool quat = a.opts.quat_error != 0;
@@ -568,8 +571,11 @@ static int k3_launch(ts_ctx* c, K3Args& a, const int64_t* N_i_host, const double
   }
   // diagonal inertia matrices (every preset of the reference): instantiations without the products by their zeros
   const bool dj = diag_inertia && !a.opts.k3_generic_inertia;
-  void (*const narrow_kernel)(const K3Args) = quat ? (dj ? k3_alilqr_quat_diag_kernel : k3_alilqr_quat_kernel)
-                                                   : (dj ? k3_alilqr_diag_kernel : k3_alilqr_kernel);
+  // a solve that exports its state runs the exporting instantiations (same results, K3StateIO written at the finish)
+  void (*const narrow_kernel)(const K3Args) =
+      a.sio ? (quat ? (dj ? k3_alilqr_quat_diag_export_kernel : k3_alilqr_quat_export_kernel)
+                    : (dj ? k3_alilqr_diag_export_kernel : k3_alilqr_export_kernel))
+            : (quat ? (dj ? k3_alilqr_quat_diag_kernel : k3_alilqr_quat_kernel) : (dj ? k3_alilqr_diag_kernel : k3_alilqr_kernel));
   void (*const wide_kernel)(const K3Args) = quat ? (dj ? k3_wide_quat_diag_kernel : k3_wide_quat_kernel)
                                                  : (dj ? k3_wide_diag_kernel : k3_wide_kernel);
   void (*const pair_kernel)(const K3Args) = dj ? k3_pair_diag_kernel : k3_pair_kernel;
@@ -664,11 +670,14 @@ static int k3_launch(ts_ctx* c, K3Args& a, const int64_t* N_i_host, const double
       arena += 4 * cap * K3_SLOT_DOUBLES_PER_KNOT;
     }
   }
-  if ((rc = scratch_reserve(c, SLOT_K3_ARENA, (size_t)(arena + 2) * sizeof(double) + 256, &p_work))) return rc;
   long long* d_woff = nullptr;
   int* d_wcap = nullptr;
-  if ((rc = upload(c, SLOT_K3_WARP_OFFS, warp_off.data(), (size_t)n_warps, &d_woff))) return rc;
-  if ((rc = upload(c, SLOT_K3_WARP_CAPS, warp_cap.data(), (size_t)n_warps, &d_wcap))) return rc;
+  p_work = nullptr;
+  if (!cont) {   // a continuation does not run the first launch
+    if ((rc = scratch_reserve(c, SLOT_K3_ARENA, (size_t)(arena + 2) * sizeof(double) + 256, &p_work))) return rc;
+    if ((rc = upload(c, SLOT_K3_WARP_OFFS, warp_off.data(), (size_t)n_warps, &d_woff))) return rc;
+    if ((rc = upload(c, SLOT_K3_WARP_CAPS, warp_cap.data(), (size_t)n_warps, &d_wcap))) return rc;
+  }
   if ((rc = scratch_reserve(c, SLOT_K3_COUNTERS, 128, &p_q))) return rc;
   if ((rc = scratch_reserve(c, SLOT_K3_CYCLES, (size_t)n_trials * 3 * sizeof(double) + 64, &p_diag))) return rc;
   {
@@ -711,10 +720,13 @@ static int k3_launch(ts_ctx* c, K3Args& a, const int64_t* N_i_host, const double
   a.park_data = nullptr;
   a.park_data_cap = 0;
   a.park_order = nullptr;
-  if (suspend_after > 0) {
+  if (cont || suspend_after > 0) {
     // a place for every trial that can be resident when the queue runs dry; array space for the `cap` longest
-    // horizons (order[] is sorted by horizon, descending), bounded by 32 GB
-    int64_t cap = early > 0.0 ? n_trials : std::min<int64_t>(n_trials, slots);
+    // horizons (order[] is sorted by horizon, descending), bounded by 32 GB.  A continuation parks every trial it
+    // continues, or fails.
+    std::vector<int64_t> cand = cont ? *cont : order_by_N;
+    if (cont) std::stable_sort(cand.begin(), cand.end(), [&](int64_t x, int64_t y) { return N_i_host[x] > N_i_host[y]; });
+    int64_t cap = cont ? (int64_t)cont->size() : (early > 0.0 ? n_trials : std::min<int64_t>(n_trials, slots));
     // memory of the hand-over: 27 N doubles of parked state per trial + a 261 N region per trial in the worst case
     // (no region is ever re-used); the parking places are limited to what fits 60% of the free device memory
     size_t free_b = 0, total_b = 0;
@@ -723,13 +735,16 @@ static int k3_launch(ts_ctx* c, K3Args& a, const int64_t* N_i_host, const double
     double need = 0.0, pool_need = 0.0;
     int64_t cap_fit = 0;
     for (int64_t i = 0; i < cap; ++i) {
-      const double Ne = (double)(N_i_host[order_by_N[(size_t)i]] + 1);
+      const double Ne = (double)(N_i_host[cand[(size_t)i]] + 1);
       const double dpk = (double)k3_wide_doubles_per_knot(a.opts.max_linesearch);
       if (need + pool_need + (27.0 + dpk) * Ne > budget) break;
       need += 27.0 * Ne;
       pool_need += dpk * Ne;
       cap_fit = i + 1;
     }
+    if (cont && cap_fit < cap)
+      return fail(c, TS_ERR_NOMEM, "continuation: the parked records of %lld trials do not fit in device memory (%lld do)",
+                  (long long)cap, (long long)cap_fit);
     cap = cap_fit;
     void *p_ps, *p_pd, *p_pool;
     if ((rc = scratch_reserve(c, SLOT_K3_POOL, (size_t)pool_need * sizeof(double) + 256, &p_pool))) return rc;
@@ -744,19 +759,47 @@ static int k3_launch(ts_ctx* c, K3Args& a, const int64_t* N_i_host, const double
     a.park_order = (int*)((char*)p_ps + (size_t)cap * (sizeof(TrialState) + 16));
     a.park_data = (double*)p_pd;
     a.park_data_cap = (long long)need;
+    if (cont && cap > 0) {   // place i = the i-th continuing trial, its record at the host-computed offset
+      std::vector<long long> off((size_t)cap);
+      unsigned long long used = 0;
+      for (int64_t i = 0; i < cap; ++i) {
+        const long long N = N_i_host[(*cont)[(size_t)i]];
+        off[(size_t)i] = (long long)used;
+        used += (unsigned long long)(27 * (N + (N & 1)));
+      }
+      const unsigned long long h_cnt[2] = {(unsigned long long)cap, used};   // park_count (low word of [4]) | park_used [5]
+      TS_CUDA(c, cudaMemcpyAsync(a.park_trial, cont->data(), (size_t)cap * sizeof(int64_t), cudaMemcpyHostToDevice, c->stream));
+      TS_CUDA(c, cudaMemcpyAsync(a.park_off, off.data(), (size_t)cap * sizeof(long long), cudaMemcpyHostToDevice, c->stream));
+      TS_CUDA(c, cudaMemcpyAsync((unsigned long long*)p_q + 4, h_cnt, sizeof(h_cnt), cudaMemcpyHostToDevice, c->stream));
+      sio->n_import = cap;
+    }
+  }
+  if (sio) {
+    TS_CUDA(c, cudaMemcpyAsync((void*)a.sio, sio, sizeof(K3StateIO), cudaMemcpyHostToDevice, c->stream));
+    // CS2: every trial's multipliers pass to the output (the continuing trials' rows are then overwritten); queued only
+    // now, so that a call that fails above leaves lam_out as it was
+    if (sio->lam_in)
+      TS_CUDA(c, cudaMemcpyAsync(sio->lam_out, sio->lam_in, (size_t)sio->lam_doubles * sizeof(double), cudaMemcpyDeviceToDevice,
+                                 c->stream));
   }
   c->k3_timed = true;
   c->d_k3_parked = a.park_count;
   c->k3_park_cap = a.park_cap;
   TS_CUDA(c, cudaEventRecord(c->ev_k3[0], c->stream));
-  narrow_kernel<<<blocks, K3_WARPS_PER_BLOCK * 32, K3_SMEM_BYTES, c->stream>>>(a);
-  c->launches++;
+  if (!cont) {
+    narrow_kernel<<<blocks, K3_WARPS_PER_BLOCK * 32, K3_SMEM_BYTES, c->stream>>>(a);
+    c->launches++;
+  }
   TS_CUDA(c, cudaGetLastError());
   TS_CUDA(c, cudaEventRecord(c->ev_k3[1], c->stream));
   TS_CUDA(c, cudaEventRecord(c->ev_k3[2], c->stream));
   if (a.park_cap > 0) {
     // one warp per parked trial; the grid cannot depend on the (device-side) count, idle blocks exit at once
     const int blocks_w = (int)std::max<int64_t>(1, std::min<int64_t>(a.park_cap, wide_warps));
+    if (cont) {
+      park_import_kernel<<<(unsigned)((sio->n_import + 3) / 4), 32, K3_SMEM_BYTES, c->stream>>>(a);
+      c->launches++;
+    }
     k3_park_order_kernel<<<1, 1024, 0, c->stream>>>(a);
     if (pair)
       pair_kernel<<<(blocks_w + K3_PAIRS_PER_BLOCK - 1) / K3_PAIRS_PER_BLOCK, 64 * K3_PAIRS_PER_BLOCK, K3_PAIR_SMEM_BYTES, c->stream>>>(a);
@@ -769,15 +812,33 @@ static int k3_launch(ts_ctx* c, K3Args& a, const int64_t* N_i_host, const double
   return TS_OK;
 }
 
+static_assert(sizeof(ts_al_state) == 104 && sizeof(ts_al_state) == sizeof(ts_al_state_dev), "ts_al_state layout");
+
 int ts_alilqr_solve_batch(ts_ctx* c, int64_t n_trials, const int64_t* N_i, const int64_t* offs, const double* x0,
                           const double* xf, const double* Jmat, const double* Qd, const double* Qfd, const double* Rd,
                           const double* B_eci, const int64_t* B_offs, const int64_t* B_rows, const double* index_scale,
                           const double* clock_rate, double dt, const double* U0, const ts_ilqr_opts* opts, double* X,
                           double* U, double* K, ts_trial_outcome* out, int pointers_are_device) {
+  return ts_alilqr_solve_state_batch(c, n_trials, N_i, offs, x0, xf, Jmat, Qd, Qfd, Rd, B_eci, B_offs, B_rows, index_scale,
+                                     clock_rate, dt, U0, opts, X, U, K, out, pointers_are_device, nullptr, nullptr, nullptr, nullptr);
+}
+
+int ts_alilqr_solve_state_batch(ts_ctx* c, int64_t n_trials, const int64_t* N_i, const int64_t* offs, const double* x0,
+                                const double* xf, const double* Jmat, const double* Qd, const double* Qfd, const double* Rd,
+                                const double* B_eci, const int64_t* B_offs, const int64_t* B_rows, const double* index_scale,
+                                const double* clock_rate, double dt, const double* U0, const ts_ilqr_opts* opts, double* X,
+                                double* U, double* K, ts_trial_outcome* out, int pointers_are_device,
+                                const ts_al_state* state_in, const double* lam_in, ts_al_state* state_out, double* lam_out) {
   if (!c) return TS_ERR_ARG;
   if (n_trials < 0 || (n_trials > 0 && (!N_i || !offs || !x0 || !xf || !Jmat || !Qd || !Qfd || !Rd || !B_eci || !B_offs || !B_rows ||
                                         !index_scale || !clock_rate || !X || !U || !out)))
     return fail(c, TS_ERR_ARG, "ts_alilqr_solve_batch: null argument");
+  if (state_in && !lam_in) return fail(c, TS_ERR_ARG, "ts_alilqr_solve_state_batch: state_in without lam_in");
+  if (state_in)
+    for (int64_t t = 0; t < n_trials; ++t)
+      if (state_in[t].status < TS_ST_CONVERGED || state_in[t].status > TS_ST_NO_CUTOFF || state_in[t].outer_iters < 1)
+        return fail(c, TS_ERR_ARG, "ts_alilqr_solve_state_batch: trial %lld: status %d / outer_iters %d is not an exported state",
+                    (long long)t, (int)state_in[t].status, (int)state_in[t].outer_iters);
   if (n_trials == 0) return TS_OK;
   if (!(dt > 0)) return fail(c, TS_ERR_ARG, "ts_alilqr_solve_batch: dt must be > 0");
   ts_ilqr_opts o;
@@ -798,12 +859,20 @@ int ts_alilqr_solve_batch(ts_ctx* c, int64_t n_trials, const int64_t* N_i, const
   TS_CUDA(c, cudaSetDevice(c->device));
   int rc;
   Staging io(c, pointers_are_device);
-  K3Args a;
+  K3Args a = {};
   a.B_eci = io.in(B_eci, (size_t)total_rows * 3);
   a.U0 = io.in(U0, (size_t)total_knots * 3);
-  a.X = io.out(X, (size_t)total_knots * 8);
-  a.U = io.out(U, (size_t)total_knots * 3);
-  a.K = io.out(K, (size_t)total_knots * 24);
+  if (state_in) {   // CS2: the rows of the trials that pass through stay as given
+    a.X = io.inout(X, (size_t)total_knots * 8);
+    a.U = io.inout(U, (size_t)total_knots * 3);
+    a.K = io.inout(K, (size_t)total_knots * 24);
+    lam_in = io.in(lam_in, (size_t)total_knots * 6);
+  } else {
+    a.X = io.out(X, (size_t)total_knots * 8);
+    a.U = io.out(U, (size_t)total_knots * 3);
+    a.K = io.out(K, (size_t)total_knots * 24);
+  }
+  double* d_lam_out = io.out(lam_out, (size_t)total_knots * 6);
   if (io.rc) return io.rc;
   // per-trial small arrays -> one packed upload
   const size_t T = (size_t)n_trials;
@@ -832,10 +901,40 @@ int ts_alilqr_solve_batch(ts_ctx* c, int64_t n_trials, const int64_t* N_i, const
   memcpy(&a.opts, &o, sizeof(o));
   a.out = (ts_trial_outcome_dev*)p_out;
   io.back(out, (const ts_trial_outcome*)p_out, T);
+  std::vector<int64_t> cont;
+  K3StateIO sio = {};
+  if (state_out || lam_out || state_in) {
+    // device block: states [0, T) imported, [T, 2T) exported | K3StateIO | the multipliers when the caller takes none
+    void* p_st;
+    const size_t b_st = 2 * T * sizeof(ts_al_state), b_lam = lam_out ? 0 : (size_t)total_knots * 6 * sizeof(double);
+    if ((rc = scratch_reserve(c, SLOT_AL_STATES, b_st + 64 + b_lam, &p_st))) return rc;
+    ts_al_state_dev* d_in = (ts_al_state_dev*)p_st;
+    sio.state_out = d_in + T;
+    sio.lam_out = lam_out ? d_lam_out : (double*)((char*)p_st + b_st + 64);
+    a.sio = (const K3StateIO*)((char*)p_st + b_st);
+    if (state_out) io.back(state_out, (const ts_al_state*)sio.state_out, T);
+    if (state_in) {
+      // CS2: which trials continue; every other trial's outcome is rebuilt from its state, and its state and multipliers
+      // are copied to the outputs (the kernels then overwrite the continuing trials' records)
+      std::vector<ts_trial_outcome> oc(T);
+      for (size_t t = 0; t < T; ++t) {
+        const ts_al_state& st = state_in[t];
+        if (st.status == TS_ST_MAX_OUTER && st.outer_iters < o.max_outer) cont.push_back((int64_t)t);
+        oc[t] = ts_trial_outcome{st.status, st.outer_iters, st.inner_iters, st.ls_rollouts, N_i[t], st.J, st.c_max, 0.0, 0.0, 0.0};
+      }
+      TS_CUDA(c, cudaMemcpyAsync(d_in, state_in, T * sizeof(ts_al_state), cudaMemcpyHostToDevice, c->stream));
+      TS_CUDA(c, cudaMemcpyAsync(p_out, oc.data(), T * sizeof(ts_trial_outcome), cudaMemcpyHostToDevice, c->stream));
+      TS_CUDA(c, cudaMemcpyAsync(sio.state_out, d_in, T * sizeof(ts_al_state), cudaMemcpyDeviceToDevice, c->stream));
+      sio.state_in = d_in;
+      sio.lam_in = lam_in;
+      sio.lam_doubles = total_knots * 6;   // copied to lam_out by k3_launch once the park records are known to fit
+    }
+  }
   std::vector<double> diff(T);
   for (size_t t = 0; t < T; ++t) diff[t] = slew_angle(x0 + 8 * t, xf + 8 * t);
   io.start();
-  if ((rc = k3_launch(c, a, N_i, diff.data(), all_inertia_diagonal(Jmat, n_trials)))) return rc;
+  if ((rc = k3_launch(c, a, N_i, diff.data(), all_inertia_diagonal(Jmat, n_trials), state_in ? &cont : nullptr, a.sio ? &sio : nullptr)))
+    return rc;
   return io.finish();
 }
 
@@ -1174,7 +1273,7 @@ int ts_monte_carlo_run(ts_ctx* c, const ts_mc_config* cfg, const double* kep6, c
     c->launches++;
     cudaEventRecord(e[3], c->stream);
     // ---- stage 4: AL-iLQR
-    K3Args ka;
+    K3Args ka = {};
     ka.n_trials = na;
     ka.N_i = d_i; ka.offs = d_i + NA; ka.B_offs = d_i + 2 * NA; ka.B_rows = d_i + 3 * NA;
     ka.x0 = d_f; ka.xf = d_f + 8 * NA; ka.Jmat = d_f + 16 * NA; ka.Qd = pa.Qd; ka.Qfd = pa.Qfd; ka.Rd = pa.Rd;

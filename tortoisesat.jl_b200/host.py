@@ -31,6 +31,17 @@ OUTCOME_DTYPE = np.dtype([("status", "<i4"), ("outer_iters", "<i4"), ("inner_ite
                           ("flops", "<f8")])
 
 
+# ts_al_state: the exported AL-iLQR solver state of one trial (CS1-CS4, DESIGN.md section 4, K3)
+AL_STATE_DTYPE = np.dtype([("mu", "<f8"), ("lam_goal", "<f8", (8,)), ("J", "<f8"), ("c_max", "<f8"), ("status", "<i4"),
+                           ("outer_iters", "<i4"), ("inner_iters", "<i4"), ("ls_rollouts", "<i4")])
+
+
+class AlState(C.Structure):
+    """ts_al_state (include/tortoise_b200.h), 104 bytes."""
+    _fields_ = [("mu", C.c_double), ("lam_goal", C.c_double * 8), ("J", C.c_double), ("c_max", C.c_double),
+                ("status", C.c_int32), ("outer_iters", C.c_int32), ("inner_iters", C.c_int32), ("ls_rollouts", C.c_int32)]
+
+
 class IlqrOpts(C.Structure):
     """ts_ilqr_opts (include/tortoise_b200.h)."""
     _fields_ = [(k, C.c_int32) for k in ("max_outer", "max_inner", "max_linesearch", "dJ_counter_limit", "stage_cost_dt",
@@ -180,6 +191,7 @@ def load_library():
     L.ts_monte_carlo_run.argtypes = [C.c_void_p, C.POINTER(McConfig)] + [C.c_void_p] * 8 + [C.POINTER(McStats)]
     L.ts_alilqr_solve_batch.argtypes = [C.c_void_p, C.c_int64] + [C.c_void_p] * 13 + [C.c_double, C.c_void_p,
                                                                                       C.POINTER(IlqrOpts)] + [C.c_void_p] * 4 + [C.c_int]
+    L.ts_alilqr_solve_state_batch.argtypes = L.ts_alilqr_solve_batch.argtypes + [C.c_void_p] * 4
     _LIB = L
     return L
 
@@ -416,34 +428,70 @@ class Engine:
 
 
     # -- K3 ---------------------------------------------------------------
+    @staticmethod
+    def _alilqr_inputs(N_i, x0, xf, Jmat, Qd, Qfd, Rd, B_eci, B_offs, B_rows, index_scale, clock_rate, dt, U0, opts):
+        """The host arrays of ts_alilqr_solve_batch / ts_alilqr_solve_state_batch up to U0 and opts, in order, plus
+        (T, offs).  The arrays are kept referenced by the returned tuple for the duration of the call."""
+        N_i = np.ascontiguousarray(N_i, dtype=np.int64)
+        T = N_i.shape[0]
+        offs = np.zeros(T + 1, dtype=np.int64)
+        offs[1:] = np.cumsum(N_i)
+        arr = lambda a, w: _f64(np.asarray(a, dtype=np.float64).reshape(T, w))
+        keep = [N_i, offs, arr(x0, 8), arr(xf, 8), arr(Jmat, 9), arr(Qd, 8), arr(Qfd, 8), arr(Rd, 3), _f64(B_eci),
+                np.ascontiguousarray(B_offs, dtype=np.int64), np.ascontiguousarray(B_rows, dtype=np.int64), _f64(index_scale),
+                _f64(clock_rate)]
+        U0a = None if U0 is None else _f64(U0)
+        o = opts if opts is not None else default_ilqr_opts()
+        args = [T] + [_ptr(a) for a in keep] + [float(dt), None if U0a is None else _ptr(U0a), C.byref(o)]
+        return T, offs, args, (keep, U0a, o)
+
     def alilqr_solve_batch(self, N_i, x0, xf, Jmat, Qd, Qfd, Rd, B_eci, B_offs, B_rows, index_scale, clock_rate, dt,
                            U0=None, opts=None, want_K=True):
         """Batched AL-iLQR solve (TortoiseSat.jl:145-146,169,178-199).  Per-trial rows in
         x0/xf (T,8), Jmat (T,9), Qd/Qfd (T,8), Rd (T,3); ragged knots addressed through
         offs = cumsum(N_i).  Returns (X, U, K, outcomes, offs): X (sum N, 8), U (sum N, 3)
         [row offs[t]+N_t-1 unused], K (sum N, 3, 8) or None."""
-        N_i = np.ascontiguousarray(N_i, dtype=np.int64)
-        T = N_i.shape[0]
-        offs = np.zeros(T + 1, dtype=np.int64)
-        offs[1:] = np.cumsum(N_i)
-        arr = lambda a, w: _f64(np.asarray(a, dtype=np.float64).reshape(T, w))
-        x0, xf, Jmat, Qd, Qfd, Rd = arr(x0, 8), arr(xf, 8), arr(Jmat, 9), arr(Qd, 8), arr(Qfd, 8), arr(Rd, 3)
-        B_eci = _f64(B_eci)
-        B_offs = np.ascontiguousarray(B_offs, dtype=np.int64)
-        B_rows = np.ascontiguousarray(B_rows, dtype=np.int64)
-        index_scale, clock_rate = _f64(index_scale), _f64(clock_rate)
+        T, offs, args, _keep = self._alilqr_inputs(N_i, x0, xf, Jmat, Qd, Qfd, Rd, B_eci, B_offs, B_rows, index_scale, clock_rate,
+                                                   dt, U0, opts)
         tot = int(offs[-1])
         X = np.zeros((tot, 8))
         U = np.zeros((tot, 3))
         K = np.zeros((tot, 3, 8)) if want_K else None
         out = np.zeros(T, dtype=OUTCOME_DTYPE)
-        o = opts if opts is not None else default_ilqr_opts()
-        U0a = None if U0 is None else _f64(U0)
-        self._check(self.lib.ts_alilqr_solve_batch(
-            self.h, T, _ptr(N_i), _ptr(offs), _ptr(x0), _ptr(xf), _ptr(Jmat), _ptr(Qd), _ptr(Qfd), _ptr(Rd), _ptr(B_eci),
-            _ptr(B_offs), _ptr(B_rows), _ptr(index_scale), _ptr(clock_rate), float(dt), None if U0a is None else _ptr(U0a),
-            C.byref(o), _ptr(X), _ptr(U), None if K is None else _ptr(K), out.ctypes.data, 0))
+        self._check(self.lib.ts_alilqr_solve_batch(self.h, *args, _ptr(X), _ptr(U), None if K is None else _ptr(K), out.ctypes.data, 0))
         return X, U, K, out, offs
+
+    def alilqr_solve_state_batch(self, N_i, x0, xf, Jmat, Qd, Qfd, Rd, B_eci, B_offs, B_rows, index_scale, clock_rate, dt,
+                                 U0=None, opts=None, want_K=True, state=None, lam=None, X=None, U=None):
+        """alilqr_solve_batch that also returns each trial's solver state and bound multipliers, and continues from them.
+        state=None: a fresh solve (the same results as alilqr_solve_batch).  With `state` (AL_STATE_DTYPE, T records)
+        and `lam` ((sum N, 6)) from an earlier call, plus that call's X and U: the trials that ended at max_outer with
+        outer_iters < opts.max_outer continue (CS2, CS3); the others pass through (their K rows stay zero here).  Returns
+        (X, U, K, out, offs, state, lam), state as AL_STATE_DTYPE records, lam (sum N, 6) [row offs[t]+N_t-1 zero]."""
+        T, offs, args, _keep = self._alilqr_inputs(N_i, x0, xf, Jmat, Qd, Qfd, Rd, B_eci, B_offs, B_rows, index_scale, clock_rate,
+                                                   dt, U0, opts)
+        tot = int(offs[-1])
+        if state is not None:
+            if lam is None or X is None or U is None:
+                raise ValueError("continuing from a state needs the lam, X and U it was exported with")
+            state = np.ascontiguousarray(state, dtype=AL_STATE_DTYPE)
+            if state.shape != (T,):
+                raise ValueError("state must hold one record per trial")
+            lam_in = np.ascontiguousarray(lam, dtype=np.float64).reshape(tot, 6)
+            X = np.array(X, dtype=np.float64, order="C").reshape(tot, 8)     # copies: the call writes X and U in place
+            U = np.array(U, dtype=np.float64, order="C").reshape(tot, 3)
+        else:
+            lam_in = None
+            X, U = np.zeros((tot, 8)), np.zeros((tot, 3))
+        K = np.zeros((tot, 3, 8)) if want_K else None
+        out = np.zeros(T, dtype=OUTCOME_DTYPE)
+        st_out = np.zeros(T, dtype=AL_STATE_DTYPE)
+        lam_out = np.zeros((tot, 6))
+        self._check(self.lib.ts_alilqr_solve_state_batch(
+            self.h, *args, _ptr(X), _ptr(U), None if K is None else _ptr(K), out.ctypes.data, 0,
+            None if state is None else state.ctypes.data, None if lam_in is None else _ptr(lam_in), st_out.ctypes.data,
+            _ptr(lam_out)))
+        return X, U, K, out, offs, st_out, lam_out
 
 
     # -- element-wise building blocks --------------------------------------
