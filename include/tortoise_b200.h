@@ -324,7 +324,9 @@ typedef struct ts_mc_config {
   int32_t eigen_axis_fix;    /* see ts_slew_weights_batch; 0 = literal reference                          */
   int32_t keep_trajectories; /* 1: X, U, X_sim, U_sim and the fine field tables of this run stay resident in HBM
                                     for ts_mc_fetch_trajectories (the `states`, `control_inputs`, `sim_states`,
-                                    `sim_control_inputs`, `B_ECI_total` arrays of monte_carlo.jl:52-66)       */
+                                    `sim_control_inputs`, `B_ECI_total` arrays of monte_carlo.jl:52-66)
+                                2: as 1, and the solver states, multipliers and per-trial inputs are kept too, for
+                                    ts_mc_fetch_state and ts_mc_continue (same results as 1)                 */
   ts_ilqr_opts ilqr;
   ts_tvlqr_opts tvlqr;
 } ts_mc_config;
@@ -351,6 +353,39 @@ int ts_monte_carlo_run(ts_ctx* ctx, const ts_mc_config* cfg, const double* kep6,
  * trial unused = 0), B_eci: rows x 3 Tesla (B_ECI_total, monte_carlo.jl:149; rows the solver cannot index are 0).   */
 int ts_mc_trajectory_layout(ts_ctx* ctx, int64_t n_trials, int64_t* knot_offs, int64_t* row_offs);
 int ts_mc_fetch_trajectories(ts_ctx* ctx, double* X, double* U, double* X_sim, double* U_sim, double* B_eci);
+
+/* ---- Monte-Carlo continuation: more outer iterations for the max-outer trials of a kept run ---------------- *
+ * A ts_monte_carlo_run with cfg->keep_trajectories = 2 keeps, besides the trajectories, every active trial's solver
+ * state (ts_al_state, CS1) and bound multipliers, its per-trial solver and replay inputs, the run's config and the final
+ * outcome records.  They stay valid until the next ts_monte_carlo_run on ctx, whatever other entries run in between.
+ * ts_mc_fetch_state copies the kept state to HOST arrays (either may be null): state gets n_trials records (a
+ * TS_ST_NO_CUTOFF trial gets a zero record with status 5), lam (sum N) x 6 doubles in the layout of
+ * ts_mc_trajectory_layout's knot_offs.  With ts_mc_fetch_trajectories that is what ts_alilqr_solve_state_batch needs
+ * to continue a trial on its own.
+ * ts_mc_continue continues the kept run in place (DESIGN.md section 4, K3):
+ *  MC1 which trials: CS2 under the continuing call's opts, status == TS_ST_MAX_OUTER && outer_iters < opts->max_outer.
+ *      Every other trial passes through unchanged, NO_CUTOFF trials included: its outcome record (byte for byte), its
+ *      rows of X, U, X_sim and U_sim, its state and its lam.
+ *  MC2 solve: the continuation path of ts_alilqr_solve_state_batch on the kept block (import, then the one-warp-per-
+ *      trial kernels), the producer-warp kernel chosen by opts->k3_pair over the run's active trials.  X, U, the states
+ *      and lam are updated in place.
+ *  MC3 replay and records: with run_tvlqr, the continuing trials alone are replayed with the run's TVLQR options (after
+ *      the fused path's overrides), stream ids and initial states; their X_sim / U_sim rows are cleared first.  A
+ *      continued record has counters, J and c_max from the solver as totals over both calls (CS3), N and t_final
+ *      unchanged, slew_time from the new replay (0 without run_tvlqr) and flops by ts_monte_carlo_run's formula over
+ *      the totals.  `out` (HOST, n_trials records) returns the whole ensemble in caller order, and the kept block holds
+ *      it: the fetch calls return the continued run and a second ts_mc_continue chains.
+ *  MC4 equivalence: the continuing trials' solver results (X, U, counters, J, c_max, state, lam) equal bit for bit
+ *      those of ts_alilqr_solve_state_batch continuing over the run's active trials from ts_mc_fetch_state and
+ *      ts_mc_fetch_trajectories with the run's inputs.  Against a direct run to the larger max_outer, CS4 applies.
+ * stats (nullable): counts and sums describe the whole ensemble after the call, as ts_monte_carlo_run reports them;
+ * ms_solve, ms_tvlqr and flops this call's work (the added iterations and the replay); ms_field = ms_prep = 0.
+ * ts_last_kernel_ms, ts_k3_last_split and ts_k3_last_parked report the continuation.  TS_ERR_ARG, with out and stats
+ * untouched, when no run on ctx had keep_trajectories = 2 (the last run decides), n_trials differs from the kept run,
+ * opts or out is null, or opts fails the checks of ts_alilqr_solve_state_batch; TS_ERR_NOMEM, nothing kept written and
+ * the run still continuable, when the parked records of the continuing trials do not fit in device memory.          */
+int ts_mc_fetch_state(ts_ctx* ctx, ts_al_state* state, double* lam);
+int ts_mc_continue(ts_ctx* ctx, int64_t n_trials, const ts_ilqr_opts* opts, ts_trial_outcome* out, ts_mc_stats* stats);
 
 /* ---- igrf12syn: the Fortran-style twin of igrf12 -------------------------------------------- *
  * igrf12syn(isv, date, itype, alt, colat, elong) [src/igrf.jl:335-534] at n points.  isv 0 = main field, 1 = secular
@@ -388,6 +423,10 @@ ts_ctx* ts_multi_ctx(ts_multi* m, int i); /* the i-th device's context (borrowed
 int ts_multi_monte_carlo_run(ts_multi* m, const ts_mc_config* cfg, const double* kep6, const ts_field_opts* fopts,
                              const double* x0, const double* xf, const double* Jmat, const double* q_noise0,
                              const uint32_t* stream_id, ts_trial_outcome* out, ts_mc_stats* stats);
+/* ts_mc_continue on every device's kept shard of a ts_multi_monte_carlo_run with keep_trajectories = 2, then the
+ * records gathered and the statistics reduced as after the run.  (Per-process multi-GPU needs no library call: each
+ * rank continues its own context and gathers as after its run.)                                                     */
+int ts_multi_mc_continue(ts_multi* m, int64_t n_trials, const ts_ilqr_opts* opts, ts_trial_outcome* out, ts_mc_stats* stats);
 
 /* ---- element-wise batch versions of the reference's building blocks (all HOST pointers) --- *
  * Correctness / drop-in paths for callers that use the small functions on their own; the fused

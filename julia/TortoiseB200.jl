@@ -330,8 +330,10 @@ end
 function monte_carlo(; number_sims = 100, alt = 400, R_E = 6371.0, inclination = 96.6, MJD_0 = 58155.0, igrf_date = 2019.0,
                      t0 = 0.0, tf = 60 * 40, cutoff = 30, N = 5000, J = [0.00125 0 0; 0 0.00125 0; 0 0 0.00125],
                      q_0 = [1.0; 0; 0; 0], q_final = [sqrt(2) / 2; sqrt(2) / 2; 0; 0], α = 1.e-1, β = 1.e3, seed = 0, run_tvlqr = true,
-                     ilqr::IlqrOpts = default_ilqr_opts(), sat_att = false, trajectories = true, e::Engine = engine())
+                     ilqr::IlqrOpts = default_ilqr_opts(), sat_att = false, trajectories = true, resumable = false,
+                     e::Engine = engine())
     # sat_att = true: the solver configuration of monte_carlo.jl:158,192 (quaternion_error / quaternion_expansion hooks)
+    # resumable = true: keep_trajectories = 2, the solver state stays on `e` for continue_monte_carlo!
     if sat_att
         ilqr = IlqrOpts((f == :quat_error ? Int32(1) : getfield(ilqr, f) for f in fieldnames(IlqrOpts))...)
     end
@@ -350,7 +352,7 @@ function monte_carlo(; number_sims = 100, alt = 400, R_E = 6371.0, inclination =
     tv = default_tvlqr_opts()
     tv = TvlqrOpts(0.2, t0, 0.0, ntuple(_ -> 10.0, 6), ntuple(_ -> 1000.0, 6), ntuple(_ -> 0.5e3, 3), tv.dt_squared, 2, seed,
                    0.05, 0.08727, 0, 0)                                            # monte_carlo.jl:69-71,216-226
-    cfg = McConfig(number_sims, 0, run_tvlqr ? 1 : 0, t0, tf, N, cutoff, 0.2, α, β, 0, trajectories ? 1 : 0, ilqr, tv)
+    cfg = McConfig(number_sims, 0, run_tvlqr ? 1 : 0, t0, tf, N, cutoff, 0.2, α, β, 0, resumable ? 2 : trajectories ? 1 : 0, ilqr, tv)
     out = Vector{TrialOutcome}(undef, number_sims); st = Ref{McStats}()
     rc = ccall((:ts_monte_carlo_run, LIB), Cint,
                (Ptr{Cvoid}, Ref{McConfig}, Ptr{Float64}, Ptr{FieldOpts}, Ptr{Float64}, Ptr{Float64}, Ptr{Float64}, Ptr{Float64},
@@ -360,6 +362,7 @@ function monte_carlo(; number_sims = 100, alt = 400, R_E = 6371.0, inclination =
     t_final = [o.t_final for o in out]; slew_time = [o.slew_time for o in out]
     fails = [o.slew_time == o.t_final ? 1.0 : 0.0 for o in out]                  # monte_carlo.jl:257-261
     res = (A = Matrix(A'), t_final = t_final, slew_time = slew_time, fails = fails, outcomes = out, stats = st[])
+    resumable && (res = merge(res, (ilqr = ilqr, run_tvlqr = run_tvlqr)))
     trajectories || return res
     # the per-trial arrays the script keeps (monte_carlo.jl:52-66,149,200-201,232-233), fetched from HBM
     ko = zeros(Int64, number_sims + 1); ro = zeros(Int64, number_sims + 1)
@@ -371,6 +374,54 @@ function monte_carlo(; number_sims = 100, alt = 400, R_E = 6371.0, inclination =
     merge(res, (states = [X[:, rng(t)] for t in 1:number_sims], control_inputs = [U[:, rng(t)[1:end-1]] for t in 1:number_sims],
                 sim_states = [Xs[:, rng(t)] for t in 1:number_sims], sim_control_inputs = [Us[:, rng(t)] for t in 1:number_sims],
                 B_ECI_total = [Matrix(B[:, (ro[t] + 1):(ro[t] + 2 * length(rng(t)))]') for t in 1:number_sims]))
+end
+
+# The kept solver state of the last monte_carlo(...; resumable = true) on `e` (ts_mc_fetch_state): one AlState per trial
+# (NO_CUTOFF: zero record with status 5) and the multipliers, 6 x (sum N) ragged like the `states` arrays.
+function mc_state(number_sims::Integer; e::Engine = engine())
+    ko = zeros(Int64, number_sims + 1)
+    check(e, ccall((:ts_mc_trajectory_layout, LIB), Cint, (Ptr{Cvoid}, Int64, Ptr{Int64}, Ptr{Int64}), e.h, number_sims, ko, C_NULL))
+    st = Vector{AlState}(undef, number_sims); lam = zeros(6, ko[end])
+    check(e, ccall((:ts_mc_fetch_state, LIB), Cint, (Ptr{Cvoid}, Ptr{AlState}, Ptr{Float64}), e.h, st, lam))
+    return st, lam
+end
+
+# ts_mc_continue: the max-outer trials of the kept run continue to ilqr.max_outer (rules MC1-MC4, DESIGN.md section 4);
+# returns the outcome records of the whole ensemble and the statistics of the call.
+function mc_continue(number_sims::Integer, ilqr::IlqrOpts; e::Engine = engine())
+    out = Vector{TrialOutcome}(undef, number_sims); st = Ref{McStats}()
+    check(e, ccall((:ts_mc_continue, LIB), Cint, (Ptr{Cvoid}, Int64, Ref{IlqrOpts}, Ptr{TrialOutcome}, Ref{McStats}),
+                   e.h, number_sims, Ref(ilqr), out, st))
+    return out, st[]
+end
+
+# Continues a monte_carlo(...; resumable = true) result `res` in place to max_outer outer iterations in all: outcomes,
+# slew_time, fails (monte_carlo.jl:257-261) and the trajectory arrays of the continued trials.  Returns their indices.
+function continue_monte_carlo!(res; max_outer = 30, ilqr::Union{Nothing,IlqrOpts} = nothing, e::Engine = engine())
+    base = ilqr === nothing ? res.ilqr : ilqr
+    o = IlqrOpts((f == :max_outer ? Int32(max_outer) : getfield(base, f) for f in fieldnames(IlqrOpts))...)
+    n = length(res.outcomes)
+    idx = [t for t in 1:n if res.outcomes[t].status == 1 && res.outcomes[t].outer_iters < max_outer]   # MC1
+    out, _ = mc_continue(n, o; e = e)
+    res.outcomes .= out
+    res.slew_time .= [r.slew_time for r in out]
+    res.fails .= [r.slew_time == r.t_final ? 1.0 : 0.0 for r in out]
+    if !isempty(idx) && haskey(res, :states)
+        ko = zeros(Int64, n + 1)
+        check(e, ccall((:ts_mc_trajectory_layout, LIB), Cint, (Ptr{Cvoid}, Int64, Ptr{Int64}, Ptr{Int64}), e.h, n, ko, C_NULL))
+        X = zeros(8, ko[end]); U = zeros(3, ko[end]); Xs = zeros(8, ko[end]); Us = zeros(3, ko[end])
+        sim = res.run_tvlqr
+        check(e, ccall((:ts_mc_fetch_trajectories, LIB), Cint, (Ptr{Cvoid}, Ptr{Float64}, Ptr{Float64}, Ptr{Float64}, Ptr{Float64}, Ptr{Float64}),
+                       e.h, X, U, sim ? Xs : C_NULL, sim ? Us : C_NULL, C_NULL))
+        for t in idx
+            r = (ko[t] + 1):ko[t + 1]
+            res.states[t] = X[:, r]; res.control_inputs[t] = U[:, r[1:end-1]]
+            if sim
+                res.sim_states[t] = Xs[:, r]; res.sim_control_inputs[t] = Us[:, r]
+            end
+        end
+    end
+    return idx
 end
 
 # igrf12syn(isv,date,itype,alt,colat,elong) -> (x,y,z,f)      reference src/igrf.jl:335-534 (scalar call = batch of one)
@@ -464,6 +515,7 @@ hat(x) = [0 -x[3] x[2]; x[3] 0 -x[1]; -x[2] x[1] 0]                             
 export Engine, params, input_parameters, igrf12, igrf12_batch, igrf_data, magnetic_simulation, magnetic_gramian, kep_ECI, OrbitPlotter,
        legendre, dlegendre, DerivFunction, gain_simulator, attitude_dynamics,
        condition_based_time, eigen_axis_slew, bryson_weights, solve_slew, attitude_simulation, monte_carlo, qmult, qrot, q_inv, hat,
-       igrf12syn, attitude_dynamics_linear, psiaki_pd_simulation, igrf_interpolant, field_map_prefilter, field_map_eval, AlState
+       igrf12syn, attitude_dynamics_linear, psiaki_pd_simulation, igrf_interpolant, field_map_prefilter, field_map_eval, AlState,
+       mc_state, mc_continue, continue_monte_carlo!
 
 end # module

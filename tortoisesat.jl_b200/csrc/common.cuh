@@ -14,7 +14,8 @@
 namespace ts {
 // Grow-only device scratch slots of a context.  Most slots hold one call's working storage and are shared between
 // entries: whatever a call leaves in them is dead once it returns.  Storage that a later call reads (the readers are
-// ts_k3_last_* and ts_mc_fetch_trajectories) lives in a slot that no other entry writes.
+// ts_k3_last_*, ts_mc_fetch_trajectories, ts_mc_fetch_state and ts_mc_continue) lives in a slot that no other entry
+// writes.
 enum Slot : int {
   SLOT_POSITIONS,                          // K2 orbit positions (ts_magnetic_simulation_batch without `pos`, Monte-Carlo)
   SLOT_ARGS_A, SLOT_ARGS_B, SLOT_ARGS_C,   // a call's small per-trial inputs; C also K3 outcomes and slew-prep outputs
@@ -23,17 +24,19 @@ enum Slot : int {
   SLOT_K3_ARENA, SLOT_ROWS_A, SLOT_ROWS_B, // K3 trajectory arena; per-row outputs (slew-prep guesses, Monte-Carlo scoping field)
   SLOT_K4_GAINS,                           // K4 gains when the caller passes none
   SLOT_ORBIT_BLOCK, SLOT_ROW_LIMITS,       // Monte-Carlo per-orbit block and table row limits
-  SLOT_PACKED_I64, SLOT_PACKED_F64,        // Monte-Carlo packed per-trial arrays
-  SLOT_STREAM_IDS,                         // Monte-Carlo Philox stream ids
+  SLOT_PACKED_I64, SLOT_PACKED_F64,        // Monte-Carlo packed per-trial arrays (read by ts_mc_continue)
+  SLOT_STREAM_IDS,                         // Monte-Carlo Philox stream ids (read by ts_mc_continue)
   SLOT_PARK_STATE, SLOT_PARK_DATA,         // K3 parking places (read by ts_k3_last_parked) and parked trajectories
   SLOT_PIPE_A, SLOT_PIPE_B,                // K1 host-pointer pipeline stages
   SLOT_K3_CYCLES,                          // K3 cycle counters (read by ts_k3_last_cycles)
-  SLOT_KEPT_XSIM, SLOT_KEPT_USIM, SLOT_KEPT_BLOCK,   // Monte-Carlo kept trajectories (read by ts_mc_fetch_trajectories)
+  SLOT_KEPT_XSIM, SLOT_KEPT_USIM, SLOT_KEPT_BLOCK,   // Monte-Carlo kept trajectories, field tables, weights and outcomes
+                                                     // (read by ts_mc_fetch_trajectories and ts_mc_continue)
   SLOT_K3_WARP_OFFS, SLOT_K3_WARP_CAPS, SLOT_K3_POOL, // K3 per-warp arena offsets and capacities, straggler pool
   SLOT_LIN_RECORDS,                        // K4 linearisation records
   SLOT_TABLE,                              // a call's lookup table: K4 linearisation offsets, K8 padded coefficients
   SLOT_K3_COUNTERS,                        // K3 queue and park counters (read by ts_k3_last_split / ts_k3_last_parked)
   SLOT_AL_STATES,                          // K3 continuation: a call's imported and exported solver states
+  SLOT_KEPT_STATE,                         // Monte-Carlo kept solver states + multipliers (ts_mc_fetch_state, ts_mc_continue)
   SLOT_COUNT
 };
 }  // namespace ts
@@ -65,6 +68,21 @@ struct ts_ctx {
     int64_t n = 0, knots = 0, rows = 0;
     std::vector<int64_t> knot_offs, row_offs;
     double *d_X = nullptr, *d_U = nullptr, *d_Xs = nullptr, *d_Us = nullptr, *d_B = nullptr;
+    // keep_trajectories = 2: what ts_mc_continue needs (device pointers into the kept slots, host copies of the
+    // run's per-trial inputs in the packed layout of ts_monte_carlo_run, and the final outcome records)
+    bool resumable = false;
+    ts_mc_config cfg = {};
+    bool diag_inertia = false;
+    std::vector<int64_t> act, hi;   // active trials (caller indices); packed int64 per-active-trial arrays
+    std::vector<double> hf;         // packed double per-active-trial arrays
+    std::vector<uint32_t> sid;      // Philox stream ids of the active trials (run_tvlqr)
+    std::vector<ts_trial_outcome> out;
+    int64_t* d_i = nullptr;
+    double *d_f = nullptr, *d_w = nullptr, *d_lam = nullptr;
+    uint32_t* d_sid = nullptr;
+    ts_trial_outcome* d_out = nullptr;
+    ts_al_state* d_state = nullptr;
+    void* d_sio = nullptr;          // the K3StateIO block of the kept states
   } mc_last;
   // grow-only scratch arenas
   void* scratch[ts::SLOT_COUNT] = {};

@@ -381,6 +381,19 @@ __global__ void __launch_bounds__(32) k4c_replay_kernel(const K4Args a) {
 }
 
 // host: the three launches of K4 (a.AB / a.lin_offs / a.lin_total must be set)
+// Zeroes the X_sim / U_sim rows of the trials about to be replayed again (ts_mc_continue): one block per trial.  A
+// replay writes only its first N_sim rows, and the kept arrays promise zeros from there on.
+__global__ void __launch_bounds__(256) k4_clear_rows_kernel(int64_t n_trials, const int64_t* N_i, const int64_t* offs, double* X_sim,
+                                                            double* U_sim) {
+  const int64_t t = blockIdx.x;
+  if (t >= n_trials) return;
+  double* xs = X_sim + offs[t] * 8;
+  double* us = U_sim + offs[t] * 3;
+  const int64_t n8 = N_i[t] * 8, n3 = N_i[t] * 3;
+  for (int64_t i = threadIdx.x; i < n8; i += blockDim.x) xs[i] = 0.0;
+  for (int64_t i = threadIdx.x; i < n3; i += blockDim.x) us[i] = 0.0;
+}
+
 inline void k4_launch(ts_ctx* c, const K4Args& a) {
   if (a.lin_total > 0) k4a_linearise_kernel<<<(unsigned)((a.lin_total + 127) / 128), 128, 0, c->stream>>>(a);
   // (a per-device attribute: set on every launch -- ts_create_multi drives several devices from one process)

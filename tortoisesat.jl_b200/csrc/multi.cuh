@@ -14,6 +14,7 @@
 extern "C" int ts_monte_carlo_run(ts_ctx* c, const ts_mc_config* cfg, const double* kep6, const ts_field_opts* fopts, const double* x0,
                                   const double* xf, const double* Jmat, const double* q_noise0, const uint32_t* stream_id,
                                   ts_trial_outcome* out, ts_mc_stats* stats);
+extern "C" int ts_mc_continue(ts_ctx* c, int64_t n_trials, const ts_ilqr_opts* opts, ts_trial_outcome* out, ts_mc_stats* stats);
 extern "C" int ts_create(ts_ctx** out, int device_id);
 extern "C" void ts_destroy(ts_ctx* c);
 extern "C" const char* ts_last_error(const ts_ctx* c);
@@ -83,6 +84,76 @@ inline void stats_unpack(const double* sum, const double* mx, ts_mc_stats& s) {
   s.sum_ls_rollouts = sum[8]; s.sum_knots = sum[9]; s.flops = sum[10];
   for (int i = 0; i < 6; ++i) s.n_status[i] = (int64_t)llround(sum[11 + i]);
   s.ms_field = mx[0]; s.ms_prep = mx[1]; s.ms_solve = mx[2]; s.ms_tvlqr = mx[3];
+}
+
+// Runs `shard(g, c, ng, shard_out, shard_stats)` for every device's shard (trials g, g+G, g+2G, ...) on the device's own
+// thread, then gathers the 64-byte outcome records with ncclAllGather and reduces the statistics with ncclAllReduce
+// (sum; ms_* max).  `out` and `stats` are written only when every shard succeeded.
+template <class Shard>
+inline int multi_shards(ts_multi* m, int64_t n, Shard&& shard, ts_trial_outcome* out, ts_mc_stats* stats) {
+  const int G = m->n;
+  const int64_t per = (n + G - 1) / G;   // records per device in the gather (short shards are padded)
+  std::vector<int> rcs(G, TS_OK);
+  std::vector<std::vector<ts_trial_outcome>> shard_out(G);
+  std::vector<ts_mc_stats> shard_stats(G);
+  std::vector<std::vector<ts_trial_outcome>> gathered(G);
+  std::vector<std::vector<double>> red(G);
+  auto worker = [&](int g) {
+    ts_ctx* c = m->ctx[g];
+    const int64_t ng = (n - g + G - 1) / G;
+    shard_out[g].assign((size_t)per, ts_trial_outcome{});
+    memset(&shard_stats[g], 0, sizeof(ts_mc_stats));
+    rcs[g] = ng > 0 ? shard(g, c, ng, shard_out[g].data(), &shard_stats[g]) : TS_OK;
+    if (G == 1) return;
+    // ---- exchange (every rank takes part even after a local failure, so that nobody hangs in the collective)
+    cudaSetDevice(m->dev[g]);
+    const size_t rec = sizeof(ts_trial_outcome);
+    const size_t b_send = (size_t)per * rec, b_recv = (size_t)per * rec * G;
+    const size_t b_red = (size_t)(MS_SUM + MS_MAX) * sizeof(double);
+    const size_t need = b_recv + 2 * b_red + 256;
+    if (m->d_bytes[g] < need) {
+      if (m->d_send[g]) cudaFree(m->d_send[g]);
+      if (m->d_recv[g]) cudaFree(m->d_recv[g]);
+      cudaMalloc(&m->d_send[g], b_send + b_red + 256);
+      cudaMalloc(&m->d_recv[g], need);
+      m->d_bytes[g] = need;
+    }
+    double hsum[MS_SUM + MS_MAX];
+    stats_pack(shard_stats[g], hsum, hsum + MS_SUM);
+    char* ds = (char*)m->d_send[g];
+    char* dr = (char*)m->d_recv[g];
+    cudaMemcpyAsync(ds, shard_out[g].data(), b_send, cudaMemcpyHostToDevice, c->stream);
+    cudaMemcpyAsync(ds + b_send, hsum, b_red, cudaMemcpyHostToDevice, c->stream);
+    int e = m->nccl.AllGather(ds, dr, b_send, NCCL_CHAR, m->comms[g], c->stream);
+    if (e == NCCL_SUCCESS) e = m->nccl.AllReduce(ds + b_send, dr + b_recv, MS_SUM, NCCL_F64, NCCL_SUM, m->comms[g], c->stream);
+    if (e == NCCL_SUCCESS)
+      e = m->nccl.AllReduce(ds + b_send + MS_SUM * sizeof(double), dr + b_recv + MS_SUM * sizeof(double), MS_MAX, NCCL_F64, NCCL_MAX,
+                            m->comms[g], c->stream);
+    if (e != NCCL_SUCCESS && rcs[g] == TS_OK) rcs[g] = TS_ERR_CUDA;
+    gathered[g].resize((size_t)per * G);
+    red[g].resize(MS_SUM + MS_MAX);
+    cudaMemcpyAsync(gathered[g].data(), dr, b_recv, cudaMemcpyDeviceToHost, c->stream);
+    cudaMemcpyAsync(red[g].data(), dr + b_recv, b_red, cudaMemcpyDeviceToHost, c->stream);
+    if (cudaStreamSynchronize(c->stream) != cudaSuccess && rcs[g] == TS_OK) rcs[g] = TS_ERR_CUDA;
+  };
+  std::vector<std::thread> th;
+  for (int g = 0; g < G; ++g) th.emplace_back(worker, g);
+  for (auto& t : th) t.join();
+  for (int g = 0; g < G; ++g)
+    if (rcs[g] != TS_OK) {
+      snprintf(m->err, sizeof(m->err), "device %d: %s", m->dev[g], ts_last_error(m->ctx[g]));
+      return rcs[g];
+    }
+  if (G == 1) {
+    memcpy(out, shard_out[0].data(), (size_t)n * sizeof(ts_trial_outcome));
+    if (stats) *stats = shard_stats[0];
+    return TS_OK;
+  }
+  // every rank now holds all records (rank-major, `per` per rank): hand rank 0's copy back in the caller's trial order
+  for (int g = 0; g < G; ++g)
+    for (int64_t a = 0; g + a * G < n; ++a) out[g + a * G] = gathered[0][(size_t)g * per + a];
+  if (stats) stats_unpack(red[0].data(), red[0].data() + MS_SUM, *stats);
+  return TS_OK;
 }
 
 }  // namespace ts
@@ -157,16 +228,7 @@ int ts_multi_monte_carlo_run(ts_multi* m, const ts_mc_config* cfg, const double*
   const int64_t n = cfg->n_trials;
   if (stats) memset(stats, 0, sizeof(*stats));
   if (n <= 0) return n == 0 ? TS_OK : TS_ERR_ARG;
-  const int64_t per = (n + G - 1) / G;   // records per device in the gather (short shards are padded)
-  std::vector<int> rcs(G, TS_OK);
-  std::vector<std::vector<ts_trial_outcome>> shard_out(G);
-  std::vector<ts_mc_stats> shard_stats(G);
-  std::vector<std::vector<ts_trial_outcome>> gathered(G);
-  std::vector<std::vector<double>> red(G);
-  auto worker = [&](int g) {
-    ts_ctx* c = m->ctx[g];
-    // ---- this device's shard: trials g, g+G, g+2G, ...
-    const int64_t ng = (n - g + G - 1) / G;
+  auto shard = [&](int g, ts_ctx* c, int64_t ng, ts_trial_outcome* so, ts_mc_stats* ss) {
     ts_mc_config cg = *cfg;
     cg.n_trials = ng;
     std::vector<double> sx0((size_t)ng * 8), sxf((size_t)ng * 8), sJ((size_t)ng * 9), sq, skep;
@@ -189,63 +251,21 @@ int ts_multi_monte_carlo_run(ts_multi* m, const ts_mc_config* cfg, const double*
         sfo[a] = fopts[t];
       }
     }
-    shard_out[g].assign((size_t)per, ts_trial_outcome{});
-    memset(&shard_stats[g], 0, sizeof(ts_mc_stats));
-    int rc = TS_OK;
-    if (ng > 0)
-      rc = ts_monte_carlo_run(c, &cg, cfg->shared_orbit ? kep6 : skep.data(), cfg->shared_orbit ? fopts : sfo.data(), sx0.data(),
-                              sxf.data(), sJ.data(), q_noise0 ? sq.data() : nullptr, sid.data(), shard_out[g].data(), &shard_stats[g]);
-    rcs[g] = rc;
-    if (G == 1) return;
-    // ---- exchange (every rank takes part even after a local failure, so that nobody hangs in the collective)
-    cudaSetDevice(m->dev[g]);
-    const size_t rec = sizeof(ts_trial_outcome);
-    const size_t b_send = (size_t)per * rec, b_recv = (size_t)per * rec * G;
-    const size_t b_red = (size_t)(MS_SUM + MS_MAX) * sizeof(double);
-    const size_t need = b_recv + 2 * b_red + 256;
-    if (m->d_bytes[g] < need) {
-      if (m->d_send[g]) cudaFree(m->d_send[g]);
-      if (m->d_recv[g]) cudaFree(m->d_recv[g]);
-      cudaMalloc(&m->d_send[g], b_send + b_red + 256);
-      cudaMalloc(&m->d_recv[g], need);
-      m->d_bytes[g] = need;
-    }
-    double hsum[MS_SUM + MS_MAX];
-    stats_pack(shard_stats[g], hsum, hsum + MS_SUM);
-    char* ds = (char*)m->d_send[g];
-    char* dr = (char*)m->d_recv[g];
-    cudaMemcpyAsync(ds, shard_out[g].data(), b_send, cudaMemcpyHostToDevice, c->stream);
-    cudaMemcpyAsync(ds + b_send, hsum, b_red, cudaMemcpyHostToDevice, c->stream);
-    int e = m->nccl.AllGather(ds, dr, b_send, NCCL_CHAR, m->comms[g], c->stream);
-    if (e == NCCL_SUCCESS) e = m->nccl.AllReduce(ds + b_send, dr + b_recv, MS_SUM, NCCL_F64, NCCL_SUM, m->comms[g], c->stream);
-    if (e == NCCL_SUCCESS)
-      e = m->nccl.AllReduce(ds + b_send + MS_SUM * sizeof(double), dr + b_recv + MS_SUM * sizeof(double), MS_MAX, NCCL_F64, NCCL_MAX,
-                            m->comms[g], c->stream);
-    if (e != NCCL_SUCCESS && rcs[g] == TS_OK) rcs[g] = TS_ERR_CUDA;
-    gathered[g].resize((size_t)per * G);
-    red[g].resize(MS_SUM + MS_MAX);
-    cudaMemcpyAsync(gathered[g].data(), dr, b_recv, cudaMemcpyDeviceToHost, c->stream);
-    cudaMemcpyAsync(red[g].data(), dr + b_recv, b_red, cudaMemcpyDeviceToHost, c->stream);
-    if (cudaStreamSynchronize(c->stream) != cudaSuccess && rcs[g] == TS_OK) rcs[g] = TS_ERR_CUDA;
+    return ts_monte_carlo_run(c, &cg, cfg->shared_orbit ? kep6 : skep.data(), cfg->shared_orbit ? fopts : sfo.data(), sx0.data(),
+                              sxf.data(), sJ.data(), q_noise0 ? sq.data() : nullptr, sid.data(), so, ss);
   };
-  std::vector<std::thread> th;
-  for (int g = 0; g < G; ++g) th.emplace_back(worker, g);
-  for (auto& t : th) t.join();
-  for (int g = 0; g < G; ++g)
-    if (rcs[g] != TS_OK) {
-      snprintf(m->err, sizeof(m->err), "device %d: %s", m->dev[g], ts_last_error(m->ctx[g]));
-      return rcs[g];
-    }
-  if (G == 1) {
-    memcpy(out, shard_out[0].data(), (size_t)n * sizeof(ts_trial_outcome));
-    if (stats) *stats = shard_stats[0];
-    return TS_OK;
+  return multi_shards(m, n, shard, out, stats);
+}
+
+int ts_multi_mc_continue(ts_multi* m, int64_t n_trials, const ts_ilqr_opts* opts, ts_trial_outcome* out, ts_mc_stats* stats) {
+  if (!m) return TS_ERR_ARG;
+  if (!opts || !out || n_trials < 0) {
+    snprintf(m->err, sizeof(m->err), "ts_multi_mc_continue: null argument or n_trials < 0");
+    return TS_ERR_ARG;
   }
-  // every rank now holds all records (rank-major, `per` per rank): hand rank 0's copy back in the caller's trial order
-  for (int g = 0; g < G; ++g)
-    for (int64_t a = 0; g + a * G < n; ++a) out[g + a * G] = gathered[0][(size_t)g * per + a];
-  if (stats) stats_unpack(red[0].data(), red[0].data() + MS_SUM, *stats);
-  return TS_OK;
+  if (n_trials == 0) return TS_OK;
+  auto shard = [&](int, ts_ctx* c, int64_t ng, ts_trial_outcome* so, ts_mc_stats* ss) { return ts_mc_continue(c, ng, opts, so, ss); };
+  return multi_shards(m, n_trials, shard, out, stats);
 }
 
 }  // extern "C"

@@ -24,7 +24,7 @@ using namespace ts;
 
 extern "C" {
 
-int ts_version(void) { return 102; }
+int ts_version(void) { return 103; }
 
 int ts_create(ts_ctx** out, int device_id) {
   if (!out) return TS_ERR_ARG;
@@ -777,8 +777,9 @@ static int k3_launch(ts_ctx* c, K3Args& a, const int64_t* N_i_host, const double
   if (sio) {
     TS_CUDA(c, cudaMemcpyAsync((void*)a.sio, sio, sizeof(K3StateIO), cudaMemcpyHostToDevice, c->stream));
     // CS2: every trial's multipliers pass to the output (the continuing trials' rows are then overwritten); queued only
-    // now, so that a call that fails above leaves lam_out as it was
-    if (sio->lam_in)
+    // now, so that a call that fails above leaves lam_out as it was.  A continuation in place (ts_mc_continue) passes
+    // lam_in == lam_out: there is nothing to copy, and an overlapping cudaMemcpyAsync is undefined.
+    if (sio->lam_in && sio->lam_in != sio->lam_out)
       TS_CUDA(c, cudaMemcpyAsync(sio->lam_out, sio->lam_in, (size_t)sio->lam_doubles * sizeof(double), cudaMemcpyDeviceToDevice,
                                  c->stream));
   }
@@ -1080,6 +1081,29 @@ int ts_tvlqr_sim_batch(ts_ctx* c, int64_t n, const int64_t* N_i, const int64_t* 
 // IGRF sample 2393 (2243 + rotations) and TVLQR ~7700 per knot are the SURVEY 8d estimates.
 static const double FL_FIELD = 2393.0, FL_ITER = 10230.0, FL_ROLL = 607.0, FL_ITER_DIAG = 9285.0, FL_ROLL_DIAG = 535.0, FL_TVLQR = 7700.0;
 
+// The counts and sums of ts_mc_stats over an ensemble's outcome records; flops starts at flops0 and adds every
+// record's.  The ms_* fields are left to the caller.
+static void mc_stats_of(const ts_trial_outcome* out, int64_t n, bool run_tvlqr, double flops0, ts_mc_stats* stats) {
+  memset(stats, 0, sizeof(*stats));
+  stats->n_trials = n;
+  stats->flops = flops0;
+  for (int64_t t = 0; t < n; ++t) {
+    const ts_trial_outcome& o = out[t];
+    if (o.status >= 0 && o.status < 6) stats->n_status[o.status]++;
+    if (o.status == TS_ST_NO_CUTOFF) { stats->n_no_cutoff++; continue; }
+    if (o.status == TS_ST_CONVERGED) stats->n_converged++;
+    stats->sum_t_final += o.t_final;
+    stats->sum_inner_iters += o.inner_iters;
+    stats->sum_ls_rollouts += o.ls_rollouts;
+    stats->sum_knots += (double)o.N;
+    stats->flops += o.flops;
+    if (run_tvlqr) {
+      if (o.slew_time == o.t_final) stats->n_fail_slew++;
+      if (o.slew_time > 0.0) { stats->sum_slew_time += o.slew_time; stats->sum_slew_time_sq += o.slew_time * o.slew_time; }
+    }
+  }
+}
+
 int ts_monte_carlo_run(ts_ctx* c, const ts_mc_config* cfg, const double* kep6, const ts_field_opts* fopts, const double* x0,
                        const double* xf, const double* Jmat, const double* q_noise0, const uint32_t* stream_id,
                        ts_trial_outcome* out, ts_mc_stats* stats) {
@@ -1098,6 +1122,7 @@ int ts_monte_carlo_run(ts_ctx* c, const ts_mc_config* cfg, const double* kep6, c
   for (int i = 0; i < 7; ++i) cudaEventCreate(&e[i]);
   struct EvGuard { cudaEvent_t* e; ~EvGuard() { for (int i = 0; i < 7; ++i) cudaEventDestroy(e[i]); } } evg{e};
   c->mc_last.valid = false;
+  c->mc_last.resumable = false;
 
   // ---- stage 1: scoping pass (2*N_scope samples per orbit) + gramian cutoff
   std::vector<ts_field_opts> fo(NF);
@@ -1283,6 +1308,17 @@ int ts_monte_carlo_run(ts_ctx* c, const ts_mc_config* cfg, const double* kep6, c
     ka.X = d_X; ka.U = d_U; ka.K = nullptr; ka.out = d_out;
     std::vector<double> diff(NA);
     for (int64_t aa = 0; aa < na; ++aa) diff[aa] = slew_angle(x0 + 8 * act[aa], xf + 8 * act[aa]);
+    // keep_trajectories = 2: the solve runs the exporting instantiations, its states and multipliers go to a kept slot
+    K3StateIO sio = {};
+    void* p_st = nullptr;
+    const bool resumable = cfg->keep_trajectories == 2;
+    const size_t b_st = NA * sizeof(ts_al_state);
+    if (resumable) {
+      if ((rc = scratch_reserve(c, SLOT_KEPT_STATE, b_st + 64 + (size_t)knots * 6 * 8, &p_st))) return rc;
+      sio.state_out = (ts_al_state_dev*)p_st;
+      sio.lam_out = (double*)((char*)p_st + b_st + 64);
+      ka.sio = (const K3StateIO*)((char*)p_st + b_st);
+    }
     // everything stage 5 needs is reserved and uploaded BEFORE the solve is queued: a cudaMalloc between the two would
     // wait for the solve and put its host latency on the device timeline
     void *p_K = nullptr, *p_xs = nullptr, *p_us = nullptr;
@@ -1299,7 +1335,7 @@ int ts_monte_carlo_run(ts_ctx* c, const ts_mc_config* cfg, const double* kep6, c
         if ((rc = scratch_reserve(c, SLOT_KEPT_USIM, (size_t)knots * 3 * 8 + 64, &p_us))) return rc;
       }
     }
-    if ((rc = k3_launch(c, ka, hi.data(), diff.data(), all_inertia_diagonal(Jmat, n)))) return rc;
+    if ((rc = k3_launch(c, ka, hi.data(), diff.data(), all_inertia_diagonal(Jmat, n), nullptr, resumable ? &sio : nullptr))) return rc;
     cudaEventRecord(e[4], c->stream);
     // ---- stage 5: TVLQR replay + slew-time rule
     double *d_Xs_keep = nullptr, *d_Us_keep = nullptr;
@@ -1359,26 +1395,37 @@ int ts_monte_carlo_run(ts_ctx* c, const ts_mc_config* cfg, const double* kep6, c
       L.d_X = d_X; L.d_U = d_U; L.d_Xs = d_Xs_keep; L.d_Us = d_Us_keep; L.d_B = d_Bf;
       L.valid = true;
     }
+    if (resumable) {
+      ts_ctx::McLast& L = c->mc_last;
+      L.diag_inertia = all_inertia_diagonal(Jmat, n);
+      L.act = act;
+      L.hi = hi;
+      L.hf = hf;
+      L.sid.clear();
+      if (cfg->run_tvlqr)
+        for (int64_t a = 0; a < na; ++a) L.sid.push_back(stream_id ? stream_id[act[a]] : (uint32_t)act[a]);
+      L.d_i = d_i; L.d_f = d_f; L.d_w = d_Qd; L.d_sid = d_sid;
+      L.d_out = (ts_trial_outcome*)d_out;
+      L.d_state = (ts_al_state*)p_st;
+      L.d_sio = (char*)p_st + b_st;
+      L.d_lam = sio.lam_out;
+    }
+  }
+  if (cfg->keep_trajectories == 2) {
+    ts_ctx::McLast& L = c->mc_last;
+    if (na == 0) {   // nothing reached the solver: a run that continues nothing
+      L.act.clear();
+      L.knots = 0;
+      L.knot_offs.assign((size_t)n + 1, 0);
+    }
+    L.n = n;
+    L.cfg = *cfg;
+    L.out.assign(out, out + n);
+    L.resumable = true;
   }
   c->last_kernel_ms = ms_field + ms_prep + ms_solve + ms_tvlqr;
   if (stats) {
-    stats->n_trials = n;
-    stats->flops = field_samples * FL_FIELD;
-    for (int64_t t = 0; t < n; ++t) {
-      const ts_trial_outcome& o = out[t];
-      if (o.status >= 0 && o.status < 6) stats->n_status[o.status]++;
-      if (o.status == TS_ST_NO_CUTOFF) { stats->n_no_cutoff++; continue; }
-      if (o.status == TS_ST_CONVERGED) stats->n_converged++;
-      stats->sum_t_final += o.t_final;
-      stats->sum_inner_iters += o.inner_iters;
-      stats->sum_ls_rollouts += o.ls_rollouts;
-      stats->sum_knots += (double)o.N;
-      stats->flops += o.flops;
-      if (cfg->run_tvlqr) {
-        if (o.slew_time == o.t_final) stats->n_fail_slew++;
-        if (o.slew_time > 0.0) { stats->sum_slew_time += o.slew_time; stats->sum_slew_time_sq += o.slew_time * o.slew_time; }
-      }
-    }
+    mc_stats_of(out, n, cfg->run_tvlqr != 0, field_samples * FL_FIELD, stats);
     stats->ms_field = ms_field; stats->ms_prep = ms_prep; stats->ms_solve = ms_solve; stats->ms_tvlqr = ms_tvlqr;
   }
   return TS_OK;
@@ -1407,6 +1454,170 @@ int ts_mc_fetch_trajectories(ts_ctx* c, double* X, double* U, double* X_sim, dou
   if (U_sim) TS_CUDA(c, cudaMemcpyAsync(U_sim, L.d_Us, K * 3 * 8, cudaMemcpyDeviceToHost, c->stream));
   if (B_eci) TS_CUDA(c, cudaMemcpyAsync(B_eci, L.d_B, (size_t)L.rows * 3 * 8, cudaMemcpyDeviceToHost, c->stream));
   TS_CUDA(c, cudaStreamSynchronize(c->stream));
+  return TS_OK;
+}
+
+int ts_mc_fetch_state(ts_ctx* c, ts_al_state* state, double* lam) {
+  if (!c) return TS_ERR_ARG;
+  const ts_ctx::McLast& L = c->mc_last;
+  if (!L.resumable) return fail(c, TS_ERR_ARG, "no Monte-Carlo run with keep_trajectories = 2 on this context");
+  TS_CUDA(c, cudaSetDevice(c->device));
+  const size_t NA = L.act.size();
+  std::vector<ts_al_state> st(NA);
+  if (state && NA) TS_CUDA(c, cudaMemcpyAsync(st.data(), L.d_state, NA * sizeof(ts_al_state), cudaMemcpyDeviceToHost, c->stream));
+  if (lam && L.knots) TS_CUDA(c, cudaMemcpyAsync(lam, L.d_lam, (size_t)L.knots * 6 * 8, cudaMemcpyDeviceToHost, c->stream));
+  TS_CUDA(c, cudaStreamSynchronize(c->stream));
+  if (state) {
+    memset(state, 0, (size_t)L.n * sizeof(ts_al_state));
+    for (int64_t t = 0; t < L.n; ++t) state[t].status = TS_ST_NO_CUTOFF;
+    for (size_t a = 0; a < NA; ++a) state[L.act[a]] = st[a];
+  }
+  return TS_OK;
+}
+
+// MC1-MC3 (DESIGN.md section 4, K3).  The continuing trials are solved on the kept block in place, exactly as
+// ts_alilqr_solve_state_batch continues them over the run's active trials, and replayed on their own.
+int ts_mc_continue(ts_ctx* c, int64_t n_trials, const ts_ilqr_opts* opts, ts_trial_outcome* out, ts_mc_stats* stats) {
+  if (!c) return TS_ERR_ARG;
+  ts_ctx::McLast& L = c->mc_last;
+  if (!L.resumable) return fail(c, TS_ERR_ARG, "ts_mc_continue: no Monte-Carlo run with keep_trajectories = 2 on this context");
+  if (n_trials != L.n) return fail(c, TS_ERR_ARG, "ts_mc_continue: the kept run had %lld trials", (long long)L.n);
+  if (!opts || !out) return fail(c, TS_ERR_ARG, "ts_mc_continue: null argument");
+  const ts_ilqr_opts& o = *opts;
+  if (o.max_linesearch < 0 || o.max_linesearch > 63) return fail(c, TS_ERR_ARG, "max_linesearch must be in [0,63]");
+  const int64_t na = (int64_t)L.act.size();
+  const size_t NA = (size_t)na;
+  const ts_mc_config& cfg = L.cfg;
+  TS_CUDA(c, cudaSetDevice(c->device));
+  if (o.quat_error && na > 0) {   // the check of ts_alilqr_solve_state_batch, on the run's weights
+    std::vector<double> w(16 * NA);
+    TS_CUDA(c, cudaMemcpy(w.data(), L.d_w, w.size() * 8, cudaMemcpyDeviceToHost));
+    for (size_t k = 0; k < 2 * NA; ++k)
+      for (int i = 4; i < 7; ++i)
+        if (w[8 * k + i] != w[8 * k + 3])
+          return fail(c, TS_ERR_ARG, "quat_error: the four quaternion weights of Q and Qf must be equal (E'QE is then diagonal)");
+  }
+  // MC1: CS2 on the kept states (their status and outer count are the kept records')
+  std::vector<int64_t> cont;
+  for (int64_t a = 0; a < na; ++a) {
+    const ts_trial_outcome& r = L.out[(size_t)L.act[(size_t)a]];
+    if (r.status == TS_ST_MAX_OUTER && r.outer_iters < o.max_outer) cont.push_back(a);
+  }
+  const size_t NC = cont.size();
+  double ms_solve = 0.0, ms_tvlqr = 0.0, flops = 0.0;
+  std::vector<ts_trial_outcome> rec = L.out;
+  if (NC == 0) c->k3_timed = false;   // no solve: ts_k3_last_split / ts_k3_last_parked report nothing
+  if (NC > 0) {
+    const int64_t* hi = L.hi.data();
+    const double* hf = L.hf.data();
+    int rc;
+    // MC3: the replay's per-trial arrays, compacted to the continuing trials in the packed layouts of the run; the knot
+    // and row offsets keep pointing into the full kept arrays
+    std::vector<int64_t> hic(4 * NC + 1);
+    std::vector<double> hfc(40 * NC);
+    for (size_t k = 0; k < NC; ++k) {
+      const size_t a = (size_t)cont[k];
+      for (int j = 0; j < 4; ++j) hic[j * NC + k] = hi[j * NA + a];
+      static const int width[] = {8, 8, 9, 1, 1, 1, 8, 4};   // x0 xf Jmat t_final index_scale clock_rate x0_lqr q_final
+      size_t base = 0;
+      for (int w : width) {
+        memcpy(&hfc[base * NC + w * k], &hf[base * NA + w * a], (size_t)w * 8);
+        base += (size_t)w;
+      }
+    }
+    hic[4 * NC] = L.knots;
+    void *p_q = nullptr, *p_K = nullptr;
+    int64_t* d_ic = nullptr;
+    double* d_fc = nullptr;
+    K4Args k4;
+    if (cfg.run_tvlqr) {
+      if ((rc = upload(c, SLOT_ARGS_A, hic.data(), hic.size(), &d_ic))) return rc;
+      if ((rc = upload(c, SLOT_ARGS_B, hfc.data(), hfc.size(), &d_fc))) return rc;
+      if ((rc = scratch_reserve(c, SLOT_ARGS_C, NC * 20 + 64, &p_q))) return rc;
+      std::vector<uint32_t> sidc(NC);
+      for (size_t k = 0; k < NC; ++k) sidc[k] = L.sid[(size_t)cont[k]];
+      TS_CUDA(c, cudaMemcpyAsync(p_q, sidc.data(), NC * 4, cudaMemcpyHostToDevice, c->stream));
+      if ((rc = scratch_reserve(c, SLOT_K4_GAINS, (size_t)L.knots * 18 * 8, &p_K))) return rc;
+      if ((rc = k4_lin_table(c, hic.data(), NC, k4))) return rc;
+    }
+    // MC2: the K3 arguments of the run, on the kept block; the states and multipliers are read and written in place
+    K3Args ka = {};
+    ka.n_trials = na;
+    ka.N_i = L.d_i; ka.offs = L.d_i + NA; ka.B_offs = L.d_i + 2 * NA; ka.B_rows = L.d_i + 3 * NA;
+    ka.x0 = L.d_f; ka.xf = L.d_f + 8 * NA; ka.Jmat = L.d_f + 16 * NA;
+    ka.Qd = L.d_w; ka.Qfd = L.d_w + 8 * NA; ka.Rd = L.d_w + 16 * NA;
+    ka.index_scale = L.d_f + 26 * NA; ka.clock_rate = L.d_f + 27 * NA;
+    ka.B_eci = L.d_B; ka.dt = cfg.dt; ka.U0 = nullptr;
+    memcpy(&ka.opts, &o, sizeof(ka.opts));
+    ka.X = L.d_X; ka.U = L.d_U; ka.K = nullptr; ka.out = (ts_trial_outcome_dev*)L.d_out;
+    ka.sio = (const K3StateIO*)L.d_sio;
+    K3StateIO sio = {};
+    sio.state_in = sio.state_out = (ts_al_state_dev*)L.d_state;
+    sio.lam_in = sio.lam_out = L.d_lam;
+    sio.lam_doubles = L.knots * 6;
+    std::vector<double> diff(NA);
+    for (size_t a = 0; a < NA; ++a) diff[a] = slew_angle(hf + 8 * a, hf + 8 * NA + 8 * a);
+    cudaEvent_t e[3];
+    for (int i = 0; i < 3; ++i) cudaEventCreate(&e[i]);
+    struct EvGuard { cudaEvent_t* e; ~EvGuard() { for (int i = 0; i < 3; ++i) cudaEventDestroy(e[i]); } } evg{e};
+    cudaEventRecord(e[0], c->stream);
+    // X, U, the states and lam are input and output of the same call.  That is safe because park_import_kernel, the
+    // first kernel k3_launch queues for a continuation, reads every imported row (X, U, lam_in, state_in) before the
+    // straggler kernel that follows it on the stream writes any.  k3_launch fails before it queues anything that writes
+    // kept storage (TS_ERR_NOMEM when the parked records do not fit), so the kept run stays continuable.
+    if ((rc = k3_launch(c, ka, hi, diff.data(), L.diag_inertia, &cont, &sio))) return rc;
+    cudaEventRecord(e[1], c->stream);
+    if (cfg.run_tvlqr) {
+      k4_clear_rows_kernel<<<(unsigned)NC, 256, 0, c->stream>>>((int64_t)NC, d_ic, d_ic + NC, L.d_Xs, L.d_Us);
+      c->launches++;
+      k4.n_trials = (int64_t)NC; k4.N_i = d_ic; k4.offs = d_ic + NC; k4.B_offs = d_ic + 2 * NC; k4.B_rows = d_ic + 3 * NC;
+      k4.X_lqr = L.d_X; k4.U_lqr = L.d_U; k4.x0_lqr = d_fc + 28 * NC; k4.Jmat = d_fc + 16 * NC; k4.B_eci = L.d_B;
+      k4.index_scale = d_fc + 26 * NC; k4.clock_rate = d_fc + 27 * NC; k4.t_final = d_fc + 25 * NC; k4.q_final = d_fc + 36 * NC;
+      k4.stream_id = (const uint32_t*)p_q;
+      memcpy(&k4.opts, &cfg.tvlqr, sizeof(k4.opts));   // with the fused run's overrides
+      k4.opts.dt = cfg.dt; k4.opts.t0 = cfg.t0;
+      if (k4.opts.noise_mode == 1) k4.opts.noise_mode = 2;
+      k4.opts.literal_postproc = 0;
+      k4.noise = nullptr; k4.dX = nullptr; k4.K = (double*)p_K;
+      k4.X_sim = L.d_Xs; k4.U_sim = L.d_Us;
+      k4.N_sim = (int64_t*)((char*)p_q + ((NC * 4 + 15) & ~(size_t)15));
+      k4.slew_time = (double*)(k4.N_sim + NC);
+      k4_launch(c, k4);
+    }
+    cudaEventRecord(e[2], c->stream);
+    TS_CUDA(c, cudaGetLastError());
+    std::vector<ts_trial_outcome> oa(NA);
+    std::vector<double> slew(NC, 0.0);
+    TS_CUDA(c, cudaMemcpyAsync(oa.data(), L.d_out, NA * sizeof(ts_trial_outcome), cudaMemcpyDeviceToHost, c->stream));
+    if (cfg.run_tvlqr) TS_CUDA(c, cudaMemcpyAsync(slew.data(), k4.slew_time, NC * 8, cudaMemcpyDeviceToHost, c->stream));
+    TS_CUDA(c, cudaStreamSynchronize(c->stream));
+    float ms = 0;
+    cudaEventElapsedTime(&ms, e[0], e[1]); ms_solve = ms;
+    if (cfg.run_tvlqr) { cudaEventElapsedTime(&ms, e[1], e[2]); ms_tvlqr = ms; }
+    const bool dj_ = L.diag_inertia && !o.k3_generic_inertia;
+    const double fl_iter = dj_ ? FL_ITER_DIAG : FL_ITER, fl_roll = dj_ ? FL_ROLL_DIAG : FL_ROLL;
+    for (size_t k = 0; k < NC; ++k) {
+      const int64_t t = L.act[(size_t)cont[k]];
+      const ts_trial_outcome& prev = L.out[(size_t)t];
+      ts_trial_outcome r = oa[(size_t)cont[k]];
+      const double kn = (double)(prev.N - 1);
+      r.N = prev.N;
+      r.t_final = prev.t_final;
+      r.slew_time = cfg.run_tvlqr ? slew[k] : 0.0;
+      r.flops = kn * ((double)r.inner_iters * fl_iter + (double)r.ls_rollouts * fl_roll) + (cfg.run_tvlqr ? kn * FL_TVLQR : 0.0);
+      flops += kn * ((double)(r.inner_iters - prev.inner_iters) * fl_iter + (double)(r.ls_rollouts - prev.ls_rollouts) * fl_roll) +
+               (cfg.run_tvlqr ? kn * FL_TVLQR : 0.0);
+      rec[(size_t)t] = r;
+    }
+    L.out = rec;
+  }
+  c->last_kernel_ms = ms_solve + ms_tvlqr;
+  memcpy(out, rec.data(), (size_t)L.n * sizeof(ts_trial_outcome));
+  if (stats) {
+    mc_stats_of(out, L.n, cfg.run_tvlqr != 0, 0.0, stats);
+    stats->flops = flops;
+    stats->ms_solve = ms_solve; stats->ms_tvlqr = ms_tvlqr;
+  }
   return TS_OK;
 }
 

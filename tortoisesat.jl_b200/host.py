@@ -156,6 +156,8 @@ def load_library():
     L.ts_fp64_latency_probe.argtypes = [C.c_void_p, c_double_p]
     L.ts_mc_trajectory_layout.argtypes = [C.c_void_p, C.c_int64, C.c_void_p, C.c_void_p]
     L.ts_mc_fetch_trajectories.argtypes = [C.c_void_p] + [C.c_void_p] * 5
+    L.ts_mc_fetch_state.argtypes = [C.c_void_p, C.c_void_p, C.c_void_p]
+    L.ts_mc_continue.argtypes = [C.c_void_p, C.c_int64, C.POINTER(IlqrOpts), C.c_void_p, C.POINTER(McStats)]
     L.ts_igrf12syn_batch.argtypes = [C.c_void_p, C.c_int, C.c_double, C.c_int, C.c_int64] + [C.c_void_p] * 7 + [C.c_int]
     L.ts_psiaki_pd_batch.argtypes = [C.c_void_p, C.c_int64] + [C.c_void_p] * 7 + [C.c_double] * 3 + [C.c_void_p] * 3
     L.ts_attitude_dynamics_linear_batch.argtypes = [C.c_void_p, C.c_int64] + [C.c_void_p] * 6
@@ -168,6 +170,7 @@ def load_library():
     L.ts_multi_ctx.argtypes = [C.c_void_p, C.c_int]
     L.ts_multi_ctx.restype = C.c_void_p
     L.ts_multi_monte_carlo_run.argtypes = [C.c_void_p, C.POINTER(McConfig)] + [C.c_void_p] * 8 + [C.POINTER(McStats)]
+    L.ts_multi_mc_continue.argtypes = [C.c_void_p, C.c_int64, C.POINTER(IlqrOpts), C.c_void_p, C.POINTER(McStats)]
     L.ts_igrf12_batch.argtypes = [C.c_void_p, C.c_double, C.c_int64] + [C.c_void_p] * 6 + [C.c_int]
     L.ts_field_map_prefilter.argtypes = [C.c_void_p, C.c_int64, C.c_int64, C.c_void_p, C.c_void_p, C.c_int]
     L.ts_field_map_eval_batch.argtypes = [C.c_void_p, C.c_int64, C.c_int64, C.c_void_p, C.c_int64] + [C.c_void_p] * 3 + [C.c_int]
@@ -637,6 +640,28 @@ class Engine:
         self._check(self.lib.ts_mc_fetch_trajectories(self.h, g("X"), g("U"), g("X_sim"), g("U_sim"), g("B_eci")))
         return res
 
+    def mc_state(self, n_trials):
+        """The kept solver state of the last monte_carlo_run with cfg.keep_trajectories = 2 (ts_mc_fetch_state): (state,
+        lam), state as AL_STATE_DTYPE records (a NO_CUTOFF trial: zero record with status 5), lam (sum N, 6) ragged by the
+        knot_offs of mc_trajectories."""
+        n = int(n_trials)
+        ko = np.zeros(n + 1, dtype=np.int64)
+        self._check(self.lib.ts_mc_trajectory_layout(self.h, n, _ptr(ko), None))
+        state = np.zeros(n, dtype=AL_STATE_DTYPE)
+        lam = np.zeros((int(ko[-1]), 6))
+        self._check(self.lib.ts_mc_fetch_state(self.h, state.ctypes.data, _ptr(lam)))
+        return state, lam
+
+    def mc_continue(self, n_trials, opts):
+        """Continues the max-outer trials of the last monte_carlo_run with cfg.keep_trajectories = 2 under `opts` (an
+        IlqrOpts with a larger max_outer; rules MC1-MC4 of ts_mc_continue).  Returns (out, stats) for the whole ensemble;
+        the kept run is updated in place, so mc_trajectories / mc_state return the continued run."""
+        n = int(n_trials)
+        out = np.zeros(n, dtype=OUTCOME_DTYPE)
+        st = McStats()
+        self._check(self.lib.ts_mc_continue(self.h, n, C.byref(opts), out.ctypes.data, C.byref(st)))
+        return out, st
+
     def igrf12syn_batch(self, isv, date, itype, alt, colat, elong):
         """igrf12syn (igrf.jl:335-534) at n points: alt km, colat/elong degrees -> x, y, z, f (nT)."""
         alt, colat, elong = _f64(np.atleast_1d(alt)), _f64(np.atleast_1d(colat)), _f64(np.atleast_1d(elong))
@@ -711,6 +736,17 @@ class MultiEngine:
         rc = self.lib.ts_multi_monte_carlo_run(self.h, C.byref(cfg), _ptr(kep6), fopts.ctypes.data, _ptr(x0), _ptr(xf), _ptr(Jmat),
                                                None if qn is None else _ptr(qn), None if sid is None else _ptr(sid),
                                                out.ctypes.data, C.byref(st))
+        if rc != 0:
+            raise TortoiseError(rc, (self.lib.ts_multi_last_error(self.h) or b"").decode())
+        return out, st
+
+    def mc_continue(self, n_trials, opts):
+        """Engine.mc_continue on every device's kept shard, records gathered and statistics reduced as after the run.
+        (With one process per GPU, each rank calls Engine.mc_continue and then parallel.gather_outcomes / reduce_stats.)"""
+        n = int(n_trials)
+        out = np.zeros(n, dtype=OUTCOME_DTYPE)
+        st = McStats()
+        rc = self.lib.ts_multi_mc_continue(self.h, n, C.byref(opts), out.ctypes.data, C.byref(st))
         if rc != 0:
             raise TortoiseError(rc, (self.lib.ts_multi_last_error(self.h) or b"").decode())
         return out, st
@@ -1010,7 +1046,7 @@ def attitude_simulation(f, f_gains, integration, X_lqr, U_lqr, dt_lqr, x0_lqr, t
 def monte_carlo(number_sims=100, alt=400.0, R_E=6371.0, inclination=96.6, MJD_0=58155.0, igrf_date=2019.0, t0=0.0, tf=60 * 40.0,
                 cutoff=30.0, N=5000, J=None, q_0=None, q_final=(np.sqrt(2) / 2, np.sqrt(2) / 2, 0.0, 0.0), alpha=1.0e-1, beta=1.0e3,
                 seed=0, run_tvlqr=True, ilqr=None, rng=None, random_attitudes=False, trajectories=True, eigen_axis_fix=False,
-                sat_att=False):
+                sat_att=False, resumable=False):
     """The loop of monte_carlo.jl:118-262 (solver block of TortoiseSat.jl:178-199) for number_sims trials in ONE
     library call.  Returns the arrays the script leaves in globals (monte_carlo.jl:52-66,237-240): A (number_sims x 6),
     t_final, slew_time, fails, and -- with trajectories=True -- the per-trial lists `states` (8 x N_i), `control_inputs`
@@ -1020,7 +1056,9 @@ def monte_carlo(number_sims=100, alt=400.0, R_E=6371.0, inclination=96.6, MJD_0=
     draws q_0 uniformly on S^3 -- the BASELINE configs[2] ensemble; initial attitude noise randn(3)*(pi/180)^2), from
     numpy's generator instead of Julia's global RNG.  sat_att=True selects the quaternion-aware solver the script asks of
     its forked TrajectoryOptimization (monte_carlo.jl:158 Model(DerivFunction, n, m, quaternion_error,
-    quaternion_expansion), :192 solver.opts.sat_att = true): ts_ilqr_opts.quat_error."""
+    quaternion_expansion), :192 solver.opts.sat_att = true): ts_ilqr_opts.quat_error.  resumable=True keeps the solver
+    state on the default engine (keep_trajectories = 2) so that continue_monte_carlo can give the max-outer trials more
+    outer iterations; the result then also holds the run's solver options as `ilqr`."""
     rng = np.random.default_rng(seed) if rng is None else rng
     n = int(number_sims)
     J = np.diag([0.00125, 0.00125, 0.00125]) if J is None else np.asarray(J, dtype=float)
@@ -1050,11 +1088,13 @@ def monte_carlo(number_sims=100, alt=400.0, R_E=6371.0, inclination=96.6, MJD_0=
         cfg.tvlqr.Qd[i], cfg.tvlqr.Qfd[i] = 10.0, 1000.0
     for i in range(3):
         cfg.tvlqr.Rd[i] = 0.5e3
-    cfg.eigen_axis_fix, cfg.keep_trajectories = int(bool(eigen_axis_fix)), int(bool(trajectories))
+    cfg.eigen_axis_fix, cfg.keep_trajectories = int(bool(eigen_axis_fix)), 2 if resumable else int(bool(trajectories))
     eng = default_engine()
     out, st = eng.monte_carlo_run(cfg, A, fo, x0, xf, np.tile(J.reshape(-1), (n, 1)), q_noise0=qn)
     fails = (out["slew_time"] == out["t_final"]).astype(float)     # monte_carlo.jl:257-261
     res = dict(A=A, t_final=out["t_final"].copy(), slew_time=out["slew_time"].copy(), fails=fails, outcomes=out, stats=st)
+    if resumable:
+        res["ilqr"] = IlqrOpts.from_buffer_copy(cfg.ilqr)
     if trajectories:
         tr = eng.mc_trajectories(n, want=("X", "U", "X_sim", "U_sim", "B_eci") if run_tvlqr else ("X", "U", "B_eci"))
         ko, ro = tr["knot_offs"], tr["row_offs"]
@@ -1067,6 +1107,38 @@ def monte_carlo(number_sims=100, alt=400.0, R_E=6371.0, inclination=96.6, MJD_0=
             res["sim_states"] = [sl(tr["X_sim"], t) for t in range(n)]           # :232
             res["sim_control_inputs"] = [sl(tr["U_sim"], t) for t in range(n)]   # :233
     return res
+
+
+def continue_monte_carlo(res, max_outer=30, ilqr=None):
+    """Gives the trials of a monte_carlo(..., resumable=True) result that ended at max_outer more outer iterations, up to
+    `max_outer` in all (ts_mc_continue on the default engine, which must not have run another Monte-Carlo call since),
+    and updates `res` in place as retry_failed does: outcomes, slew_time, fails (monte_carlo.jl:257-261) and the trajectory
+    lists of the continued trials.  `ilqr` (default: the run's options) supplies the other solver options.  Returns the
+    0-based indices of the continued trials."""
+    if "ilqr" not in res:
+        raise ValueError("continue_monte_carlo needs a monte_carlo(..., resumable=True) result")
+    o = IlqrOpts.from_buffer_copy(res["ilqr"] if ilqr is None else ilqr)
+    o.max_outer = int(max_outer)
+    prev = res["outcomes"]
+    n = prev.shape[0]
+    idx = np.nonzero((prev["status"] == 1) & (prev["outer_iters"] < o.max_outer))[0]   # MC1
+    eng = default_engine()
+    out, st = eng.mc_continue(n, o)
+    res["outcomes"], res["stats"], res["ilqr"] = out, st, o
+    res["slew_time"] = out["slew_time"].copy()
+    res["fails"] = (out["slew_time"] == out["t_final"]).astype(float)
+    if idx.size and "states" in res:
+        run_tvlqr = "sim_states" in res
+        tr = eng.mc_trajectories(n, want=("X", "U", "X_sim", "U_sim") if run_tvlqr else ("X", "U"))
+        ko = tr["knot_offs"]
+        sl = lambda a, t, last=0: a[ko[t]:ko[t + 1] - last].T.copy()
+        for t in idx:
+            res["states"][t] = sl(tr["X"], t)
+            res["control_inputs"][t] = sl(tr["U"], t, 1)
+            if run_tvlqr:
+                res["sim_states"][t] = sl(tr["X_sim"], t)
+                res["sim_control_inputs"][t] = sl(tr["U_sim"], t)
+    return idx
 
 
 # ---------------------------------------------------------------------------
