@@ -387,6 +387,40 @@ int ts_mc_fetch_trajectories(ts_ctx* ctx, double* X, double* U, double* X_sim, d
 int ts_mc_fetch_state(ts_ctx* ctx, ts_al_state* state, double* lam);
 int ts_mc_continue(ts_ctx* ctx, int64_t n_trials, const ts_ilqr_opts* opts, ts_trial_outcome* out, ts_mc_stats* stats);
 
+/* ---- disturbance ensembles: the kept run's slews under many independent noise draws ------------------------- *
+ * ts_mc_replay_ensemble replays every selected trial of the kept run n_real times, each time under an independent draw
+ * of the simulator.jl disturbances, with the trial's kept optimised trajectory and its TVLQR gains (computed once per
+ * call), and returns the slew time and final state of every (trial, realisation) pair (DESIGN.md section 4, K4):
+ *  RE1 the kept run: the most recent ts_monte_carlo_run on ctx with keep_trajectories >= 1, continued by
+ *      ts_mc_continue or not (after a continuation the continued trajectories are replayed).
+ *  RE2 the draws of realisation r (0 <= r < 2^30), key = the run's tvlqr.seed, stream = the trial's stream id: the stage
+ *      disturbances of step k, stage s are tvlqr_noise's with counter (stream, k, s, block + 4r), block 0..2 (r = 0 is
+ *      the run's own stream); realisation r >= 1 starts from the trial's unperturbed x0 perturbed, as ts_monte_carlo_run
+ *      applies q_noise0, by q_noise = q_noise_scale * (z0, z1, z2), (z0, z1) = box_muller(o0, o1), z2 = the first of
+ *      box_muller(o2, o3), o = Philox4x32-10 of counter (stream, 0xFFFFFFFF, 0, 4r) (q_noise_scale = 0: x0 itself);
+ *      realisation 0 starts from the run's x0_lqr.  Realisations always draw (noise mode 2), whatever the run's
+ *      noise_mode; the run's TVLQR options apply with the fused path's overrides (dt, t0, literal_postproc = 0).
+ *  RE3 realisation 0 is the run: when the run drew noise (noise_mode 1 or 2), realisation 0 of a trial has the kept
+ *      record's slew_time and the kept X_sim row N_sim - 1 as x_final, bit for bit.
+ *  RE4 row (trial t, realisation r) depends on the kept run, t, r and q_noise_scale alone, bit for bit: not on r_first
+ *      or n_real (chunking), the other selected trials or their order, or the number of devices.
+ *  RE5 isolation: nothing a later call reads is written; the kept run (records, trajectories, states) is unchanged.
+ * trials (HOST, caller indices, repeats allowed; null = all n_trials, then n_sel == n_trials).  HOST outputs: slew_time
+ * (n_sel x n_real, == t_final when the realisation "fails", monte_carlo.jl:257-261), x_final (n_sel x n_real x 8,
+ * nullable): the state at the last simulated step.  A TS_ST_NO_CUTOFF trial gets NaN rows.  ts_last_kernel_ms is the
+ * device time of the call (gains + ensemble replay); ts_mc_replay_ensemble_last_split gives the two parts.
+ * TS_ERR_ARG, outputs untouched: no kept run, n_trials differs from the kept run's, n_real < 1, r_first < 0,
+ * r_first + n_real > 2^30, a trial index out of range, opts or slew_time null.  TS_ERR_NOMEM, outputs untouched, when
+ * the device outputs do not fit: chunk the realisations with r_first (RE4 makes that exact).                          */
+typedef struct ts_replay_ensemble_opts {
+  int64_t n_real;        /* realisations per selected trial, >= 1                     */
+  int64_t r_first;       /* first realisation index; r_first + n_real <= 2^30         */
+  double  q_noise_scale; /* initial attitude perturbation of realisations r >= 1 (RE2) */
+} ts_replay_ensemble_opts;
+int ts_mc_replay_ensemble(ts_ctx* ctx, int64_t n_trials, const ts_replay_ensemble_opts* opts, int64_t n_sel,
+                          const int64_t* trials, double* slew_time, double* x_final);
+int ts_mc_replay_ensemble_last_split(ts_ctx* ctx, double* gains_ms, double* replay_ms);
+
 /* ---- igrf12syn: the Fortran-style twin of igrf12 -------------------------------------------- *
  * igrf12syn(isv, date, itype, alt, colat, elong) [src/igrf.jl:335-534] at n points.  isv 0 = main field, 1 = secular
  * variation; itype 1 = geodetic (alt = height above the WGS-84 ellipsoid, km), 2 = geocentric (alt = radius, km);
@@ -427,6 +461,12 @@ int ts_multi_monte_carlo_run(ts_multi* m, const ts_mc_config* cfg, const double*
  * records gathered and the statistics reduced as after the run.  (Per-process multi-GPU needs no library call: each
  * rank continues its own context and gathers as after its run.)                                                     */
 int ts_multi_mc_continue(ts_multi* m, int64_t n_trials, const ts_ilqr_opts* opts, ts_trial_outcome* out, ts_mc_stats* stats);
+/* ts_mc_replay_ensemble over a ts_multi_monte_carlo_run kept with keep_trajectories >= 1: each selected trial is replayed
+ * on the device that holds it (t mod n_devices), all devices at once, and the rows come back in the caller's order,
+ * equal bit for bit to the single-device rows (RE4).  No collective is needed; per-process multi-GPU needs no library
+ * call (each rank replays the trials of its own context).  ts_last_kernel_ms of device i's context is its own part.    */
+int ts_multi_mc_replay_ensemble(ts_multi* m, int64_t n_trials, const ts_replay_ensemble_opts* opts, int64_t n_sel,
+                                const int64_t* trials, double* slew_time, double* x_final);
 
 /* ---- element-wise batch versions of the reference's building blocks (all HOST pointers) --- *
  * Correctness / drop-in paths for callers that use the small functions on their own; the fused

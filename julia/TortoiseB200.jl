@@ -75,6 +75,9 @@ struct McStats              # ts_mc_stats
     ms_field::Float64; ms_prep::Float64; ms_solve::Float64; ms_tvlqr::Float64
     n_status::NTuple{6,Int64}          # trials per TS_ST_* code
 end
+struct ReplayEnsembleOpts   # ts_replay_ensemble_opts
+    n_real::Int64; r_first::Int64; q_noise_scale::Float64
+end
 function default_ilqr_opts()
     r = Ref{IlqrOpts}()
     ccall((:ts_ilqr_default_opts, LIB), Cvoid, (Ref{IlqrOpts},), r); r[]
@@ -395,6 +398,37 @@ function mc_continue(number_sims::Integer, ilqr::IlqrOpts; e::Engine = engine())
     return out, st[]
 end
 
+# ts_mc_replay_ensemble: the kept run's slews (last monte_carlo with trajectories or resumable on `e`) replayed under
+# n_real independent disturbance draws each, realisations r_first .. r_first + n_real - 1 (rules RE1-RE5, DESIGN.md
+# section 4).  trials: 1-based indices (repeats allowed; nothing = all).  Returns slew_time (n_real x n_sel) and, with
+# want_x_final, x_final (8 x n_real x n_sel); a NO_CUTOFF trial gets NaN columns.
+function mc_replay_ensemble(number_sims::Integer, n_real::Integer; r_first::Integer = 0, trials = nothing,
+                            q_noise_scale::Float64 = (pi / 180)^2, want_x_final::Bool = false, e::Engine = engine())
+    sel = trials === nothing ? C_NULL : Int64[t - 1 for t in trials]
+    ns = trials === nothing ? number_sims : length(trials)
+    slew = zeros(n_real, ns); xf = want_x_final ? zeros(8, n_real, ns) : nothing
+    o = ReplayEnsembleOpts(n_real, r_first, q_noise_scale)
+    check(e, ccall((:ts_mc_replay_ensemble, LIB), Cint,
+                   (Ptr{Cvoid}, Int64, Ref{ReplayEnsembleOpts}, Int64, Ptr{Int64}, Ptr{Float64}, Ptr{Float64}),
+                   e.h, number_sims, Ref(o), ns, sel, slew, xf === nothing ? C_NULL : xf))
+    return slew, xf
+end
+
+# The slew-time distribution of a monte_carlo result's optimised slews under the disturbances: slew_time (n_real x n_sel),
+# fails (slew_time == t_final), fail_rate, slew_mean / slew_std over the non-failing draws, trials (1-based).
+function replay_ensemble(res; n_real::Integer = 100, trials = nothing, r_first::Integer = 0, q_noise_scale::Float64 = (pi / 180)^2,
+                         e::Engine = engine())
+    n = length(res.outcomes)
+    sel = trials === nothing ? collect(1:n) : collect(trials)
+    slew, _ = mc_replay_ensemble(n, n_real; r_first = r_first, trials = sel, q_noise_scale = q_noise_scale, e = e)
+    fails = slew .== reshape([res.outcomes[t].t_final for t in sel], 1, :)
+    fail_rate = [all(isnan, slew[:, k]) ? NaN : sum(fails[:, k]) / count(!isnan, slew[:, k]) for k in eachindex(sel)]
+    ok(k) = [slew[i, k] for i in 1:n_real if !isnan(slew[i, k]) && !fails[i, k]]
+    mean_ = [isempty(ok(k)) ? NaN : sum(ok(k)) / length(ok(k)) for k in eachindex(sel)]
+    std_ = [isempty(ok(k)) ? NaN : sqrt(sum((ok(k) .- mean_[k]) .^ 2) / length(ok(k))) for k in eachindex(sel)]
+    return (slew_time = slew, fails = fails, fail_rate = fail_rate, slew_mean = mean_, slew_std = std_, trials = sel)
+end
+
 # Continues a monte_carlo(...; resumable = true) result `res` in place to max_outer outer iterations in all: outcomes,
 # slew_time, fails (monte_carlo.jl:257-261) and the trajectory arrays of the continued trials.  Returns their indices.
 function continue_monte_carlo!(res; max_outer = 30, ilqr::Union{Nothing,IlqrOpts} = nothing, e::Engine = engine())
@@ -516,6 +550,6 @@ export Engine, params, input_parameters, igrf12, igrf12_batch, igrf_data, magnet
        legendre, dlegendre, DerivFunction, gain_simulator, attitude_dynamics,
        condition_based_time, eigen_axis_slew, bryson_weights, solve_slew, attitude_simulation, monte_carlo, qmult, qrot, q_inv, hat,
        igrf12syn, attitude_dynamics_linear, psiaki_pd_simulation, igrf_interpolant, field_map_prefilter, field_map_eval, AlState,
-       mc_state, mc_continue, continue_monte_carlo!
+       mc_state, mc_continue, continue_monte_carlo!, ReplayEnsembleOpts, mc_replay_ensemble, replay_ensemble
 
 end # module

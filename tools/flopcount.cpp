@@ -56,6 +56,7 @@ CD_ONLY inline CD floor(const T& a) { return CD(::floor(a.v)); }
 CD_ONLY inline CD sin(const T& a) { return CD(::sin(a.v)); }
 CD_ONLY inline CD cos(const T& a) { return CD(::cos(a.v)); }
 CD_ONLY inline CD acos(const T& a) { return CD(::acos(a.v)); }
+CD_ONLY inline CD log(const T& a) { return CD(::log(a.v)); }
 inline CD fmax(const CD& a, const CD& b) { ++g_cnt.cmp; return CD(::fmax(a.v, b.v)); }
 inline CD fmin(const CD& a, const CD& b) { ++g_cnt.cmp; return CD(::fmin(a.v, b.v)); }
 namespace std {
@@ -64,6 +65,7 @@ inline CD fabs(const CD& a) { return CD(::fabs(a.v)); }
 inline CD floor(const CD& a) { return CD(::floor(a.v)); }
 inline CD sin(const CD& a) { return CD(::sin(a.v)); }
 inline CD cos(const CD& a) { return CD(::cos(a.v)); }
+inline CD log(const CD& a) { return CD(::log(a.v)); }
 inline CD max(const CD& a, const CD& b) { ++g_cnt.cmp; return a.v < b.v ? b : a; }
 inline CD min(const CD& a, const CD& b) { ++g_cnt.cmp; return b.v < a.v ? b : a; }
 }  // namespace std
@@ -73,6 +75,7 @@ inline CD min(const CD& a, const CD& b) { ++g_cnt.cmp; return b.v < a.v ? b : a;
 #define volatile
 #include "orc_ilqr.hpp"          // (a) the oracle: literal reference algorithm
 #include "ilqr_solver.cuh"       // (b) the kernels' lane-local math (host build)
+#include "tvlqr_solver.cuh"      // (c) the TVLQR replay step with its inline draws (the disturbance ensemble, K4e)
 #undef volatile
 #undef double
 
@@ -218,5 +221,36 @@ int main() {
          "\"oracle_per_knot_iteration\": %.0f, \"oracle_per_rollout_knot\": %.0f, \"oracle_jacobians\": %.0f, \"oracle_backward\": %.0f}\n",
          k_iter, k_rollf, k_iter_d, k_rollf_d, k_lin.flops(), k_lin_d.flops(), k_grad.flops(), k_ric.flops(), k_gradm, orc_iter, orc_roll,
          c_jac.flops() / K, c_bwd.flops() / K);
+  // (c) one step of the replay with inline draws, as K4e runs it per lane: feedback, four stage records (Philox +
+  // Box-Muller draws, perturbation quaternion, field row) and the rk4 step of the simulator.  Counted as the difference
+  // of two replays of 65 and 33 knots over the 32 extra steps; log / sin / cos calls are not FLOPs in this count.
+  auto replay = [&](int n) {
+    std::vector<CD> Xr(8 * n), Ur(3 * n), Kr(18 * n);
+    for (int k = 0; k < n; ++k) for (int i = 0; i < 8; ++i) Xr[k * 8 + i] = CD(x0[i]);
+    for (int i = 0; i < 18 * n; ++i) Kr[i] = CD(0.01);
+    ts::TvlqrIn ti;
+    ti.N = n; ti.X_lqr = Xr.data(); ti.U_lqr = Ur.data();
+    for (int i = 0; i < 8; ++i) ti.x0[i] = CD(x0[i]);
+    for (int i = 0; i < 9; ++i) { ti.I.J[i] = p.dyn.J[i]; ti.I.Jinv[i] = p.dyn.Jinv[i]; }
+    ti.Bt = Bt.data(); ti.B_rows = 4 * N; ti.index_scale = CD((double)N); ti.clock_rate = CD(1.0 / 2400.0);
+    ti.noise = nullptr; ti.trial = 3; ti.real = 5;
+    for (int i = 0; i < 4; ++i) ti.q_final[i] = CD(xf[3 + i]);
+    ti.t_final = CD(0.2 * (n - 1)); ti.time_step = CD(0.2); ti.trial_index_1based = 4;
+    ts_tvlqr_opts_dev to = {};
+    to.dt = CD(0.2); to.t0 = CD(0.0); to.tf = ti.t_final; to.noise_mode = 2; to.seed = 7; to.w_limit = CD(0.05); to.ang_limit = CD(0.08727);
+    CD slew(0.0);
+    const Counters a = g_cnt;
+    ts::tvlqr_replay(ti, to, Kr.data(), nullptr, nullptr, nullptr, &slew);
+    return diff(g_cnt, a);
+  };
+  const Counters r65 = replay(65), r33 = replay(33);
+  const Counters c_step = diff(r65, r33);
+  c0 = g_cnt;
+  { CD nz[9]; ts::tvlqr_noise(7, 3, 1, 2, nz, 5); }
+  const Counters c_draw = diff(g_cnt, c0);
+  printf("\n(c) TVLQR replay with inline draws (disturbance ensemble, K4e), per replay step:\n");
+  show("replay step (feedback + 4 stage records with draws + rk4)", c_step, 32);
+  show("draws of one stage (tvlqr_noise: 3 Philox blocks, 3 Box-Muller pairs, scaling)", c_draw, 1);
+  printf("JSON {\"ensemble_replay_step\": %.0f, \"stage_draws\": %lld}\n", c_step.flops() / 32.0, c_draw.flops());
   return 0;
 }

@@ -37,6 +37,7 @@ enum Slot : int {
   SLOT_K3_COUNTERS,                        // K3 queue and park counters (read by ts_k3_last_split / ts_k3_last_parked)
   SLOT_AL_STATES,                          // K3 continuation: a call's imported and exported solver states
   SLOT_KEPT_STATE,                         // Monte-Carlo kept solver states + multipliers (ts_mc_fetch_state, ts_mc_continue)
+  SLOT_ENSEMBLE_OUT,                       // a disturbance ensemble's slew times and final states (ts_mc_replay_ensemble)
   SLOT_COUNT
 };
 }  // namespace ts
@@ -57,6 +58,7 @@ struct ts_ctx {
   char name[128] = {0};
   int64_t launches = 0;
   double last_kernel_ms = 0.0;
+  double ens_ms[2] = {0.0, 0.0};  // the last ts_mc_replay_ensemble: gains (K4a + K4b) | ensemble replay (K4e)
   double* d_tabG = nullptr;  // 104 x 25
   double* d_tabH = nullptr;  // 91 x 25
   double* d_tabGH = nullptr; // 3450 (igrf12syn)
@@ -68,15 +70,17 @@ struct ts_ctx {
     int64_t n = 0, knots = 0, rows = 0;
     std::vector<int64_t> knot_offs, row_offs;
     double *d_X = nullptr, *d_U = nullptr, *d_Xs = nullptr, *d_Us = nullptr, *d_B = nullptr;
-    // keep_trajectories = 2: what ts_mc_continue needs (device pointers into the kept slots, host copies of the
-    // run's per-trial inputs in the packed layout of ts_monte_carlo_run, and the final outcome records)
-    bool resumable = false;
+    // keep_trajectories >= 1: what ts_mc_replay_ensemble needs (host copies of the run's config, active trials,
+    // per-trial inputs in the packed layout of ts_monte_carlo_run, stream ids and final outcome records)
+    bool replayable = false;
     ts_mc_config cfg = {};
     bool diag_inertia = false;
     std::vector<int64_t> act, hi;   // active trials (caller indices); packed int64 per-active-trial arrays
     std::vector<double> hf;         // packed double per-active-trial arrays
-    std::vector<uint32_t> sid;      // Philox stream ids of the active trials (run_tvlqr)
+    std::vector<uint32_t> sid;      // Philox stream ids of the active trials
     std::vector<ts_trial_outcome> out;
+    // keep_trajectories = 2: what ts_mc_continue needs besides (device pointers into the kept slots)
+    bool resumable = false;
     int64_t* d_i = nullptr;
     double *d_f = nullptr, *d_w = nullptr, *d_lam = nullptr;
     uint32_t* d_sid = nullptr;

@@ -394,7 +394,8 @@ __global__ void __launch_bounds__(256) k4_clear_rows_kernel(int64_t n_trials, co
   for (int64_t i = threadIdx.x; i < n3; i += blockDim.x) us[i] = 0.0;
 }
 
-inline void k4_launch(ts_ctx* c, const K4Args& a) {
+// K4a + K4b: the gains and the replay clock sequence
+inline void k4_gains_launch(ts_ctx* c, const K4Args& a) {
   if (a.lin_total > 0) k4a_linearise_kernel<<<(unsigned)((a.lin_total + 127) / 128), 128, 0, c->stream>>>(a);
   // (a per-device attribute: set on every launch -- ts_create_multi drives several devices from one process)
   cudaFuncSetAttribute(k4b_riccati_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, K4B_SMEM_BYTES);
@@ -404,9 +405,142 @@ inline void k4_launch(ts_ctx* c, const K4Args& a) {
                               c->stream>>>(a);
   else
     k4b_riccati_kernel<<<(unsigned)((a.n_trials + 31) / 32), 32, K4B_SMEM_BYTES, c->stream>>>(a);
+  c->launches += 2;
+}
+
+inline void k4_launch(ts_ctx* c, const K4Args& a) {
+  k4_gains_launch(c, a);
   if (a.lin_total > 0) k4n_records_kernel<<<(unsigned)((4 * a.lin_total + 127) / 128), 128, 0, c->stream>>>(a);
   k4c_replay_kernel<<<(unsigned)((a.n_trials + 31) / 32), 32, K4C_SMEM_BYTES, c->stream>>>(a);
-  c->launches += 4;
+  c->launches += 2;
+}
+
+// ---- K4e: the disturbance ensemble of a kept Monte-Carlo run (ts_mc_replay_ensemble, RE1-RE5 of DESIGN.md section 4,
+// K4).  One warp per (slew, 32 consecutive realisations), one realisation per lane, warps of the longest slews first.
+// The reference row, the gain, the reference control and the clock state of a step (K4b's sequence) are the same for
+// every lane: the warp stages them K4_RING_D steps ahead into one shared slot per step (30 doubles, one 8-byte cp.async
+// per lane) and the lanes read them by broadcast.  The clock state is noise-free, so the four stage field rows are the
+// same for every lane too (uniform loads).  The stage records cannot be pre-generated as K4n does (40 doubles per step
+// and realisation): each lane builds its own at the step, with K4n's Philox / Box-Muller / stage-record code and its
+// realisation's counters, into its own slice of shared memory (one stage at a time, so the draws never compete with
+// the integration for registers), and then runs K4c's replay step and slew-time rule on them (tvlqr_replay_src<true>).
+// Stored and reloaded like K4n's records, the draws enter the integration exactly as in the kept run (RE3).
+constexpr int K4E_W = 32;            // ring slot: x_ref 8 | K 18 | u_ref 3 | clock 1
+constexpr int K4E_R = 4 * TV_REC + 1;   // a lane's stage records (odd stride: 64-bit accesses without bank conflicts)
+constexpr int K4E_WARPS = 4;
+struct K4eArgs {
+  int64_t n_sel;                     // selected active trials, compacted (longest horizon first)
+  const int64_t *N_i, *offs, *B_offs, *B_rows;
+  const double *X_lqr, *U_lqr, *K;   // kept trajectories (knot offsets offs), gains of K4a + K4b
+  const double* clk;                 // K4b's replay clock sequence, at lin_offs
+  const int64_t* lin_offs;
+  const double *x0, *x0_lqr, *Jmat, *B_eci, *index_scale, *clock_rate, *t_final, *q_final;
+  const uint32_t* stream_id;
+  ts_tvlqr_opts_dev opts;            // the run's options after the fused path's overrides, noise_mode 2
+  int64_t n_real, r_first, n_blk;    // n_blk = ceil(n_real / 32) warps per trial
+  double q_noise_scale;
+  double* slew_time;                 // n_sel x n_real
+  double* x_final;                   // n_sel x n_real x 8, nullable
+};
+struct K4eWarpSrc {
+  const TvlqrIn* in;
+  const ts_tvlqr_opts_dev* o;
+  const double *X, *U, *K, *clk;
+  double* ring;                      // this warp's K4_RING_D slots of K4E_W doubles
+  double* recs;                      // this lane's K4E_R doubles
+  long long n_steps;
+  int lane;
+  __device__ __forceinline__ void issue(long long k) const {
+    if (k < n_steps && lane < 30) {
+      const double* src = lane < 8 ? X + k * 8 + lane
+                        : lane < 26 ? K + k * 18 + (lane - 8)
+                        : lane < 29 ? U + k * 3 + (lane - 26)
+                                    : clk + k;
+      k4_cp8(ring + (int)(k % K4_RING_D) * K4E_W + lane, src);
+    }
+    k4_commit();
+  }
+  __device__ __forceinline__ void fetch(long long k, const double*& xr, const double*& Kk, const double*& ul, const double*& rk) const {
+    k4_wait_oldest();
+    __syncwarp();                    // the other lanes' copies of slot k are complete and visible
+    const double* p = ring + (int)(k % K4_RING_D) * K4E_W;
+    double tcl[4], nxt;
+    clock_rk4(p[29], in->clock_rate, o->dt, tcl, nxt);
+#pragma unroll 1
+    for (int s = 0; s < 4; ++s) {
+      double rec[TV_REC];
+      const double tc = s == 0 ? tcl[0] : (s == 3 ? tcl[3] : tcl[1]);   // (no dynamic index: tcl stays in registers)
+      tvlqr_stage_record_at(*in, *o, k, s, tc, rec);
+#pragma unroll
+      for (int i = 0; i < TV_REC; ++i) recs[s * TV_REC + i] = rec[i];
+    }
+    xr = p;
+    Kk = p + 8;
+    ul = p + 26;
+    rk = recs;
+  }
+  __device__ __forceinline__ void done(long long k) const {
+    __syncwarp();                    // every lane has read slot k: it may be refilled
+    issue(k + K4_RING_D);
+  }
+};
+__global__ void __launch_bounds__(32 * K4E_WARPS) k4e_ensemble_replay_kernel(const K4eArgs a) {
+  __shared__ __align__(16) double ring_all[K4E_WARPS * K4_RING_D * K4E_W];
+  __shared__ double recs_all[32 * K4E_WARPS * K4E_R];
+  const int lane = threadIdx.x & 31, wib = threadIdx.x >> 5;
+  const int64_t w = (int64_t)blockIdx.x * K4E_WARPS + wib;
+  if (w >= a.n_sel * a.n_blk) return;   // whole warps leave together
+  const int64_t t = w / a.n_blk;
+  const int64_t j = (w % a.n_blk) * 32 + lane;             // realisation r_first + j of trial t
+  const int64_t jc = j < a.n_real ? j : a.n_real - 1;      // lanes past n_real replay a copy and store nothing
+  const uint32_t r = (uint32_t)(a.r_first + jc);
+  TvlqrIn in;
+  in.N = (int)a.N_i[t];
+  in.X_lqr = a.X_lqr + a.offs[t] * 8;
+  in.U_lqr = a.U_lqr + a.offs[t] * 3;
+  in.trial = a.stream_id[t];
+  in.real = r;
+  if (r == 0) {
+    for (int i = 0; i < 8; ++i) in.x0[i] = a.x0_lqr[t * 8 + i];
+  } else {
+    double qn[3];
+    tvlqr_initial_qnoise(a.opts.seed, in.trial, r, a.q_noise_scale, qn);
+    tvlqr_x0_lqr(a.x0 + t * 8, qn, in.x0);
+  }
+  for (int i = 0; i < 9; ++i) in.I.J[i] = a.Jmat[t * 9 + i];
+  inv3_gj(in.I.J, in.I.Jinv);
+  in.Bt = a.B_eci + a.B_offs[t] * 3;
+  in.B_rows = a.B_rows[t];
+  in.index_scale = a.index_scale[t];
+  in.clock_rate = a.clock_rate[t];
+  in.noise = nullptr;
+  for (int i = 0; i < 4; ++i) in.q_final[i] = a.q_final[t * 4 + i];
+  in.t_final = a.t_final[t];
+  in.time_step = a.opts.dt;
+  in.trial_index_1based = (long long)in.trial + 1;
+  ts_tvlqr_opts_dev o = a.opts;
+  o.tf = a.t_final[t];
+  K4eWarpSrc src;
+  src.in = &in;
+  src.o = &o;
+  src.X = in.X_lqr;
+  src.U = in.U_lqr;
+  src.K = a.K + a.offs[t] * 18;
+  src.clk = a.clk + a.lin_offs[t];
+  src.ring = ring_all + wib * (K4_RING_D * K4E_W);
+  src.recs = recs_all + threadIdx.x * K4E_R;
+  src.n_steps = in.N - 1;
+  src.lane = lane;
+  for (int d = 0; d < K4_RING_D; ++d) src.issue(d);
+  double slew = 0.0, xl[8];
+  tvlqr_replay_src<true>(in, o, src, nullptr, nullptr, nullptr, &slew, xl);
+  asm volatile("cp.async.wait_all;\n" ::: "memory");
+  if (j < a.n_real) {
+    const int64_t row = t * a.n_real + j;
+    a.slew_time[row] = slew;
+    if (a.x_final)
+      for (int i = 0; i < 8; ++i) a.x_final[row * 8 + i] = xl[i];
+  }
 }
 
 // eigen_axis_slew + Bryson weights, one thread per trial.  t_k = t0 + k*dt, k = 0..nt-1 with

@@ -268,4 +268,50 @@ int ts_multi_mc_continue(ts_multi* m, int64_t n_trials, const ts_ilqr_opts* opts
   return multi_shards(m, n_trials, shard, out, stats);
 }
 
+int ts_multi_mc_replay_ensemble(ts_multi* m, int64_t n_trials, const ts_replay_ensemble_opts* opts, int64_t n_sel, const int64_t* trials,
+                                double* slew_time, double* x_final) {
+  if (!m) return TS_ERR_ARG;
+  const int G = m->n;
+  // the argument checks of ts_mc_replay_ensemble, before any device runs: a failure leaves the outputs untouched
+  bool bad = n_trials < 0 || !opts || !slew_time || (trials ? n_sel < 0 : n_sel != n_trials);
+  if (!bad) bad = opts->n_real < 1 || opts->r_first < 0 || opts->r_first + opts->n_real > ((int64_t)1 << 30);
+  for (int64_t p = 0; !bad && trials && p < n_sel; ++p) bad = trials[p] < 0 || trials[p] >= n_trials;
+  if (bad) {
+    snprintf(m->err, sizeof(m->err), "ts_multi_mc_replay_ensemble: bad argument");
+    return TS_ERR_ARG;
+  }
+  const size_t RR = (size_t)opts->n_real;
+  std::vector<std::vector<int64_t>> pos(G), loc(G);   // caller rows and device-local trial indices per device
+  for (int64_t p = 0; p < n_sel; ++p) {
+    const int64_t t = trials ? trials[p] : p;
+    pos[t % G].push_back(p);
+    loc[t % G].push_back(t / G);
+  }
+  std::vector<int> rcs(G, TS_OK);
+  std::vector<std::vector<double>> hs(G), hx(G);
+  auto worker = [&](int g) {
+    if (pos[g].empty()) return;
+    const int64_t ng = (n_trials - g + G - 1) / G;
+    const size_t k = pos[g].size();
+    hs[g].resize(k * RR);
+    if (x_final) hx[g].resize(k * RR * 8);
+    rcs[g] = ts_mc_replay_ensemble(m->ctx[g], ng, opts, (int64_t)k, loc[g].data(), hs[g].data(), x_final ? hx[g].data() : nullptr);
+  };
+  std::vector<std::thread> th;
+  for (int g = 0; g < G; ++g) th.emplace_back(worker, g);
+  for (auto& t : th) t.join();
+  for (int g = 0; g < G; ++g)
+    if (rcs[g] != TS_OK) {
+      snprintf(m->err, sizeof(m->err), "device %d: %s", m->dev[g], ts_last_error(m->ctx[g]));
+      return rcs[g];
+    }
+  for (int g = 0; g < G; ++g)
+    for (size_t k = 0; k < pos[g].size(); ++k) {
+      const size_t p = (size_t)pos[g][k];
+      memcpy(slew_time + p * RR, &hs[g][k * RR], RR * 8);
+      if (x_final) memcpy(x_final + p * RR * 8, &hx[g][k * RR * 8], RR * 64);
+    }
+  return TS_OK;
+}
+
 }  // extern "C"

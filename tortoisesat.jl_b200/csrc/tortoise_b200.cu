@@ -24,7 +24,7 @@ using namespace ts;
 
 extern "C" {
 
-int ts_version(void) { return 103; }
+int ts_version(void) { return 104; }
 
 int ts_create(ts_ctx** out, int device_id) {
   if (!out) return TS_ERR_ARG;
@@ -1123,6 +1123,7 @@ int ts_monte_carlo_run(ts_ctx* c, const ts_mc_config* cfg, const double* kep6, c
   struct EvGuard { cudaEvent_t* e; ~EvGuard() { for (int i = 0; i < 7; ++i) cudaEventDestroy(e[i]); } } evg{e};
   c->mc_last.valid = false;
   c->mc_last.resumable = false;
+  c->mc_last.replayable = false;
 
   // ---- stage 1: scoping pass (2*N_scope samples per orbit) + gramian cutoff
   std::vector<ts_field_opts> fo(NF);
@@ -1244,23 +1245,7 @@ int ts_monte_carlo_run(ts_ctx* c, const ts_mc_config* cfg, const double* kep6, c
       hf[26 * NA + a] = (double)Nf[f];
       hf[27 * NA + a] = 1.0 / (cfg->tf - cfg->t0);
       // x0_lqr (TortoiseSat.jl:227-234): omega from x0, attitude perturbed by q_noise0, clock 0
-      double* xl = &hf[28 * NA + 8 * a];
-      for (int i = 0; i < 3; ++i) xl[i] = x0[8 * t + i];
-      const double* q0 = x0 + 8 * t + 3;
-      if (q_noise0) {
-        const double* qn = q_noise0 + 3 * t;
-        const double th = sqrt(qn[0] * qn[0] + qn[1] * qn[1] + qn[2] * qn[2]);
-        if (th > 1e-300) {
-          const double sh = sin(th / 2);
-          const double qp[4] = {cos(th / 2), qn[0] / th * sh, qn[1] / th * sh, qn[2] / th * sh};
-          ts::qmult(q0, qp, xl + 3);
-        } else {  // a zero row = "no initial perturbation" (the reference's r_noise = q_noise/0 would be NaN)
-          for (int i = 0; i < 4; ++i) xl[3 + i] = q0[i];
-        }
-      } else {
-        for (int i = 0; i < 4; ++i) xl[3 + i] = q0[i];
-      }
-      xl[7] = 0.0;
+      tvlqr_x0_lqr(x0 + 8 * t, q_noise0 ? q_noise0 + 3 * t : nullptr, &hf[28 * NA + 8 * a]);
       memcpy(&hf[36 * NA + 4 * a], xf + 8 * t + 3, 32);
     }
     hi[4 * NA] = knots;
@@ -1394,16 +1379,16 @@ int ts_monte_carlo_run(ts_ctx* c, const ts_mc_config* cfg, const double* kep6, c
       L.row_offs[n] = offs_f[nf];
       L.d_X = d_X; L.d_U = d_U; L.d_Xs = d_Xs_keep; L.d_Us = d_Us_keep; L.d_B = d_Bf;
       L.valid = true;
-    }
-    if (resumable) {
-      ts_ctx::McLast& L = c->mc_last;
+      // the host side of the kept run: what ts_mc_replay_ensemble (and, with keep_trajectories = 2, ts_mc_continue) needs
       L.diag_inertia = all_inertia_diagonal(Jmat, n);
       L.act = act;
       L.hi = hi;
       L.hf = hf;
       L.sid.clear();
-      if (cfg->run_tvlqr)
-        for (int64_t a = 0; a < na; ++a) L.sid.push_back(stream_id ? stream_id[act[a]] : (uint32_t)act[a]);
+      for (int64_t a = 0; a < na; ++a) L.sid.push_back(stream_id ? stream_id[act[a]] : (uint32_t)act[a]);
+    }
+    if (resumable) {
+      ts_ctx::McLast& L = c->mc_last;
       L.d_i = d_i; L.d_f = d_f; L.d_w = d_Qd; L.d_sid = d_sid;
       L.d_out = (ts_trial_outcome*)d_out;
       L.d_state = (ts_al_state*)p_st;
@@ -1411,17 +1396,19 @@ int ts_monte_carlo_run(ts_ctx* c, const ts_mc_config* cfg, const double* kep6, c
       L.d_lam = sio.lam_out;
     }
   }
-  if (cfg->keep_trajectories == 2) {
+  if (cfg->keep_trajectories >= 1) {
     ts_ctx::McLast& L = c->mc_last;
-    if (na == 0) {   // nothing reached the solver: a run that continues nothing
+    if (na == 0) {   // nothing reached the solver: a run that continues nothing and replays only NO_CUTOFF rows
       L.act.clear();
+      L.sid.clear();
       L.knots = 0;
       L.knot_offs.assign((size_t)n + 1, 0);
     }
     L.n = n;
     L.cfg = *cfg;
     L.out.assign(out, out + n);
-    L.resumable = true;
+    L.replayable = true;
+    L.resumable = cfg->keep_trajectories == 2;
   }
   c->last_kernel_ms = ms_field + ms_prep + ms_solve + ms_tvlqr;
   if (stats) {
@@ -1475,6 +1462,30 @@ int ts_mc_fetch_state(ts_ctx* c, ts_al_state* state, double* lam) {
   return TS_OK;
 }
 
+// The packed per-trial arrays of the kept run (ts_monte_carlo_run's layouts: hi = N | offs | B_offs | B_rows, hf = x0 xf
+// Jmat t_final index_scale clock_rate x0_lqr q_final) and stream ids, compacted to the active trials sel (indices into
+// L.act, repeats allowed) for a replay of those trials alone; the knot and row offsets keep pointing into the full kept
+// arrays.  hic[4 NC] = the kept run's knot count.
+static void compact_kept(const ts_ctx::McLast& L, const std::vector<int64_t>& sel, std::vector<int64_t>& hic, std::vector<double>& hfc,
+                         std::vector<uint32_t>& sidc) {
+  const size_t NA = L.act.size(), NC = sel.size();
+  hic.assign(4 * NC + 1, 0);
+  hfc.assign(40 * NC, 0.0);
+  sidc.assign(NC, 0u);
+  for (size_t k = 0; k < NC; ++k) {
+    const size_t a = (size_t)sel[k];
+    for (int j = 0; j < 4; ++j) hic[j * NC + k] = L.hi[j * NA + a];
+    static const int width[] = {8, 8, 9, 1, 1, 1, 8, 4};   // x0 xf Jmat t_final index_scale clock_rate x0_lqr q_final
+    size_t base = 0;
+    for (int w : width) {
+      memcpy(&hfc[base * NC + w * k], &L.hf[base * NA + w * a], (size_t)w * 8);
+      base += (size_t)w;
+    }
+    sidc[k] = L.sid[a];
+  }
+  hic[4 * NC] = L.knots;
+}
+
 // MC1-MC3 (DESIGN.md section 4, K3).  The continuing trials are solved on the kept block in place, exactly as
 // ts_alilqr_solve_state_batch continues them over the run's active trials, and replayed on their own.
 int ts_mc_continue(ts_ctx* c, int64_t n_trials, const ts_ilqr_opts* opts, ts_trial_outcome* out, ts_mc_stats* stats) {
@@ -1511,21 +1522,11 @@ int ts_mc_continue(ts_ctx* c, int64_t n_trials, const ts_ilqr_opts* opts, ts_tri
     const int64_t* hi = L.hi.data();
     const double* hf = L.hf.data();
     int rc;
-    // MC3: the replay's per-trial arrays, compacted to the continuing trials in the packed layouts of the run; the knot
-    // and row offsets keep pointing into the full kept arrays
-    std::vector<int64_t> hic(4 * NC + 1);
-    std::vector<double> hfc(40 * NC);
-    for (size_t k = 0; k < NC; ++k) {
-      const size_t a = (size_t)cont[k];
-      for (int j = 0; j < 4; ++j) hic[j * NC + k] = hi[j * NA + a];
-      static const int width[] = {8, 8, 9, 1, 1, 1, 8, 4};   // x0 xf Jmat t_final index_scale clock_rate x0_lqr q_final
-      size_t base = 0;
-      for (int w : width) {
-        memcpy(&hfc[base * NC + w * k], &hf[base * NA + w * a], (size_t)w * 8);
-        base += (size_t)w;
-      }
-    }
-    hic[4 * NC] = L.knots;
+    // MC3: the replay's per-trial arrays, compacted to the continuing trials
+    std::vector<int64_t> hic;
+    std::vector<double> hfc;
+    std::vector<uint32_t> sidc;
+    compact_kept(L, cont, hic, hfc, sidc);
     void *p_q = nullptr, *p_K = nullptr;
     int64_t* d_ic = nullptr;
     double* d_fc = nullptr;
@@ -1534,8 +1535,6 @@ int ts_mc_continue(ts_ctx* c, int64_t n_trials, const ts_ilqr_opts* opts, ts_tri
       if ((rc = upload(c, SLOT_ARGS_A, hic.data(), hic.size(), &d_ic))) return rc;
       if ((rc = upload(c, SLOT_ARGS_B, hfc.data(), hfc.size(), &d_fc))) return rc;
       if ((rc = scratch_reserve(c, SLOT_ARGS_C, NC * 20 + 64, &p_q))) return rc;
-      std::vector<uint32_t> sidc(NC);
-      for (size_t k = 0; k < NC; ++k) sidc[k] = L.sid[(size_t)cont[k]];
       TS_CUDA(c, cudaMemcpyAsync(p_q, sidc.data(), NC * 4, cudaMemcpyHostToDevice, c->stream));
       if ((rc = scratch_reserve(c, SLOT_K4_GAINS, (size_t)L.knots * 18 * 8, &p_K))) return rc;
       if ((rc = k4_lin_table(c, hic.data(), NC, k4))) return rc;
@@ -1618,6 +1617,120 @@ int ts_mc_continue(ts_ctx* c, int64_t n_trials, const ts_ilqr_opts* opts, ts_tri
     stats->flops = flops;
     stats->ms_solve = ms_solve; stats->ms_tvlqr = ms_tvlqr;
   }
+  return TS_OK;
+}
+
+// RE1-RE5 (DESIGN.md section 4, K4): the kept run's slews replayed under n_real disturbance draws each.  The gains of
+// the selected trials come from the unchanged K4a + K4b on host-compacted arrays (as ts_mc_continue replays), then K4e
+// replays every (trial, realisation) pair.  Only per-call slots are written: the kept run stays as it was (RE5).
+int ts_mc_replay_ensemble(ts_ctx* c, int64_t n_trials, const ts_replay_ensemble_opts* opts, int64_t n_sel, const int64_t* trials,
+                          double* slew_time, double* x_final) {
+  if (!c) return TS_ERR_ARG;
+  const ts_ctx::McLast& L = c->mc_last;
+  if (!L.replayable) return fail(c, TS_ERR_ARG, "ts_mc_replay_ensemble: no Monte-Carlo run with keep_trajectories >= 1 on this context");
+  if (n_trials != L.n) return fail(c, TS_ERR_ARG, "ts_mc_replay_ensemble: the kept run had %lld trials", (long long)L.n);
+  if (!opts || !slew_time) return fail(c, TS_ERR_ARG, "ts_mc_replay_ensemble: null argument");
+  const int64_t R = opts->n_real, r0 = opts->r_first;
+  if (R < 1 || r0 < 0 || r0 + R > ((int64_t)1 << 30))
+    return fail(c, TS_ERR_ARG, "ts_mc_replay_ensemble: need n_real >= 1, r_first >= 0, r_first + n_real <= 2^30");
+  if (trials ? n_sel < 0 : n_sel != n_trials)
+    return fail(c, TS_ERR_ARG, "ts_mc_replay_ensemble: n_sel must be >= 0 (= n_trials without a trial list)");
+  for (int64_t p = 0; trials && p < n_sel; ++p)
+    if (trials[p] < 0 || trials[p] >= n_trials) return fail(c, TS_ERR_ARG, "ts_mc_replay_ensemble: trial %lld out of range", (long long)trials[p]);
+  // selected active trials, longest horizon first (stable: repeats and the caller's order decide nothing about a row, RE4)
+  std::vector<int64_t> act_of((size_t)n_trials, -1);
+  for (size_t a = 0; a < L.act.size(); ++a) act_of[(size_t)L.act[a]] = (int64_t)a;
+  std::vector<int64_t> pos;   // caller rows with an active trial
+  for (int64_t p = 0; p < n_sel; ++p)
+    if (act_of[(size_t)(trials ? trials[p] : p)] >= 0) pos.push_back(p);
+  auto act_at = [&](int64_t p) { return act_of[(size_t)(trials ? trials[p] : p)]; };
+  std::stable_sort(pos.begin(), pos.end(), [&](int64_t u, int64_t v) { return L.hi[(size_t)act_at(u)] > L.hi[(size_t)act_at(v)]; });
+  const size_t NC = pos.size(), RR = (size_t)R;
+  const size_t per = x_final ? 9 : 1;   // doubles per (trial, realisation) row
+  std::vector<double> hs(NC * RR), hx(x_final ? NC * RR * 8 : 0);
+  c->ens_ms[0] = c->ens_ms[1] = 0.0;
+  c->last_kernel_ms = 0.0;
+  if (NC > 0) {
+    TS_CUDA(c, cudaSetDevice(c->device));
+    std::vector<int64_t> sel(NC);
+    for (size_t k = 0; k < NC; ++k) sel[k] = act_at(pos[k]);
+    std::vector<int64_t> hic;
+    std::vector<double> hfc;
+    std::vector<uint32_t> sidc;
+    compact_kept(L, sel, hic, hfc, sidc);
+    int rc;
+    void *p_out, *p_K, *p_s;
+    if ((rc = scratch_reserve(c, SLOT_ENSEMBLE_OUT, NC * RR * per * 8 + 64, &p_out))) return rc;
+    if ((rc = scratch_reserve(c, SLOT_K4_GAINS, (size_t)L.knots * 18 * 8, &p_K))) return rc;
+    int64_t* d_ic;
+    double* d_fc;
+    if ((rc = upload(c, SLOT_ARGS_A, hic.data(), hic.size(), &d_ic))) return rc;
+    if ((rc = upload(c, SLOT_ARGS_B, hfc.data(), hfc.size(), &d_fc))) return rc;
+    if ((rc = upload(c, SLOT_ARGS_C, sidc.data(), NC, (uint32_t**)&p_s))) return rc;
+    K4Args k4;
+    if ((rc = k4_lin_table(c, hic.data(), NC, k4))) return rc;
+    const ts_mc_config& cfg = L.cfg;
+    k4.n_trials = (int64_t)NC; k4.N_i = d_ic; k4.offs = d_ic + NC; k4.B_offs = d_ic + 2 * NC; k4.B_rows = d_ic + 3 * NC;
+    k4.X_lqr = L.d_X; k4.U_lqr = L.d_U; k4.x0_lqr = d_fc + 28 * NC; k4.Jmat = d_fc + 16 * NC; k4.B_eci = L.d_B;
+    k4.index_scale = d_fc + 26 * NC; k4.clock_rate = d_fc + 27 * NC; k4.t_final = d_fc + 25 * NC; k4.q_final = d_fc + 36 * NC;
+    k4.stream_id = (const uint32_t*)p_s;
+    memcpy(&k4.opts, &cfg.tvlqr, sizeof(k4.opts));   // RE2: the run's options with the fused path's overrides
+    k4.opts.dt = cfg.dt; k4.opts.t0 = cfg.t0;
+    k4.opts.noise_mode = 2;                          // realisations always draw
+    k4.opts.literal_postproc = 0;
+    k4.noise = nullptr; k4.X_sim = nullptr; k4.U_sim = nullptr; k4.dX = nullptr; k4.K = (double*)p_K;
+    k4.N_sim = nullptr; k4.slew_time = nullptr;
+    K4eArgs e;
+    e.n_sel = (int64_t)NC; e.N_i = k4.N_i; e.offs = k4.offs; e.B_offs = k4.B_offs; e.B_rows = k4.B_rows;
+    e.X_lqr = L.d_X; e.U_lqr = L.d_U; e.K = k4.K;
+    e.clk = k4.clk; e.lin_offs = k4.lin_offs;
+    e.x0 = d_fc; e.x0_lqr = k4.x0_lqr; e.Jmat = k4.Jmat; e.B_eci = L.d_B; e.index_scale = k4.index_scale;
+    e.clock_rate = k4.clock_rate; e.t_final = k4.t_final; e.q_final = k4.q_final; e.stream_id = k4.stream_id;
+    e.opts = k4.opts;
+    e.n_real = R; e.r_first = r0; e.n_blk = (R + 31) / 32;
+    e.q_noise_scale = opts->q_noise_scale;
+    e.slew_time = (double*)p_out;
+    e.x_final = x_final ? e.slew_time + NC * RR : nullptr;
+    cudaEvent_t ev[3];
+    for (int i = 0; i < 3; ++i) cudaEventCreate(&ev[i]);
+    struct EvGuard { cudaEvent_t* e; ~EvGuard() { for (int i = 0; i < 3; ++i) cudaEventDestroy(e[i]); } } evg{ev};
+    cudaEventRecord(ev[0], c->stream);
+    k4_gains_launch(c, k4);
+    cudaEventRecord(ev[1], c->stream);
+    const int64_t warps = (int64_t)NC * e.n_blk;
+    k4e_ensemble_replay_kernel<<<(unsigned)((warps + K4E_WARPS - 1) / K4E_WARPS), 32 * K4E_WARPS, 0, c->stream>>>(e);
+    c->launches++;
+    cudaEventRecord(ev[2], c->stream);
+    TS_CUDA(c, cudaGetLastError());
+    TS_CUDA(c, cudaMemcpyAsync(hs.data(), e.slew_time, NC * RR * 8, cudaMemcpyDeviceToHost, c->stream));
+    if (x_final) TS_CUDA(c, cudaMemcpyAsync(hx.data(), e.x_final, NC * RR * 64, cudaMemcpyDeviceToHost, c->stream));
+    TS_CUDA(c, cudaStreamSynchronize(c->stream));
+    float ms = 0;
+    cudaEventElapsedTime(&ms, ev[0], ev[1]); c->ens_ms[0] = ms;
+    cudaEventElapsedTime(&ms, ev[1], ev[2]); c->ens_ms[1] = ms;
+    c->last_kernel_ms = c->ens_ms[0] + c->ens_ms[1];
+  }
+  // rows in the caller's order; a NO_CUTOFF trial gets NaN rows
+  std::vector<char> done((size_t)n_sel, 0);
+  for (size_t k = 0; k < NC; ++k) {
+    const size_t p = (size_t)pos[k];
+    done[p] = 1;
+    memcpy(slew_time + p * RR, &hs[k * RR], RR * 8);
+    if (x_final) memcpy(x_final + p * RR * 8, &hx[k * RR * 8], RR * 64);
+  }
+  for (int64_t p = 0; p < n_sel; ++p)
+    if (!done[(size_t)p]) {
+      for (size_t i = 0; i < RR; ++i) slew_time[(size_t)p * RR + i] = NAN;
+      if (x_final)
+        for (size_t i = 0; i < RR * 8; ++i) x_final[(size_t)p * RR * 8 + i] = NAN;
+    }
+  return TS_OK;
+}
+
+int ts_mc_replay_ensemble_last_split(ts_ctx* c, double* gains_ms, double* replay_ms) {
+  if (!c) return TS_ERR_ARG;
+  if (gains_ms) *gains_ms = c->ens_ms[0];
+  if (replay_ms) *replay_ms = c->ens_ms[1];
   return TS_OK;
 }
 

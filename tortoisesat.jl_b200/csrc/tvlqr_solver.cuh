@@ -98,6 +98,7 @@ struct TvlqrIn {
   double index_scale, clock_rate;
   const double* noise;   // (N_sim-1) x 4 x 9 or null
   uint32_t trial;        // Philox stream id
+  uint32_t real = 0;     // realisation of a disturbance ensemble (counter blocks 4 real + {0,1,2}); 0 = the single replay
   double q_final[4];
   double t_final, time_step;
   long long trial_index_1based;
@@ -337,21 +338,37 @@ TS_HD void tvlqr_gains(const TvlqrIn& in, const ts_tvlqr_opts_dev& o, double* K,
   }
 }
 
-// The four stage records of step k (40 doubles) when they are not pre-generated: clock -> field rows -> noise -> records.
-TS_HD void tvlqr_step_records(const TvlqrIn& in, const ts_tvlqr_opts_dev& o, long long k, double x8, double recs[4 * TV_REC]) {
-  double tcl[4], nxt;
-  clock_rk4(x8, in.clock_rate, o.dt, tcl, nxt);
-  for (int s = 0; s < 4; ++s) {
-    const double* Bn = in.Bt + (long long)field_row(tcl[s], in.index_scale, in.B_rows) * 3;
+// Stage record s of step k when it is not pre-generated (tcl_s: the stage's clock value): field row -> noise -> record.
+TS_HD void tvlqr_stage_record_at(const TvlqrIn& in, const ts_tvlqr_opts_dev& o, long long k, int s, double tcl_s, double rec[TV_REC]) {
+  const double* Bn = in.Bt + (long long)field_row(tcl_s, in.index_scale, in.B_rows) * 3;
+  if (o.noise_mode == 2) {   // (its own call: the draws stay in registers, no pointer may alias them)
     double nzb[9];
-    const double* nz = nullptr;
-    if (o.noise_mode == 1) nz = in.noise + (k * 4 + s) * 9;
-    if (o.noise_mode == 2) {
-      tvlqr_noise(o.seed, in.trial, (uint32_t)k, (uint32_t)s, nzb);
-      nz = nzb;
-    }
-    tvlqr_stage_record(nz, Bn, recs + s * TV_REC);
+    tvlqr_noise(o.seed, in.trial, (uint32_t)k, (uint32_t)s, nzb, in.real);
+    tvlqr_stage_record(nzb, Bn, rec);
+  } else {
+    tvlqr_stage_record(o.noise_mode == 1 ? in.noise + (k * 4 + s) * 9 : nullptr, Bn, rec);
   }
+}
+
+// The replay's initial state (TortoiseSat.jl:227-234): omega from x0, attitude x0's perturbed by the rotation of q_noise
+// (qn, nullable; a zero row = no perturbation: the reference's r_noise = q_noise/0 would be NaN), clock 0.  Built so by
+// ts_monte_carlo_run from q_noise0 and by the disturbance ensemble (K4e) from its initial draw.
+TS_HD void tvlqr_x0_lqr(const double* x0, const double* qn, double xl[8]) {
+  for (int i = 0; i < 3; ++i) xl[i] = x0[i];
+  const double* q0 = x0 + 3;
+  bool rotated = false;
+  if (qn) {
+    const double th = sqrt(qn[0] * qn[0] + qn[1] * qn[1] + qn[2] * qn[2]);
+    if (th > 1e-300) {
+      const double sh = sin(th / 2);
+      const double qp[4] = {cos(th / 2), qn[0] / th * sh, qn[1] / th * sh, qn[2] / th * sh};
+      qmult(q0, qp, xl + 3);
+      rotated = true;
+    }
+  }
+  if (!rotated)
+    for (int i = 0; i < 4; ++i) xl[3 + i] = q0[i];
+  xl[7] = 0.0;
 }
 
 // Closed-loop replay + slew-time detection.  Outputs nullable.  Returns N_sim; *slew_time_out as
@@ -359,9 +376,11 @@ TS_HD void tvlqr_step_records(const TvlqrIn& in, const ts_tvlqr_opts_dev& o, lon
 // K4n) or null -> built on the fly.  The slew-time rule is evaluated without sqrt / acos: |w| < w_limit is w.w < w_limit^2
 // and 2 acos(min(q_e1,1)) < ang_limit is q_e1 > cos(ang_limit/2) (acos is decreasing; identical decisions except within one
 // rounding of the thresholds).
-// Where the replay reads the per-step inputs from (reference state 8, gain 18, reference control 3, stage records 40):
+// Where the replay reads the per-step inputs from (reference state 8, gain 18, reference control 3, stage records 40 if
+// pre-generated):
 // straight from the arrays (host twin, unit entries), or from a per-thread staging ring filled ahead of the sequential
-// loop by asynchronous copies (K4c, k4_tvlqr.cuh).
+// loop by asynchronous copies (K4c, k4_tvlqr.cuh), or from a per-warp ring when the 32 lanes replay the same slew under
+// 32 noise draws (K4e).  x_last (nullable): the state at the last simulated step, X_sim row N_sim - 1.
 struct TvlqrDirectSrc {
   const double *X, *U, *K, *recs;
   TS_HD void fetch(long long k, const double*& xr, const double*& Kk, const double*& ul, const double*& rk) const {
@@ -374,7 +393,7 @@ struct TvlqrDirectSrc {
 };
 template <bool PRE, class Src>
 TS_HD long long tvlqr_replay_src(const TvlqrIn& in, const ts_tvlqr_opts_dev& o, Src& src, double* X_sim, double* U_sim,
-                                 double* dX, double* slew_time_out) {
+                                 double* dX, double* slew_time_out, double* x_last = nullptr) {
   const int N = in.N;
   long long N_sim = range_len(o.t0, o.dt, o.tf);
   if (N_sim > N) N_sim = range_len(o.t0, o.dt, o.tf - o.dt);
@@ -397,6 +416,8 @@ TS_HD long long tvlqr_replay_src(const TvlqrIn& in, const ts_tvlqr_opts_dev& o, 
       if (j > 10 && w2 < w2_limit && qe0 > cos_limit && slew == in.t_final) slew = in.time_step * (double)j;
     }
     if (k == N_sim - 1) {
+      if (x_last)
+        for (int i = 0; i < 8; ++i) x_last[i] = x[i];
       if (U_sim) U_sim[k * 3 + 0] = U_sim[k * 3 + 1] = U_sim[k * 3 + 2] = 0.0;
       if (dX)
         for (int i = 0; i < 6; ++i) dX[k * 6 + i] = 0.0;
@@ -426,20 +447,27 @@ TS_HD long long tvlqr_replay_src(const TvlqrIn& in, const ts_tvlqr_opts_dev& o, 
     // rk4(simulator) with per-stage records
     double tcl[4], nxt;
     clock_rk4(x[7], in.clock_rate, o.dt, tcl, nxt);
-    double rbuf[PRE ? 1 : 4 * TV_REC];
-    const double* rk = PRE ? rk_src : rbuf;
-    if (!PRE) tvlqr_step_records(in, o, k, x[7], rbuf);
+    // stage record s: pre-generated, or built right before its stage (10 live doubles rather than a step's 40)
+    double rbuf[TV_REC];
+    auto rec = [&](int s) -> const double* {
+      if constexpr (PRE) {
+        return rk_src + s * TV_REC;
+      } else {
+        tvlqr_stage_record_at(in, o, k, s, tcl[s], rbuf);
+        return rbuf;
+      }
+    };
     double k1[7], k2[7], k3[7], k4[7], xs[7];
-    simulator7_rec(in.I, x, u, rk, k1);
+    simulator7_rec(in.I, x, u, rec(0), k1);
     for (int i = 0; i < 7; ++i) k1[i] = k1[i] * o.dt;
     for (int i = 0; i < 7; ++i) xs[i] = x[i] + k1[i] / 2.0;
-    simulator7_rec(in.I, xs, u, rk + TV_REC, k2);
+    simulator7_rec(in.I, xs, u, rec(1), k2);
     for (int i = 0; i < 7; ++i) k2[i] = k2[i] * o.dt;
     for (int i = 0; i < 7; ++i) xs[i] = x[i] + k2[i] / 2.0;
-    simulator7_rec(in.I, xs, u, rk + 2 * TV_REC, k3);
+    simulator7_rec(in.I, xs, u, rec(2), k3);
     for (int i = 0; i < 7; ++i) k3[i] = k3[i] * o.dt;
     for (int i = 0; i < 7; ++i) xs[i] = x[i] + k3[i];
-    simulator7_rec(in.I, xs, u, rk + 3 * TV_REC, k4);
+    simulator7_rec(in.I, xs, u, rec(3), k4);
     for (int i = 0; i < 7; ++i) k4[i] = k4[i] * o.dt;
     for (int i = 0; i < 7; ++i) x[i] = x[i] + (k1[i] + 2.0 * k2[i] + 2.0 * k3[i] + k4[i]) * TS_SIXTH;
     x[7] = nxt;

@@ -85,6 +85,14 @@ class McStats(C.Structure):
                                           "ms_tvlqr")] + [("n_status", C.c_int64 * 6)]
 
 
+class ReplayEnsembleOpts(C.Structure):
+    """ts_replay_ensemble_opts (include/tortoise_b200.h)."""
+    _fields_ = [("n_real", C.c_int64), ("r_first", C.c_int64), ("q_noise_scale", C.c_double)]
+
+
+Q_NOISE_SCALE = (np.pi / 180) ** 2   # initial attitude noise of monte_carlo.jl: randn(3)*(pi/180)^2
+
+
 def default_tvlqr_opts():
     o = TvlqrOpts()
     load_library().ts_tvlqr_default_opts(C.byref(o))
@@ -158,6 +166,8 @@ def load_library():
     L.ts_mc_fetch_trajectories.argtypes = [C.c_void_p] + [C.c_void_p] * 5
     L.ts_mc_fetch_state.argtypes = [C.c_void_p, C.c_void_p, C.c_void_p]
     L.ts_mc_continue.argtypes = [C.c_void_p, C.c_int64, C.POINTER(IlqrOpts), C.c_void_p, C.POINTER(McStats)]
+    L.ts_mc_replay_ensemble.argtypes = [C.c_void_p, C.c_int64, C.POINTER(ReplayEnsembleOpts), C.c_int64] + [C.c_void_p] * 3
+    L.ts_mc_replay_ensemble_last_split.argtypes = [C.c_void_p, c_double_p, c_double_p]
     L.ts_igrf12syn_batch.argtypes = [C.c_void_p, C.c_int, C.c_double, C.c_int, C.c_int64] + [C.c_void_p] * 7 + [C.c_int]
     L.ts_psiaki_pd_batch.argtypes = [C.c_void_p, C.c_int64] + [C.c_void_p] * 7 + [C.c_double] * 3 + [C.c_void_p] * 3
     L.ts_attitude_dynamics_linear_batch.argtypes = [C.c_void_p, C.c_int64] + [C.c_void_p] * 6
@@ -171,6 +181,7 @@ def load_library():
     L.ts_multi_ctx.restype = C.c_void_p
     L.ts_multi_monte_carlo_run.argtypes = [C.c_void_p, C.POINTER(McConfig)] + [C.c_void_p] * 8 + [C.POINTER(McStats)]
     L.ts_multi_mc_continue.argtypes = [C.c_void_p, C.c_int64, C.POINTER(IlqrOpts), C.c_void_p, C.POINTER(McStats)]
+    L.ts_multi_mc_replay_ensemble.argtypes = [C.c_void_p, C.c_int64, C.POINTER(ReplayEnsembleOpts), C.c_int64] + [C.c_void_p] * 3
     L.ts_igrf12_batch.argtypes = [C.c_void_p, C.c_double, C.c_int64] + [C.c_void_p] * 6 + [C.c_int]
     L.ts_field_map_prefilter.argtypes = [C.c_void_p, C.c_int64, C.c_int64, C.c_void_p, C.c_void_p, C.c_int]
     L.ts_field_map_eval_batch.argtypes = [C.c_void_p, C.c_int64, C.c_int64, C.c_void_p, C.c_int64] + [C.c_void_p] * 3 + [C.c_int]
@@ -662,6 +673,20 @@ class Engine:
         self._check(self.lib.ts_mc_continue(self.h, n, C.byref(opts), out.ctypes.data, C.byref(st)))
         return out, st
 
+    def mc_replay_ensemble(self, n_trials, n_real, r_first=0, trials=None, q_noise_scale=Q_NOISE_SCALE, want_x_final=False):
+        """The kept run's slews (last monte_carlo_run with cfg.keep_trajectories >= 1) replayed under n_real independent
+        disturbance draws each (ts_mc_replay_ensemble, rules RE1-RE5): realisations r_first .. r_first + n_real - 1 of the
+        selected trials (caller indices, repeats allowed; None = all).  Returns (slew_time (n_sel, n_real), x_final
+        (n_sel, n_real, 8) or None); a NO_CUTOFF trial gets NaN rows."""
+        return _replay_ensemble(self.lib.ts_mc_replay_ensemble, self.h, n_trials, n_real, r_first, trials, q_noise_scale,
+                                want_x_final, self._check)
+
+    def mc_replay_ensemble_split(self):
+        """Device ms of the last mc_replay_ensemble: (gains, ensemble replay)."""
+        g, r = C.c_double(), C.c_double()
+        self._check(self.lib.ts_mc_replay_ensemble_last_split(self.h, C.byref(g), C.byref(r)))
+        return g.value, r.value
+
     def igrf12syn_batch(self, isv, date, itype, alt, colat, elong):
         """igrf12syn (igrf.jl:335-534) at n points: alt km, colat/elong degrees -> x, y, z, f (nT)."""
         alt, colat, elong = _f64(np.atleast_1d(alt)), _f64(np.atleast_1d(colat)), _f64(np.atleast_1d(elong))
@@ -750,6 +775,27 @@ class MultiEngine:
         if rc != 0:
             raise TortoiseError(rc, (self.lib.ts_multi_last_error(self.h) or b"").decode())
         return out, st
+
+    def mc_replay_ensemble(self, n_trials, n_real, r_first=0, trials=None, q_noise_scale=Q_NOISE_SCALE, want_x_final=False):
+        """Engine.mc_replay_ensemble over the devices' kept shards: each trial on the device that holds it (t mod
+        n_devices); the rows equal the single-device rows bit for bit (RE4)."""
+        def check(rc):
+            if rc != 0:
+                raise TortoiseError(rc, (self.lib.ts_multi_last_error(self.h) or b"").decode())
+        return _replay_ensemble(self.lib.ts_multi_mc_replay_ensemble, self.h, n_trials, n_real, r_first, trials, q_noise_scale,
+                                want_x_final, check)
+
+
+def _replay_ensemble(fn, h, n_trials, n_real, r_first, trials, q_noise_scale, want_x_final, check):
+    n = int(n_trials)
+    o = ReplayEnsembleOpts(int(n_real), int(r_first), float(q_noise_scale))
+    sel = None if trials is None else np.ascontiguousarray(trials, dtype=np.int64).reshape(-1)
+    ns = n if sel is None else sel.shape[0]
+    R = max(int(n_real), 0)
+    slew = np.zeros((ns, R))
+    xf = np.zeros((ns, R, 8)) if want_x_final else None
+    check(fn(h, n, C.byref(o), ns, None if sel is None else _ptr(sel), _ptr(slew), None if xf is None else _ptr(xf)))
+    return slew, xf
 
 
 # ---------------------------------------------------------------------------
@@ -1139,6 +1185,34 @@ def continue_monte_carlo(res, max_outer=30, ilqr=None):
                 res["sim_states"][t] = sl(tr["X_sim"], t)
                 res["sim_control_inputs"][t] = sl(tr["U_sim"], t)
     return idx
+
+
+def replay_ensemble(res, n_real=100, trials=None, r_first=0, q_noise_scale=Q_NOISE_SCALE):
+    """The slew-time distribution of the optimised slews of a monte_carlo() result under the simulator's disturbances:
+    every selected trial (None = all) replayed n_real times with independent draws (ts_mc_replay_ensemble on the default
+    engine, which must not have run another Monte-Carlo call since; the result must come from monte_carlo with
+    trajectories=True, the default, or resumable=True).  Realisation 0 repeats the run's own replay (RE3).  Returns a dict:
+    slew_time (n_sel, n_real), fails (slew_time == t_final, monte_carlo.jl:257-261), fail_rate (n_sel: the share of failing
+    draws), slew_mean / slew_std (n_sel: over the non-failing draws, NaN if none) and trials (the selected indices).  A
+    NO_CUTOFF trial has NaN slew times, no fails and a NaN fail_rate."""
+    if "states" not in res and "ilqr" not in res:
+        raise ValueError("replay_ensemble needs a monte_carlo(..., trajectories=True) or monte_carlo(..., resumable=True) result")
+    out = res["outcomes"]
+    n = out.shape[0]
+    sel = np.arange(n, dtype=np.int64) if trials is None else np.ascontiguousarray(trials, dtype=np.int64).reshape(-1)
+    slew, _ = default_engine().mc_replay_ensemble(n, n_real, r_first=r_first, trials=sel, q_noise_scale=q_noise_scale)
+    tf = out["t_final"][sel][:, None]
+    fails = slew == tf
+    valid = ~np.isnan(slew)
+    ok = valid & ~fails
+    with np.errstate(invalid="ignore", divide="ignore"):
+        nv = valid.sum(axis=1)
+        fail_rate = np.where(nv > 0, fails.sum(axis=1) / np.maximum(nv, 1), np.nan)
+        k = ok.sum(axis=1)
+        s = np.where(ok, slew, 0.0)
+        mean = np.where(k > 0, s.sum(axis=1) / np.maximum(k, 1), np.nan)
+        var = np.where(k > 0, (np.where(ok, slew - mean[:, None], 0.0) ** 2).sum(axis=1) / np.maximum(k, 1), np.nan)
+    return dict(slew_time=slew, fails=fails, fail_rate=fail_rate, slew_mean=mean, slew_std=np.sqrt(var), trials=sel)
 
 
 # ---------------------------------------------------------------------------
