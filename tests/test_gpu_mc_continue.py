@@ -348,6 +348,36 @@ def test_errors_leave_out_and_stats_untouched(engine):
     assert out["status"].size == n
 
 
+def test_kept_run_without_active_trials(engine):
+    """A keep = 2 run in which no trial reaches the solver, after one in which some did: nothing of the first run leaks
+    through.  The fetched states are zero records with status 5, a continuation returns the run's records and does no
+    work, the ensemble gives NaN rows, and the trajectory layout (hence mc_trajectories and mc_state) refuses the run."""
+    import tortoisesat.jl_b200 as tb
+    from tortoisesat.jl_b200 import host
+    e = shared_ensemble()
+    n = len(e["x0"])
+    out1, _ = run(engine, e, 4)
+    assert np.all(out1["status"] != 5)
+    e["cfg"].cutoff = 1.0   # a condition number is >= 1: no orbit reaches this cutoff
+    out2, _ = run(engine, e, 4)
+    ref = np.zeros(n, dtype=host.OUTCOME_DTYPE)
+    ref["status"] = 5
+    assert out2.tobytes() == ref.tobytes()
+    state = np.frombuffer(np.full(n * host.AL_STATE_DTYPE.itemsize, 0x5A, dtype=np.uint8).tobytes(), dtype=host.AL_STATE_DTYPE).copy()
+    assert engine.lib.ts_mc_fetch_state(engine.h, state.ctypes.data, None) == 0
+    ref_state = np.zeros(n, dtype=host.AL_STATE_DTYPE)
+    ref_state["status"] = 5
+    assert state.tobytes() == ref_state.tobytes()
+    oc, st = engine.mc_continue(n, cont_opts(e, 9))
+    assert oc.tobytes() == out2.tobytes() and st.ms_solve == 0 and st.ms_tvlqr == 0 and st.flops == 0
+    slew, xfin = engine.mc_replay_ensemble(n, 3, want_x_final=True)
+    assert slew.shape == (n, 3) and np.all(np.isnan(slew)) and np.all(np.isnan(xfin))
+    with pytest.raises(tb.TortoiseError):
+        engine.mc_trajectories(n)
+    with pytest.raises(tb.TortoiseError):
+        engine.mc_state(n)
+
+
 def test_no_replay(engine):
     """A kept run with run_tvlqr = 0 continues, with slew_time 0; fetching X_sim still fails."""
     import tortoisesat.jl_b200 as tb

@@ -25,7 +25,7 @@ enum Slot : int {
   SLOT_K4_GAINS,                           // K4 gains when the caller passes none
   SLOT_ORBIT_BLOCK, SLOT_ROW_LIMITS,       // Monte-Carlo per-orbit block and table row limits
   SLOT_PACKED_I64, SLOT_PACKED_F64,        // Monte-Carlo packed per-trial arrays (read by ts_mc_continue)
-  SLOT_STREAM_IDS,                         // Monte-Carlo Philox stream ids (read by ts_mc_continue)
+  SLOT_STREAM_IDS,                         // Monte-Carlo Philox stream ids (the run's own replay)
   SLOT_PARK_STATE, SLOT_PARK_DATA,         // K3 parking places (read by ts_k3_last_parked) and parked trajectories
   SLOT_PIPE_A, SLOT_PIPE_B,                // K1 host-pointer pipeline stages
   SLOT_K3_CYCLES,                          // K3 cycle counters (read by ts_k3_last_cycles)
@@ -39,6 +39,48 @@ enum Slot : int {
   SLOT_KEPT_STATE,                         // Monte-Carlo kept solver states + multipliers (ts_mc_fetch_state, ts_mc_continue)
   SLOT_ENSEMBLE_OUT,                       // a disturbance ensemble's slew times and final states (ts_mc_replay_ensemble)
   SLOT_COUNT
+};
+
+// The per-trial inputs of a fused Monte-Carlo run's n active trials, packed column by column: hi holds the int64 columns
+// and then the run's total knot count, hf the double columns, column k at [F_COL[k] * n, F_COL[k + 1] * n) (trial a's
+// entries at F_COL[k] * n + width(k) * a).  ts_monte_carlo_run fills and uploads it, and ts_mc_continue and
+// ts_mc_replay_ensemble compact the kept copy to the trials they replay.
+enum McColI : int { I_N, I_OFFS, I_B_OFFS, I_B_ROWS, I_COLS };
+enum McColF : int { F_X0, F_XF, F_JMAT, F_T_FINAL, F_INDEX_SCALE, F_CLOCK_RATE, F_X0LQR, F_Q_FINAL, F_COLS };
+constexpr size_t F_COL[F_COLS + 1] = {0, 8, 16, 25, 26, 27, 28, 36, 40};
+
+struct McPacked {
+  size_t n;
+  std::vector<int64_t> hi;
+  std::vector<double> hf;
+  std::vector<uint32_t> sid;   // Philox stream ids
+  McPacked(size_t n = 0) : n(n), hi(I_COLS * n + 1), hf(F_COL[F_COLS] * n), sid(n) {}
+  static size_t width(McColF k) { return F_COL[k + 1] - F_COL[k]; }
+  int64_t* col(McColI k) { return hi.data() + k * n; }
+  const int64_t* col(McColI k) const { return hi.data() + k * n; }
+  double* at(McColF k, size_t a) { return hf.data() + F_COL[k] * n + width(k) * a; }
+  const double* at(McColF k, size_t a) const { return hf.data() + F_COL[k] * n + width(k) * a; }
+  // the trials sel (indices, repeats allowed) alone; their knot and row offsets keep pointing into the full arrays
+  McPacked compact(const std::vector<int64_t>& sel) const {
+    McPacked p(sel.size());
+    for (size_t k = 0; k < p.n; ++k) {
+      const size_t a = (size_t)sel[k];
+      for (int j = 0; j < I_COLS; ++j) p.col((McColI)j)[k] = col((McColI)j)[a];
+      for (int j = 0; j < F_COLS; ++j) memcpy(p.at((McColF)j, k), at((McColF)j, a), width((McColF)j) * sizeof(double));
+      p.sid[k] = sid[a];
+    }
+    p.hi.back() = hi.back();
+    return p;
+  }
+};
+
+// an uploaded McPacked: the columns as device pointers
+struct McPackedView {
+  const int64_t* i = nullptr;
+  const double* f = nullptr;
+  size_t n = 0;
+  const int64_t* col(McColI k) const { return i + k * n; }
+  const double* col(McColF k) const { return f + F_COL[k] * n; }
 };
 }  // namespace ts
 
@@ -64,26 +106,20 @@ struct ts_ctx {
   double* d_tabGH = nullptr; // 3450 (igrf12syn)
   int* d_flag = nullptr;     // generic device error/flag word
   void* d_gh_stage = nullptr; // K1: the call's interpolated coefficient table (2 x 104 double2)
-  // trajectories of the last ts_monte_carlo_run with keep_trajectories (device pointers into the scratch arenas)
+  // the last ts_monte_carlo_run with keep_trajectories, cleared when a run starts (device pointers into the kept slots).
+  // The kept level cfg.keep_trajectories: 1 the trajectories and what ts_mc_replay_ensemble needs, 2 also ts_mc_continue's.
   struct McLast {
-    bool valid = false;
+    ts_mc_config cfg = {};
     int64_t n = 0, knots = 0, rows = 0;
     std::vector<int64_t> knot_offs, row_offs;
     double *d_X = nullptr, *d_U = nullptr, *d_Xs = nullptr, *d_Us = nullptr, *d_B = nullptr;
-    // keep_trajectories >= 1: what ts_mc_replay_ensemble needs (host copies of the run's config, active trials,
-    // per-trial inputs in the packed layout of ts_monte_carlo_run, stream ids and final outcome records)
-    bool replayable = false;
-    ts_mc_config cfg = {};
     bool diag_inertia = false;
-    std::vector<int64_t> act, hi;   // active trials (caller indices); packed int64 per-active-trial arrays
-    std::vector<double> hf;         // packed double per-active-trial arrays
-    std::vector<uint32_t> sid;      // Philox stream ids of the active trials
+    std::vector<int64_t> act;       // active trials (caller indices); none reached the solver: no trajectories kept
+    ts::McPacked in;                // their packed inputs and stream ids
     std::vector<ts_trial_outcome> out;
-    // keep_trajectories = 2: what ts_mc_continue needs besides (device pointers into the kept slots)
-    bool resumable = false;
-    int64_t* d_i = nullptr;
-    double *d_f = nullptr, *d_w = nullptr, *d_lam = nullptr;
-    uint32_t* d_sid = nullptr;
+    // keep_trajectories = 2
+    ts::McPackedView d_in;
+    double *d_w = nullptr, *d_lam = nullptr;
     ts_trial_outcome* d_out = nullptr;
     ts_al_state* d_state = nullptr;
     void* d_sio = nullptr;          // the K3StateIO block of the kept states
@@ -210,5 +246,18 @@ inline int upload(ts_ctx* c, Slot slot, const T* host, size_t count, T** dev) {
   *dev = (T*)d;
   return TS_OK;
 }
+
+// a call's N timing events, destroyed when it returns; ms(a, b) is the time between the a-th and the b-th
+template <int N> struct Events {
+  cudaEvent_t e[N];
+  Events() { for (cudaEvent_t& x : e) cudaEventCreate(&x); }
+  ~Events() { for (cudaEvent_t x : e) cudaEventDestroy(x); }
+  cudaEvent_t operator[](int i) const { return e[i]; }
+  float ms(int a, int b) const {
+    float t = 0.f;
+    cudaEventElapsedTime(&t, e[a], e[b]);
+    return t;
+  }
+};
 
 }  // namespace ts

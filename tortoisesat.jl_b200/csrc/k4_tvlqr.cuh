@@ -442,6 +442,18 @@ struct K4eArgs {
   double* slew_time;                 // n_sel x n_real
   double* x_final;                   // n_sel x n_real x 8, nullable
 };
+// The K4e arguments over the trials, kept trajectories, gains and options of a's replay (x0: the trials' unperturbed
+// initial states); the realisations and the outputs are left to the caller.
+inline K4eArgs k4e_args(const K4Args& a, const double* x0) {
+  K4eArgs e;
+  e.n_sel = a.n_trials; e.N_i = a.N_i; e.offs = a.offs; e.B_offs = a.B_offs; e.B_rows = a.B_rows;
+  e.X_lqr = a.X_lqr; e.U_lqr = a.U_lqr; e.K = a.K;
+  e.clk = a.clk; e.lin_offs = a.lin_offs;
+  e.x0 = x0; e.x0_lqr = a.x0_lqr; e.Jmat = a.Jmat; e.B_eci = a.B_eci; e.index_scale = a.index_scale;
+  e.clock_rate = a.clock_rate; e.t_final = a.t_final; e.q_final = a.q_final; e.stream_id = a.stream_id;
+  e.opts = a.opts;
+  return e;
+}
 struct K4eWarpSrc {
   const TvlqrIn* in;
   const ts_tvlqr_opts_dev* o;

@@ -815,6 +815,17 @@ static int k3_launch(ts_ctx* c, K3Args& a, const int64_t* N_i_host, const double
 
 static_assert(sizeof(ts_al_state) == 104 && sizeof(ts_al_state) == sizeof(ts_al_state_dev), "ts_al_state layout");
 
+// The option checks of an AL-iLQR solve of n trials with the state weights Qd, Qfd (8 per trial)
+static int check_ilqr_opts(ts_ctx* c, const ts_ilqr_opts& o, int64_t n, const double* Qd, const double* Qfd) {
+  if (o.max_linesearch < 0 || o.max_linesearch > 63) return fail(c, TS_ERR_ARG, "max_linesearch must be in [0,63]");
+  if (o.quat_error)
+    for (int64_t t = 0; t < n; ++t)
+      for (int i = 4; i < 7; ++i)
+        if (Qd[t * 8 + i] != Qd[t * 8 + 3] || Qfd[t * 8 + i] != Qfd[t * 8 + 3])
+          return fail(c, TS_ERR_ARG, "quat_error: the four quaternion weights of Q and Qf must be equal (E'QE is then diagonal)");
+  return TS_OK;
+}
+
 int ts_alilqr_solve_batch(ts_ctx* c, int64_t n_trials, const int64_t* N_i, const int64_t* offs, const double* x0,
                           const double* xf, const double* Jmat, const double* Qd, const double* Qfd, const double* Rd,
                           const double* B_eci, const int64_t* B_offs, const int64_t* B_rows, const double* index_scale,
@@ -844,12 +855,8 @@ int ts_alilqr_solve_state_batch(ts_ctx* c, int64_t n_trials, const int64_t* N_i,
   if (!(dt > 0)) return fail(c, TS_ERR_ARG, "ts_alilqr_solve_batch: dt must be > 0");
   ts_ilqr_opts o;
   if (opts) o = *opts; else ts_ilqr_default_opts(&o);
-  if (o.max_linesearch < 0 || o.max_linesearch > 63) return fail(c, TS_ERR_ARG, "max_linesearch must be in [0,63]");
-  if (o.quat_error)
-    for (int64_t t = 0; t < n_trials; ++t)
-      for (int i = 4; i < 7; ++i)
-        if (Qd[t * 8 + i] != Qd[t * 8 + 3] || Qfd[t * 8 + i] != Qfd[t * 8 + 3])
-          return fail(c, TS_ERR_ARG, "quat_error: the four quaternion weights of Q and Qf must be equal (E'QE is then diagonal)");
+  int rc;
+  if ((rc = check_ilqr_opts(c, o, n_trials, Qd, Qfd))) return rc;
   int64_t total_knots = 0, total_rows = 0;
   for (int64_t t = 0; t < n_trials; ++t) {
     if (N_i[t] < 2) return fail(c, TS_ERR_ARG, "trial %lld: N < 2", (long long)t);
@@ -858,7 +865,6 @@ int ts_alilqr_solve_state_batch(ts_ctx* c, int64_t n_trials, const int64_t* N_i,
     if (B_rows[t] < 1) return fail(c, TS_ERR_ARG, "trial %lld: empty field table", (long long)t);
   }
   TS_CUDA(c, cudaSetDevice(c->device));
-  int rc;
   Staging io(c, pointers_are_device);
   K3Args a = {};
   a.B_eci = io.in(B_eci, (size_t)total_rows * 3);
@@ -1104,6 +1110,66 @@ static void mc_stats_of(const ts_trial_outcome* out, int64_t n, bool run_tvlqr, 
   }
 }
 
+// FLOP of a trial of N knots over `inner` inner iterations and `ls` line-search rollouts (diag: the diagonal-inertia
+// instantiation) and, with tvlqr, its replay: a record's flops, or with the counters' increments a continuation's work
+static double trial_flops(bool diag, int64_t N, int64_t inner, int64_t ls, bool tvlqr) {
+  const double kn = (double)(N - 1);
+  return kn * ((double)inner * (diag ? FL_ITER_DIAG : FL_ITER) + (double)ls * (diag ? FL_ROLL_DIAG : FL_ROLL)) + (tvlqr ? kn * FL_TVLQR : 0.0);
+}
+
+static int upload_packed(ts_ctx* c, const McPacked& p, Slot si, Slot sf, McPackedView& v) {
+  int64_t* d_i;
+  double* d_f;
+  int rc;
+  if ((rc = upload(c, si, p.hi.data(), p.hi.size(), &d_i))) return rc;
+  if ((rc = upload(c, sf, p.hf.data(), p.hf.size(), &d_f))) return rc;
+  v = {d_i, d_f, p.n};
+  return TS_OK;
+}
+
+// The fused path's weights block, written by k_slew_prep: Qd (8 per trial) | Qfd (8) | Rd (3) of the n active trials
+struct McWeights {
+  double *Qd, *Qfd, *Rd;
+  McWeights(double* w, size_t n) : Qd(w), Qfd(w + 8 * n), Rd(w + 16 * n) {}
+};
+
+// The K3 arguments of the fused path: packed trials v, their weights w, field table B, trajectories X, U, outcome records
+static K3Args fused_k3_args(const McPackedView& v, const McWeights& w, const double* B, double* X, double* U, ts_trial_outcome_dev* out,
+                            const ts_ilqr_opts& opts, double dt) {
+  K3Args a = {};
+  a.n_trials = (int64_t)v.n;
+  a.N_i = v.col(I_N); a.offs = v.col(I_OFFS); a.B_offs = v.col(I_B_OFFS); a.B_rows = v.col(I_B_ROWS);
+  a.x0 = v.col(F_X0); a.xf = v.col(F_XF); a.Jmat = v.col(F_JMAT); a.Qd = w.Qd; a.Qfd = w.Qfd; a.Rd = w.Rd;
+  a.index_scale = v.col(F_INDEX_SCALE); a.clock_rate = v.col(F_CLOCK_RATE);
+  a.B_eci = B; a.dt = dt; a.U0 = nullptr;
+  memcpy(&a.opts, &opts, sizeof(a.opts));
+  a.X = X; a.U = U; a.K = nullptr; a.out = out;
+  return a;
+}
+
+// The run's TVLQR options with the fused path's overrides
+static ts_tvlqr_opts_dev fused_tvlqr_opts(const ts_mc_config& cfg) {
+  ts_tvlqr_opts_dev o;
+  memcpy(&o, &cfg.tvlqr, sizeof(o));
+  o.dt = cfg.dt; o.t0 = cfg.t0;
+  if (o.noise_mode == 1) o.noise_mode = 2;  // no explicit array in the fused path
+  o.literal_postproc = 0;                   // needs X_sim storage; fused path uses the fixed rule (Q12)
+  return o;
+}
+
+// Completes a (holding k4_lin_table's table) to the K4 arguments of a fused replay of the packed trials v on trajectories
+// X, U, field table B, gains K and stream ids sid; X_sim, U_sim, N_sim and slew_time are null until the caller sets them.
+static void fused_k4_args(K4Args& a, const McPackedView& v, const double* X, const double* U, const double* B, double* K,
+                          const uint32_t* sid, const ts_mc_config& cfg) {
+  a.n_trials = (int64_t)v.n; a.N_i = v.col(I_N); a.offs = v.col(I_OFFS); a.B_offs = v.col(I_B_OFFS); a.B_rows = v.col(I_B_ROWS);
+  a.X_lqr = X; a.U_lqr = U; a.x0_lqr = v.col(F_X0LQR); a.Jmat = v.col(F_JMAT); a.B_eci = B;
+  a.index_scale = v.col(F_INDEX_SCALE); a.clock_rate = v.col(F_CLOCK_RATE); a.t_final = v.col(F_T_FINAL); a.q_final = v.col(F_Q_FINAL);
+  a.stream_id = sid;
+  a.opts = fused_tvlqr_opts(cfg);
+  a.noise = nullptr; a.X_sim = nullptr; a.U_sim = nullptr; a.dX = nullptr; a.K = K;
+  a.N_sim = nullptr; a.slew_time = nullptr;
+}
+
 int ts_monte_carlo_run(ts_ctx* c, const ts_mc_config* cfg, const double* kep6, const ts_field_opts* fopts, const double* x0,
                        const double* xf, const double* Jmat, const double* q_noise0, const uint32_t* stream_id,
                        ts_trial_outcome* out, ts_mc_stats* stats) {
@@ -1118,12 +1184,9 @@ int ts_monte_carlo_run(ts_ctx* c, const ts_mc_config* cfg, const double* kep6, c
   const int64_t nf = cfg->shared_orbit ? 1 : n;
   const size_t NF = (size_t)nf;
   int rc;
-  cudaEvent_t e[7];
-  for (int i = 0; i < 7; ++i) cudaEventCreate(&e[i]);
-  struct EvGuard { cudaEvent_t* e; ~EvGuard() { for (int i = 0; i < 7; ++i) cudaEventDestroy(e[i]); } } evg{e};
-  c->mc_last.valid = false;
-  c->mc_last.resumable = false;
-  c->mc_last.replayable = false;
+  Events<7> e;
+  ts_ctx::McLast& L = c->mc_last;
+  L = {};
 
   // ---- stage 1: scoping pass (2*N_scope samples per orbit) + gramian cutoff
   std::vector<ts_field_opts> fo(NF);
@@ -1228,30 +1291,29 @@ int ts_monte_carlo_run(ts_ctx* c, const ts_mc_config* cfg, const double* kep6, c
     void* p_pos2;
     if ((rc = scratch_reserve(c, SLOT_POSITIONS, std::max((size_t)(offs_s[nf] + nf) * 3 * 8, (size_t)(offs_f[nf] + nf) * 3 * 8), &p_pos2))) return rc;
     // per-trial layout
-    std::vector<int64_t> hi(4 * NA + 1);
-    std::vector<double> hf((8 + 8 + 9 + 1 + 1 + 1 + 8 + 4) * NA);
+    McPacked P(NA);
     int64_t knots = 0;
     for (int64_t a = 0; a < na; ++a) {
       const int64_t t = act[a], f = cfg->shared_orbit ? 0 : t;
-      hi[a] = Nf[f];
-      hi[NA + a] = knots;
-      hi[2 * NA + a] = offs_f[f];
-      hi[3 * NA + a] = 2 * Nf[f];
+      P.col(I_N)[a] = Nf[f];
+      P.col(I_OFFS)[a] = knots;
+      P.col(I_B_OFFS)[a] = offs_f[f];
+      P.col(I_B_ROWS)[a] = 2 * Nf[f];
       knots += Nf[f];
-      memcpy(&hf[8 * a], x0 + 8 * t, 64);
-      memcpy(&hf[8 * NA + 8 * a], xf + 8 * t, 64);
-      memcpy(&hf[16 * NA + 9 * a], Jmat + 9 * t, 72);
-      hf[25 * NA + a] = tfin[f];
-      hf[26 * NA + a] = (double)Nf[f];
-      hf[27 * NA + a] = 1.0 / (cfg->tf - cfg->t0);
+      memcpy(P.at(F_X0, a), x0 + 8 * t, 64);
+      memcpy(P.at(F_XF, a), xf + 8 * t, 64);
+      memcpy(P.at(F_JMAT, a), Jmat + 9 * t, 72);
+      *P.at(F_T_FINAL, a) = tfin[f];
+      *P.at(F_INDEX_SCALE, a) = (double)Nf[f];
+      *P.at(F_CLOCK_RATE, a) = 1.0 / (cfg->tf - cfg->t0);
       // x0_lqr (TortoiseSat.jl:227-234): omega from x0, attitude perturbed by q_noise0, clock 0
-      tvlqr_x0_lqr(x0 + 8 * t, q_noise0 ? q_noise0 + 3 * t : nullptr, &hf[28 * NA + 8 * a]);
-      memcpy(&hf[36 * NA + 4 * a], xf + 8 * t + 3, 32);
+      tvlqr_x0_lqr(x0 + 8 * t, q_noise0 ? q_noise0 + 3 * t : nullptr, P.at(F_X0LQR, a));
+      memcpy(P.at(F_Q_FINAL, a), xf + 8 * t + 3, 32);
+      P.sid[a] = stream_id ? stream_id[t] : (uint32_t)t;
     }
-    hi[4 * NA] = knots;
-    int64_t* d_i; double* d_f;
-    if ((rc = upload(c, SLOT_PACKED_I64, hi.data(), hi.size(), &d_i))) return rc;
-    if ((rc = upload(c, SLOT_PACKED_F64, hf.data(), hf.size(), &d_f))) return rc;
+    P.hi.back() = knots;
+    McPackedView v;
+    if ((rc = upload_packed(c, P, SLOT_PACKED_I64, SLOT_PACKED_F64, v))) return rc;
     // device block: fine field tables, weights, X, U, outcomes, slew times
     const size_t b_B = (size_t)offs_f[nf] * 3 * 8, b_w = 19 * NA * 8, b_X = (size_t)knots * 8 * 8, b_U = (size_t)knots * 3 * 8,
                  b_o = NA * sizeof(ts_trial_outcome), b_s = NA * 16;
@@ -1274,31 +1336,25 @@ int ts_monte_carlo_run(ts_ctx* c, const ts_mc_config* cfg, const double* kep6, c
     }
     cudaEventRecord(e[2], c->stream);
     // ---- stage 3: eigen-axis guess + Bryson weights
+    const McWeights wt(d_Qd, NA);
     PrepArgs pa;
-    pa.n_trials = na; pa.x0 = d_f; pa.xf = d_f + 8 * NA; pa.Jmat = d_f + 16 * NA; pa.t_final = d_f + 25 * NA;
+    pa.n_trials = na; pa.x0 = v.col(F_X0); pa.xf = v.col(F_XF); pa.Jmat = v.col(F_JMAT); pa.t_final = v.col(F_T_FINAL);
     pa.t0 = cfg->t0; pa.dt = cfg->dt; pa.alpha = cfg->alpha; pa.beta = cfg->beta; pa.conj_fix = cfg->eigen_axis_fix ? 1 : 0;
-    pa.Qd = d_Qd; pa.Qfd = d_Qd + 8 * NA; pa.Rd = d_Qd + 16 * NA;
+    pa.Qd = wt.Qd; pa.Qfd = wt.Qfd; pa.Rd = wt.Rd;
     pa.goffs = nullptr; pa.w_guess = nullptr; pa.q_guess = nullptr;
     k_slew_prep<<<(unsigned)((na + 127) / 128), 128, 0, c->stream>>>(pa);
     c->launches++;
     cudaEventRecord(e[3], c->stream);
     // ---- stage 4: AL-iLQR
-    K3Args ka = {};
-    ka.n_trials = na;
-    ka.N_i = d_i; ka.offs = d_i + NA; ka.B_offs = d_i + 2 * NA; ka.B_rows = d_i + 3 * NA;
-    ka.x0 = d_f; ka.xf = d_f + 8 * NA; ka.Jmat = d_f + 16 * NA; ka.Qd = pa.Qd; ka.Qfd = pa.Qfd; ka.Rd = pa.Rd;
-    ka.index_scale = d_f + 26 * NA; ka.clock_rate = d_f + 27 * NA;
-    ka.B_eci = d_Bf; ka.dt = cfg->dt; ka.U0 = nullptr;
-    memcpy(&ka.opts, &cfg->ilqr, sizeof(ka.opts));
-    ka.X = d_X; ka.U = d_U; ka.K = nullptr; ka.out = d_out;
+    K3Args ka = fused_k3_args(v, wt, d_Bf, d_X, d_U, d_out, cfg->ilqr, cfg->dt);
     std::vector<double> diff(NA);
     for (int64_t aa = 0; aa < na; ++aa) diff[aa] = slew_angle(x0 + 8 * act[aa], xf + 8 * act[aa]);
     // keep_trajectories = 2: the solve runs the exporting instantiations, its states and multipliers go to a kept slot
     K3StateIO sio = {};
     void* p_st = nullptr;
-    const bool resumable = cfg->keep_trajectories == 2;
+    const bool keep_state = cfg->keep_trajectories == 2;
     const size_t b_st = NA * sizeof(ts_al_state);
-    if (resumable) {
+    if (keep_state) {
       if ((rc = scratch_reserve(c, SLOT_KEPT_STATE, b_st + 64 + (size_t)knots * 6 * 8, &p_st))) return rc;
       sio.state_out = (ts_al_state_dev*)p_st;
       sio.lam_out = (double*)((char*)p_st + b_st + 64);
@@ -1311,29 +1367,19 @@ int ts_monte_carlo_run(ts_ctx* c, const ts_mc_config* cfg, const double* kep6, c
     K4Args k4;
     if (cfg->run_tvlqr) {
       if ((rc = scratch_reserve(c, SLOT_K4_GAINS, (size_t)knots * 18 * 8, &p_K))) return rc;
-      std::vector<uint32_t> sid(NA);
-      for (int64_t a = 0; a < na; ++a) sid[a] = stream_id ? stream_id[act[a]] : (uint32_t)act[a];
-      if ((rc = upload(c, SLOT_STREAM_IDS, sid.data(), NA, &d_sid))) return rc;
-      if ((rc = k4_lin_table(c, hi.data(), NA, k4))) return rc;
+      if ((rc = upload(c, SLOT_STREAM_IDS, P.sid.data(), NA, &d_sid))) return rc;
+      if ((rc = k4_lin_table(c, P.col(I_N), NA, k4))) return rc;
       if (cfg->keep_trajectories) {
         if ((rc = scratch_reserve(c, SLOT_KEPT_XSIM, (size_t)knots * 8 * 8 + 64, &p_xs))) return rc;
         if ((rc = scratch_reserve(c, SLOT_KEPT_USIM, (size_t)knots * 3 * 8 + 64, &p_us))) return rc;
       }
     }
-    if ((rc = k3_launch(c, ka, hi.data(), diff.data(), all_inertia_diagonal(Jmat, n), nullptr, resumable ? &sio : nullptr))) return rc;
+    if ((rc = k3_launch(c, ka, P.col(I_N), diff.data(), all_inertia_diagonal(Jmat, n), nullptr, keep_state ? &sio : nullptr))) return rc;
     cudaEventRecord(e[4], c->stream);
     // ---- stage 5: TVLQR replay + slew-time rule
     double *d_Xs_keep = nullptr, *d_Us_keep = nullptr;
     if (cfg->run_tvlqr) {
-      k4.n_trials = na; k4.N_i = d_i; k4.offs = d_i + NA; k4.B_offs = d_i + 2 * NA; k4.B_rows = d_i + 3 * NA;
-      k4.X_lqr = d_X; k4.U_lqr = d_U; k4.x0_lqr = d_f + 28 * NA; k4.Jmat = d_f + 16 * NA; k4.B_eci = d_Bf;
-      k4.index_scale = d_f + 26 * NA; k4.clock_rate = d_f + 27 * NA; k4.t_final = d_f + 25 * NA; k4.q_final = d_f + 36 * NA;
-      k4.stream_id = d_sid;
-      memcpy(&k4.opts, &cfg->tvlqr, sizeof(k4.opts));
-      k4.opts.dt = cfg->dt; k4.opts.t0 = cfg->t0;
-      if (k4.opts.noise_mode == 1) k4.opts.noise_mode = 2;  // no explicit array in the fused path
-      k4.opts.literal_postproc = 0;                          // needs X_sim storage; fused path uses the fixed rule (Q12)
-      k4.noise = nullptr; k4.X_sim = nullptr; k4.U_sim = nullptr; k4.dX = nullptr; k4.K = (double*)p_K;
+      fused_k4_args(k4, v, d_X, d_U, d_Bf, (double*)p_K, d_sid, *cfg);
       if (cfg->keep_trajectories) {
         TS_CUDA(c, cudaMemsetAsync(p_xs, 0, (size_t)knots * 8 * 8, c->stream));
         TS_CUDA(c, cudaMemsetAsync(p_us, 0, (size_t)knots * 3 * 8, c->stream));
@@ -1350,25 +1396,21 @@ int ts_monte_carlo_run(ts_ctx* c, const ts_mc_config* cfg, const double* kep6, c
     TS_CUDA(c, cudaMemcpyAsync(oa.data(), d_out, b_o, cudaMemcpyDeviceToHost, c->stream));
     if (cfg->run_tvlqr) TS_CUDA(c, cudaMemcpyAsync(slew.data(), d_slew, NA * 8, cudaMemcpyDeviceToHost, c->stream));
     TS_CUDA(c, cudaStreamSynchronize(c->stream));
-    float ms = 0;
-    cudaEventElapsedTime(&ms, e[0], e[6]); ms_field = ms;
-    cudaEventElapsedTime(&ms, e[1], e[2]); ms_field += ms;
-    cudaEventElapsedTime(&ms, e[2], e[3]); ms_prep = ms;
-    cudaEventElapsedTime(&ms, e[3], e[4]); ms_solve = ms;
-    cudaEventElapsedTime(&ms, e[4], e[5]); ms_tvlqr = ms;
-    const bool dj_ = all_inertia_diagonal(Jmat, n) && !cfg->ilqr.k3_generic_inertia;
-    const double fl_iter = dj_ ? FL_ITER_DIAG : FL_ITER, fl_roll = dj_ ? FL_ROLL_DIAG : FL_ROLL;
+    ms_field = e.ms(0, 6);
+    ms_field += e.ms(1, 2);
+    ms_prep = e.ms(2, 3);
+    ms_solve = e.ms(3, 4);
+    ms_tvlqr = e.ms(4, 5);
+    const bool dj = all_inertia_diagonal(Jmat, n) && !cfg->ilqr.k3_generic_inertia;
     for (int64_t a = 0; a < na; ++a) {
       const int64_t t = act[a], f = cfg->shared_orbit ? 0 : t;
       out[t] = oa[a];
       out[t].t_final = tfin[f];
       out[t].slew_time = cfg->run_tvlqr ? slew[a] : 0.0;
-      const double kn = (double)(Nf[f] - 1);
-      out[t].flops = kn * ((double)oa[a].inner_iters * fl_iter + (double)oa[a].ls_rollouts * fl_roll) + (cfg->run_tvlqr ? kn * FL_TVLQR : 0.0);
+      out[t].flops = trial_flops(dj, Nf[f], oa[a].inner_iters, oa[a].ls_rollouts, cfg->run_tvlqr != 0);
     }
     if (cfg->keep_trajectories) {
-      ts_ctx::McLast& L = c->mc_last;
-      L.n = n; L.knots = knots; L.rows = offs_f[nf];
+      L.knots = knots; L.rows = offs_f[nf];
       L.knot_offs.assign((size_t)n + 1, 0);
       L.row_offs.assign((size_t)n + 1, 0);
       for (int64_t t = 0; t < n; ++t) {
@@ -1378,37 +1420,23 @@ int ts_monte_carlo_run(ts_ctx* c, const ts_mc_config* cfg, const double* kep6, c
       }
       L.row_offs[n] = offs_f[nf];
       L.d_X = d_X; L.d_U = d_U; L.d_Xs = d_Xs_keep; L.d_Us = d_Us_keep; L.d_B = d_Bf;
-      L.valid = true;
       // the host side of the kept run: what ts_mc_replay_ensemble (and, with keep_trajectories = 2, ts_mc_continue) needs
       L.diag_inertia = all_inertia_diagonal(Jmat, n);
       L.act = act;
-      L.hi = hi;
-      L.hf = hf;
-      L.sid.clear();
-      for (int64_t a = 0; a < na; ++a) L.sid.push_back(stream_id ? stream_id[act[a]] : (uint32_t)act[a]);
+      L.in = std::move(P);
     }
-    if (resumable) {
-      ts_ctx::McLast& L = c->mc_last;
-      L.d_i = d_i; L.d_f = d_f; L.d_w = d_Qd; L.d_sid = d_sid;
+    if (keep_state) {
+      L.d_in = v; L.d_w = d_Qd;
       L.d_out = (ts_trial_outcome*)d_out;
       L.d_state = (ts_al_state*)p_st;
       L.d_sio = (char*)p_st + b_st;
       L.d_lam = sio.lam_out;
     }
   }
-  if (cfg->keep_trajectories >= 1) {
-    ts_ctx::McLast& L = c->mc_last;
-    if (na == 0) {   // nothing reached the solver: a run that continues nothing and replays only NO_CUTOFF rows
-      L.act.clear();
-      L.sid.clear();
-      L.knots = 0;
-      L.knot_offs.assign((size_t)n + 1, 0);
-    }
-    L.n = n;
+  if (cfg->keep_trajectories) {
     L.cfg = *cfg;
+    L.n = n;
     L.out.assign(out, out + n);
-    L.replayable = true;
-    L.resumable = cfg->keep_trajectories == 2;
   }
   c->last_kernel_ms = ms_field + ms_prep + ms_solve + ms_tvlqr;
   if (stats) {
@@ -1421,7 +1449,7 @@ int ts_monte_carlo_run(ts_ctx* c, const ts_mc_config* cfg, const double* kep6, c
 int ts_mc_trajectory_layout(ts_ctx* c, int64_t n_trials, int64_t* knot_offs, int64_t* row_offs) {
   if (!c) return TS_ERR_ARG;
   const ts_ctx::McLast& L = c->mc_last;
-  if (!L.valid) return fail(c, TS_ERR_ARG, "no Monte-Carlo run with keep_trajectories = 1 on this context");
+  if (!L.cfg.keep_trajectories || L.act.empty()) return fail(c, TS_ERR_ARG, "no Monte-Carlo run with keep_trajectories = 1 on this context");
   if (n_trials != L.n) return fail(c, TS_ERR_ARG, "the kept run had %lld trials", (long long)L.n);
   if (knot_offs) memcpy(knot_offs, L.knot_offs.data(), (size_t)(L.n + 1) * 8);
   if (row_offs) memcpy(row_offs, L.row_offs.data(), (size_t)(L.n + 1) * 8);
@@ -1431,7 +1459,7 @@ int ts_mc_trajectory_layout(ts_ctx* c, int64_t n_trials, int64_t* knot_offs, int
 int ts_mc_fetch_trajectories(ts_ctx* c, double* X, double* U, double* X_sim, double* U_sim, double* B_eci) {
   if (!c) return TS_ERR_ARG;
   const ts_ctx::McLast& L = c->mc_last;
-  if (!L.valid) return fail(c, TS_ERR_ARG, "no Monte-Carlo run with keep_trajectories = 1 on this context");
+  if (!L.cfg.keep_trajectories || L.act.empty()) return fail(c, TS_ERR_ARG, "no Monte-Carlo run with keep_trajectories = 1 on this context");
   if ((X_sim || U_sim) && !L.d_Xs) return fail(c, TS_ERR_ARG, "the kept run had run_tvlqr = 0: no X_sim / U_sim");
   TS_CUDA(c, cudaSetDevice(c->device));
   const size_t K = (size_t)L.knots;
@@ -1447,7 +1475,7 @@ int ts_mc_fetch_trajectories(ts_ctx* c, double* X, double* U, double* X_sim, dou
 int ts_mc_fetch_state(ts_ctx* c, ts_al_state* state, double* lam) {
   if (!c) return TS_ERR_ARG;
   const ts_ctx::McLast& L = c->mc_last;
-  if (!L.resumable) return fail(c, TS_ERR_ARG, "no Monte-Carlo run with keep_trajectories = 2 on this context");
+  if (L.cfg.keep_trajectories != 2) return fail(c, TS_ERR_ARG, "no Monte-Carlo run with keep_trajectories = 2 on this context");
   TS_CUDA(c, cudaSetDevice(c->device));
   const size_t NA = L.act.size();
   std::vector<ts_al_state> st(NA);
@@ -1462,52 +1490,26 @@ int ts_mc_fetch_state(ts_ctx* c, ts_al_state* state, double* lam) {
   return TS_OK;
 }
 
-// The packed per-trial arrays of the kept run (ts_monte_carlo_run's layouts: hi = N | offs | B_offs | B_rows, hf = x0 xf
-// Jmat t_final index_scale clock_rate x0_lqr q_final) and stream ids, compacted to the active trials sel (indices into
-// L.act, repeats allowed) for a replay of those trials alone; the knot and row offsets keep pointing into the full kept
-// arrays.  hic[4 NC] = the kept run's knot count.
-static void compact_kept(const ts_ctx::McLast& L, const std::vector<int64_t>& sel, std::vector<int64_t>& hic, std::vector<double>& hfc,
-                         std::vector<uint32_t>& sidc) {
-  const size_t NA = L.act.size(), NC = sel.size();
-  hic.assign(4 * NC + 1, 0);
-  hfc.assign(40 * NC, 0.0);
-  sidc.assign(NC, 0u);
-  for (size_t k = 0; k < NC; ++k) {
-    const size_t a = (size_t)sel[k];
-    for (int j = 0; j < 4; ++j) hic[j * NC + k] = L.hi[j * NA + a];
-    static const int width[] = {8, 8, 9, 1, 1, 1, 8, 4};   // x0 xf Jmat t_final index_scale clock_rate x0_lqr q_final
-    size_t base = 0;
-    for (int w : width) {
-      memcpy(&hfc[base * NC + w * k], &L.hf[base * NA + w * a], (size_t)w * 8);
-      base += (size_t)w;
-    }
-    sidc[k] = L.sid[a];
-  }
-  hic[4 * NC] = L.knots;
-}
-
 // MC1-MC3 (DESIGN.md section 4, K3).  The continuing trials are solved on the kept block in place, exactly as
 // ts_alilqr_solve_state_batch continues them over the run's active trials, and replayed on their own.
 int ts_mc_continue(ts_ctx* c, int64_t n_trials, const ts_ilqr_opts* opts, ts_trial_outcome* out, ts_mc_stats* stats) {
   if (!c) return TS_ERR_ARG;
   ts_ctx::McLast& L = c->mc_last;
-  if (!L.resumable) return fail(c, TS_ERR_ARG, "ts_mc_continue: no Monte-Carlo run with keep_trajectories = 2 on this context");
+  if (L.cfg.keep_trajectories != 2) return fail(c, TS_ERR_ARG, "ts_mc_continue: no Monte-Carlo run with keep_trajectories = 2 on this context");
   if (n_trials != L.n) return fail(c, TS_ERR_ARG, "ts_mc_continue: the kept run had %lld trials", (long long)L.n);
   if (!opts || !out) return fail(c, TS_ERR_ARG, "ts_mc_continue: null argument");
   const ts_ilqr_opts& o = *opts;
-  if (o.max_linesearch < 0 || o.max_linesearch > 63) return fail(c, TS_ERR_ARG, "max_linesearch must be in [0,63]");
   const int64_t na = (int64_t)L.act.size();
   const size_t NA = (size_t)na;
   const ts_mc_config& cfg = L.cfg;
   TS_CUDA(c, cudaSetDevice(c->device));
-  if (o.quat_error && na > 0) {   // the check of ts_alilqr_solve_state_batch, on the run's weights
-    std::vector<double> w(16 * NA);
-    TS_CUDA(c, cudaMemcpy(w.data(), L.d_w, w.size() * 8, cudaMemcpyDeviceToHost));
-    for (size_t k = 0; k < 2 * NA; ++k)
-      for (int i = 4; i < 7; ++i)
-        if (w[8 * k + i] != w[8 * k + 3])
-          return fail(c, TS_ERR_ARG, "quat_error: the four quaternion weights of Q and Qf must be equal (E'QE is then diagonal)");
-  }
+  int rc;
+  // the option checks of ts_alilqr_solve_state_batch; quat_error's reads the run's weights back
+  const size_t nw = o.quat_error ? NA : 0;
+  std::vector<double> w(16 * nw);
+  if (nw) TS_CUDA(c, cudaMemcpy(w.data(), L.d_w, w.size() * 8, cudaMemcpyDeviceToHost));
+  const McWeights hw(w.data(), nw);
+  if ((rc = check_ilqr_opts(c, o, (int64_t)nw, hw.Qd, hw.Qfd))) return rc;
   // MC1: CS2 on the kept states (their status and outer count are the kept records')
   std::vector<int64_t> cont;
   for (int64_t a = 0; a < na; ++a) {
@@ -1519,65 +1521,39 @@ int ts_mc_continue(ts_ctx* c, int64_t n_trials, const ts_ilqr_opts* opts, ts_tri
   std::vector<ts_trial_outcome> rec = L.out;
   if (NC == 0) c->k3_timed = false;   // no solve: ts_k3_last_split / ts_k3_last_parked report nothing
   if (NC > 0) {
-    const int64_t* hi = L.hi.data();
-    const double* hf = L.hf.data();
-    int rc;
     // MC3: the replay's per-trial arrays, compacted to the continuing trials
-    std::vector<int64_t> hic;
-    std::vector<double> hfc;
-    std::vector<uint32_t> sidc;
-    compact_kept(L, cont, hic, hfc, sidc);
+    const McPacked P = L.in.compact(cont);
+    McPackedView v;
     void *p_q = nullptr, *p_K = nullptr;
-    int64_t* d_ic = nullptr;
-    double* d_fc = nullptr;
     K4Args k4;
     if (cfg.run_tvlqr) {
-      if ((rc = upload(c, SLOT_ARGS_A, hic.data(), hic.size(), &d_ic))) return rc;
-      if ((rc = upload(c, SLOT_ARGS_B, hfc.data(), hfc.size(), &d_fc))) return rc;
+      if ((rc = upload_packed(c, P, SLOT_ARGS_A, SLOT_ARGS_B, v))) return rc;
       if ((rc = scratch_reserve(c, SLOT_ARGS_C, NC * 20 + 64, &p_q))) return rc;
-      TS_CUDA(c, cudaMemcpyAsync(p_q, sidc.data(), NC * 4, cudaMemcpyHostToDevice, c->stream));
+      TS_CUDA(c, cudaMemcpyAsync(p_q, P.sid.data(), NC * 4, cudaMemcpyHostToDevice, c->stream));
       if ((rc = scratch_reserve(c, SLOT_K4_GAINS, (size_t)L.knots * 18 * 8, &p_K))) return rc;
-      if ((rc = k4_lin_table(c, hic.data(), NC, k4))) return rc;
+      if ((rc = k4_lin_table(c, P.col(I_N), NC, k4))) return rc;
     }
     // MC2: the K3 arguments of the run, on the kept block; the states and multipliers are read and written in place
-    K3Args ka = {};
-    ka.n_trials = na;
-    ka.N_i = L.d_i; ka.offs = L.d_i + NA; ka.B_offs = L.d_i + 2 * NA; ka.B_rows = L.d_i + 3 * NA;
-    ka.x0 = L.d_f; ka.xf = L.d_f + 8 * NA; ka.Jmat = L.d_f + 16 * NA;
-    ka.Qd = L.d_w; ka.Qfd = L.d_w + 8 * NA; ka.Rd = L.d_w + 16 * NA;
-    ka.index_scale = L.d_f + 26 * NA; ka.clock_rate = L.d_f + 27 * NA;
-    ka.B_eci = L.d_B; ka.dt = cfg.dt; ka.U0 = nullptr;
-    memcpy(&ka.opts, &o, sizeof(ka.opts));
-    ka.X = L.d_X; ka.U = L.d_U; ka.K = nullptr; ka.out = (ts_trial_outcome_dev*)L.d_out;
+    K3Args ka = fused_k3_args(L.d_in, McWeights(L.d_w, NA), L.d_B, L.d_X, L.d_U, (ts_trial_outcome_dev*)L.d_out, o, cfg.dt);
     ka.sio = (const K3StateIO*)L.d_sio;
     K3StateIO sio = {};
     sio.state_in = sio.state_out = (ts_al_state_dev*)L.d_state;
     sio.lam_in = sio.lam_out = L.d_lam;
     sio.lam_doubles = L.knots * 6;
     std::vector<double> diff(NA);
-    for (size_t a = 0; a < NA; ++a) diff[a] = slew_angle(hf + 8 * a, hf + 8 * NA + 8 * a);
-    cudaEvent_t e[3];
-    for (int i = 0; i < 3; ++i) cudaEventCreate(&e[i]);
-    struct EvGuard { cudaEvent_t* e; ~EvGuard() { for (int i = 0; i < 3; ++i) cudaEventDestroy(e[i]); } } evg{e};
+    for (size_t a = 0; a < NA; ++a) diff[a] = slew_angle(L.in.at(F_X0, a), L.in.at(F_XF, a));
+    Events<3> e;
     cudaEventRecord(e[0], c->stream);
     // X, U, the states and lam are input and output of the same call.  That is safe because park_import_kernel, the
     // first kernel k3_launch queues for a continuation, reads every imported row (X, U, lam_in, state_in) before the
     // straggler kernel that follows it on the stream writes any.  k3_launch fails before it queues anything that writes
     // kept storage (TS_ERR_NOMEM when the parked records do not fit), so the kept run stays continuable.
-    if ((rc = k3_launch(c, ka, hi, diff.data(), L.diag_inertia, &cont, &sio))) return rc;
+    if ((rc = k3_launch(c, ka, L.in.col(I_N), diff.data(), L.diag_inertia, &cont, &sio))) return rc;
     cudaEventRecord(e[1], c->stream);
     if (cfg.run_tvlqr) {
-      k4_clear_rows_kernel<<<(unsigned)NC, 256, 0, c->stream>>>((int64_t)NC, d_ic, d_ic + NC, L.d_Xs, L.d_Us);
+      k4_clear_rows_kernel<<<(unsigned)NC, 256, 0, c->stream>>>((int64_t)NC, v.col(I_N), v.col(I_OFFS), L.d_Xs, L.d_Us);
       c->launches++;
-      k4.n_trials = (int64_t)NC; k4.N_i = d_ic; k4.offs = d_ic + NC; k4.B_offs = d_ic + 2 * NC; k4.B_rows = d_ic + 3 * NC;
-      k4.X_lqr = L.d_X; k4.U_lqr = L.d_U; k4.x0_lqr = d_fc + 28 * NC; k4.Jmat = d_fc + 16 * NC; k4.B_eci = L.d_B;
-      k4.index_scale = d_fc + 26 * NC; k4.clock_rate = d_fc + 27 * NC; k4.t_final = d_fc + 25 * NC; k4.q_final = d_fc + 36 * NC;
-      k4.stream_id = (const uint32_t*)p_q;
-      memcpy(&k4.opts, &cfg.tvlqr, sizeof(k4.opts));   // with the fused run's overrides
-      k4.opts.dt = cfg.dt; k4.opts.t0 = cfg.t0;
-      if (k4.opts.noise_mode == 1) k4.opts.noise_mode = 2;
-      k4.opts.literal_postproc = 0;
-      k4.noise = nullptr; k4.dX = nullptr; k4.K = (double*)p_K;
+      fused_k4_args(k4, v, L.d_X, L.d_U, L.d_B, (double*)p_K, (const uint32_t*)p_q, cfg);
       k4.X_sim = L.d_Xs; k4.U_sim = L.d_Us;
       k4.N_sim = (int64_t*)((char*)p_q + ((NC * 4 + 15) & ~(size_t)15));
       k4.slew_time = (double*)(k4.N_sim + NC);
@@ -1590,22 +1566,18 @@ int ts_mc_continue(ts_ctx* c, int64_t n_trials, const ts_ilqr_opts* opts, ts_tri
     TS_CUDA(c, cudaMemcpyAsync(oa.data(), L.d_out, NA * sizeof(ts_trial_outcome), cudaMemcpyDeviceToHost, c->stream));
     if (cfg.run_tvlqr) TS_CUDA(c, cudaMemcpyAsync(slew.data(), k4.slew_time, NC * 8, cudaMemcpyDeviceToHost, c->stream));
     TS_CUDA(c, cudaStreamSynchronize(c->stream));
-    float ms = 0;
-    cudaEventElapsedTime(&ms, e[0], e[1]); ms_solve = ms;
-    if (cfg.run_tvlqr) { cudaEventElapsedTime(&ms, e[1], e[2]); ms_tvlqr = ms; }
-    const bool dj_ = L.diag_inertia && !o.k3_generic_inertia;
-    const double fl_iter = dj_ ? FL_ITER_DIAG : FL_ITER, fl_roll = dj_ ? FL_ROLL_DIAG : FL_ROLL;
+    ms_solve = e.ms(0, 1);
+    if (cfg.run_tvlqr) ms_tvlqr = e.ms(1, 2);
+    const bool dj = L.diag_inertia && !o.k3_generic_inertia, tv = cfg.run_tvlqr != 0;
     for (size_t k = 0; k < NC; ++k) {
       const int64_t t = L.act[(size_t)cont[k]];
       const ts_trial_outcome& prev = L.out[(size_t)t];
       ts_trial_outcome r = oa[(size_t)cont[k]];
-      const double kn = (double)(prev.N - 1);
       r.N = prev.N;
       r.t_final = prev.t_final;
       r.slew_time = cfg.run_tvlqr ? slew[k] : 0.0;
-      r.flops = kn * ((double)r.inner_iters * fl_iter + (double)r.ls_rollouts * fl_roll) + (cfg.run_tvlqr ? kn * FL_TVLQR : 0.0);
-      flops += kn * ((double)(r.inner_iters - prev.inner_iters) * fl_iter + (double)(r.ls_rollouts - prev.ls_rollouts) * fl_roll) +
-               (cfg.run_tvlqr ? kn * FL_TVLQR : 0.0);
+      r.flops = trial_flops(dj, prev.N, r.inner_iters, r.ls_rollouts, tv);
+      flops += trial_flops(dj, prev.N, r.inner_iters - prev.inner_iters, r.ls_rollouts - prev.ls_rollouts, tv);
       rec[(size_t)t] = r;
     }
     L.out = rec;
@@ -1627,7 +1599,7 @@ int ts_mc_replay_ensemble(ts_ctx* c, int64_t n_trials, const ts_replay_ensemble_
                           double* slew_time, double* x_final) {
   if (!c) return TS_ERR_ARG;
   const ts_ctx::McLast& L = c->mc_last;
-  if (!L.replayable) return fail(c, TS_ERR_ARG, "ts_mc_replay_ensemble: no Monte-Carlo run with keep_trajectories >= 1 on this context");
+  if (L.cfg.keep_trajectories < 1) return fail(c, TS_ERR_ARG, "ts_mc_replay_ensemble: no Monte-Carlo run with keep_trajectories >= 1 on this context");
   if (n_trials != L.n) return fail(c, TS_ERR_ARG, "ts_mc_replay_ensemble: the kept run had %lld trials", (long long)L.n);
   if (!opts || !slew_time) return fail(c, TS_ERR_ARG, "ts_mc_replay_ensemble: null argument");
   const int64_t R = opts->n_real, r0 = opts->r_first;
@@ -1644,7 +1616,7 @@ int ts_mc_replay_ensemble(ts_ctx* c, int64_t n_trials, const ts_replay_ensemble_
   for (int64_t p = 0; p < n_sel; ++p)
     if (act_of[(size_t)(trials ? trials[p] : p)] >= 0) pos.push_back(p);
   auto act_at = [&](int64_t p) { return act_of[(size_t)(trials ? trials[p] : p)]; };
-  std::stable_sort(pos.begin(), pos.end(), [&](int64_t u, int64_t v) { return L.hi[(size_t)act_at(u)] > L.hi[(size_t)act_at(v)]; });
+  std::stable_sort(pos.begin(), pos.end(), [&](int64_t u, int64_t v) { return L.in.col(I_N)[act_at(u)] > L.in.col(I_N)[act_at(v)]; });
   const size_t NC = pos.size(), RR = (size_t)R;
   const size_t per = x_final ? 9 : 1;   // doubles per (trial, realisation) row
   std::vector<double> hs(NC * RR), hx(x_final ? NC * RR * 8 : 0);
@@ -1654,46 +1626,25 @@ int ts_mc_replay_ensemble(ts_ctx* c, int64_t n_trials, const ts_replay_ensemble_
     TS_CUDA(c, cudaSetDevice(c->device));
     std::vector<int64_t> sel(NC);
     for (size_t k = 0; k < NC; ++k) sel[k] = act_at(pos[k]);
-    std::vector<int64_t> hic;
-    std::vector<double> hfc;
-    std::vector<uint32_t> sidc;
-    compact_kept(L, sel, hic, hfc, sidc);
+    const McPacked P = L.in.compact(sel);
     int rc;
-    void *p_out, *p_K, *p_s;
+    void *p_out, *p_K;
     if ((rc = scratch_reserve(c, SLOT_ENSEMBLE_OUT, NC * RR * per * 8 + 64, &p_out))) return rc;
     if ((rc = scratch_reserve(c, SLOT_K4_GAINS, (size_t)L.knots * 18 * 8, &p_K))) return rc;
-    int64_t* d_ic;
-    double* d_fc;
-    if ((rc = upload(c, SLOT_ARGS_A, hic.data(), hic.size(), &d_ic))) return rc;
-    if ((rc = upload(c, SLOT_ARGS_B, hfc.data(), hfc.size(), &d_fc))) return rc;
-    if ((rc = upload(c, SLOT_ARGS_C, sidc.data(), NC, (uint32_t**)&p_s))) return rc;
+    McPackedView v;
+    uint32_t* d_sid;
+    if ((rc = upload_packed(c, P, SLOT_ARGS_A, SLOT_ARGS_B, v))) return rc;
+    if ((rc = upload(c, SLOT_ARGS_C, P.sid.data(), NC, &d_sid))) return rc;
     K4Args k4;
-    if ((rc = k4_lin_table(c, hic.data(), NC, k4))) return rc;
-    const ts_mc_config& cfg = L.cfg;
-    k4.n_trials = (int64_t)NC; k4.N_i = d_ic; k4.offs = d_ic + NC; k4.B_offs = d_ic + 2 * NC; k4.B_rows = d_ic + 3 * NC;
-    k4.X_lqr = L.d_X; k4.U_lqr = L.d_U; k4.x0_lqr = d_fc + 28 * NC; k4.Jmat = d_fc + 16 * NC; k4.B_eci = L.d_B;
-    k4.index_scale = d_fc + 26 * NC; k4.clock_rate = d_fc + 27 * NC; k4.t_final = d_fc + 25 * NC; k4.q_final = d_fc + 36 * NC;
-    k4.stream_id = (const uint32_t*)p_s;
-    memcpy(&k4.opts, &cfg.tvlqr, sizeof(k4.opts));   // RE2: the run's options with the fused path's overrides
-    k4.opts.dt = cfg.dt; k4.opts.t0 = cfg.t0;
-    k4.opts.noise_mode = 2;                          // realisations always draw
-    k4.opts.literal_postproc = 0;
-    k4.noise = nullptr; k4.X_sim = nullptr; k4.U_sim = nullptr; k4.dX = nullptr; k4.K = (double*)p_K;
-    k4.N_sim = nullptr; k4.slew_time = nullptr;
-    K4eArgs e;
-    e.n_sel = (int64_t)NC; e.N_i = k4.N_i; e.offs = k4.offs; e.B_offs = k4.B_offs; e.B_rows = k4.B_rows;
-    e.X_lqr = L.d_X; e.U_lqr = L.d_U; e.K = k4.K;
-    e.clk = k4.clk; e.lin_offs = k4.lin_offs;
-    e.x0 = d_fc; e.x0_lqr = k4.x0_lqr; e.Jmat = k4.Jmat; e.B_eci = L.d_B; e.index_scale = k4.index_scale;
-    e.clock_rate = k4.clock_rate; e.t_final = k4.t_final; e.q_final = k4.q_final; e.stream_id = k4.stream_id;
-    e.opts = k4.opts;
+    if ((rc = k4_lin_table(c, P.col(I_N), NC, k4))) return rc;
+    fused_k4_args(k4, v, L.d_X, L.d_U, L.d_B, (double*)p_K, d_sid, L.cfg);   // RE2: the run's options with the overrides
+    k4.opts.noise_mode = 2;                                                  // realisations always draw
+    K4eArgs e = k4e_args(k4, v.col(F_X0));
     e.n_real = R; e.r_first = r0; e.n_blk = (R + 31) / 32;
     e.q_noise_scale = opts->q_noise_scale;
     e.slew_time = (double*)p_out;
     e.x_final = x_final ? e.slew_time + NC * RR : nullptr;
-    cudaEvent_t ev[3];
-    for (int i = 0; i < 3; ++i) cudaEventCreate(&ev[i]);
-    struct EvGuard { cudaEvent_t* e; ~EvGuard() { for (int i = 0; i < 3; ++i) cudaEventDestroy(e[i]); } } evg{ev};
+    Events<3> ev;
     cudaEventRecord(ev[0], c->stream);
     k4_gains_launch(c, k4);
     cudaEventRecord(ev[1], c->stream);
@@ -1705,9 +1656,8 @@ int ts_mc_replay_ensemble(ts_ctx* c, int64_t n_trials, const ts_replay_ensemble_
     TS_CUDA(c, cudaMemcpyAsync(hs.data(), e.slew_time, NC * RR * 8, cudaMemcpyDeviceToHost, c->stream));
     if (x_final) TS_CUDA(c, cudaMemcpyAsync(hx.data(), e.x_final, NC * RR * 64, cudaMemcpyDeviceToHost, c->stream));
     TS_CUDA(c, cudaStreamSynchronize(c->stream));
-    float ms = 0;
-    cudaEventElapsedTime(&ms, ev[0], ev[1]); c->ens_ms[0] = ms;
-    cudaEventElapsedTime(&ms, ev[1], ev[2]); c->ens_ms[1] = ms;
+    c->ens_ms[0] = ev.ms(0, 1);
+    c->ens_ms[1] = ev.ms(1, 2);
     c->last_kernel_ms = c->ens_ms[0] + c->ens_ms[1];
   }
   // rows in the caller's order; a NO_CUTOFF trial gets NaN rows
