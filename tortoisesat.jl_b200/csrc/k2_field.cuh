@@ -315,7 +315,8 @@ k2c_gramian_cutoff(int64_t n_trials, const double* __restrict__ B_eci, const int
 // previous chunks / of an earlier call, `carry` 6 doubles per orbit) -> cond() of every prefix in parallel -> the first
 // sample below the cutoff by ballot.  The prefix sums are formed pairwise instead of left to right, i.e. they differ from
 // the sequential gramian in the last bits (relative 1e-16) -- far below the ~1e-4 by which cond() moves per sample, so
-// the index is the same (tests compare it with the oracle's on every trial).  tf_index[t] != 0 on entry: nothing to do.
+// the index is the same (tests/test_gpu_scoping.py: hits on chunk and range edges, the benchmark sweep's second-range
+// orbits).  tf_index[t] != 0 on entry: nothing to do.
 constexpr int K2C_THREADS = 128;
 __global__ void __launch_bounds__(K2C_THREADS)
 k2c_cutoff_scan(const double* __restrict__ B_eci, const int64_t* __restrict__ B_offs, const int64_t* __restrict__ rows,
