@@ -421,6 +421,38 @@ int ts_mc_replay_ensemble(ts_ctx* ctx, int64_t n_trials, const ts_replay_ensembl
                           const int64_t* trials, double* slew_time, double* x_final);
 int ts_mc_replay_ensemble_last_split(ts_ctx* ctx, double* gains_ms, double* replay_ms);
 
+/* ---- dispersion ensembles: the kept run's slews under drawn truth-model errors ----------------------------------- *
+ * ts_mc_dispersion_ensemble replays the kept run's slews as ts_mc_replay_ensemble does, with the TVLQR gains of the
+ * nominal model, but each realisation's "truth" dynamics carry drawn errors of the inertia, the torquer gains and the
+ * field model (DESIGN.md section 4, K4):
+ *  DE1 the kept run: as RE1, with the argument checks of ts_mc_replay_ensemble.
+ *  DE2 the draws of realisation r: the stage noise and (r >= 1) the initial attitude of RE2, and ten standard normals
+ *      z0..z9 with key = the run's tvlqr.seed, counters (stream, 0xFFFFFFFE, 0, 4r + b), b = 0, 1, 2: (z0, z1) and
+ *      (z2, z3) = box_muller of block 0's (o0, o1) and (o2, o3), (z4 .. z7) the same of block 1, (z8, z9) = box_muller
+ *      of block 2's (o0, o1).  Parameters: d_i = exp(sigma_inertia z_i / 2) (i = 0..2), truth inertia
+ *      J_true[i][j] = (d_i J[i][j]) d_j; g_i = exp(sigma_torquer z_{3+i}), truth torque ((u_i * 0.01) g_i) x B_B;
+ *      s_B = exp(sigma_field_scale z6) and phi = sigma_field_angle (z7, z8, z9) rad, p = [cos(|phi|/2);
+ *      phi/|phi| sin(|phi|/2)] (identity for |phi| <= 1e-300): truth field of a stage = s_B qrot(p, B_row) + B_noise.
+ *      A group with sigma 0 keeps its nominal value exactly (1, 1, 1 / no rotation); each group reads fixed normals,
+ *      so one sigma leaves the other groups' parameters and the stage noise unchanged (paired one-factor studies).
+ *  DE3 realisation 0 carries no dispersion whatever the sigmas: its row is RE3's, bit for bit.
+ *  DE4 with all four sigmas 0 every row equals ts_mc_replay_ensemble's row for the same (trial, r, q_noise_scale).
+ *  DE5 a row depends on the kept run, t, r, q_noise_scale and the sigmas alone (as RE4).
+ *  DE6 isolation, as RE5: later calls behave as if this call never ran.
+ * Outputs as ts_mc_replay_ensemble, plus params (HOST, nullable): n_sel x n_real x 10, in the order d0 d1 d2 g0 g1 g2
+ * s_B phi0 phi1 phi2.  A TS_ST_NO_CUTOFF trial gets NaN rows in every output.  ts_last_kernel_ms and
+ * ts_mc_replay_ensemble_last_split report this call.  TS_ERR_ARG, outputs untouched: every case of
+ * ts_mc_replay_ensemble, a null disp, a sigma negative or not finite, sigma_inertia, sigma_torquer or sigma_field_scale
+ * above 1, sigma_field_angle above pi.  TS_ERR_NOMEM as ts_mc_replay_ensemble.                                       */
+typedef struct ts_dispersion_opts {
+  double sigma_inertia;     /* log-standard deviation of each principal inertia scale (J_true = D J D, D = diag(d)) */
+  double sigma_torquer;     /* log-standard deviation of each torquer gain                                          */
+  double sigma_field_scale; /* log-standard deviation of the field magnitude                                        */
+  double sigma_field_angle; /* standard deviation of each field rotation-vector component, rad                      */
+} ts_dispersion_opts;
+int ts_mc_dispersion_ensemble(ts_ctx* ctx, int64_t n_trials, const ts_replay_ensemble_opts* opts, const ts_dispersion_opts* disp,
+                              int64_t n_sel, const int64_t* trials, double* slew_time, double* x_final, double* params);
+
 /* ---- igrf12syn: the Fortran-style twin of igrf12 -------------------------------------------- *
  * igrf12syn(isv, date, itype, alt, colat, elong) [src/igrf.jl:335-534] at n points.  isv 0 = main field, 1 = secular
  * variation; itype 1 = geodetic (alt = height above the WGS-84 ellipsoid, km), 2 = geocentric (alt = radius, km);
@@ -467,6 +499,10 @@ int ts_multi_mc_continue(ts_multi* m, int64_t n_trials, const ts_ilqr_opts* opts
  * call (each rank replays the trials of its own context).  ts_last_kernel_ms of device i's context is its own part.    */
 int ts_multi_mc_replay_ensemble(ts_multi* m, int64_t n_trials, const ts_replay_ensemble_opts* opts, int64_t n_sel,
                                 const int64_t* trials, double* slew_time, double* x_final);
+/* ts_mc_dispersion_ensemble over a ts_multi_monte_carlo_run kept with keep_trajectories >= 1, dispatched as
+ * ts_multi_mc_replay_ensemble; the rows equal the single-device rows bit for bit (DE5).                              */
+int ts_multi_mc_dispersion_ensemble(ts_multi* m, int64_t n_trials, const ts_replay_ensemble_opts* opts, const ts_dispersion_opts* disp,
+                                    int64_t n_sel, const int64_t* trials, double* slew_time, double* x_final, double* params);
 
 /* ---- element-wise batch versions of the reference's building blocks (all HOST pointers) --- *
  * Correctness / drop-in paths for callers that use the small functions on their own; the fused

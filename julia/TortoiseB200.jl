@@ -78,6 +78,9 @@ end
 struct ReplayEnsembleOpts   # ts_replay_ensemble_opts
     n_real::Int64; r_first::Int64; q_noise_scale::Float64
 end
+struct DispersionOpts   # ts_dispersion_opts
+    sigma_inertia::Float64; sigma_torquer::Float64; sigma_field_scale::Float64; sigma_field_angle::Float64
+end
 function default_ilqr_opts()
     r = Ref{IlqrOpts}()
     ccall((:ts_ilqr_default_opts, LIB), Cvoid, (Ref{IlqrOpts},), r); r[]
@@ -421,12 +424,47 @@ function replay_ensemble(res; n_real::Integer = 100, trials = nothing, r_first::
     n = length(res.outcomes)
     sel = trials === nothing ? collect(1:n) : collect(trials)
     slew, _ = mc_replay_ensemble(n, n_real; r_first = r_first, trials = sel, q_noise_scale = q_noise_scale, e = e)
+    return ensemble_stats(res, sel, slew, n_real)
+end
+function ensemble_stats(res, sel, slew, n_real)
     fails = slew .== reshape([res.outcomes[t].t_final for t in sel], 1, :)
     fail_rate = [all(isnan, slew[:, k]) ? NaN : sum(fails[:, k]) / count(!isnan, slew[:, k]) for k in eachindex(sel)]
     ok(k) = [slew[i, k] for i in 1:n_real if !isnan(slew[i, k]) && !fails[i, k]]
     mean_ = [isempty(ok(k)) ? NaN : sum(ok(k)) / length(ok(k)) for k in eachindex(sel)]
     std_ = [isempty(ok(k)) ? NaN : sqrt(sum((ok(k) .- mean_[k]) .^ 2) / length(ok(k))) for k in eachindex(sel)]
     return (slew_time = slew, fails = fails, fail_rate = fail_rate, slew_mean = mean_, slew_std = std_, trials = sel)
+end
+
+# ts_mc_dispersion_ensemble: mc_replay_ensemble with drawn truth-model errors of the inertia, torquer gains and field
+# model per realisation (rules DE1-DE6, DESIGN.md section 4; sigma_field_angle in radians), the gains of the nominal
+# model.  Returns slew_time (n_real x n_sel), x_final (8 x n_real x n_sel) with want_x_final, and params
+# (10 x n_real x n_sel: d0 d1 d2 g0 g1 g2 s_B phi0 phi1 phi2) with want_params.  Realisation 0 carries no dispersion.
+function mc_dispersion_ensemble(number_sims::Integer, n_real::Integer; sigma_inertia::Float64 = 0.0, sigma_torquer::Float64 = 0.0,
+                                sigma_field_scale::Float64 = 0.0, sigma_field_angle::Float64 = 0.0, r_first::Integer = 0,
+                                trials = nothing, q_noise_scale::Float64 = (pi / 180)^2, want_x_final::Bool = false,
+                                want_params::Bool = false, e::Engine = engine())
+    sel = trials === nothing ? C_NULL : Int64[t - 1 for t in trials]
+    ns = trials === nothing ? number_sims : length(trials)
+    slew = zeros(n_real, ns); xf = want_x_final ? zeros(8, n_real, ns) : nothing; prm = want_params ? zeros(10, n_real, ns) : nothing
+    o = ReplayEnsembleOpts(n_real, r_first, q_noise_scale)
+    d = DispersionOpts(sigma_inertia, sigma_torquer, sigma_field_scale, sigma_field_angle)
+    check(e, ccall((:ts_mc_dispersion_ensemble, LIB), Cint,
+                   (Ptr{Cvoid}, Int64, Ref{ReplayEnsembleOpts}, Ref{DispersionOpts}, Int64, Ptr{Int64}, Ptr{Float64}, Ptr{Float64},
+                    Ptr{Float64}),
+                   e.h, number_sims, Ref(o), Ref(d), ns, sel, slew, xf === nothing ? C_NULL : xf, prm === nothing ? C_NULL : prm))
+    return slew, xf, prm
+end
+
+# replay_ensemble's statistics of a dispersion ensemble, plus params; r_first = 1 leaves the nominal realisation 0 out.
+function dispersion_ensemble(res; n_real::Integer = 100, trials = nothing, r_first::Integer = 1, sigma_inertia::Float64 = 0.0,
+                             sigma_torquer::Float64 = 0.0, sigma_field_scale::Float64 = 0.0, sigma_field_angle::Float64 = 0.0,
+                             q_noise_scale::Float64 = (pi / 180)^2, e::Engine = engine())
+    n = length(res.outcomes)
+    sel = trials === nothing ? collect(1:n) : collect(trials)
+    slew, _, prm = mc_dispersion_ensemble(n, n_real; sigma_inertia = sigma_inertia, sigma_torquer = sigma_torquer,
+                                          sigma_field_scale = sigma_field_scale, sigma_field_angle = sigma_field_angle,
+                                          r_first = r_first, trials = sel, q_noise_scale = q_noise_scale, want_params = true, e = e)
+    return merge(ensemble_stats(res, sel, slew, n_real), (params = prm,))
 end
 
 # Continues a monte_carlo(...; resumable = true) result `res` in place to max_outer outer iterations in all: outcomes,
@@ -550,6 +588,7 @@ export Engine, params, input_parameters, igrf12, igrf12_batch, igrf_data, magnet
        legendre, dlegendre, DerivFunction, gain_simulator, attitude_dynamics,
        condition_based_time, eigen_axis_slew, bryson_weights, solve_slew, attitude_simulation, monte_carlo, qmult, qrot, q_inv, hat,
        igrf12syn, attitude_dynamics_linear, psiaki_pd_simulation, igrf_interpolant, field_map_prefilter, field_map_eval, AlState,
-       mc_state, mc_continue, continue_monte_carlo!, ReplayEnsembleOpts, mc_replay_ensemble, replay_ensemble
+       mc_state, mc_continue, continue_monte_carlo!, ReplayEnsembleOpts, mc_replay_ensemble, replay_ensemble,
+       DispersionOpts, mc_dispersion_ensemble, dispersion_ensemble
 
 end # module

@@ -54,6 +54,7 @@ CD_ONLY inline CD sqrt(const T& a) { ++g_cnt.sqrt_; return CD(::sqrt(a.v)); }
 CD_ONLY inline CD fabs(const T& a) { return CD(::fabs(a.v)); }
 CD_ONLY inline CD floor(const T& a) { return CD(::floor(a.v)); }
 CD_ONLY inline CD sin(const T& a) { return CD(::sin(a.v)); }
+CD_ONLY inline CD exp(const T& a) { return CD(::exp(a.v)); }
 CD_ONLY inline CD cos(const T& a) { return CD(::cos(a.v)); }
 CD_ONLY inline CD acos(const T& a) { return CD(::acos(a.v)); }
 CD_ONLY inline CD log(const T& a) { return CD(::log(a.v)); }
@@ -224,7 +225,7 @@ int main() {
   // (c) one step of the replay with inline draws, as K4e runs it per lane: feedback, four stage records (Philox +
   // Box-Muller draws, perturbation quaternion, field row) and the rk4 step of the simulator.  Counted as the difference
   // of two replays of 65 and 33 knots over the 32 extra steps; log / sin / cos calls are not FLOPs in this count.
-  auto replay = [&](int n) {
+  auto replay = [&](int n, const CD* prm = nullptr) {
     std::vector<CD> Xr(8 * n), Ur(3 * n), Kr(18 * n);
     for (int k = 0; k < n; ++k) for (int i = 0; i < 8; ++i) Xr[k * 8 + i] = CD(x0[i]);
     for (int i = 0; i < 18 * n; ++i) Kr[i] = CD(0.01);
@@ -239,8 +240,17 @@ int main() {
     ts_tvlqr_opts_dev to = {};
     to.dt = CD(0.2); to.t0 = CD(0.0); to.tf = ti.t_final; to.noise_mode = 2; to.seed = 7; to.w_limit = CD(0.05); to.ang_limit = CD(0.08727);
     CD slew(0.0);
+    if (prm) {   // (d): a dispersed realisation; its once-per-lane setup is outside the counted replay
+      ts::tvlqr_disp_setup(prm, ti.I.J, ti.disp);
+      ts::inv3_gj(ti.I.J, ti.I.Jinv);
+    }
     const Counters a = g_cnt;
-    ts::tvlqr_replay(ti, to, Kr.data(), nullptr, nullptr, nullptr, &slew);
+    if (prm) {
+      ts::TvlqrDirectSrc src = {ti.X_lqr, ti.U_lqr, Kr.data(), nullptr};
+      ts::tvlqr_replay_src<false, ts::TvlqrDirectSrc, true>(ti, to, src, nullptr, nullptr, nullptr, &slew);
+    } else {
+      ts::tvlqr_replay(ti, to, Kr.data(), nullptr, nullptr, nullptr, &slew);
+    }
     return diff(g_cnt, a);
   };
   const Counters r65 = replay(65), r33 = replay(33);
@@ -252,5 +262,12 @@ int main() {
   show("replay step (feedback + 4 stage records with draws + rk4)", c_step, 32);
   show("draws of one stage (tvlqr_noise: 3 Philox blocks, 3 Box-Muller pairs, scaling)", c_draw, 1);
   printf("JSON {\"ensemble_replay_step\": %.0f, \"stage_draws\": %lld}\n", c_step.flops() / 32.0, c_draw.flops());
+  // (d) the same step of a dispersed realisation (K4d) with every group active: truth inertia, torquer gains, field
+  // scale and rotation (per stage: qrot of the field row, its scaling, the gains on the torque)
+  const CD prm[10] = {CD(1.05), CD(0.97), CD(1.02), CD(1.03), CD(0.98), CD(1.01), CD(1.04), CD(0.02), CD(-0.01), CD(0.03)};
+  const Counters c_dstep = diff(replay(65, prm), replay(33, prm));
+  printf("\n(d) TVLQR replay of a dispersed realisation (dispersion ensemble, K4d), per replay step:\n");
+  show("replay step (as (c) + field transform and torquer gains in every stage)", c_dstep, 32);
+  printf("JSON {\"dispersion_replay_step\": %.0f}\n", c_dstep.flops() / 32.0);
   return 0;
 }

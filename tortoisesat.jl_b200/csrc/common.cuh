@@ -37,7 +37,7 @@ enum Slot : int {
   SLOT_K3_COUNTERS,                        // K3 queue and park counters (read by ts_k3_last_split / ts_k3_last_parked)
   SLOT_AL_STATES,                          // K3 continuation: a call's imported and exported solver states
   SLOT_KEPT_STATE,                         // Monte-Carlo kept solver states + multipliers (ts_mc_fetch_state, ts_mc_continue)
-  SLOT_ENSEMBLE_OUT,                       // a disturbance ensemble's slew times and final states (ts_mc_replay_ensemble)
+  SLOT_ENSEMBLE_OUT,                       // an ensemble's slew times, final states and parameters (ts_mc_replay_ensemble, ts_mc_dispersion_ensemble)
   SLOT_COUNT
 };
 
@@ -100,7 +100,7 @@ struct ts_ctx {
   char name[128] = {0};
   int64_t launches = 0;
   double last_kernel_ms = 0.0;
-  double ens_ms[2] = {0.0, 0.0};  // the last ts_mc_replay_ensemble: gains (K4a + K4b) | ensemble replay (K4e)
+  double ens_ms[2] = {0.0, 0.0};  // the last ts_mc_replay_ensemble / ts_mc_dispersion_ensemble: gains (K4a + K4b) | replay (K4e / K4d)
   double* d_tabG = nullptr;  // 104 x 25
   double* d_tabH = nullptr;  // 91 x 25
   double* d_tabGH = nullptr; // 3450 (igrf12syn)
@@ -139,6 +139,15 @@ inline int fail(ts_ctx* ctx, int code, const char* fmt, ...) {
     va_end(ap);
   }
   return code;
+}
+
+// The sigmas a dispersion ensemble accepts (ts_mc_dispersion_ensemble): finite and >= 0, the three log-standard
+// deviations <= 1 and the field angle <= pi.
+inline bool dispersion_opts_ok(const ts_dispersion_opts* d) {
+  const double s[4] = {d->sigma_inertia, d->sigma_torquer, d->sigma_field_scale, d->sigma_field_angle};
+  for (int i = 0; i < 4; ++i)
+    if (!std::isfinite(s[i]) || s[i] < 0.0 || s[i] > (i < 3 ? 1.0 : 3.14159265358979323846)) return false;
+  return true;
 }
 
 #define TS_CUDA(ctx, call)                                                                              \

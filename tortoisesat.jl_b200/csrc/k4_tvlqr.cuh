@@ -454,6 +454,7 @@ inline K4eArgs k4e_args(const K4Args& a, const double* x0) {
   e.opts = a.opts;
   return e;
 }
+template <bool DISP>
 struct K4eWarpSrc {
   const TvlqrIn* in;
   const ts_tvlqr_opts_dev* o;
@@ -482,7 +483,7 @@ struct K4eWarpSrc {
     for (int s = 0; s < 4; ++s) {
       double rec[TV_REC];
       const double tc = s == 0 ? tcl[0] : (s == 3 ? tcl[3] : tcl[1]);   // (no dynamic index: tcl stays in registers)
-      tvlqr_stage_record_at(*in, *o, k, s, tc, rec);
+      tvlqr_stage_record_at<DISP>(*in, *o, k, s, tc, rec);
 #pragma unroll
       for (int i = 0; i < TV_REC; ++i) recs[s * TV_REC + i] = rec[i];
     }
@@ -496,63 +497,27 @@ struct K4eWarpSrc {
     issue(k + K4_RING_D);
   }
 };
+// K4d: the dispersion ensemble of a kept run (ts_mc_dispersion_ensemble, DE1-DE6): K4e's layout, ring and replay; each
+// lane draws its realisation's truth-model parameters once before the step loop (dispersion_params, tvlqr_disp_setup:
+// truth inertia in TvlqrIn::I, gains of the nominal model).  Per stage the lane transforms the (uniformly loaded) field
+// row of its record and scales the torque (tvlqr_disp_field, simulator7_rec<true>).
+struct K4dArgs {
+  K4eArgs e;
+  double sigma[4];                   // sigma_inertia, sigma_torquer, sigma_field_scale, sigma_field_angle
+  double* params;                    // n_sel x n_real x DISP_NP, nullable
+};
 __global__ void __launch_bounds__(32 * K4E_WARPS) k4e_ensemble_replay_kernel(const K4eArgs a) {
-  __shared__ __align__(16) double ring_all[K4E_WARPS * K4_RING_D * K4E_W];
-  __shared__ double recs_all[32 * K4E_WARPS * K4E_R];
-  const int lane = threadIdx.x & 31, wib = threadIdx.x >> 5;
-  const int64_t w = (int64_t)blockIdx.x * K4E_WARPS + wib;
-  if (w >= a.n_sel * a.n_blk) return;   // whole warps leave together
-  const int64_t t = w / a.n_blk;
-  const int64_t j = (w % a.n_blk) * 32 + lane;             // realisation r_first + j of trial t
-  const int64_t jc = j < a.n_real ? j : a.n_real - 1;      // lanes past n_real replay a copy and store nothing
-  const uint32_t r = (uint32_t)(a.r_first + jc);
-  TvlqrIn in;
-  in.N = (int)a.N_i[t];
-  in.X_lqr = a.X_lqr + a.offs[t] * 8;
-  in.U_lqr = a.U_lqr + a.offs[t] * 3;
-  in.trial = a.stream_id[t];
-  in.real = r;
-  if (r == 0) {
-    for (int i = 0; i < 8; ++i) in.x0[i] = a.x0_lqr[t * 8 + i];
-  } else {
-    double qn[3];
-    tvlqr_initial_qnoise(a.opts.seed, in.trial, r, a.q_noise_scale, qn);
-    tvlqr_x0_lqr(a.x0 + t * 8, qn, in.x0);
-  }
-  for (int i = 0; i < 9; ++i) in.I.J[i] = a.Jmat[t * 9 + i];
-  inv3_gj(in.I.J, in.I.Jinv);
-  in.Bt = a.B_eci + a.B_offs[t] * 3;
-  in.B_rows = a.B_rows[t];
-  in.index_scale = a.index_scale[t];
-  in.clock_rate = a.clock_rate[t];
-  in.noise = nullptr;
-  for (int i = 0; i < 4; ++i) in.q_final[i] = a.q_final[t * 4 + i];
-  in.t_final = a.t_final[t];
-  in.time_step = a.opts.dt;
-  in.trial_index_1based = (long long)in.trial + 1;
-  ts_tvlqr_opts_dev o = a.opts;
-  o.tf = a.t_final[t];
-  K4eWarpSrc src;
-  src.in = &in;
-  src.o = &o;
-  src.X = in.X_lqr;
-  src.U = in.U_lqr;
-  src.K = a.K + a.offs[t] * 18;
-  src.clk = a.clk + a.lin_offs[t];
-  src.ring = ring_all + wib * (K4_RING_D * K4E_W);
-  src.recs = recs_all + threadIdx.x * K4E_R;
-  src.n_steps = in.N - 1;
-  src.lane = lane;
-  for (int d = 0; d < K4_RING_D; ++d) src.issue(d);
-  double slew = 0.0, xl[8];
-  tvlqr_replay_src<true>(in, o, src, nullptr, nullptr, nullptr, &slew, xl);
-  asm volatile("cp.async.wait_all;\n" ::: "memory");
-  if (j < a.n_real) {
-    const int64_t row = t * a.n_real + j;
-    a.slew_time[row] = slew;
-    if (a.x_final)
-      for (int i = 0; i < 8; ++i) a.x_final[row * 8 + i] = xl[i];
-  }
+  constexpr bool DISP = false;
+  const double* sigma = nullptr;
+  double* params = nullptr;
+#include "k4e_replay_body.inc"
+}
+__global__ void __launch_bounds__(32 * K4E_WARPS) k4d_dispersion_replay_kernel(const K4dArgs ad) {
+  constexpr bool DISP = true;
+  const K4eArgs& a = ad.e;
+  const double* sigma = ad.sigma;
+  double* params = ad.params;
+#include "k4e_replay_body.inc"
 }
 
 // eigen_axis_slew + Bryson weights, one thread per trial.  t_k = t0 + k*dt, k = 0..nt-1 with

@@ -268,19 +268,23 @@ int ts_multi_mc_continue(ts_multi* m, int64_t n_trials, const ts_ilqr_opts* opts
   return multi_shards(m, n_trials, shard, out, stats);
 }
 
-int ts_multi_mc_replay_ensemble(ts_multi* m, int64_t n_trials, const ts_replay_ensemble_opts* opts, int64_t n_sel, const int64_t* trials,
-                                double* slew_time, double* x_final) {
+// ts_multi_mc_replay_ensemble and ts_multi_mc_dispersion_ensemble (disp non-null): each trial on the device that holds
+// it, all devices at once, rows back in the caller's order.  The argument checks of the single-device entry run before
+// any device does: a failure leaves the outputs untouched.
+static int multi_ensemble(ts_multi* m, const char* fn, int64_t n_trials, const ts_replay_ensemble_opts* opts, bool dispersed,
+                          const ts_dispersion_opts* disp, int64_t n_sel, const int64_t* trials, double* slew_time, double* x_final,
+                          double* params) {
   if (!m) return TS_ERR_ARG;
   const int G = m->n;
-  // the argument checks of ts_mc_replay_ensemble, before any device runs: a failure leaves the outputs untouched
-  bool bad = n_trials < 0 || !opts || !slew_time || (trials ? n_sel < 0 : n_sel != n_trials);
+  bool bad = n_trials < 0 || !opts || !slew_time || (trials ? n_sel < 0 : n_sel != n_trials) || (dispersed && !disp);
   if (!bad) bad = opts->n_real < 1 || opts->r_first < 0 || opts->r_first + opts->n_real > ((int64_t)1 << 30);
+  if (!bad && dispersed) bad = !ts::dispersion_opts_ok(disp);
   for (int64_t p = 0; !bad && trials && p < n_sel; ++p) bad = trials[p] < 0 || trials[p] >= n_trials;
   if (bad) {
-    snprintf(m->err, sizeof(m->err), "ts_multi_mc_replay_ensemble: bad argument");
+    snprintf(m->err, sizeof(m->err), "%s: bad argument", fn);
     return TS_ERR_ARG;
   }
-  const size_t RR = (size_t)opts->n_real;
+  const size_t RR = (size_t)opts->n_real, NP = ts::DISP_NP;
   std::vector<std::vector<int64_t>> pos(G), loc(G);   // caller rows and device-local trial indices per device
   for (int64_t p = 0; p < n_sel; ++p) {
     const int64_t t = trials ? trials[p] : p;
@@ -288,14 +292,18 @@ int ts_multi_mc_replay_ensemble(ts_multi* m, int64_t n_trials, const ts_replay_e
     loc[t % G].push_back(t / G);
   }
   std::vector<int> rcs(G, TS_OK);
-  std::vector<std::vector<double>> hs(G), hx(G);
+  std::vector<std::vector<double>> hs(G), hx(G), hp(G);
   auto worker = [&](int g) {
     if (pos[g].empty()) return;
     const int64_t ng = (n_trials - g + G - 1) / G;
     const size_t k = pos[g].size();
     hs[g].resize(k * RR);
     if (x_final) hx[g].resize(k * RR * 8);
-    rcs[g] = ts_mc_replay_ensemble(m->ctx[g], ng, opts, (int64_t)k, loc[g].data(), hs[g].data(), x_final ? hx[g].data() : nullptr);
+    if (params) hp[g].resize(k * RR * NP);
+    double* px = x_final ? hx[g].data() : nullptr;
+    rcs[g] = dispersed ? ts_mc_dispersion_ensemble(m->ctx[g], ng, opts, disp, (int64_t)k, loc[g].data(), hs[g].data(), px,
+                                                   params ? hp[g].data() : nullptr)
+                       : ts_mc_replay_ensemble(m->ctx[g], ng, opts, (int64_t)k, loc[g].data(), hs[g].data(), px);
   };
   std::vector<std::thread> th;
   for (int g = 0; g < G; ++g) th.emplace_back(worker, g);
@@ -310,8 +318,19 @@ int ts_multi_mc_replay_ensemble(ts_multi* m, int64_t n_trials, const ts_replay_e
       const size_t p = (size_t)pos[g][k];
       memcpy(slew_time + p * RR, &hs[g][k * RR], RR * 8);
       if (x_final) memcpy(x_final + p * RR * 8, &hx[g][k * RR * 8], RR * 64);
+      if (params) memcpy(params + p * RR * NP, &hp[g][k * RR * NP], RR * NP * 8);
     }
   return TS_OK;
+}
+
+int ts_multi_mc_replay_ensemble(ts_multi* m, int64_t n_trials, const ts_replay_ensemble_opts* opts, int64_t n_sel, const int64_t* trials,
+                                double* slew_time, double* x_final) {
+  return multi_ensemble(m, "ts_multi_mc_replay_ensemble", n_trials, opts, false, nullptr, n_sel, trials, slew_time, x_final, nullptr);
+}
+
+int ts_multi_mc_dispersion_ensemble(ts_multi* m, int64_t n_trials, const ts_replay_ensemble_opts* opts, const ts_dispersion_opts* disp,
+                                    int64_t n_sel, const int64_t* trials, double* slew_time, double* x_final, double* params) {
+  return multi_ensemble(m, "ts_multi_mc_dispersion_ensemble", n_trials, opts, true, disp, n_sel, trials, slew_time, x_final, params);
 }
 
 }  // extern "C"

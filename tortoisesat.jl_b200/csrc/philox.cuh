@@ -91,4 +91,36 @@ TS_HD void tvlqr_initial_qnoise(uint64_t seed, uint32_t trial, uint32_t real, do
   qn[2] = scale * z2;
 }
 
+// The ten truth-model parameters of realisation real of a dispersion ensemble (ts_mc_dispersion_ensemble, DE2), in the
+// order d0 d1 d2 g0 g1 g2 s_B phi0 phi1 phi2, for sig = (sigma_inertia, sigma_torquer, sigma_field_scale,
+// sigma_field_angle).  Normals z0..z9 from counter blocks (stream, 0xFFFFFFFE, 0, 4 real + {0, 1, 2}) (no replay step
+// reaches that step word; the initial draw uses 0xFFFFFFFF): (z0, z1), (z2, z3) from block 0's two Box-Muller pairs,
+// (z4 .. z7) from block 1's, (z8, z9) from block 2's first.  d_i = exp(sig0 z_i / 2), g_i = exp(sig1 z_{3+i}),
+// s_B = exp(sig2 z6), phi = sig3 (z7, z8, z9).  Each group reads fixed normals, so one sigma leaves the others' values
+// alone; a group with sigma 0, and every group of realisation 0, keeps its nominal value (1 or 0) exactly.
+constexpr int DISP_NP = 10;
+TS_HD void dispersion_params(uint64_t seed, uint32_t stream, uint32_t real, const double sig[4], double p[DISP_NP]) {
+  for (int i = 0; i < 7; ++i) p[i] = 1.0;
+  p[7] = p[8] = p[9] = 0.0;
+  if (real == 0) return;
+  const uint32_t k0 = (uint32_t)seed, k1 = (uint32_t)(seed >> 32), b = 4u * real;
+  uint32_t o0[4], o1[4], o2[4];
+  philox4x32_10(stream, 0xFFFFFFFEu, 0u, b, k0, k1, o0);
+  philox4x32_10(stream, 0xFFFFFFFEu, 0u, b + 1u, k0, k1, o1);
+  philox4x32_10(stream, 0xFFFFFFFEu, 0u, b + 2u, k0, k1, o2);
+  double z[DISP_NP];
+  box_muller(o0[0], o0[1], z[0], z[1]);
+  box_muller(o0[2], o0[3], z[2], z[3]);
+  box_muller(o1[0], o1[1], z[4], z[5]);
+  box_muller(o1[2], o1[3], z[6], z[7]);
+  box_muller(o2[0], o2[1], z[8], z[9]);
+  if (sig[0] > 0.0)
+    for (int i = 0; i < 3; ++i) p[i] = exp(sig[0] * z[i] / 2);
+  if (sig[1] > 0.0)
+    for (int i = 0; i < 3; ++i) p[3 + i] = exp(sig[1] * z[3 + i]);
+  if (sig[2] > 0.0) p[6] = exp(sig[2] * z[6]);
+  if (sig[3] > 0.0)
+    for (int i = 0; i < 3; ++i) p[7 + i] = sig[3] * z[7 + i];
+}
+
 }  // namespace ts

@@ -24,7 +24,7 @@ using namespace ts;
 
 extern "C" {
 
-int ts_version(void) { return 104; }
+int ts_version(void) { return 105; }
 
 int ts_create(ts_ctx** out, int device_id) {
   if (!out) return TS_ERR_ARG;
@@ -1592,23 +1592,28 @@ int ts_mc_continue(ts_ctx* c, int64_t n_trials, const ts_ilqr_opts* opts, ts_tri
   return TS_OK;
 }
 
-// RE1-RE5 (DESIGN.md section 4, K4): the kept run's slews replayed under n_real disturbance draws each.  The gains of
-// the selected trials come from the unchanged K4a + K4b on host-compacted arrays (as ts_mc_continue replays), then K4e
-// replays every (trial, realisation) pair.  Only per-call slots are written: the kept run stays as it was (RE5).
-int ts_mc_replay_ensemble(ts_ctx* c, int64_t n_trials, const ts_replay_ensemble_opts* opts, int64_t n_sel, const int64_t* trials,
-                          double* slew_time, double* x_final) {
+// RE1-RE5 and DE1-DE6 (DESIGN.md section 4, K4): the body of ts_mc_replay_ensemble and, with disp, of
+// ts_mc_dispersion_ensemble.  The kept run's slews replayed under n_real disturbance draws each (and, with disp, under
+// drawn truth-model errors).  The gains of the selected trials come from the unchanged K4a + K4b on host-compacted arrays
+// (as ts_mc_continue replays), then K4e (K4d) replays every (trial, realisation) pair.  Only per-call slots are written:
+// the kept run stays as it was (RE5, DE6).
+static int mc_ensemble(ts_ctx* c, const char* fn, int64_t n_trials, const ts_replay_ensemble_opts* opts, bool dispersed,
+                       const ts_dispersion_opts* disp, int64_t n_sel, const int64_t* trials, double* slew_time, double* x_final,
+                       double* params) {
   if (!c) return TS_ERR_ARG;
   const ts_ctx::McLast& L = c->mc_last;
-  if (L.cfg.keep_trajectories < 1) return fail(c, TS_ERR_ARG, "ts_mc_replay_ensemble: no Monte-Carlo run with keep_trajectories >= 1 on this context");
-  if (n_trials != L.n) return fail(c, TS_ERR_ARG, "ts_mc_replay_ensemble: the kept run had %lld trials", (long long)L.n);
-  if (!opts || !slew_time) return fail(c, TS_ERR_ARG, "ts_mc_replay_ensemble: null argument");
+  if (L.cfg.keep_trajectories < 1) return fail(c, TS_ERR_ARG, "%s: no Monte-Carlo run with keep_trajectories >= 1 on this context", fn);
+  if (n_trials != L.n) return fail(c, TS_ERR_ARG, "%s: the kept run had %lld trials", fn, (long long)L.n);
+  if (!opts || !slew_time || (dispersed && !disp)) return fail(c, TS_ERR_ARG, "%s: null argument", fn);
   const int64_t R = opts->n_real, r0 = opts->r_first;
   if (R < 1 || r0 < 0 || r0 + R > ((int64_t)1 << 30))
-    return fail(c, TS_ERR_ARG, "ts_mc_replay_ensemble: need n_real >= 1, r_first >= 0, r_first + n_real <= 2^30");
+    return fail(c, TS_ERR_ARG, "%s: need n_real >= 1, r_first >= 0, r_first + n_real <= 2^30", fn);
   if (trials ? n_sel < 0 : n_sel != n_trials)
-    return fail(c, TS_ERR_ARG, "ts_mc_replay_ensemble: n_sel must be >= 0 (= n_trials without a trial list)");
+    return fail(c, TS_ERR_ARG, "%s: n_sel must be >= 0 (= n_trials without a trial list)", fn);
   for (int64_t p = 0; trials && p < n_sel; ++p)
-    if (trials[p] < 0 || trials[p] >= n_trials) return fail(c, TS_ERR_ARG, "ts_mc_replay_ensemble: trial %lld out of range", (long long)trials[p]);
+    if (trials[p] < 0 || trials[p] >= n_trials) return fail(c, TS_ERR_ARG, "%s: trial %lld out of range", fn, (long long)trials[p]);
+  if (dispersed && !dispersion_opts_ok(disp))
+    return fail(c, TS_ERR_ARG, "%s: need finite sigmas >= 0, the three log-sigmas <= 1 and sigma_field_angle <= pi", fn);
   // selected active trials, longest horizon first (stable: repeats and the caller's order decide nothing about a row, RE4)
   std::vector<int64_t> act_of((size_t)n_trials, -1);
   for (size_t a = 0; a < L.act.size(); ++a) act_of[(size_t)L.act[a]] = (int64_t)a;
@@ -1618,8 +1623,8 @@ int ts_mc_replay_ensemble(ts_ctx* c, int64_t n_trials, const ts_replay_ensemble_
   auto act_at = [&](int64_t p) { return act_of[(size_t)(trials ? trials[p] : p)]; };
   std::stable_sort(pos.begin(), pos.end(), [&](int64_t u, int64_t v) { return L.in.col(I_N)[act_at(u)] > L.in.col(I_N)[act_at(v)]; });
   const size_t NC = pos.size(), RR = (size_t)R;
-  const size_t per = x_final ? 9 : 1;   // doubles per (trial, realisation) row
-  std::vector<double> hs(NC * RR), hx(x_final ? NC * RR * 8 : 0);
+  const size_t per = 1 + (x_final ? 8 : 0) + (params ? DISP_NP : 0);   // doubles per (trial, realisation) row
+  std::vector<double> hs(NC * RR), hx(x_final ? NC * RR * 8 : 0), hp(params ? NC * RR * DISP_NP : 0);
   c->ens_ms[0] = c->ens_ms[1] = 0.0;
   c->last_kernel_ms = 0.0;
   if (NC > 0) {
@@ -1644,17 +1649,29 @@ int ts_mc_replay_ensemble(ts_ctx* c, int64_t n_trials, const ts_replay_ensemble_
     e.q_noise_scale = opts->q_noise_scale;
     e.slew_time = (double*)p_out;
     e.x_final = x_final ? e.slew_time + NC * RR : nullptr;
+    double* d_params = params ? e.slew_time + NC * RR * (x_final ? 9 : 1) : nullptr;
     Events<3> ev;
     cudaEventRecord(ev[0], c->stream);
     k4_gains_launch(c, k4);
     cudaEventRecord(ev[1], c->stream);
     const int64_t warps = (int64_t)NC * e.n_blk;
-    k4e_ensemble_replay_kernel<<<(unsigned)((warps + K4E_WARPS - 1) / K4E_WARPS), 32 * K4E_WARPS, 0, c->stream>>>(e);
+    const unsigned blocks = (unsigned)((warps + K4E_WARPS - 1) / K4E_WARPS);
+    if (dispersed) {
+      K4dArgs d;
+      d.e = e;
+      d.sigma[0] = disp->sigma_inertia; d.sigma[1] = disp->sigma_torquer;
+      d.sigma[2] = disp->sigma_field_scale; d.sigma[3] = disp->sigma_field_angle;
+      d.params = d_params;
+      k4d_dispersion_replay_kernel<<<blocks, 32 * K4E_WARPS, 0, c->stream>>>(d);
+    } else {
+      k4e_ensemble_replay_kernel<<<blocks, 32 * K4E_WARPS, 0, c->stream>>>(e);
+    }
     c->launches++;
     cudaEventRecord(ev[2], c->stream);
     TS_CUDA(c, cudaGetLastError());
     TS_CUDA(c, cudaMemcpyAsync(hs.data(), e.slew_time, NC * RR * 8, cudaMemcpyDeviceToHost, c->stream));
     if (x_final) TS_CUDA(c, cudaMemcpyAsync(hx.data(), e.x_final, NC * RR * 64, cudaMemcpyDeviceToHost, c->stream));
+    if (params) TS_CUDA(c, cudaMemcpyAsync(hp.data(), d_params, NC * RR * DISP_NP * 8, cudaMemcpyDeviceToHost, c->stream));
     TS_CUDA(c, cudaStreamSynchronize(c->stream));
     c->ens_ms[0] = ev.ms(0, 1);
     c->ens_ms[1] = ev.ms(1, 2);
@@ -1667,14 +1684,27 @@ int ts_mc_replay_ensemble(ts_ctx* c, int64_t n_trials, const ts_replay_ensemble_
     done[p] = 1;
     memcpy(slew_time + p * RR, &hs[k * RR], RR * 8);
     if (x_final) memcpy(x_final + p * RR * 8, &hx[k * RR * 8], RR * 64);
+    if (params) memcpy(params + p * RR * DISP_NP, &hp[k * RR * DISP_NP], RR * DISP_NP * 8);
   }
   for (int64_t p = 0; p < n_sel; ++p)
     if (!done[(size_t)p]) {
       for (size_t i = 0; i < RR; ++i) slew_time[(size_t)p * RR + i] = NAN;
       if (x_final)
         for (size_t i = 0; i < RR * 8; ++i) x_final[(size_t)p * RR * 8 + i] = NAN;
+      if (params)
+        for (size_t i = 0; i < RR * DISP_NP; ++i) params[(size_t)p * RR * DISP_NP + i] = NAN;
     }
   return TS_OK;
+}
+
+int ts_mc_replay_ensemble(ts_ctx* c, int64_t n_trials, const ts_replay_ensemble_opts* opts, int64_t n_sel, const int64_t* trials,
+                          double* slew_time, double* x_final) {
+  return mc_ensemble(c, "ts_mc_replay_ensemble", n_trials, opts, false, nullptr, n_sel, trials, slew_time, x_final, nullptr);
+}
+
+int ts_mc_dispersion_ensemble(ts_ctx* c, int64_t n_trials, const ts_replay_ensemble_opts* opts, const ts_dispersion_opts* disp,
+                              int64_t n_sel, const int64_t* trials, double* slew_time, double* x_final, double* params) {
+  return mc_ensemble(c, "ts_mc_dispersion_ensemble", n_trials, opts, true, disp, n_sel, trials, slew_time, x_final, params);
 }
 
 int ts_mc_replay_ensemble_last_split(ts_ctx* c, double* gains_ms, double* replay_ms) {

@@ -87,6 +87,14 @@ TS_HD void inv3_adj(const double A[9], double out[9]) {
   out[8] = (A[0] * A[4] - A[1] * A[3]) * id;
 }
 
+// The truth-model errors of one realisation of a dispersion ensemble (K4d, DE2 of DESIGN.md section 4, K4) that act in
+// the stage dynamics: torquer gains, and the field transform s_B * qrot(p, row).  A group at its nominal value is
+// skipped (torq / scale / rot false), so a realisation without errors runs K4e's arithmetic exactly (DE3, DE4).
+struct TvlqrDisp {
+  double g[3], sB, p[4];
+  bool torq, scale, rot;
+};
+
 struct TvlqrIn {
   int N;                 // knots of the optimised trajectory
   const double* X_lqr;   // N x 8
@@ -102,7 +110,40 @@ struct TvlqrIn {
   double q_final[4];
   double t_final, time_step;
   long long trial_index_1based;
+  TvlqrDisp disp;        // read by the dispersed instantiations (DISP = true) only
 };
+
+// A dispersed realisation's truth model from its ten parameters (dispersion_params): J_true[i][j] = (d_i J[i][j]) d_j in
+// place of J (positive definite for any draw; the caller inverts it as for the nominal J), the torquer gains, and the
+// field rotation p = [cos(|phi|/2); phi/|phi| sin(|phi|/2)] (the identity for |phi| <= 1e-300, tvlqr_stage_record's guard).
+TS_HD void tvlqr_disp_setup(const double prm[10], double J[9], TvlqrDisp& d) {
+  for (int i = 0; i < 3; ++i)
+    for (int j = 0; j < 3; ++j) J[i * 3 + j] = (prm[i] * J[i * 3 + j]) * prm[j];
+  for (int i = 0; i < 3; ++i) d.g[i] = prm[3 + i];
+  d.torq = prm[3] != 1.0 || prm[4] != 1.0 || prm[5] != 1.0;
+  d.sB = prm[6];
+  d.scale = prm[6] != 1.0;
+  const double th = sqrt(prm[7] * prm[7] + prm[8] * prm[8] + prm[9] * prm[9]);
+  d.rot = th > 1e-300;
+  d.p[0] = 1.0;
+  d.p[1] = d.p[2] = d.p[3] = 0.0;
+  if (d.rot) {
+    const double sh = sin(th / 2);
+    d.p[0] = cos(th / 2);
+    for (int i = 0; i < 3; ++i) d.p[1 + i] = prm[7 + i] / th * sh;
+  }
+}
+
+// The truth field row of a dispersed stage: s_B * qrot(p, row); tvlqr_stage_record then adds the stage's field noise.
+TS_HD void tvlqr_disp_field(const TvlqrDisp& d, const double* Bn, double out[3]) {
+  if (d.rot) {
+    qrot(d.p, Bn, out);
+  } else {
+    for (int i = 0; i < 3; ++i) out[i] = Bn[i];
+  }
+  if (d.scale)
+    for (int i = 0; i < 3; ++i) out[i] = mul_rn(d.sB, out[i]);
+}
 
 // stage clocks of rk4 on the decoupled clock state: c = rate*h; x8, x8+c/2, x8+c/2, x8+c; next = x8 + (c+2c+2c+c)/6
 TS_HD void clock_rk4(double x8, double rate, double h, double t[4], double& next) {
@@ -160,7 +201,10 @@ TS_HD void tvlqr_stage_record(const double* nz9, const double* Bn, double rec[TV
 
 // simulator(dx,x,u) (simulator.jl:1-42) for the 7 dynamic states, from a stage record.  q/|q| is x * rsqrt(q.q) (one
 // rounding apart from the reference's four divisions, like the solver kernels; inside the 1e-10 rollout bar).
-TS_HD void simulator7_rec(const Inertia& I, const double x[7], const double u[3], const double* rec, double dx[7]) {
+// DISP: a dispersed realisation's torque ((u_i * 0.01) * g_i) x B_B (I is then its truth inertia).
+template <bool DISP = false>
+TS_HD void simulator7_rec(const Inertia& I, const double x[7], const double u[3], const double* rec, double dx[7],
+                          const TvlqrDisp* disp = nullptr) {
   const double om[3] = {x[0] + rec[0], x[1] + rec[1], x[2] + rec[2]};
   const double inq = rnorm(x[3] * x[3] + x[4] * x[4] + x[5] * x[5] + x[6] * x[6]);
   const double q0[4] = {x[3] * inq, x[4] * inq, x[5] * inq, x[6] * inq};
@@ -170,7 +214,11 @@ TS_HD void simulator7_rec(const Inertia& I, const double x[7], const double u[3]
   double qd[4], BB[3], tau[3], Jw[3], wJw[3];
   qmult(q, w4, qd);
   qrot(q, rec + 7, BB);
-  const double us[3] = {u[0] * 0.01, u[1] * 0.01, u[2] * 0.01};
+  double us[3] = {u[0] * 0.01, u[1] * 0.01, u[2] * 0.01};
+  if constexpr (DISP) {
+    if (disp->torq)
+      for (int i = 0; i < 3; ++i) us[i] = mul_rn(us[i], disp->g[i]);
+  }
   cross3(us, BB, tau);
   for (int i = 0; i < 3; ++i) Jw[i] = I.J[i * 3 + 0] * om[0] + I.J[i * 3 + 1] * om[1] + I.J[i * 3 + 2] * om[2];
   cross3(om, Jw, wJw);
@@ -339,8 +387,15 @@ TS_HD void tvlqr_gains(const TvlqrIn& in, const ts_tvlqr_opts_dev& o, double* K,
 }
 
 // Stage record s of step k when it is not pre-generated (tcl_s: the stage's clock value): field row -> noise -> record.
+// DISP: the row goes through the realisation's field transform (tvlqr_disp_field) before the noise is added.
+template <bool DISP = false>
 TS_HD void tvlqr_stage_record_at(const TvlqrIn& in, const ts_tvlqr_opts_dev& o, long long k, int s, double tcl_s, double rec[TV_REC]) {
   const double* Bn = in.Bt + (long long)field_row(tcl_s, in.index_scale, in.B_rows) * 3;
+  double Bd[3];
+  if constexpr (DISP) {
+    tvlqr_disp_field(in.disp, Bn, Bd);
+    Bn = Bd;
+  }
   if (o.noise_mode == 2) {   // (its own call: the draws stay in registers, no pointer may alias them)
     double nzb[9];
     tvlqr_noise(o.seed, in.trial, (uint32_t)k, (uint32_t)s, nzb, in.real);
@@ -391,7 +446,9 @@ struct TvlqrDirectSrc {
   }
   TS_HD void done(long long) const {}
 };
-template <bool PRE, class Src>
+// DISP: a dispersed realisation (in.disp; in.I holds its truth inertia): transformed field rows when the records are
+// built here, and the scaled torque in every stage.
+template <bool PRE, class Src, bool DISP = false>
 TS_HD long long tvlqr_replay_src(const TvlqrIn& in, const ts_tvlqr_opts_dev& o, Src& src, double* X_sim, double* U_sim,
                                  double* dX, double* slew_time_out, double* x_last = nullptr) {
   const int N = in.N;
@@ -453,21 +510,21 @@ TS_HD long long tvlqr_replay_src(const TvlqrIn& in, const ts_tvlqr_opts_dev& o, 
       if constexpr (PRE) {
         return rk_src + s * TV_REC;
       } else {
-        tvlqr_stage_record_at(in, o, k, s, tcl[s], rbuf);
+        tvlqr_stage_record_at<DISP>(in, o, k, s, tcl[s], rbuf);
         return rbuf;
       }
     };
     double k1[7], k2[7], k3[7], k4[7], xs[7];
-    simulator7_rec(in.I, x, u, rec(0), k1);
+    simulator7_rec<DISP>(in.I, x, u, rec(0), k1, &in.disp);
     for (int i = 0; i < 7; ++i) k1[i] = k1[i] * o.dt;
     for (int i = 0; i < 7; ++i) xs[i] = x[i] + k1[i] / 2.0;
-    simulator7_rec(in.I, xs, u, rec(1), k2);
+    simulator7_rec<DISP>(in.I, xs, u, rec(1), k2, &in.disp);
     for (int i = 0; i < 7; ++i) k2[i] = k2[i] * o.dt;
     for (int i = 0; i < 7; ++i) xs[i] = x[i] + k2[i] / 2.0;
-    simulator7_rec(in.I, xs, u, rec(2), k3);
+    simulator7_rec<DISP>(in.I, xs, u, rec(2), k3, &in.disp);
     for (int i = 0; i < 7; ++i) k3[i] = k3[i] * o.dt;
     for (int i = 0; i < 7; ++i) xs[i] = x[i] + k3[i];
-    simulator7_rec(in.I, xs, u, rec(3), k4);
+    simulator7_rec<DISP>(in.I, xs, u, rec(3), k4, &in.disp);
     for (int i = 0; i < 7; ++i) k4[i] = k4[i] * o.dt;
     for (int i = 0; i < 7; ++i) x[i] = x[i] + (k1[i] + 2.0 * k2[i] + 2.0 * k3[i] + k4[i]) * TS_SIXTH;
     x[7] = nxt;

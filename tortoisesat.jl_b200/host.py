@@ -90,6 +90,14 @@ class ReplayEnsembleOpts(C.Structure):
     _fields_ = [("n_real", C.c_int64), ("r_first", C.c_int64), ("q_noise_scale", C.c_double)]
 
 
+class DispersionOpts(C.Structure):
+    """ts_dispersion_opts (include/tortoise_b200.h): the truth-model error sigmas of a dispersion ensemble (DE2)."""
+    _fields_ = [(k, C.c_double) for k in ("sigma_inertia", "sigma_torquer", "sigma_field_scale", "sigma_field_angle")]
+
+
+DISPERSION_PARAMS = ("d0", "d1", "d2", "g0", "g1", "g2", "s_B", "phi0", "phi1", "phi2")   # order of a params row
+
+
 Q_NOISE_SCALE = (np.pi / 180) ** 2   # initial attitude noise of monte_carlo.jl: randn(3)*(pi/180)^2
 
 
@@ -168,6 +176,8 @@ def load_library():
     L.ts_mc_continue.argtypes = [C.c_void_p, C.c_int64, C.POINTER(IlqrOpts), C.c_void_p, C.POINTER(McStats)]
     L.ts_mc_replay_ensemble.argtypes = [C.c_void_p, C.c_int64, C.POINTER(ReplayEnsembleOpts), C.c_int64] + [C.c_void_p] * 3
     L.ts_mc_replay_ensemble_last_split.argtypes = [C.c_void_p, c_double_p, c_double_p]
+    L.ts_mc_dispersion_ensemble.argtypes = [C.c_void_p, C.c_int64, C.POINTER(ReplayEnsembleOpts), C.POINTER(DispersionOpts),
+                                            C.c_int64] + [C.c_void_p] * 4
     L.ts_igrf12syn_batch.argtypes = [C.c_void_p, C.c_int, C.c_double, C.c_int, C.c_int64] + [C.c_void_p] * 7 + [C.c_int]
     L.ts_psiaki_pd_batch.argtypes = [C.c_void_p, C.c_int64] + [C.c_void_p] * 7 + [C.c_double] * 3 + [C.c_void_p] * 3
     L.ts_attitude_dynamics_linear_batch.argtypes = [C.c_void_p, C.c_int64] + [C.c_void_p] * 6
@@ -182,6 +192,8 @@ def load_library():
     L.ts_multi_monte_carlo_run.argtypes = [C.c_void_p, C.POINTER(McConfig)] + [C.c_void_p] * 8 + [C.POINTER(McStats)]
     L.ts_multi_mc_continue.argtypes = [C.c_void_p, C.c_int64, C.POINTER(IlqrOpts), C.c_void_p, C.POINTER(McStats)]
     L.ts_multi_mc_replay_ensemble.argtypes = [C.c_void_p, C.c_int64, C.POINTER(ReplayEnsembleOpts), C.c_int64] + [C.c_void_p] * 3
+    L.ts_multi_mc_dispersion_ensemble.argtypes = [C.c_void_p, C.c_int64, C.POINTER(ReplayEnsembleOpts), C.POINTER(DispersionOpts),
+                                                  C.c_int64] + [C.c_void_p] * 4
     L.ts_igrf12_batch.argtypes = [C.c_void_p, C.c_double, C.c_int64] + [C.c_void_p] * 6 + [C.c_int]
     L.ts_field_map_prefilter.argtypes = [C.c_void_p, C.c_int64, C.c_int64, C.c_void_p, C.c_void_p, C.c_int]
     L.ts_field_map_eval_batch.argtypes = [C.c_void_p, C.c_int64, C.c_int64, C.c_void_p, C.c_int64] + [C.c_void_p] * 3 + [C.c_int]
@@ -681,6 +693,17 @@ class Engine:
         return _replay_ensemble(self.lib.ts_mc_replay_ensemble, self.h, n_trials, n_real, r_first, trials, q_noise_scale,
                                 want_x_final, self._check)
 
+    def mc_dispersion_ensemble(self, n_trials, n_real, sigma_inertia=0.0, sigma_torquer=0.0, sigma_field_scale=0.0,
+                               sigma_field_angle=0.0, r_first=0, trials=None, q_noise_scale=Q_NOISE_SCALE, want_x_final=False,
+                               want_params=False):
+        """The kept run's slews replayed as mc_replay_ensemble does, each realisation with drawn truth-model errors of the
+        inertia, torquer gains and field model (ts_mc_dispersion_ensemble, rules DE1-DE6; sigma_field_angle in radians).
+        Returns (slew_time (n_sel, n_real), x_final (n_sel, n_real, 8) or None, params (n_sel, n_real, 10) in the order
+        DISPERSION_PARAMS, or None); a NO_CUTOFF trial gets NaN rows.  Realisation 0 carries no dispersion (DE3)."""
+        d = DispersionOpts(float(sigma_inertia), float(sigma_torquer), float(sigma_field_scale), float(sigma_field_angle))
+        return _dispersion_ensemble(self.lib.ts_mc_dispersion_ensemble, self.h, n_trials, n_real, d, r_first, trials,
+                                    q_noise_scale, want_x_final, want_params, self._check)
+
     def mc_replay_ensemble_split(self):
         """Device ms of the last mc_replay_ensemble: (gains, ensemble replay)."""
         g, r = C.c_double(), C.c_double()
@@ -786,6 +809,18 @@ class MultiEngine:
                                 want_x_final, check)
 
 
+    def mc_dispersion_ensemble(self, n_trials, n_real, sigma_inertia=0.0, sigma_torquer=0.0, sigma_field_scale=0.0,
+                               sigma_field_angle=0.0, r_first=0, trials=None, q_noise_scale=Q_NOISE_SCALE, want_x_final=False,
+                               want_params=False):
+        """Engine.mc_dispersion_ensemble over the devices' kept shards; the rows equal the single-device rows (DE5)."""
+        def check(rc):
+            if rc != 0:
+                raise TortoiseError(rc, (self.lib.ts_multi_last_error(self.h) or b"").decode())
+        d = DispersionOpts(float(sigma_inertia), float(sigma_torquer), float(sigma_field_scale), float(sigma_field_angle))
+        return _dispersion_ensemble(self.lib.ts_multi_mc_dispersion_ensemble, self.h, n_trials, n_real, d, r_first, trials,
+                                    q_noise_scale, want_x_final, want_params, check)
+
+
 def _replay_ensemble(fn, h, n_trials, n_real, r_first, trials, q_noise_scale, want_x_final, check):
     n = int(n_trials)
     o = ReplayEnsembleOpts(int(n_real), int(r_first), float(q_noise_scale))
@@ -796,6 +831,20 @@ def _replay_ensemble(fn, h, n_trials, n_real, r_first, trials, q_noise_scale, wa
     xf = np.zeros((ns, R, 8)) if want_x_final else None
     check(fn(h, n, C.byref(o), ns, None if sel is None else _ptr(sel), _ptr(slew), None if xf is None else _ptr(xf)))
     return slew, xf
+
+
+def _dispersion_ensemble(fn, h, n_trials, n_real, disp, r_first, trials, q_noise_scale, want_x_final, want_params, check):
+    n = int(n_trials)
+    o = ReplayEnsembleOpts(int(n_real), int(r_first), float(q_noise_scale))
+    sel = None if trials is None else np.ascontiguousarray(trials, dtype=np.int64).reshape(-1)
+    ns = n if sel is None else sel.shape[0]
+    R = max(int(n_real), 0)
+    slew = np.zeros((ns, R))
+    xf = np.zeros((ns, R, 8)) if want_x_final else None
+    prm = np.zeros((ns, R, 10)) if want_params else None
+    check(fn(h, n, C.byref(o), C.byref(disp), ns, None if sel is None else _ptr(sel), _ptr(slew), None if xf is None else _ptr(xf),
+             None if prm is None else _ptr(prm)))
+    return slew, xf, prm
 
 
 # ---------------------------------------------------------------------------
@@ -1201,6 +1250,10 @@ def replay_ensemble(res, n_real=100, trials=None, r_first=0, q_noise_scale=Q_NOI
     n = out.shape[0]
     sel = np.arange(n, dtype=np.int64) if trials is None else np.ascontiguousarray(trials, dtype=np.int64).reshape(-1)
     slew, _ = default_engine().mc_replay_ensemble(n, n_real, r_first=r_first, trials=sel, q_noise_scale=q_noise_scale)
+    return _ensemble_stats(out, sel, slew)
+
+
+def _ensemble_stats(out, sel, slew):
     tf = out["t_final"][sel][:, None]
     fails = slew == tf
     valid = ~np.isnan(slew)
@@ -1213,6 +1266,27 @@ def replay_ensemble(res, n_real=100, trials=None, r_first=0, q_noise_scale=Q_NOI
         mean = np.where(k > 0, s.sum(axis=1) / np.maximum(k, 1), np.nan)
         var = np.where(k > 0, (np.where(ok, slew - mean[:, None], 0.0) ** 2).sum(axis=1) / np.maximum(k, 1), np.nan)
     return dict(slew_time=slew, fails=fails, fail_rate=fail_rate, slew_mean=mean, slew_std=np.sqrt(var), trials=sel)
+
+
+def dispersion_ensemble(res, n_real=100, trials=None, r_first=1, sigma_inertia=0.0, sigma_torquer=0.0, sigma_field_scale=0.0,
+                        sigma_field_angle=0.0, q_noise_scale=Q_NOISE_SCALE):
+    """replay_ensemble with truth-model errors (ts_mc_dispersion_ensemble on the default engine, rules DE1-DE6): every
+    selected trial's slew replayed n_real times with the nominal TVLQR gains, each realisation under drawn inertia
+    (J_true = D J D, d_i = exp(sigma_inertia z / 2)), torquer-gain (exp(sigma_torquer z)) and field-model errors
+    (magnitude exp(sigma_field_scale z), rotation vector sigma_field_angle z, radians) on top of the simulator's
+    disturbances.  r_first = 1 by default: realisation 0 carries no dispersion (DE3) and would bias the statistics.
+    Returns replay_ensemble's dict plus params (n_sel, n_real, 10), in the order DISPERSION_PARAMS."""
+    if "states" not in res and "ilqr" not in res:
+        raise ValueError("dispersion_ensemble needs a monte_carlo(..., trajectories=True) or monte_carlo(..., resumable=True) result")
+    out = res["outcomes"]
+    n = out.shape[0]
+    sel = np.arange(n, dtype=np.int64) if trials is None else np.ascontiguousarray(trials, dtype=np.int64).reshape(-1)
+    slew, _, prm = default_engine().mc_dispersion_ensemble(n, n_real, sigma_inertia, sigma_torquer, sigma_field_scale,
+                                                           sigma_field_angle, r_first=r_first, trials=sel,
+                                                           q_noise_scale=q_noise_scale, want_params=True)
+    d = _ensemble_stats(out, sel, slew)
+    d["params"] = prm
+    return d
 
 
 # ---------------------------------------------------------------------------
