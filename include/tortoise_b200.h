@@ -453,6 +453,36 @@ typedef struct ts_dispersion_opts {
 int ts_mc_dispersion_ensemble(ts_ctx* ctx, int64_t n_trials, const ts_replay_ensemble_opts* opts, const ts_dispersion_opts* disp,
                               int64_t n_sel, const int64_t* trials, double* slew_time, double* x_final, double* params);
 
+/* ---- weight-sweep ensembles: the kept run's slews under the TVLQR gains of many tracking weightings ---------------- *
+ * ts_mc_weight_ensemble replays the kept run's slews as ts_mc_dispersion_ensemble does, once per weighting of sets:
+ * the gains of set w come from the kept trajectory, linearised once, and a Riccati sweep with set w's diagonals of Q,
+ * Qf and R (DESIGN.md section 4, K4):
+ *  WE1 the kept run: as RE1, with the argument checks of ts_mc_replay_ensemble.
+ *  WE2 paired draws: row (t, w, r) uses DE2's draws for (t, r) -- stage noise, initial attitude (r >= 1) and the ten
+ *      truth-model normals; a null disp means all four sigmas 0.  The draws do not depend on w.  Every TVLQR option
+ *      other than the weights is the run's, with the fused path's overrides.
+ *  WE3 a set equal to the run's cfg.tvlqr weights, with u_limit 0, gives ts_mc_dispersion_ensemble's rows bit for bit
+ *      (ts_mc_replay_ensemble's with a null disp); its realisation 0 is the kept record.
+ *  WE4 torquer limit: u_limit 0 = none (simulator.jl); u_limit > 0 clamps each component of u = U_lqr - K dx to
+ *      [-u_limit, u_limit] before it drives the step's four rk4 stages (a NaN stays NaN).  It acts in the truth model
+ *      only; the gains are unchanged.  The planner's bound cfg.ilqr.u_max is the physical choice.
+ *  WE5 a row depends on the kept run, t, r, q_noise_scale, the sigmas, set w's weights and u_limit alone: not on the
+ *      other sets, their number or order, chunking, the other selected trials, their order or the number of devices.
+ *  WE6 isolation, as RE5: later calls behave as if this call never ran.
+ *  WE7 TS_ERR_ARG, outputs untouched: every case of ts_mc_dispersion_ensemble (the sigma checks when disp is
+ *      non-null), n_sets < 1, a null sets, a Qd or Qfd entry negative or not finite, an Rd entry <= 0 or not finite, a
+ *      u_limit negative or not finite.  TS_ERR_NOMEM, outputs untouched, when the gains of all sets (144 bytes per kept
+ *      knot and set) or the device outputs do not fit: chunk the sets or the realisations (exact by WE5).
+ * Outputs (HOST): slew_time n_sel x n_sets x n_real, x_final (nullable) n_sel x n_sets x n_real x 8.  A TS_ST_NO_CUTOFF
+ * trial gets NaN rows in every set.  ts_last_kernel_ms and ts_mc_replay_ensemble_last_split report this call (gains:
+ * the linearisation and every set's Riccati sweep; replay: the ensemble replay).                                        */
+typedef struct ts_tvlqr_weights {   /* one tracking weighting: the diagonals of ts_tvlqr_opts' Q, Qf, R (120 bytes)   */
+  double Qd[6], Qfd[6], Rd[3];
+} ts_tvlqr_weights;
+int ts_mc_weight_ensemble(ts_ctx* ctx, int64_t n_trials, const ts_replay_ensemble_opts* opts, const ts_dispersion_opts* disp,
+                          int64_t n_sets, const ts_tvlqr_weights* sets, double u_limit, int64_t n_sel, const int64_t* trials,
+                          double* slew_time, double* x_final);
+
 /* ---- igrf12syn: the Fortran-style twin of igrf12 -------------------------------------------- *
  * igrf12syn(isv, date, itype, alt, colat, elong) [src/igrf.jl:335-534] at n points.  isv 0 = main field, 1 = secular
  * variation; itype 1 = geodetic (alt = height above the WGS-84 ellipsoid, km), 2 = geocentric (alt = radius, km);
@@ -503,6 +533,11 @@ int ts_multi_mc_replay_ensemble(ts_multi* m, int64_t n_trials, const ts_replay_e
  * ts_multi_mc_replay_ensemble; the rows equal the single-device rows bit for bit (DE5).                              */
 int ts_multi_mc_dispersion_ensemble(ts_multi* m, int64_t n_trials, const ts_replay_ensemble_opts* opts, const ts_dispersion_opts* disp,
                                     int64_t n_sel, const int64_t* trials, double* slew_time, double* x_final, double* params);
+/* ts_mc_weight_ensemble over a ts_multi_monte_carlo_run kept with keep_trajectories >= 1, dispatched as
+ * ts_multi_mc_replay_ensemble; the rows equal the single-device rows bit for bit (WE5).                                  */
+int ts_multi_mc_weight_ensemble(ts_multi* m, int64_t n_trials, const ts_replay_ensemble_opts* opts, const ts_dispersion_opts* disp,
+                                int64_t n_sets, const ts_tvlqr_weights* sets, double u_limit, int64_t n_sel, const int64_t* trials,
+                                double* slew_time, double* x_final);
 
 /* ---- element-wise batch versions of the reference's building blocks (all HOST pointers) --- *
  * Correctness / drop-in paths for callers that use the small functions on their own; the fused

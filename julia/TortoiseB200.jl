@@ -81,6 +81,9 @@ end
 struct DispersionOpts   # ts_dispersion_opts
     sigma_inertia::Float64; sigma_torquer::Float64; sigma_field_scale::Float64; sigma_field_angle::Float64
 end
+struct TvlqrWeights   # ts_tvlqr_weights: one tracking weighting, the diagonals of Q, Qf, R (120 bytes)
+    Qd::NTuple{6, Float64}; Qfd::NTuple{6, Float64}; Rd::NTuple{3, Float64}
+end
 function default_ilqr_opts()
     r = Ref{IlqrOpts}()
     ccall((:ts_ilqr_default_opts, LIB), Cvoid, (Ref{IlqrOpts},), r); r[]
@@ -467,6 +470,46 @@ function dispersion_ensemble(res; n_real::Integer = 100, trials = nothing, r_fir
     return merge(ensemble_stats(res, sel, slew, n_real), (params = prm,))
 end
 
+# ts_mc_weight_ensemble: mc_dispersion_ensemble once per tracking weighting of `sets` (a vector of TvlqrWeights), the
+# gains of each from its own Riccati sweep and the same draws for every set (rules WE1-WE7, DESIGN.md section 4).
+# u_limit > 0 clamps each dipole command component to [-u_limit, u_limit] in the truth model (the planner's u_max is the
+# physical choice); disp = nothing: no truth-model error.  Returns slew_time (n_real x n_sets x n_sel) and, with
+# want_x_final, x_final (8 x n_real x n_sets x n_sel); a NO_CUTOFF trial gets NaN columns.
+function mc_weight_ensemble(number_sims::Integer, n_real::Integer, sets::Vector{TvlqrWeights}; u_limit::Float64 = 0.0,
+                            disp::Union{Nothing,DispersionOpts} = nothing, r_first::Integer = 0, trials = nothing,
+                            q_noise_scale::Float64 = (pi / 180)^2, want_x_final::Bool = false, e::Engine = engine())
+    sel = trials === nothing ? C_NULL : Int64[t - 1 for t in trials]
+    ns = trials === nothing ? number_sims : length(trials)
+    nw = length(sets)
+    slew = zeros(n_real, nw, ns); xf = want_x_final ? zeros(8, n_real, nw, ns) : nothing
+    o = ReplayEnsembleOpts(n_real, r_first, q_noise_scale)
+    dp = disp === nothing ? Ptr{DispersionOpts}(C_NULL) : Ref(disp)
+    check(e, ccall((:ts_mc_weight_ensemble, LIB), Cint,
+                   (Ptr{Cvoid}, Int64, Ref{ReplayEnsembleOpts}, Ptr{DispersionOpts}, Int64, Ptr{TvlqrWeights}, Float64, Int64,
+                    Ptr{Int64}, Ptr{Float64}, Ptr{Float64}),
+                   e.h, number_sims, Ref(o), dp, nw, sets, u_limit, ns, sel, slew, xf === nothing ? C_NULL : xf))
+    return slew, xf
+end
+
+# replay_ensemble's statistics per weighting (each field gains a set dimension after the realisations), plus
+# set_fail_rate (one per set, over every selected trial); r_first = 1 leaves the nominal realisation 0 out.
+function weight_ensemble(res, sets::Vector{TvlqrWeights}; n_real::Integer = 100, trials = nothing, r_first::Integer = 1,
+                         u_limit::Float64 = 0.0, sigma_inertia::Float64 = 0.0, sigma_torquer::Float64 = 0.0,
+                         sigma_field_scale::Float64 = 0.0, sigma_field_angle::Float64 = 0.0, q_noise_scale::Float64 = (pi / 180)^2,
+                         e::Engine = engine())
+    n = length(res.outcomes)
+    sel = trials === nothing ? collect(1:n) : collect(trials)
+    d = DispersionOpts(sigma_inertia, sigma_torquer, sigma_field_scale, sigma_field_angle)
+    slew, _ = mc_weight_ensemble(n, n_real, sets; u_limit = u_limit, disp = d, r_first = r_first, trials = sel,
+                                 q_noise_scale = q_noise_scale, e = e)
+    per = [ensemble_stats(res, sel, slew[:, w, :], n_real) for w in eachindex(sets)]
+    fails = cat([p.fails for p in per]...; dims = 3)                # n_real x n_sel x n_sets
+    set_fail_rate = [sum(fails[:, :, w]) / count(!isnan, slew[:, w, :]) for w in eachindex(sets)]
+    return (slew_time = slew, fails = permutedims(fails, (1, 3, 2)),
+            fail_rate = permutedims(hcat([p.fail_rate for p in per]...)), slew_mean = permutedims(hcat([p.slew_mean for p in per]...)),
+            slew_std = permutedims(hcat([p.slew_std for p in per]...)), set_fail_rate = set_fail_rate, trials = sel)
+end
+
 # Continues a monte_carlo(...; resumable = true) result `res` in place to max_outer outer iterations in all: outcomes,
 # slew_time, fails (monte_carlo.jl:257-261) and the trajectory arrays of the continued trials.  Returns their indices.
 function continue_monte_carlo!(res; max_outer = 30, ilqr::Union{Nothing,IlqrOpts} = nothing, e::Engine = engine())
@@ -589,6 +632,6 @@ export Engine, params, input_parameters, igrf12, igrf12_batch, igrf_data, magnet
        condition_based_time, eigen_axis_slew, bryson_weights, solve_slew, attitude_simulation, monte_carlo, qmult, qrot, q_inv, hat,
        igrf12syn, attitude_dynamics_linear, psiaki_pd_simulation, igrf_interpolant, field_map_prefilter, field_map_eval, AlState,
        mc_state, mc_continue, continue_monte_carlo!, ReplayEnsembleOpts, mc_replay_ensemble, replay_ensemble,
-       DispersionOpts, mc_dispersion_ensemble, dispersion_ensemble
+       DispersionOpts, mc_dispersion_ensemble, dispersion_ensemble, TvlqrWeights, mc_weight_ensemble, weight_ensemble
 
 end # module

@@ -38,6 +38,7 @@ enum Slot : int {
   SLOT_AL_STATES,                          // K3 continuation: a call's imported and exported solver states
   SLOT_KEPT_STATE,                         // Monte-Carlo kept solver states + multipliers (ts_mc_fetch_state, ts_mc_continue)
   SLOT_ENSEMBLE_OUT,                       // an ensemble's slew times, final states and parameters (ts_mc_replay_ensemble, ts_mc_dispersion_ensemble)
+  SLOT_WEIGHT_SETS,                        // a weight-sweep ensemble's weightings (ts_mc_weight_ensemble)
   SLOT_COUNT
 };
 
@@ -100,7 +101,7 @@ struct ts_ctx {
   char name[128] = {0};
   int64_t launches = 0;
   double last_kernel_ms = 0.0;
-  double ens_ms[2] = {0.0, 0.0};  // the last ts_mc_replay_ensemble / ts_mc_dispersion_ensemble: gains (K4a + K4b) | replay (K4e / K4d)
+  double ens_ms[2] = {0.0, 0.0};  // the last replay / dispersion / weight ensemble: gains (K4a + K4b / K4w) | replay (K4e / K4d / K4w)
   double* d_tabG = nullptr;  // 104 x 25
   double* d_tabH = nullptr;  // 91 x 25
   double* d_tabGH = nullptr; // 3450 (igrf12syn)
@@ -147,6 +148,19 @@ inline bool dispersion_opts_ok(const ts_dispersion_opts* d) {
   const double s[4] = {d->sigma_inertia, d->sigma_torquer, d->sigma_field_scale, d->sigma_field_angle};
   for (int i = 0; i < 4; ++i)
     if (!std::isfinite(s[i]) || s[i] < 0.0 || s[i] > (i < 3 ? 1.0 : 3.14159265358979323846)) return false;
+  return true;
+}
+
+// The weightings and torquer limit a weight-sweep ensemble accepts (ts_mc_weight_ensemble, WE7): n_sets >= 1, every Qd
+// and Qfd entry finite and >= 0, every Rd entry finite and > 0 (B'SB + R stays invertible), u_limit finite and >= 0.
+inline bool weight_sets_ok(int64_t n_sets, const ts_tvlqr_weights* sets, double u_limit) {
+  if (n_sets < 1 || !sets || !std::isfinite(u_limit) || u_limit < 0.0) return false;
+  for (int64_t w = 0; w < n_sets; ++w) {
+    for (int i = 0; i < 6; ++i)
+      if (!std::isfinite(sets[w].Qd[i]) || sets[w].Qd[i] < 0.0 || !std::isfinite(sets[w].Qfd[i]) || sets[w].Qfd[i] < 0.0) return false;
+    for (int i = 0; i < 3; ++i)
+      if (!std::isfinite(sets[w].Rd[i]) || !(sets[w].Rd[i] > 0.0)) return false;
+  }
   return true;
 }
 

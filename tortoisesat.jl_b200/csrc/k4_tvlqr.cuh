@@ -147,131 +147,40 @@ __global__ void __launch_bounds__(K4B_TEAM * K4B_TEAMS_PER_BLOCK) k4b_riccati_te
   const int team = threadIdx.x / K4B_TEAM, c = threadIdx.x % K4B_TEAM;
   const int64_t t = (int64_t)blockIdx.x * K4B_TEAMS_PER_BLOCK + team;
   if (t >= a.n_trials) return;   // the whole team leaves together
-  const unsigned mask = 0xFFFFu << (16 * ((threadIdx.x / K4B_TEAM) & 1));
-  double* ring = sm_all + team * K4B_TEAM_DOUBLES;
-  double* xBSB = ring + K4B_XB;
-  double* xK = xBSB + 12;
-  double* xAcl = xK + 20;
-  double* xSn = xAcl + 36;
-  const int N = (int)a.N_i[t];
-  double S[36];
+#define K4B_QD(i) a.opts.Qd[i]
+#define K4B_QFD(i) a.opts.Qfd[i]
+#define K4B_RD(i) a.opts.Rd[i]
+#define K4B_GAINS a.K
+#define K4B_CLOCK true
+#include "k4b_riccati_body.inc"
+}
+
+// ---- K4w gains: K4b's team step with one team per (slew, weighting) of a weight-sweep ensemble (ts_mc_weight_ensemble,
+// WE2 of DESIGN.md section 4, K4).  The teams of one slew are adjacent and share its [A|B] records in L2.  Team (t, w)
+// reads weighting w (Qd 6 | Qfd 6 | Rd 3 doubles at sets + 15 w) into registers and writes its gains at K + w k_stride +
+// offs[t] * 18; the team of weighting 0 alone writes the slew's replay clock sequence.
+struct K4wGainsArgs {
+  K4Args a;                          // the selected slews' K4 arguments (a.K unused)
+  const double* sets;                // n_sets x 15
+  int64_t n_sets, k_stride;          // k_stride: doubles per weighting's gains region
+  double* K;
+};
+__global__ void __launch_bounds__(K4B_TEAM * K4B_TEAMS_PER_BLOCK) k4w_riccati_sets_kernel(const K4wGainsArgs aw) {
+  __shared__ __align__(16) double sm_all[K4B_TEAMS_PER_BLOCK * K4B_TEAM_DOUBLES];
+  const K4Args& a = aw.a;
+  const int team = threadIdx.x / K4B_TEAM, c = threadIdx.x % K4B_TEAM;
+  const int64_t g = (int64_t)blockIdx.x * K4B_TEAMS_PER_BLOCK + team;
+  if (g >= a.n_trials * aw.n_sets) return;   // the whole team leaves together
+  const int64_t t = g / aw.n_sets, ws = g - t * aw.n_sets;
+  double wq[15];
 #pragma unroll
-  for (int i = 0; i < 36; ++i) S[i] = 0.0;
-#pragma unroll
-  for (int i = 0; i < 6; ++i) S[i * 6 + i] = a.opts.Qfd[i];
-  const double* ab = a.AB + a.lin_offs[t] * 54;
-  double* K = a.K + a.offs[t] * 18;
-  auto issue = [&](int k) {   // record k -> slot (k mod D): 27 pieces of 16 bytes, lanes 0..13 take two each
-    if (k >= 0) {
-      const unsigned dst = (unsigned)__cvta_generic_to_shared(ring + (k % K4_RING_D) * 54);
-      const double* src = ab + (long long)k * 54;
-      for (int pc = c; pc < 27; pc += 14)
-        if (c < 14) asm volatile("cp.async.cg.shared.global [%0], [%1], 16;\n" ::"r"(dst + 16u * pc), "l"(src + 2 * pc) : "memory");
-    }
-    k4_commit();
-  };
-  for (int d = 0; d < K4_RING_D; ++d) issue(N - 2 - d);
-  const bool isA = c < 6, isB = c >= 6 && c < 9;
-  const int cc = isA ? c : (isB ? c - 6 : 0);
-#pragma unroll 1
-  for (int k = N - 2; k >= 0; --k) {
-    k4_wait_oldest();
-    __syncwarp(mask);
-    const double* A = ring + (k % K4_RING_D) * 54;
-    const double* B = A + 36;
-    // ---- stage 1: SX = S col, BX = B' SX  (col = column cc of A, or of B on lanes 6..8)
-    double col[6], SX[6], BX[3];
-#pragma unroll
-    for (int l = 0; l < 6; ++l) col[l] = isB ? B[l * 3 + cc] : A[l * 6 + cc];
-#pragma unroll
-    for (int i = 0; i < 6; ++i) {
-      double s = 0.0;
-#pragma unroll
-      for (int l = 0; l < 6; ++l) s += S[i * 6 + l] * col[l];
-      SX[i] = s;
-    }
-#pragma unroll
-    for (int r = 0; r < 3; ++r) {
-      double s = 0.0;
-#pragma unroll
-      for (int l = 0; l < 6; ++l) s += B[l * 3 + r] * SX[l];
-      BX[r] = s;
-    }
-    if (isB)
-#pragma unroll
-      for (int r = 0; r < 3; ++r) xBSB[r * 3 + cc] = BX[r] + ((r == cc) ? a.opts.Rd[r] : 0.0);
-    __syncwarp(mask);
-    // ---- stage 2: gain column, closed-loop column, S Acl column
-    double BSB[9], Minv[9], Kc[3], Ac[6], SAc[6];
-#pragma unroll
-    for (int i = 0; i < 9; ++i) BSB[i] = xBSB[i];
-    inv3_adj(BSB, Minv);
-#pragma unroll
-    for (int r = 0; r < 3; ++r) {
-      double s = 0.0;
-#pragma unroll
-      for (int l = 0; l < 3; ++l) s += Minv[r * 3 + l] * BX[l];
-      Kc[r] = s;
-    }
-#pragma unroll
-    for (int i = 0; i < 6; ++i) {
-      double s = 0.0;
-#pragma unroll
-      for (int l = 0; l < 3; ++l) s += B[i * 3 + l] * Kc[l];
-      Ac[i] = col[i] - s;
-    }
-#pragma unroll
-    for (int i = 0; i < 6; ++i) {
-      double s = 0.0;
-#pragma unroll
-      for (int l = 0; l < 6; ++l) s += S[i * 6 + l] * Ac[l];
-      SAc[i] = s;
-    }
-    if (isA) {
-      double* Kout = K + (long long)k * 18;
-#pragma unroll
-      for (int r = 0; r < 3; ++r) {
-        xK[r * 6 + cc] = Kc[r];
-        Kout[r * 6 + cc] = Kc[r];
-      }
-#pragma unroll
-      for (int i = 0; i < 6; ++i) xAcl[i * 6 + cc] = Ac[i];
-    }
-    __syncwarp(mask);
-    // ---- stage 3: column cc of the new S
-    if (isA) {
-#pragma unroll
-      for (int i = 0; i < 6; ++i) {
-        double s = (i == cc) ? a.opts.Qd[i] : 0.0;
-        double kr = 0.0;
-#pragma unroll
-        for (int l = 0; l < 3; ++l) kr += xK[l * 6 + i] * a.opts.Rd[l] * Kc[l];
-        s += kr;
-        double tt = 0.0;
-#pragma unroll
-        for (int l = 0; l < 6; ++l) tt += xAcl[l * 6 + i] * SAc[l];
-        xSn[i * 6 + cc] = s + tt;
-      }
-    }
-    __syncwarp(mask);
-#pragma unroll
-    for (int i = 0; i < 36; ++i) S[i] = xSn[i];
-    __syncwarp(mask);   // everybody has read the record and the exchange area: the slot may be refilled
-    issue(k - K4_RING_D);
-  }
-  asm volatile("cp.async.wait_all;\n" ::: "memory");
-  if (c == 0) {
-    // the replay's clock state at every step (the reference accumulates it through rk4: sequential, exact replica)
-    double x8 = a.x0_lqr[t * 8 + 7];
-    double* clk = a.clk + a.lin_offs[t];
-#pragma unroll 1
-    for (int k = 0; k < N - 1; ++k) {
-      clk[k] = x8;
-      double tcl[4], nxt;
-      clock_rk4(x8, a.clock_rate[t], a.opts.dt, tcl, nxt);
-      x8 = nxt;
-    }
-  }
+  for (int i = 0; i < 15; ++i) wq[i] = aw.sets[ws * 15 + i];
+#define K4B_QD(i) wq[i]
+#define K4B_QFD(i) wq[6 + (i)]
+#define K4B_RD(i) wq[12 + (i)]
+#define K4B_GAINS (aw.K + ws * aw.k_stride)
+#define K4B_CLOCK (ws == 0)
+#include "k4b_riccati_body.inc"
 }
 
 // ---- K4n: the stage records of the replay (tvlqr_solver.cuh): for every rk4 stage of every step the disturbance draws of
@@ -506,17 +415,40 @@ struct K4dArgs {
   double sigma[4];                   // sigma_inertia, sigma_torquer, sigma_field_scale, sigma_field_angle
   double* params;                    // n_sel x n_real x DISP_NP, nullable
 };
+// K4w: the weight-sweep ensemble of a kept run (ts_mc_weight_ensemble, WE1-WE7): K4d's replay (DISP = true; a null
+// dispersion is four zero sigmas) with one warp per (slew, weighting, 32 realisations).  The warps of one slew are
+// adjacent, its weightings in order, so they share the slew's reference rows in L2; the staging ring reads weighting w's
+// gains (K4w gains layout).  CLAMP: the torquer limit u_limit (WE4).
+struct K4wArgs {
+  K4dArgs d;                         // d.e.n_sel slews; d.params unused
+  int64_t n_sets, k_stride;
+  double u_limit;
+};
 __global__ void __launch_bounds__(32 * K4E_WARPS) k4e_ensemble_replay_kernel(const K4eArgs a) {
-  constexpr bool DISP = false;
+  constexpr bool DISP = false, CLAMP = false;
+  constexpr int64_t n_sets = 1, k_stride = 0;
+  constexpr double u_limit = 0.0;
   const double* sigma = nullptr;
   double* params = nullptr;
 #include "k4e_replay_body.inc"
 }
 __global__ void __launch_bounds__(32 * K4E_WARPS) k4d_dispersion_replay_kernel(const K4dArgs ad) {
-  constexpr bool DISP = true;
+  constexpr bool DISP = true, CLAMP = false;
+  constexpr int64_t n_sets = 1, k_stride = 0;
+  constexpr double u_limit = 0.0;
   const K4eArgs& a = ad.e;
   const double* sigma = ad.sigma;
   double* params = ad.params;
+#include "k4e_replay_body.inc"
+}
+template <bool CLAMP>
+__global__ void __launch_bounds__(32 * K4E_WARPS) k4w_weight_replay_kernel(const K4wArgs aw) {
+  constexpr bool DISP = true;
+  const int64_t n_sets = aw.n_sets, k_stride = aw.k_stride;
+  const double u_limit = aw.u_limit;
+  const K4eArgs& a = aw.d.e;
+  const double* sigma = aw.d.sigma;
+  double* params = nullptr;
 #include "k4e_replay_body.inc"
 }
 

@@ -268,23 +268,24 @@ int ts_multi_mc_continue(ts_multi* m, int64_t n_trials, const ts_ilqr_opts* opts
   return multi_shards(m, n_trials, shard, out, stats);
 }
 
-// ts_multi_mc_replay_ensemble and ts_multi_mc_dispersion_ensemble (disp non-null): each trial on the device that holds
-// it, all devices at once, rows back in the caller's order.  The argument checks of the single-device entry run before
-// any device does: a failure leaves the outputs untouched.
+// ts_multi_mc_replay_ensemble, ts_multi_mc_dispersion_ensemble (dispersed) and ts_multi_mc_weight_ensemble (ws): each
+// trial on the device that holds it, all devices at once, rows back in the caller's order.  The argument checks of the
+// single-device entry run before any device does: a failure leaves the outputs untouched.
 static int multi_ensemble(ts_multi* m, const char* fn, int64_t n_trials, const ts_replay_ensemble_opts* opts, bool dispersed,
                           const ts_dispersion_opts* disp, int64_t n_sel, const int64_t* trials, double* slew_time, double* x_final,
-                          double* params) {
+                          double* params, const WeightSets* ws = nullptr) {
   if (!m) return TS_ERR_ARG;
   const int G = m->n;
   bool bad = n_trials < 0 || !opts || !slew_time || (trials ? n_sel < 0 : n_sel != n_trials) || (dispersed && !disp);
   if (!bad) bad = opts->n_real < 1 || opts->r_first < 0 || opts->r_first + opts->n_real > ((int64_t)1 << 30);
-  if (!bad && dispersed) bad = !ts::dispersion_opts_ok(disp);
+  if (!bad && disp) bad = !ts::dispersion_opts_ok(disp);
+  if (!bad && ws) bad = !ts::weight_sets_ok(ws->n, ws->sets, ws->u_limit);
   for (int64_t p = 0; !bad && trials && p < n_sel; ++p) bad = trials[p] < 0 || trials[p] >= n_trials;
   if (bad) {
     snprintf(m->err, sizeof(m->err), "%s: bad argument", fn);
     return TS_ERR_ARG;
   }
-  const size_t RR = (size_t)opts->n_real, NP = ts::DISP_NP;
+  const size_t RR = (size_t)opts->n_real * (ws ? (size_t)ws->n : 1), NP = ts::DISP_NP;   // RR: slew times per trial
   std::vector<std::vector<int64_t>> pos(G), loc(G);   // caller rows and device-local trial indices per device
   for (int64_t p = 0; p < n_sel; ++p) {
     const int64_t t = trials ? trials[p] : p;
@@ -301,9 +302,11 @@ static int multi_ensemble(ts_multi* m, const char* fn, int64_t n_trials, const t
     if (x_final) hx[g].resize(k * RR * 8);
     if (params) hp[g].resize(k * RR * NP);
     double* px = x_final ? hx[g].data() : nullptr;
-    rcs[g] = dispersed ? ts_mc_dispersion_ensemble(m->ctx[g], ng, opts, disp, (int64_t)k, loc[g].data(), hs[g].data(), px,
-                                                   params ? hp[g].data() : nullptr)
-                       : ts_mc_replay_ensemble(m->ctx[g], ng, opts, (int64_t)k, loc[g].data(), hs[g].data(), px);
+    rcs[g] = ws          ? ts_mc_weight_ensemble(m->ctx[g], ng, opts, disp, ws->n, ws->sets, ws->u_limit, (int64_t)k, loc[g].data(),
+                                                 hs[g].data(), px)
+             : dispersed ? ts_mc_dispersion_ensemble(m->ctx[g], ng, opts, disp, (int64_t)k, loc[g].data(), hs[g].data(), px,
+                                                     params ? hp[g].data() : nullptr)
+                         : ts_mc_replay_ensemble(m->ctx[g], ng, opts, (int64_t)k, loc[g].data(), hs[g].data(), px);
   };
   std::vector<std::thread> th;
   for (int g = 0; g < G; ++g) th.emplace_back(worker, g);
@@ -331,6 +334,13 @@ int ts_multi_mc_replay_ensemble(ts_multi* m, int64_t n_trials, const ts_replay_e
 int ts_multi_mc_dispersion_ensemble(ts_multi* m, int64_t n_trials, const ts_replay_ensemble_opts* opts, const ts_dispersion_opts* disp,
                                     int64_t n_sel, const int64_t* trials, double* slew_time, double* x_final, double* params) {
   return multi_ensemble(m, "ts_multi_mc_dispersion_ensemble", n_trials, opts, true, disp, n_sel, trials, slew_time, x_final, params);
+}
+
+int ts_multi_mc_weight_ensemble(ts_multi* m, int64_t n_trials, const ts_replay_ensemble_opts* opts, const ts_dispersion_opts* disp,
+                                int64_t n_sets, const ts_tvlqr_weights* sets, double u_limit, int64_t n_sel, const int64_t* trials,
+                                double* slew_time, double* x_final) {
+  const WeightSets ws = {n_sets, sets, u_limit};
+  return multi_ensemble(m, "ts_multi_mc_weight_ensemble", n_trials, opts, false, disp, n_sel, trials, slew_time, x_final, nullptr, &ws);
 }
 
 }  // extern "C"

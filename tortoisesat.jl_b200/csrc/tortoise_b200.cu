@@ -24,7 +24,7 @@ using namespace ts;
 
 extern "C" {
 
-int ts_version(void) { return 105; }
+int ts_version(void) { return 106; }
 
 int ts_create(ts_ctx** out, int device_id) {
   if (!out) return TS_ERR_ARG;
@@ -1592,14 +1592,20 @@ int ts_mc_continue(ts_ctx* c, int64_t n_trials, const ts_ilqr_opts* opts, ts_tri
   return TS_OK;
 }
 
-// RE1-RE5 and DE1-DE6 (DESIGN.md section 4, K4): the body of ts_mc_replay_ensemble and, with disp, of
-// ts_mc_dispersion_ensemble.  The kept run's slews replayed under n_real disturbance draws each (and, with disp, under
-// drawn truth-model errors).  The gains of the selected trials come from the unchanged K4a + K4b on host-compacted arrays
-// (as ts_mc_continue replays), then K4e (K4d) replays every (trial, realisation) pair.  Only per-call slots are written:
-// the kept run stays as it was (RE5, DE6).
+// RE1-RE5, DE1-DE6 and WE1-WE7 (DESIGN.md section 4, K4): the body of ts_mc_replay_ensemble, with disp of
+// ts_mc_dispersion_ensemble, and with weight sets (ws) of ts_mc_weight_ensemble.  The kept run's slews replayed under
+// n_real disturbance draws each (and, with disp, under drawn truth-model errors).  The gains of the selected trials come
+// from the unchanged K4a + K4b on host-compacted arrays (as ts_mc_continue replays), then K4e (K4d) replays every (trial,
+// realisation) pair; with weight sets, K4a and one K4w Riccati sweep per (trial, set), then K4w replays every (trial,
+// set, realisation) triple.  Only per-call slots are written: the kept run stays as it was (RE5, DE6, WE6).
+struct WeightSets {
+  int64_t n;
+  const ts_tvlqr_weights* sets;
+  double u_limit;
+};
 static int mc_ensemble(ts_ctx* c, const char* fn, int64_t n_trials, const ts_replay_ensemble_opts* opts, bool dispersed,
                        const ts_dispersion_opts* disp, int64_t n_sel, const int64_t* trials, double* slew_time, double* x_final,
-                       double* params) {
+                       double* params, const WeightSets* ws = nullptr) {
   if (!c) return TS_ERR_ARG;
   const ts_ctx::McLast& L = c->mc_last;
   if (L.cfg.keep_trajectories < 1) return fail(c, TS_ERR_ARG, "%s: no Monte-Carlo run with keep_trajectories >= 1 on this context", fn);
@@ -1612,8 +1618,10 @@ static int mc_ensemble(ts_ctx* c, const char* fn, int64_t n_trials, const ts_rep
     return fail(c, TS_ERR_ARG, "%s: n_sel must be >= 0 (= n_trials without a trial list)", fn);
   for (int64_t p = 0; trials && p < n_sel; ++p)
     if (trials[p] < 0 || trials[p] >= n_trials) return fail(c, TS_ERR_ARG, "%s: trial %lld out of range", fn, (long long)trials[p]);
-  if (dispersed && !dispersion_opts_ok(disp))
+  if (disp && !dispersion_opts_ok(disp))
     return fail(c, TS_ERR_ARG, "%s: need finite sigmas >= 0, the three log-sigmas <= 1 and sigma_field_angle <= pi", fn);
+  if (ws && !weight_sets_ok(ws->n, ws->sets, ws->u_limit))
+    return fail(c, TS_ERR_ARG, "%s: need n_sets >= 1, sets, finite Qd, Qfd >= 0, finite Rd > 0 and a finite u_limit >= 0", fn);
   // selected active trials, longest horizon first (stable: repeats and the caller's order decide nothing about a row, RE4)
   std::vector<int64_t> act_of((size_t)n_trials, -1);
   for (size_t a = 0; a < L.act.size(); ++a) act_of[(size_t)L.act[a]] = (int64_t)a;
@@ -1622,8 +1630,10 @@ static int mc_ensemble(ts_ctx* c, const char* fn, int64_t n_trials, const ts_rep
     if (act_of[(size_t)(trials ? trials[p] : p)] >= 0) pos.push_back(p);
   auto act_at = [&](int64_t p) { return act_of[(size_t)(trials ? trials[p] : p)]; };
   std::stable_sort(pos.begin(), pos.end(), [&](int64_t u, int64_t v) { return L.in.col(I_N)[act_at(u)] > L.in.col(I_N)[act_at(v)]; });
-  const size_t NC = pos.size(), RR = (size_t)R;
-  const size_t per = 1 + (x_final ? 8 : 0) + (params ? DISP_NP : 0);   // doubles per (trial, realisation) row
+  const size_t NC = pos.size(), NS = ws ? (size_t)ws->n : 1, RR = (size_t)R * NS;   // RR: doubles of slew time per trial
+  const size_t per = 1 + (x_final ? 8 : 0) + (params ? DISP_NP : 0);   // doubles per (trial, set, realisation) row
+  if ((double)NS * (double)L.knots * 144.0 > 0x1p62 || (double)NC * (double)RR * 72.0 > 0x1p62)   // (no size_t wrap below)
+    return fail(c, TS_ERR_NOMEM, "%s: the gains of %zu sets or the outputs do not fit", fn, NS);
   std::vector<double> hs(NC * RR), hx(x_final ? NC * RR * 8 : 0), hp(params ? NC * RR * DISP_NP : 0);
   c->ens_ms[0] = c->ens_ms[1] = 0.0;
   c->last_kernel_ms = 0.0;
@@ -1635,7 +1645,9 @@ static int mc_ensemble(ts_ctx* c, const char* fn, int64_t n_trials, const ts_rep
     int rc;
     void *p_out, *p_K;
     if ((rc = scratch_reserve(c, SLOT_ENSEMBLE_OUT, NC * RR * per * 8 + 64, &p_out))) return rc;
-    if ((rc = scratch_reserve(c, SLOT_K4_GAINS, (size_t)L.knots * 18 * 8, &p_K))) return rc;
+    if ((rc = scratch_reserve(c, SLOT_K4_GAINS, NS * (size_t)L.knots * 18 * 8, &p_K))) return rc;
+    double* d_sets = nullptr;
+    if (ws && (rc = upload(c, SLOT_WEIGHT_SETS, &ws->sets[0].Qd[0], NS * 15, &d_sets))) return rc;
     McPackedView v;
     uint32_t* d_sid;
     if ((rc = upload_packed(c, P, SLOT_ARGS_A, SLOT_ARGS_B, v))) return rc;
@@ -1645,23 +1657,45 @@ static int mc_ensemble(ts_ctx* c, const char* fn, int64_t n_trials, const ts_rep
     fused_k4_args(k4, v, L.d_X, L.d_U, L.d_B, (double*)p_K, d_sid, L.cfg);   // RE2: the run's options with the overrides
     k4.opts.noise_mode = 2;                                                  // realisations always draw
     K4eArgs e = k4e_args(k4, v.col(F_X0));
-    e.n_real = R; e.r_first = r0; e.n_blk = (R + 31) / 32;
+    e.n_real = R; e.r_first = r0; e.n_blk = (R + 31) / 32;   // (per set)
     e.q_noise_scale = opts->q_noise_scale;
     e.slew_time = (double*)p_out;
     e.x_final = x_final ? e.slew_time + NC * RR : nullptr;
     double* d_params = params ? e.slew_time + NC * RR * (x_final ? 9 : 1) : nullptr;
     Events<3> ev;
     cudaEventRecord(ev[0], c->stream);
-    k4_gains_launch(c, k4);
+    K4wGainsArgs g;
+    if (ws) {   // K4a once, then one K4b team per (trial, set) (WE2)
+      g.a = k4; g.sets = d_sets; g.n_sets = (int64_t)NS; g.k_stride = L.knots * 18; g.K = (double*)p_K;
+      if (k4.lin_total > 0) {
+        k4a_linearise_kernel<<<(unsigned)((k4.lin_total + 127) / 128), 128, 0, c->stream>>>(k4);
+        const int64_t teams = (int64_t)NC * g.n_sets;
+        k4w_riccati_sets_kernel<<<(unsigned)((teams + K4B_TEAMS_PER_BLOCK - 1) / K4B_TEAMS_PER_BLOCK), K4B_TEAM * K4B_TEAMS_PER_BLOCK, 0,
+                                  c->stream>>>(g);
+        c->launches += 2;
+      }
+    } else {
+      k4_gains_launch(c, k4);
+    }
     cudaEventRecord(ev[1], c->stream);
-    const int64_t warps = (int64_t)NC * e.n_blk;
+    const int64_t warps = (int64_t)(NC * NS) * e.n_blk;
     const unsigned blocks = (unsigned)((warps + K4E_WARPS - 1) / K4E_WARPS);
-    if (dispersed) {
-      K4dArgs d;
-      d.e = e;
+    K4dArgs d;
+    d.e = e;
+    d.sigma[0] = d.sigma[1] = d.sigma[2] = d.sigma[3] = 0.0;   // a null disp of the weight ensemble (WE2)
+    if (disp) {
       d.sigma[0] = disp->sigma_inertia; d.sigma[1] = disp->sigma_torquer;
       d.sigma[2] = disp->sigma_field_scale; d.sigma[3] = disp->sigma_field_angle;
-      d.params = d_params;
+    }
+    d.params = d_params;
+    if (ws) {
+      K4wArgs w;
+      w.d = d; w.n_sets = g.n_sets; w.k_stride = g.k_stride; w.u_limit = ws->u_limit;
+      if (w.u_limit > 0.0)
+        k4w_weight_replay_kernel<true><<<blocks, 32 * K4E_WARPS, 0, c->stream>>>(w);
+      else
+        k4w_weight_replay_kernel<false><<<blocks, 32 * K4E_WARPS, 0, c->stream>>>(w);
+    } else if (dispersed) {
       k4d_dispersion_replay_kernel<<<blocks, 32 * K4E_WARPS, 0, c->stream>>>(d);
     } else {
       k4e_ensemble_replay_kernel<<<blocks, 32 * K4E_WARPS, 0, c->stream>>>(e);
@@ -1705,6 +1739,15 @@ int ts_mc_replay_ensemble(ts_ctx* c, int64_t n_trials, const ts_replay_ensemble_
 int ts_mc_dispersion_ensemble(ts_ctx* c, int64_t n_trials, const ts_replay_ensemble_opts* opts, const ts_dispersion_opts* disp,
                               int64_t n_sel, const int64_t* trials, double* slew_time, double* x_final, double* params) {
   return mc_ensemble(c, "ts_mc_dispersion_ensemble", n_trials, opts, true, disp, n_sel, trials, slew_time, x_final, params);
+}
+
+int ts_mc_weight_ensemble(ts_ctx* c, int64_t n_trials, const ts_replay_ensemble_opts* opts, const ts_dispersion_opts* disp,
+                          int64_t n_sets, const ts_tvlqr_weights* sets, double u_limit, int64_t n_sel, const int64_t* trials,
+                          double* slew_time, double* x_final) {
+  const WeightSets ws = {n_sets, sets, u_limit};
+  const int rc = mc_ensemble(c, "ts_mc_weight_ensemble", n_trials, opts, false, disp, n_sel, trials, slew_time, x_final, nullptr, &ws);
+  if (rc == TS_ERR_NOMEM) cudaGetLastError();   // the failed allocation is not a fault: a chunked retry may follow (WE7)
+  return rc;
 }
 
 int ts_mc_replay_ensemble_last_split(ts_ctx* c, double* gains_ms, double* replay_ms) {

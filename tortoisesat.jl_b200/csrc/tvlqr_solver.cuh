@@ -447,10 +447,12 @@ struct TvlqrDirectSrc {
   TS_HD void done(long long) const {}
 };
 // DISP: a dispersed realisation (in.disp; in.I holds its truth inertia): transformed field rows when the records are
-// built here, and the scaled torque in every stage.
-template <bool PRE, class Src, bool DISP = false>
+// built here, and the scaled torque in every stage.  CLAMP: the torquer limit of a weight-sweep ensemble (WE4 of DESIGN.md
+// section 4, K4): each component of u = U_lqr - K dx is clamped to [-u_lim, u_lim] before it drives the step (a NaN
+// stays NaN); the gains are unchanged.
+template <bool PRE, class Src, bool DISP = false, bool CLAMP = false>
 TS_HD long long tvlqr_replay_src(const TvlqrIn& in, const ts_tvlqr_opts_dev& o, Src& src, double* X_sim, double* U_sim,
-                                 double* dX, double* slew_time_out, double* x_last = nullptr) {
+                                 double* dX, double* slew_time_out, double* x_last = nullptr, double u_lim = 0.0) {
   const int N = in.N;
   long long N_sim = range_len(o.t0, o.dt, o.tf);
   if (N_sim > N) N_sim = range_len(o.t0, o.dt, o.tf - o.dt);
@@ -497,6 +499,8 @@ TS_HD long long tvlqr_replay_src(const TvlqrIn& in, const ts_tvlqr_opts_dev& o, 
       for (int j = 0; j < 6; ++j) s += Kk[i * 6 + j] * d6[j];
       u[i] = ul[i] - s;
     }
+    if constexpr (CLAMP)
+      for (int i = 0; i < 3; ++i) u[i] = u[i] < -u_lim ? -u_lim : (u[i] > u_lim ? u_lim : u[i]);
     if (U_sim)
       for (int i = 0; i < 3; ++i) U_sim[k * 3 + i] = u[i];
     if (dX)

@@ -98,6 +98,27 @@ class DispersionOpts(C.Structure):
 DISPERSION_PARAMS = ("d0", "d1", "d2", "g0", "g1", "g2", "s_B", "phi0", "phi1", "phi2")   # order of a params row
 
 
+class TvlqrWeights(C.Structure):
+    """ts_tvlqr_weights (include/tortoise_b200.h): one tracking weighting of a weight-sweep ensemble, the diagonals of
+    TvlqrOpts' Q, Qf and R (120 bytes)."""
+    _fields_ = [("Qd", C.c_double * 6), ("Qfd", C.c_double * 6), ("Rd", C.c_double * 3)]
+
+
+def weight_sets(sets):
+    """A ctypes array of TvlqrWeights from an (n_sets, 15) array in the order Qd 6 | Qfd 6 | Rd 3, a sequence of
+    TvlqrWeights, or such a ctypes array (returned as is)."""
+    if isinstance(sets, C.Array) and sets._type_ is TvlqrWeights:
+        return sets
+    if len(sets) and all(isinstance(w, TvlqrWeights) for w in sets):
+        return (TvlqrWeights * len(sets))(*sets)
+    a = np.ascontiguousarray(sets, dtype=np.float64)
+    if a.ndim != 2 or a.shape[1] != 15:
+        raise ValueError("weight sets: need an (n_sets, 15) array in the order Qd 6 | Qfd 6 | Rd 3")
+    out = (TvlqrWeights * a.shape[0])()
+    C.memmove(out, a.ctypes.data, a.nbytes)
+    return out
+
+
 Q_NOISE_SCALE = (np.pi / 180) ** 2   # initial attitude noise of monte_carlo.jl: randn(3)*(pi/180)^2
 
 
@@ -178,6 +199,8 @@ def load_library():
     L.ts_mc_replay_ensemble_last_split.argtypes = [C.c_void_p, c_double_p, c_double_p]
     L.ts_mc_dispersion_ensemble.argtypes = [C.c_void_p, C.c_int64, C.POINTER(ReplayEnsembleOpts), C.POINTER(DispersionOpts),
                                             C.c_int64] + [C.c_void_p] * 4
+    L.ts_mc_weight_ensemble.argtypes = [C.c_void_p, C.c_int64, C.POINTER(ReplayEnsembleOpts), C.POINTER(DispersionOpts), C.c_int64,
+                                        C.POINTER(TvlqrWeights), C.c_double, C.c_int64] + [C.c_void_p] * 3
     L.ts_igrf12syn_batch.argtypes = [C.c_void_p, C.c_int, C.c_double, C.c_int, C.c_int64] + [C.c_void_p] * 7 + [C.c_int]
     L.ts_psiaki_pd_batch.argtypes = [C.c_void_p, C.c_int64] + [C.c_void_p] * 7 + [C.c_double] * 3 + [C.c_void_p] * 3
     L.ts_attitude_dynamics_linear_batch.argtypes = [C.c_void_p, C.c_int64] + [C.c_void_p] * 6
@@ -194,6 +217,8 @@ def load_library():
     L.ts_multi_mc_replay_ensemble.argtypes = [C.c_void_p, C.c_int64, C.POINTER(ReplayEnsembleOpts), C.c_int64] + [C.c_void_p] * 3
     L.ts_multi_mc_dispersion_ensemble.argtypes = [C.c_void_p, C.c_int64, C.POINTER(ReplayEnsembleOpts), C.POINTER(DispersionOpts),
                                                   C.c_int64] + [C.c_void_p] * 4
+    L.ts_multi_mc_weight_ensemble.argtypes = [C.c_void_p, C.c_int64, C.POINTER(ReplayEnsembleOpts), C.POINTER(DispersionOpts),
+                                              C.c_int64, C.POINTER(TvlqrWeights), C.c_double, C.c_int64] + [C.c_void_p] * 3
     L.ts_igrf12_batch.argtypes = [C.c_void_p, C.c_double, C.c_int64] + [C.c_void_p] * 6 + [C.c_int]
     L.ts_field_map_prefilter.argtypes = [C.c_void_p, C.c_int64, C.c_int64, C.c_void_p, C.c_void_p, C.c_int]
     L.ts_field_map_eval_batch.argtypes = [C.c_void_p, C.c_int64, C.c_int64, C.c_void_p, C.c_int64] + [C.c_void_p] * 3 + [C.c_int]
@@ -704,6 +729,19 @@ class Engine:
         return _dispersion_ensemble(self.lib.ts_mc_dispersion_ensemble, self.h, n_trials, n_real, d, r_first, trials,
                                     q_noise_scale, want_x_final, want_params, self._check)
 
+    def mc_weight_ensemble(self, n_trials, n_real, sets, u_limit=0.0, disp=None, r_first=0, trials=None, q_noise_scale=Q_NOISE_SCALE,
+                           want_x_final=False):
+        """The kept run's slews replayed as mc_dispersion_ensemble does, once per tracking weighting of sets (an
+        (n_sets, 15) array Qd 6 | Qfd 6 | Rd 3, or TvlqrWeights): the gains of each set from its own Riccati sweep, the same
+        draws for every set (ts_mc_weight_ensemble, rules WE1-WE7).  u_limit > 0 clamps each dipole command component to
+        [-u_limit, u_limit] in the truth model (0: no limit); cfg.ilqr.u_max, the planner's own bound, is the physically
+        meaningful limit.  disp: the truth-model sigmas (DispersionOpts or a dict of mc_dispersion_ensemble's sigma_*
+        keywords), None for none (a null dispersion).  Returns (slew_time
+        (n_sel, n_sets, n_real), x_final (n_sel, n_sets, n_real, 8) or None); a NO_CUTOFF trial gets NaN rows."""
+        return _weight_ensemble(self.lib.ts_mc_weight_ensemble, self.h, n_trials, n_real, sets, u_limit,
+                                _dispersion_opts(disp), r_first, trials,
+                                q_noise_scale, want_x_final, self._check)
+
     def mc_replay_ensemble_split(self):
         """Device ms of the last mc_replay_ensemble: (gains, ensemble replay)."""
         g, r = C.c_double(), C.c_double()
@@ -820,6 +858,16 @@ class MultiEngine:
         return _dispersion_ensemble(self.lib.ts_multi_mc_dispersion_ensemble, self.h, n_trials, n_real, d, r_first, trials,
                                     q_noise_scale, want_x_final, want_params, check)
 
+    def mc_weight_ensemble(self, n_trials, n_real, sets, u_limit=0.0, disp=None, r_first=0, trials=None, q_noise_scale=Q_NOISE_SCALE,
+                           want_x_final=False):
+        """Engine.mc_weight_ensemble over the devices' kept shards; the rows equal the single-device rows (WE5)."""
+        def check(rc):
+            if rc != 0:
+                raise TortoiseError(rc, (self.lib.ts_multi_last_error(self.h) or b"").decode())
+        return _weight_ensemble(self.lib.ts_multi_mc_weight_ensemble, self.h, n_trials, n_real, sets, u_limit,
+                                _dispersion_opts(disp), r_first, trials,
+                                q_noise_scale, want_x_final, check)
+
 
 def _replay_ensemble(fn, h, n_trials, n_real, r_first, trials, q_noise_scale, want_x_final, check):
     n = int(n_trials)
@@ -845,6 +893,27 @@ def _dispersion_ensemble(fn, h, n_trials, n_real, disp, r_first, trials, q_noise
     check(fn(h, n, C.byref(o), C.byref(disp), ns, None if sel is None else _ptr(sel), _ptr(slew), None if xf is None else _ptr(xf),
              None if prm is None else _ptr(prm)))
     return slew, xf, prm
+
+
+def _dispersion_opts(disp):
+    """None, a DispersionOpts, or a dict of sigma_* keywords -> None or a DispersionOpts."""
+    if disp is None or isinstance(disp, DispersionOpts):
+        return disp
+    return DispersionOpts(*[float(disp.get(k, 0.0)) for k, _ in DispersionOpts._fields_])
+
+
+def _weight_ensemble(fn, h, n_trials, n_real, sets, u_limit, disp, r_first, trials, q_noise_scale, want_x_final, check):
+    n = int(n_trials)
+    o = ReplayEnsembleOpts(int(n_real), int(r_first), float(q_noise_scale))
+    ws = weight_sets(sets)
+    sel = None if trials is None else np.ascontiguousarray(trials, dtype=np.int64).reshape(-1)
+    ns = n if sel is None else sel.shape[0]
+    R = max(int(n_real), 0)
+    slew = np.zeros((ns, len(ws), R))
+    xf = np.zeros((ns, len(ws), R, 8)) if want_x_final else None
+    check(fn(h, n, C.byref(o), None if disp is None else C.byref(disp), len(ws), ws, float(u_limit), ns,
+             None if sel is None else _ptr(sel), _ptr(slew), None if xf is None else _ptr(xf)))
+    return slew, xf
 
 
 # ---------------------------------------------------------------------------
@@ -1286,6 +1355,33 @@ def dispersion_ensemble(res, n_real=100, trials=None, r_first=1, sigma_inertia=0
                                                            q_noise_scale=q_noise_scale, want_params=True)
     d = _ensemble_stats(out, sel, slew)
     d["params"] = prm
+    return d
+
+
+def weight_ensemble(res, sets, n_real=100, trials=None, r_first=1, u_limit=0.0, sigma_inertia=0.0, sigma_torquer=0.0,
+                    sigma_field_scale=0.0, sigma_field_angle=0.0, q_noise_scale=Q_NOISE_SCALE):
+    """dispersion_ensemble once per tracking weighting (ts_mc_weight_ensemble on the default engine, rules WE1-WE7):
+    sets is an (n_sets, 15) array Qd 6 | Qfd 6 | Rd 3 (or TvlqrWeights); every set's gains come from its own Riccati
+    sweep on the kept trajectory, and every set meets the same disturbances and truth models, draw for draw.  u_limit > 0
+    clamps each dipole command component to [-u_limit, u_limit] in the truth model; the planner's bound
+    (IlqrOpts.u_max, 1 by default) is the physically meaningful limit, and without one larger gains are free.  Returns
+    replay_ensemble's statistics per set: slew_time (n_sel, n_sets, n_real), fails, fail_rate / slew_mean / slew_std
+    (n_sel, n_sets), set_fail_rate (n_sets: the share of failing draws over every selected trial) and trials."""
+    if "states" not in res and "ilqr" not in res:
+        raise ValueError("weight_ensemble needs a monte_carlo(..., trajectories=True) or monte_carlo(..., resumable=True) result")
+    out = res["outcomes"]
+    n = out.shape[0]
+    sel = np.arange(n, dtype=np.int64) if trials is None else np.ascontiguousarray(trials, dtype=np.int64).reshape(-1)
+    disp = DispersionOpts(float(sigma_inertia), float(sigma_torquer), float(sigma_field_scale), float(sigma_field_angle))
+    slew, _ = default_engine().mc_weight_ensemble(n, n_real, sets, u_limit, disp, r_first=r_first, trials=sel,
+                                                  q_noise_scale=q_noise_scale)
+    per = [_ensemble_stats(out, sel, slew[:, w]) for w in range(slew.shape[1])]
+    d = {k: np.stack([p[k] for p in per], axis=1) for k in ("fails", "fail_rate", "slew_mean", "slew_std")}
+    valid = ~np.isnan(slew)
+    with np.errstate(invalid="ignore", divide="ignore"):
+        d["set_fail_rate"] = d["fails"].sum(axis=(0, 2)) / valid.sum(axis=(0, 2))
+    d["slew_time"] = slew
+    d["trials"] = sel
     return d
 
 
